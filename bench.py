@@ -37,6 +37,8 @@ sys.path.insert(0, os.path.join(ROOT, "smart-chess-rust_b200"))
 FLOP_PER_LEAF = 2 * 1463895040            # BASELINE.md section 2
 FLOP_PER_LEAF_CONV3 = 2 * 64 * 256 * 2304  # one 3x3 256->256 layer, per leaf
 N_BLOCKS = 19
+DUMP_BYTES = 64_000_000                    # --dump-outputs: at most this much over all ranks, headers included
+NPY_HEADER = 128                           # bytes before the data of a 1-D .npy file
 
 
 def _peaks():
@@ -69,6 +71,30 @@ def make_blob(tmpdir: str, n_blocks: int = N_BLOCKS):
     path = os.path.join(tmpdir, f"seed0_{n_blocks}.scw")
     scb200.write_blob(sd, path)
     return sd, path
+
+
+def dump_outputs(out_dir: str, pri, val, off, rank: int, world: int):
+    """Writes what one step returns to its caller: priors.npy (float32, per legal move, leaf after leaf) and values.npy
+    (float32, per leaf), with leaves.npy (each leaf's index in the step) and offsets.npy (where each leaf's priors start
+    in priors.npy, plus the end), both float64.  Above DUMP_BYTES, a fixed seeded sample of whole leaves in leaf order."""
+    import numpy as np
+
+    names = ("priors", "values", "leaves", "offsets")
+    budget = DUMP_BYTES // world - len(names) * NPY_HEADER - 8   # bytes per rank, less the headers and the end offset
+    lens = np.diff(off).astype(np.int64)
+    leaves = np.arange(len(val))
+    if 4 * int(lens.sum()) + 20 * len(val) > budget:
+        order = np.random.default_rng(0).permutation(len(val))
+        cost = np.cumsum(4 * lens[order] + 20)      # a leaf's priors and value (float32), index and offset (float64)
+        leaves = np.sort(order[: int(np.searchsorted(cost, budget, side="right"))])
+    lens = lens[leaves]
+    starts = np.concatenate([[0], np.cumsum(lens)])
+    pri = pri[np.arange(int(starts[-1])) + np.repeat(off[leaves] - starts[:-1], lens)]
+    arrays = (pri.astype(np.float32), val[leaves].astype(np.float32), leaves.astype(np.float64), starts.astype(np.float64))
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = "" if world == 1 else f"_rank{rank}"
+    for name, a in zip(names, arrays):
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), a)
 
 
 def oracle_sample(n: int, seed: int):
@@ -300,7 +326,13 @@ def main():
                     help="plies of one game through the one-leaf interface (BASELINE configs[0] settings) to time (0 = skip)")
     ap.add_argument("--sustain", type=float, default=5.0,
                     help="seconds of back-to-back steps for the sustained roofline leg and the clock samples (0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the priors and values of the last timed step as DIR/priors.npy and DIR/values.npy "
+                         "(float32), with DIR/leaves.npy and DIR/offsets.npy to split the priors by leaf; at most 64 MB "
+                         "(a seeded sample of the leaves beyond that); with several ranks, _rank<r> before .npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs dumps the b200 arm's timed step; the reference arm does not keep its outputs")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     if args.impl == "reference":
@@ -417,6 +449,8 @@ def main():
         t_wall = time.perf_counter() - t_wall0
         launches = eng.launch_count() - launches0
         eng_timed_flops = eng.timed_flops_per_leaf()
+        # the sustained leg below overwrites d_pri / d_val: keep the last timed step's results
+        dumped = (d_pri.cpu().numpy(), d_val.cpu().numpy()) if args.dump_outputs else None
         # ---- sustained leg: the same step back to back for >= args.sustain seconds, no flush, no idle gap beyond the
         #      engine's own event read-back: what the kernel does under continuous load (power cap); its roofline
         #      fraction is taken against the SUSTAINED peak, the event-bracketed steps above against the BURST peak.
@@ -514,6 +548,8 @@ def main():
     # sanity: the timed output is a real evaluation (not part of the timed region)
     pri_chk = d_pri.cpu().numpy()
     assert np.isfinite(pri_chk).all() and abs(float(pri_chk[: int(off[1])].sum()) - 1.0) < 0.05
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, *dumped, off, rank, world)
 
     if rank == 0:
         peaks = _peaks()

@@ -81,3 +81,31 @@ def test_bench_reference_arm_prints_the_contract_line():
     assert cb["kind"] == "port" and cb["cores"] >= 1 and cb["value"] == d["value"] and cb["leaves_per_step_run"] == 64
     assert cb["batch1_value"] > 0
     assert d["e2e"] == {"value": d["value"], "unit": "leaf evals/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
+
+
+def test_bench_dump_outputs_refused_on_the_reference_arm(tmp_path):
+    """The reference arm keeps no outputs: --dump-outputs there is an error, not an empty directory."""
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--dump-outputs",
+                        str(tmp_path / "d")], capture_output=True, text=True, timeout=120)
+    assert r.returncode == 2 and "--dump-outputs" in r.stderr and not (tmp_path / "d").exists()
+
+
+def test_bench_dump_outputs_sample_stays_under_the_cap_and_splits_by_leaf(tmp_path, monkeypatch):
+    import numpy as np
+
+    import bench
+
+    rng = np.random.default_rng(1)
+    off = np.concatenate([[0], np.cumsum(rng.integers(0, 60, 3000))]).astype(np.int32)
+    pri, val = rng.random(off[-1]).astype(np.float32), rng.random(3000).astype(np.float32)
+    monkeypatch.setattr(bench, "DUMP_BYTES", 200_000)
+    for world, rank in ((1, 0), (2, 1)):
+        d = tmp_path / str(world)
+        bench.dump_outputs(str(d), pri, val, off, rank, world)
+        assert sum(f.stat().st_size for f in d.iterdir()) <= 200_000 // world
+        s = "" if world == 1 else "_rank1"
+        p, v, lv, o = (np.load(d / f"{n}{s}.npy") for n in ("priors", "values", "leaves", "offsets"))
+        lv, o = lv.astype(np.int64), o.astype(np.int64)
+        assert 0 < len(lv) < 3000 and (np.diff(lv) > 0).all() and np.array_equal(v, val[lv]) and o[-1] == len(p)
+        for k, i in enumerate(lv):
+            assert np.array_equal(p[o[k]:o[k + 1]], pri[off[i]:off[i + 1]])

@@ -140,23 +140,35 @@ def test_sample_games_replay_digest(co, sample_games):
         assert h.hexdigest() == game["sha256"]
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/py/validation/sample.csv"), reason="reference tree absent")
 def test_sample_csv_san_resolution(co, sample_games):
-    import csv
+    """The oracle's SAN parser on the 60 games of the reference's py/validation/sample.csv: tests/golden/sample_san.json
+    holds either the CSV's own text (oracle/make_golden_chess.py) or, as its `source` says, a reconstruction written
+    without the oracle (oracle/make_golden_san.py).  The totals are the ones recorded from the CSV."""
+    import json
 
-    with open("/root/reference/py/validation/sample.csv") as f:
-        rows = list(csv.DictReader(f))
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "sample_san.json")) as f:
+        rows = json.load(f)["games"]
     assert len(rows) == 60
+    sans = [s for row in rows for s in row["moves"].split()]
+    tot = sample_games["totals"]
+    assert len(sans) == tot["plies"] and sum(s[-1] in "+#" for s in sans) == tot["check"]
+    assert sum(s.endswith("#") for s in sans) == tot["mate"]
+    assert sum(s.startswith("O-O") for s in sans) == tot["castle"] and sum("=" in s for s in sans) == tot["promo"]
+    ep = 0
     for row, game in zip(rows, sample_games["games"]):
+        assert row["id"] == game["id"]
         g = co.Game()
         ucis = []
         for san in row["moves"].split():
             m = g.parse_san(san)
+            f, t = int(m[0]), int(m[1])
+            ep += abs(g.piece_at(f)) == 1 and (f & 7) != (t & 7) and g.piece_at(t) == 0
             g.push(m)
             ucis.append(co.uci(m))
             assert g.is_check() == (san[-1] in "+#")
             assert (len(g.legal_moves()) == 0 and g.is_check()) == san.endswith("#")
         assert " ".join(ucis) == game["uci"]
+    assert ep == tot["ep"]
 
 
 def test_repetition_flags(co):
