@@ -123,7 +123,7 @@ struct TcTowerLayerDesc {
 };
 int tc_tower_create(TcTower **out, const TcTowerLayerDesc *descs, int n, int boards_alloc);
 // group = tiles per CTA carried through all layers together (0 = all of the CTA's tiles)
-// max_layers > 0: only the first max_layers layers (debug hook)
+// max_layers > 0: only the first max_layers layers (sc_debug_tower's layer-by-layer comparison)
 int tc_tower_launch(TcTower *t, int n_boards, int num_sms, int group, cudaStream_t st, int max_layers = 0);
 void tc_tower_destroy(TcTower *t);
 

@@ -132,7 +132,7 @@ struct sc_engine {
     int device = 0, mode = 0, max_batch = 0, n_blocks = 0, num_sms = 148;
     int mode_requested = 0;
     // FP32 parity mode: the 256-wide convolutions as bf16x3 split GEMMs on the tensor cores (fp32 accumulate), LayerNorm /
-    // SE / the narrow head layers in fp32 on the CUDA cores.  SC_MODE_FP32_FFMA (or SCB200_FP32_TC=0) = everything FFMA.
+    // SE / the narrow head layers in fp32 on the CUDA cores.  SC_MODE_FP32_FFMA = everything FFMA.
     bool fp32_tc = false;
     __nv_bfloat16 *p_x = nullptr, *p_t = nullptr;  // fp32_tc: activations as three bf16 planes [boards][64][768]
     int alloc_boards = 0;
@@ -197,11 +197,11 @@ struct sc_engine {
     cudaStream_t head_stream = nullptr;
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
     int64_t n_submits = 0;
-    // small batches (sc_eval with n <= SC_SMALL_N): inputs are packed into ONE pinned staging buffer and travel in one
-    // copy, values + priors come back in one copy (a caller's Vec / numpy array is pageable memory, which would
-    // otherwise make every one of the five copies a staged, blocking one)
+    // small batches (sc_eval with n <= SC_SMALL_N): inputs are packed into ONE pinned staging buffer and travel in at
+    // most one copy, the kernels write values + priors straight into another (a caller's Vec / numpy array is pageable
+    // memory, which would otherwise make every one of the five copies a staged, blocking one)
     uint8_t *h_small_in = nullptr, *d_small_in = nullptr;
-    float *h_small_out = nullptr, *d_small_out = nullptr;
+    float *h_small_out = nullptr;
     std::vector<cudaEvent_t> kev;  // level-2 timing: event pairs around the 3x3 256->256 convs
     int kev_used = 0;
     float last_conv_avg_ms = 0.f;
@@ -466,7 +466,6 @@ static int alloc_buffers(sc_engine *e)
         const size_t in_bytes = (size_t)SC_SMALL_N * (sizeof(sc_position) + 4 + SC_MAX_MOVES * sizeof(sc_move)) + 64;
         const size_t out_floats = (size_t)SC_SMALL_N * (1 + SC_MAX_MOVES);
         SCB_CHECK(dev_alloc(e, &e->d_small_in, in_bytes));
-        SCB_CHECK(dev_alloc(e, &e->d_small_out, out_floats));
         SCB_CUDA(cudaMallocHost(&e->h_small_in, in_bytes));
         SCB_CUDA(cudaMallocHost(&e->h_small_out, out_floats * sizeof(float)));
     }
@@ -705,7 +704,7 @@ int sc_create(const char *weights_blob_path, int device, int mode, int max_batch
     e->device = device;
     e->mode_requested = mode;
     e->mode = mode == SC_MODE_FP32_FFMA ? SC_MODE_FP32 : mode;
-    e->fp32_tc = mode == SC_MODE_FP32 && !(getenv("SCB200_FP32_TC") && getenv("SCB200_FP32_TC")[0] == '0');
+    e->fp32_tc = mode == SC_MODE_FP32;
     e->max_batch = max_batch;
     e->num_sms = prop.multiProcessorCount;
     int rc = SC_OK;
@@ -884,19 +883,14 @@ int sc_eval(sc_engine *e, int n, const sc_position *pos, const sc_move *moves, c
         memcpy(e->h_small_in + pos_b + off_b, moves, mv_b);
         // inputs: up to 16 leaves are read by the kernels straight from the pinned staging buffer (a few hundred bytes per
         // leaf over PCIe inside the encode / gather kernels instead of a copy engine round trip before the first launch)
-        static const bool zero_copy_in = !(getenv("SCB200_ZERO_COPY_IN") && getenv("SCB200_ZERO_COPY_IN")[0] == '0');
         const uint8_t *in_dev = e->d_small_in;
-        if (zero_copy_in && n <= 16)
+        if (n <= 16)
             in_dev = e->h_small_in;
         else
             SCB_CUDA(cudaMemcpyAsync(e->d_small_in, e->h_small_in, pos_b + off_b + mv_b, cudaMemcpyHostToDevice, st));
         // results: the kernels store priors and values straight into the pinned (device-mapped under UVA) staging buffer --
         // posted writes over PCIe instead of a device buffer + a copy; the stream sync makes them visible to the host
-        static const bool zero_copy_out = !(getenv("SCB200_ZERO_COPY_OUT") && getenv("SCB200_ZERO_COPY_OUT")[0] == '0');
-        float *out_dev = zero_copy_out ? e->h_small_out : e->d_small_out;
-        SCB_CHECK(sc_eval_device(e, n, in_dev, in_dev + pos_b + off_b, in_dev + pos_b, total, out_dev + n, out_dev, st));
-        if (!zero_copy_out)
-            SCB_CUDA(cudaMemcpyAsync(e->h_small_out, e->d_small_out, sizeof(float) * (size_t)(n + total), cudaMemcpyDeviceToHost, st));
+        SCB_CHECK(sc_eval_device(e, n, in_dev, in_dev + pos_b + off_b, in_dev + pos_b, total, e->h_small_out + n, e->h_small_out, st));
         SCB_CUDA(cudaStreamSynchronize(st));
         memcpy(value_out, e->h_small_out, sizeof(float) * (size_t)n);
         memcpy(priors_out, e->h_small_out + n, sizeof(float) * (size_t)total);

@@ -219,41 +219,6 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16])
     asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 }
 
-// Sum over the 32 lanes of a warp of 32 per-lane values, result for index `lane` lands in
-// lane `lane` (recursive halving: 16+8+4+2+1 = 31 shuffles instead of 32 x 5).
-__device__ __forceinline__ float warp_transpose_reduce(float (&v)[32], int lane)
-{
-    const bool b16 = lane & 16, b8 = lane & 8, b4 = lane & 4, b2 = lane & 2, b1 = lane & 1;
-    float w16[16], w8[8], w4[4], w2[2];
-#pragma unroll
-    for (int i = 0; i < 16; i++) {
-        float send = b16 ? v[i] : v[i + 16];
-        float keep = b16 ? v[i + 16] : v[i];
-        w16[i] = keep + __shfl_xor_sync(0xffffffffu, send, 16);
-    }
-#pragma unroll
-    for (int i = 0; i < 8; i++) {
-        float send = b8 ? w16[i] : w16[i + 8];
-        float keep = b8 ? w16[i + 8] : w16[i];
-        w8[i] = keep + __shfl_xor_sync(0xffffffffu, send, 8);
-    }
-#pragma unroll
-    for (int i = 0; i < 4; i++) {
-        float send = b4 ? w8[i] : w8[i + 4];
-        float keep = b4 ? w8[i + 4] : w8[i];
-        w4[i] = keep + __shfl_xor_sync(0xffffffffu, send, 4);
-    }
-#pragma unroll
-    for (int i = 0; i < 2; i++) {
-        float send = b2 ? w4[i] : w4[i + 2];
-        float keep = b2 ? w4[i + 2] : w4[i];
-        w2[i] = keep + __shfl_xor_sync(0xffffffffu, send, 2);
-    }
-    float send = b1 ? w2[0] : w2[1];
-    float keep = b1 ? w2[1] : w2[0];
-    return keep + __shfl_xor_sync(0xffffffffu, send, 1);
-}
-
 __device__ __forceinline__ void bf16x8_to_float(const uint4 &u, float (&f)[8])
 {
     const uint32_t w[4] = {u.x, u.y, u.z, u.w};

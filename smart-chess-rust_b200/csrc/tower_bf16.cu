@@ -7,26 +7,26 @@
 // SqueezeExcitation(256, 128) = sigmoid(fc2(relu(fc1(avgpool)))) * x (torchvision).
 //
 // GEMM view of one 3x3 layer: M = 64 * boards, N = 256 output channels, K = 9 taps x Cin.
-//   A (activations, bf16 NHWC [board][rank][file][C]) is never materialised as im2col.  Single-CTA
-//   kernels: for tap (dy,dx) and channel chunk kc the TMA loads the 4-D box {64 ch, 8 files, 8 ranks,
-//   2 boards} at coordinates (64*kc, dx, dy, board0).  Pair kernels (the tower): ONE box {64 ch,
-//   8 files, 2 boards, 10 ranks} at (64*kc, dx, board0, -1) serves the three dy taps of (kc, dx); it
-//   lands as 160 rows ordered (rank, board, file) and tap dy is the 128-row tile 2 KB * (dy + 1) into it.
+//   A (activations, bf16 NHWC [board][rank][file][C]) is never materialised as im2col.  The 256-wide
+//   convolutions (pair kernels): ONE box {64 ch, 8 files, 2 boards, 10 ranks} at (64*kc, dx, board0, -1)
+//   serves the three dy taps of channel chunk kc and column shift dx; it lands as 160 rows ordered
+//   (rank, board, file) and tap dy is the 128-row tile 2 KB * (dy + 1) into it.  The policy head (a
+//   single-CTA 1x1 convolution) loads the 4-D box {64 ch, 8 files, 8 ranks, 2 boards} at (64*kc, 0, 0, board0).
 //   Ranks/files outside [0,8) are zero-filled by the TMA unit, which IS the conv padding; 128B swizzle
 //   makes every tile the canonical K-major UMMA operand.
 //   B (weights, bf16 [tap][cout][cin]) is a plain 2-D box.
 //   D accumulates in TMEM (128 lanes x 256 fp32 columns per tile, two tiles = all 512
 //   columns, so the epilogue of tile i overlaps the MMAs of tile i+1).
 // One kernel template, tc_gemm_kernel<BN, EPI, A4D, CTA2, TOWER>:
-//   * CTA2: clusters of two CTAs issue tcgen05.mma.cta_group::2 (256-row tiles, each CTA
-//     stages its own rows of A and half of the weight rows);
+//   * CTA2: every 256-wide convolution; clusters of two CTAs issue tcgen05.mma.cta_group::2 (256-row
+//     tiles, each CTA stages its own rows of A and half of the weight rows);
 //   * TOWER: the stem, all residual blocks and the two 256-wide head 1x1 convolutions run
 //     in ONE persistent launch; a tile's layers are chained by a per-tile mbarrier inside
 //     the CTA (boards never interact inside the tower), tiles are carried through all
 //     layers in groups of 3-4 so that layer outputs are re-read from L2;
 //   * the narrow head GEMMs (256->73 with LayerNorm(73), optionally followed in the same epilogue
 //     by log-softmax + legal-move gather + renormalisation; value FC 16384->128 as a split-K
-//     GEMM whose rows are boards) are single-CTA instantiations of the same kernel.
+//     GEMM whose rows are boards) are the single-CTA instantiations of the same kernel.
 // Producer and MMA warps run warp-uniform loops and elect one lane around the TMA / MMA / commit
 // instructions only, which keeps descriptors and barrier addresses in uniform registers.
 // Warp roles (320 threads): warp 0 = TMA producer, warp 1 = TMEM allocator + MMA issuer,
@@ -53,9 +53,6 @@ namespace scb {
 constexpr int TC_BN = 256;
 constexpr int TC_STAGES = 4;
 constexpr int TC_A_BYTES = TC_BM * TC_BK * 2;  // 16 KB
-#ifndef SCB_AREUSE
-#define SCB_AREUSE 1
-#endif
 constexpr int TC_THREADS = 320;      // warp 0 TMA, warp 1 MMA, warps 2..9 epilogue (two per TMEM lane quadrant)
 
 // ---- the kernel ---------------------------------------------------------------------------
@@ -138,7 +135,7 @@ __device__ __forceinline__ void staged_store_64B(uint8_t *stg, int lane, const u
     __syncwarp();
 }
 
-// Same, for accumulator rows ordered (rank, board, file) (pair mode with the shared activation box): the warp of
+// Same, for accumulator rows ordered (rank, board, file) (pair kernels, shared activation box): the warp of
 // TMEM quadrant `quad` holds ranks 2 quad and 2 quad + 1 of both boards; its 8-row group k is rank 2 quad + k / 2
 // of board k % 2, i.e. tile rows 64 (k % 2) + 8 (2 quad + k / 2) .. + 7 in memory.
 __device__ __forceinline__ void staged_store_64B_hbw(uint8_t *stg, int lane, const uint4 (&v)[4], uint8_t *tile_base,
@@ -157,26 +154,14 @@ __device__ __forceinline__ void staged_store_64B_hbw(uint8_t *stg, int lane, con
     __syncwarp();
 }
 
-// 4 registers loaded with the coalesced mapping (row (lane>>2)+8k, chunk lane&3) -> lane's own row
-__device__ __forceinline__ void staged_gather_64B(uint8_t *stg, int lane, const uint4 *coal /*[4]*/, uint4 (&mine)[4])
-{
-#pragma unroll
-    for (int k = 0; k < 4; k++) *reinterpret_cast<uint4 *>(stg + stg_off((lane >> 2) + 8 * k, lane & 3)) = coal[k];
-    __syncwarp();
-#pragma unroll
-    for (int q = 0; q < 4; q++) mine[q] = *reinterpret_cast<const uint4 *>(stg + stg_off(lane, q));
-    __syncwarp();
-}
-
 template <int BN, bool CTA2 = false, bool YSMEM = false> struct TcCfg {
-    // cta_group::2: the pair computes a 256-row tile; each CTA stages its own 128 rows of A and HALF of
-    // the weight rows, so a stage is 32 KB instead of 48 KB and six of them fit.  The SE variant spends
-    // two of those stages on a 64 KB bf16 copy of the tile's LayerNorm output (YSMEM), see the epilogue.
-    static constexpr int STAGES = CTA2 ? (YSMEM ? 4 : 6) : TC_STAGES;
-    // Pair mode, A re-use: the three dy taps of a (channel chunk, dx) read ONE activation box of 10 board rows
-    // (rank -1..8, zero-filled outside the board) instead of three boxes of 8: separate rings for the 20 KB
-    // activation boxes (NA) and the 16 KB weight tiles (NB), 29 % fewer bytes from L2 per tile.
-    static constexpr bool AREUSE = CTA2 && (SCB_AREUSE != 0);
+    // single CTA (the narrow heads): one ring of stages, each holding an A tile and a B tile
+    static constexpr int STAGES = TC_STAGES;
+    // cta_group::2: the pair computes a 256-row tile; each CTA stages its own 128 rows of A and HALF of the weight rows.
+    // The three dy taps of a (channel chunk, dx) read ONE activation box of 10 board rows (rank -1..8, zero-filled
+    // outside the board) instead of three boxes of 8: separate rings for the 20 KB activation boxes (NA) and the 16 KB
+    // weight tiles (NB), 29 % fewer bytes from L2 per tile.  The SE variant gives up ring slots for a 64 KB bf16 copy of
+    // the tile's LayerNorm output (YSMEM), see the epilogue.
     static constexpr int NA = YSMEM ? 3 : 4, NB = YSMEM ? 4 : 7;
     static constexpr int A_BOX_BYTES = 160 * TC_BK * 2;  // rows ordered (rank, board, file): 10 x 2 x 8
     // BN == LD_POLICY: room for the fp32 logits of the tile's two leaves ([128][81], odd row stride = no bank
@@ -185,10 +170,10 @@ template <int BN, bool CTA2 = false, bool YSMEM = false> struct TcCfg {
     static constexpr int Y_BYTES = YSMEM ? TC_BM * 256 * 2 : G_BYTES;
     static constexpr int B_BYTES = (CTA2 ? BN / 2 : BN) * TC_BK * 2;
     static constexpr int STAGE_BYTES = TC_A_BYTES + B_BYTES;
-    static constexpr int SMEM_EPI = 3 * 256 * 4 /*bias,gamma,beta*/ + (4 * 256 + 2 * 256 + 2 * 128 + 2 * 256) * 4 /*SE*/ +
+    static constexpr int SMEM_EPI = 3 * 256 * 4 /*bias,gamma,beta*/ + (4 * 256 /*unused*/ + 2 * 256 + 2 * 128 + 2 * 256) * 4 /*SE*/ +
                                     (2 * 256 + 4 * 128) * 4 /*LN partials, FC1 partials*/ + 8 * 2048 /*store staging*/;
-    static constexpr int RING_BYTES = AREUSE ? NA * A_BOX_BYTES + NB * B_BYTES : STAGES * STAGE_BYTES;
-    static constexpr int N_RING_BARS = AREUSE ? 2 * (NA + NB) : 2 * STAGES;
+    static constexpr int RING_BYTES = CTA2 ? NA * A_BOX_BYTES + NB * B_BYTES : STAGES * STAGE_BYTES;
+    static constexpr int N_RING_BARS = CTA2 ? 2 * (NA + NB) : 2 * STAGES;
     static constexpr int SMEM_BYTES = RING_BYTES + SMEM_EPI + Y_BYTES + 768;
 };
 
@@ -204,12 +189,14 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     // produced: the hand-over is a per-tile mbarrier inside the CTA, there is no grid-wide barrier, no
     // per-layer launch gap and no per-layer tail.
     static_assert(!TOWER || (CTA2 && EPI == EPI_LN_SE), "tower kernel = pair mode with both epilogues compiled in");
-    constexpr bool YSMEM = CTA2 && EPI == EPI_LN_SE;
+    constexpr bool YSMEM = EPI == EPI_LN_SE;
     using Cfg = TcCfg<BN, CTA2, YSMEM>;
     constexpr int STAGE_BYTES = Cfg::STAGE_BYTES;
     constexpr int NSTAGES = Cfg::STAGES;
     static_assert(!CTA2 || (A4D && BN == 256 && (EPI == EPI_LN || EPI == EPI_LN_SE || EPI == EPI_F32)),
                   "pair mode: tower convs only");
+    static_assert(CTA2 || ((BN == LD_POLICY && (EPI == EPI_LN73 || EPI == EPI_LN73_GATHER)) || (BN == N_VALUE_HIDDEN && EPI == EPI_RAW)),
+                  "single CTA: narrow head GEMMs only");
     const uint32_t cta_rank = CTA2 ? __shfl_sync(0xffffffffu, cluster_ctarank(), 0) : 0u;
     const int work0 = CTA2 ? (int)(blockIdx.x >> 1) : (int)blockIdx.x;
     const int work_stride = CTA2 ? (int)(gridDim.x >> 1) : (int)gridDim.x;
@@ -218,14 +205,12 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     // the pointers directly from the __shared__ symbol keeps every access an LDS/STS (a pointer
     // laundered through an integer cast degrades to generic LD/ST).
     extern __shared__ __align__(1024) uint8_t smem[];
-    constexpr bool AREUSE = Cfg::AREUSE;
     constexpr int NA = Cfg::NA, NB = Cfg::NB, A_BOX = Cfg::A_BOX_BYTES, B_TILE = Cfg::B_BYTES;
     constexpr int NRB = Cfg::N_RING_BARS;
     float *s_bias = reinterpret_cast<float *>(smem + Cfg::RING_BYTES);
     float *s_gamma = s_bias + 256;
     float *s_beta = s_gamma + 256;
-    float *s_pool = s_beta + 256;   // [4 quads][256]
-    float *s_mean = s_pool + 1024;  // [2 boards][256]
+    float *s_mean = s_beta + 256 + 1024;  // [2 boards][256] (the 4 KB before it are unused)
     float *s_hid = s_mean + 512;    // [2][128]
     float *s_gate = s_hid + 256;    // [2][256]
     float *s_stat = s_gate + 512;   // [2 column halves][128 rows][sum, sumsq]
@@ -247,7 +232,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     auto tfull_bar = [&](int s) { return bar_base + 8u * (NRB + s); };
     auto tempty_bar = [&](int s) { return bar_base + 8u * (NRB + 2 + s); };
     auto ready_bar = [&](int s) { return bar_base + 8u * (NRB + 4 + s); };  // TOWER: tile s written by layer l
-    // AREUSE rings: activation boxes first, then weight tiles
+    // pair rings: activation boxes first, then weight tiles
     auto afull_bar = [&](int s) { return bar_base + 8u * s; };
     auto aempty_bar = [&](int s) { return bar_base + 8u * (NA + s); };
     auto bfull_bar = [&](int s) { return bar_base + 8u * (2 * NA + s); };
@@ -349,7 +334,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                 if (TOWER && layer > 0) mbar_wait(ready_bar(slot), (uint32_t)(layer - 1) & 1u);  // this tile's input is written
                 const int tile = EPI == EPI_RAW ? work / args.n_splits : (CTA2 ? work * 2 + (int)cta_rank : work);
                 const int split = EPI == EPI_RAW ? work % args.n_splits : 0;
-                if constexpr (AREUSE) {
+                if constexpr (CTA2) {
                     const int nd = P.taps == 9 ? 3 : 1;
                     for (int kc = 0; kc < P.kchunks; kc++) {
                         // channel chunk of the A / B tensor this k step reads (the same one unless the operands are split)
@@ -404,12 +389,6 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                         const uint32_t a_dst = smem_base + stage * STAGE_BYTES;
                         const uint32_t b_dst = a_dst + TC_A_BYTES;
                         if (!elect_one()) {
-                        } else if (CTA2) {
-                            // both CTAs load into their own shared memory and complete on the LEADER's barrier,
-                            // which the leader alone arms with the bytes of both
-                            if (cta_rank == 0) mbar_expect_tx(full_bar(stage), 2 * STAGE_BYTES);
-                            tma2_load_4d(a_dst, P.ma, full_bar(stage), kc * TC_BK, dx, dy, tile * 2);
-                            tma2_load_2d(b_dst, P.mw, full_bar(stage), kc * TC_BK, tap * BN + (int)cta_rank * (BN / 2));
                         } else if (A4D) {
                             mbar_expect_tx(full_bar(stage), STAGE_BYTES);
                             tma_load_4d(a_dst, &map_a, full_bar(stage), kc * TC_BK, dx, dy, tile * 2);
@@ -449,7 +428,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                 if (args.prof) pc_wait_tempty += clock64() - t0;
                 tc_fence_after();
                 const uint32_t d_tmem = tmem_base + (uint32_t)(as * 256);
-                if constexpr (AREUSE) {
+                if constexpr (CTA2) {
                     const int nd = P.taps == 9 ? 3 : 1;
                     uint32_t acc = 0;
                     for (int g = 0; g < P.kchunks * nd; g++) {
@@ -498,17 +477,10 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                     const uint64_t db = umma_desc_sw128(a_addr + TC_A_BYTES);
                     if (elect_one()) {
 #pragma unroll
-                        for (int k = 0; k < TC_BK / 16; k++) {
-                            // +32 bytes per K=16 slice inside the 128-byte swizzle row
-                            if (CTA2)
-                                tc2_mma_bf16(d_tmem, da + (uint64_t)(k * 2), db + (uint64_t)(k * 2), idesc,
-                                             (uint32_t)((kb | k) != 0));
-                            else
-                                tc_mma_bf16(d_tmem, da + (uint64_t)(k * 2), db + (uint64_t)(k * 2), idesc,
-                                            (uint32_t)((kb | k) != 0));
-                        }
-                        if (CTA2) tc2_commit_mc(empty_bar(stage));
-                        else tc_commit(empty_bar(stage));
+                        for (int k = 0; k < TC_BK / 16; k++)  // +32 bytes per K=16 slice inside the 128-byte swizzle row
+                            tc_mma_bf16(d_tmem, da + (uint64_t)(k * 2), db + (uint64_t)(k * 2), idesc,
+                                        (uint32_t)((kb | k) != 0));
+                        tc_commit(empty_bar(stage));
                     }
                     __syncwarp();
                     if (++stage == NSTAGES) {
@@ -516,10 +488,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                         phase ^= 1u;
                     }
                 }
-                if (elect_one()) {
-                    if (CTA2) tc2_commit_mc(tfull_bar(as));
-                    else tc_commit(tfull_bar(as));
-                }
+                if (elect_one()) tc_commit(tfull_bar(as));
                 __syncwarp();
             }
             }
@@ -533,8 +502,8 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     } else if ((EPI == EPI_LN || EPI == EPI_LN_SE || EPI == EPI_LN73_GATHER || EPI == EPI_F32) || warp < 6) {
         const int quad = warp & 3;
         const int row = quad * 32 + lane;
-        // pair mode with the shared activation box: accumulator row = (rank, board, file); orow = its row in memory
-        const int orow = AREUSE ? ((row >> 3) & 1) * 64 + (row >> 4) * 8 + (row & 7) : row;
+        // pair kernels (shared activation box): accumulator row = (rank, board, file); orow = its row in memory
+        const int orow = ((row >> 3) & 1) * 64 + (row >> 4) * 8 + (row & 7);
         const int te = (warp - 2) * 32 + lane;  // 0..255 (0..127 for the 4-warp epilogues)
         const int chalf = (warp - 2) >> 2;      // which 128-column half of the tile this warp owns
         int it = 0;
@@ -583,7 +552,6 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
 
             if constexpr (EPI == EPI_F32) {
                 // ---- bias only: the fp32 accumulator goes to memory (this warp: 128 columns of its 32 rows) ----
-                static_assert(EPI != EPI_F32 || AREUSE, "fp32 output: pair mode only");
                 uint32_t r[32];
                 const int c0 = chalf * 128;
                 uint8_t *stg = s_stage + (warp - 2) * 2048;
@@ -872,12 +840,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                 }
                 long long tp2 = prof ? clock64() : 0;
                 pe_stats += tp2 - tp1;
-                // residual: this warp's 32 rows x 128 columns, requested now with a coalesced mapping
-                // (xa[ch*4+k] = row (lane>>2)+8k, 16-byte chunk lane&3 of 32-column chunk ch), consumed
-                // after the SE phase through the staging tile
                 uint8_t *stg = s_stage + (warp - 2) * 2048;
-                const size_t wrow0 = (size_t)tile * TC_BM + quad * 32;  // first global row of this warp
-                uint4 xa[16];
                 // FC1 weights do not depend on anything computed here: request them before the pooling pass
                 // so their L2 latency is hidden (thread = (hidden unit j, channel half hc))
                 uint4 w1v[16];
@@ -917,16 +880,13 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                                     make_uint4(pw[0], pw[1], pw[2], pw[3]);
                             }
                         }
-                        if (!se_fc) {
-                            // residual-only block (use_se=False): no pooling
-                        } else if constexpr (AREUSE) {
+                        if (se_fc) {  // (a residual-only block, use_se=False, has no pooling)
                             // partial sums per (quadrant, board) live in the (idle) store-staging area
                             int i0;
                             const float2 ps = warp_transpose_reduce_2boards(y, lane, i0);
                             float *s_poolx = reinterpret_cast<float *>(s_stage);
                             *reinterpret_cast<float2 *>(s_poolx + (quad * 2 + ((lane >> 3) & 1)) * 256 + c0 + ch * 32 + i0) = ps;
-                        } else
-                            s_pool[quad * 256 + c0 + ch * 32 + lane] = warp_transpose_reduce(y, lane);
+                        }
                         if (ch < 3) tmem_wait_ld();
                     }
                     if constexpr (YSMEM) {
@@ -947,12 +907,9 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                     for (int i = 0; i < 2; i++) {
                         const int idx = te + 256 * i;  // [board][channel]
                         const int b = idx >> 8, c = idx & 255;
-                        if constexpr (AREUSE) {
-                            const float *s_poolx = reinterpret_cast<const float *>(s_stage);
-                            s_mean[idx] = ((s_poolx[b * 256 + c] + s_poolx[(2 + b) * 256 + c]) +
-                                           (s_poolx[(4 + b) * 256 + c] + s_poolx[(6 + b) * 256 + c])) * (1.f / 64.f);
-                        } else
-                            s_mean[idx] = (s_pool[(2 * b) * 256 + c] + s_pool[(2 * b + 1) * 256 + c]) * (1.f / 64.f);
+                        const float *s_poolx = reinterpret_cast<const float *>(s_stage);
+                        s_mean[idx] = ((s_poolx[b * 256 + c] + s_poolx[(2 + b) * 256 + c]) +
+                                       (s_poolx[(4 + b) * 256 + c] + s_poolx[(6 + b) * 256 + c])) * (1.f / 64.f);
                     }
                     epi_bar_sync();
                     // ---- excitation FC1 (256 -> 128): thread = (hidden unit j, channel half hc), both boards
@@ -985,17 +942,9 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                         s_hidp[(hc * 2 + 0) * 128 + j] = h0;
                         s_hidp[(hc * 2 + 1) * 128 + j] = h1;
                     }
-                    // FC2 weights (thread = channel te) and the residual rows are requested now; both are
-                    // consumed two barriers later
+                    // FC2 weights (thread = channel te) are requested now and consumed two barriers later
 #pragma unroll
                     for (int u = 0; u < 16; u++) w2v[u] = __ldg(P.w2p + u * 256 + te);
-                    if constexpr (!YSMEM) {
-                        const uint4 *xw = reinterpret_cast<const uint4 *>(P.resid + (wrow0 + (lane >> 2)) * BN + c0) + (lane & 3);
-#pragma unroll
-                        for (int ch = 0; ch < 4; ch++)
-#pragma unroll
-                            for (int k = 0; k < 4; k++) xa[ch * 4 + k] = xw[(size_t)k * 8 * (BN / 8) + ch * 4];
-                    }
                     epi_bar_sync();
                     {
                         const int b = te >> 7, j = te & 127;  // [board][hidden unit]
@@ -1033,13 +982,6 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                     epi_bar_sync();
                     } else {
                         // residual-only block: gate = 1, so the final pass computes relu(y + x) exactly
-                    if constexpr (!YSMEM) {
-                        const uint4 *xw = reinterpret_cast<const uint4 *>(P.resid + (wrow0 + (lane >> 2)) * BN + c0) + (lane & 3);
-#pragma unroll
-                        for (int ch = 0; ch < 4; ch++)
-#pragma unroll
-                            for (int k = 0; k < 4; k++) xa[ch * 4 + k] = xw[(size_t)k * 8 * (BN / 8) + ch * 4];
-                    }
                         s_gate[te] = 1.f;
                         s_gate[256 + te] = 1.f;
                         epi_bar_sync();
@@ -1091,19 +1033,14 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                     tile_done(slot);
                     continue;  // the accumulator was released after the pooling pass
                 }
-                // ---- final pass: y (recomputed from TMEM), [gate * y + x], ReLU, bf16 store ------
-                const float *gate = s_gate + (quad >> 1) * 256;
-                uint8_t *gout = reinterpret_cast<uint8_t *>(static_cast<__nv_bfloat16 *>(P.out) + wrow0 * BN + c0);
+                // ---- final pass of the LayerNorm-only layers: y (recomputed from TMEM), ReLU, bf16 store ------
                 uint8_t *gtile = reinterpret_cast<uint8_t *>(static_cast<__nv_bfloat16 *>(P.out) + (size_t)tile * TC_BM * BN + c0);
-                (void)gtile;
                 uint32_t rm[32];
                 tmem_ld32(tcol, r);
 #pragma unroll
                 for (int ch = 0; ch < 4; ch++) {
                     if (ch < 3) tmem_ld32_nowait(tcol + (ch + 1) * 32, (ch & 1) ? r : rm);
                     const uint32_t(&cur)[32] = (ch & 1) ? rm : r;
-                    uint4 xr[4];
-                    if (!YSMEM && is_se) staged_gather_64B(stg, lane, xa + ch * 4, xr);
                     uint4 pk[4];
 #pragma unroll
                     for (int j = 0; j < 16; j++) {
@@ -1111,12 +1048,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                         float y0 = ln_apply(__fadd_rn(__uint_as_float(cur[2 * j]), s_bias[c]), mean, rstd, s_gamma[c], s_beta[c]);
                         float y1 = ln_apply(__fadd_rn(__uint_as_float(cur[2 * j + 1]), s_bias[c + 1]), mean, rstd, s_gamma[c + 1],
                                             s_beta[c + 1]);
-                        if (!YSMEM && is_se) {
-                            const uint4 xq = xr[j >> 2];
-                            const uint32_t xw = (j & 3) == 0 ? xq.x : ((j & 3) == 1 ? xq.y : ((j & 3) == 2 ? xq.z : xq.w));
-                            y0 = fmaxf(fmaf(gate[c], y0, __uint_as_float(xw << 16)), 0.f);
-                            y1 = fmaxf(fmaf(gate[c + 1], y1, __uint_as_float(xw & 0xffff0000u)), 0.f);
-                        } else if (P.relu) {
+                        if (P.relu) {
                             y0 = fmaxf(y0, 0.f);
                             y1 = fmaxf(y1, 0.f);
                         }
@@ -1127,10 +1059,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                         else if ((j & 3) == 2) pk[j >> 2].z = hv;
                         else pk[j >> 2].w = hv;
                     }
-                    if constexpr (AREUSE)
-                        staged_store_64B_hbw(stg, lane, pk, gtile + ch * 64, (size_t)BN * 2, quad);
-                    else
-                        staged_store_64B(stg, lane, pk, gout + ch * 64, (size_t)BN * 2, 32);
+                    staged_store_64B_hbw(stg, lane, pk, gtile + ch * 64, (size_t)BN * 2, quad);
                     if (ch < 3) tmem_wait_ld();
                 }
                 if (prof) pe_final += clock64() - tp2;
@@ -1185,14 +1114,13 @@ static EncodeTiledFn get_encode()
 struct ActMap {
     const void *ptr;
     int rows, c;
-    bool hbw;
     CUtensorMap map;
 };
 
+// bn == 256: a convolution of the CTA-pair kernels, whose weight box {64, 128} is the half of the weight rows one CTA of
+// the pair stages; otherwise a single-CTA head GEMM with the weight box {64, bn}
 struct TcConv {
     CUtensorMap map_w;
-    CUtensorMap map_w_half;  // box {64, 128}: the half of the weight rows one CTA of a pair stages
-    bool pair_ok = false;
     int taps, k_per_tap, bn, epi;
     int split_pairs = 0, split_kreal = 0;  // FP32 parity mode: (A plane, B plane) pairs of the bf16x3 split
     uint8_t split_ap[8] = {0}, split_bp[8] = {0};
@@ -1271,20 +1199,11 @@ int tc_conv_create(TcConv **out, const __nv_bfloat16 *w, int taps, int k_per_tap
     // weights [taps * bn rows][k_per_tap], K-major
     cuuint64_t dims[2] = {(cuuint64_t)k_per_tap, (cuuint64_t)taps * bn};
     cuuint64_t strides[1] = {(cuuint64_t)k_per_tap * 2};
-    cuuint32_t box[2] = {TC_BK, (cuuint32_t)bn};
+    cuuint32_t box[2] = {TC_BK, (cuuint32_t)(bn == 256 ? bn / 2 : bn)};
     int rc = tc_encode_map(&c->map_w, w, 2, dims, strides, box, "weights");
     if (rc != SC_OK) {
         delete c;
         return rc;
-    }
-    if (bn == 256 && (epi == EPI_LN || epi == EPI_LN_SE)) {
-        cuuint32_t box2[2] = {TC_BK, 128};
-        rc = tc_encode_map(&c->map_w_half, w, 2, dims, strides, box2, "weights (pair half)");
-        if (rc != SC_OK) {
-            delete c;
-            return rc;
-        }
-        c->pair_ok = true;
     }
     // function attributes belong to the device (context): set them once per device, not once per process
     static std::mutex attr_mu;
@@ -1294,8 +1213,6 @@ int tc_conv_create(TcConv **out, const __nv_bfloat16 *w, int taps, int k_per_tap
     std::lock_guard<std::mutex> lk(attr_mu);
     bool &attr_set = attr_done[dev];
     if (!attr_set) {
-        SCB_CHECK((set_smem_attr<256, EPI_LN, true>()));
-        SCB_CHECK((set_smem_attr<256, EPI_LN_SE, true>()));
         SCB_CUDA(cudaFuncSetAttribute(tc_gemm_kernel<256, EPI_LN, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                       TcCfg<256, true>::SMEM_BYTES));
         SCB_CUDA(cudaFuncSetAttribute(tc_gemm_kernel<256, EPI_LN_SE, true, true>,
@@ -1330,12 +1247,11 @@ int tc_split_conv_create(TcConv **out, const __nv_bfloat16 *w3, int taps, int ci
     cuuint64_t dims[2] = {(cuuint64_t)3 * cin_pad, (cuuint64_t)taps * 256};
     cuuint64_t strides[1] = {(cuuint64_t)3 * cin_pad * 2};
     cuuint32_t box2[2] = {TC_BK, 128};
-    int rc = tc_encode_map(&c->map_w_half, w3, 2, dims, strides, box2, "split weights (pair half)");
+    int rc = tc_encode_map(&c->map_w, w3, 2, dims, strides, box2, "split weights (pair half)");
     if (rc != SC_OK) {
         delete c;
         return rc;
     }
-    c->pair_ok = true;
     c->split_kreal = cin_pad / TC_BK;
     if (a_planes == 3) {
         static const uint8_t ap[6] = {0, 1, 2, 0, 1, 0}, bp[6] = {2, 1, 0, 1, 0, 0};
@@ -1398,16 +1314,13 @@ int tc_tower_create(TcTower **out, const TcTowerLayerDesc *descs, int n, int boa
     std::vector<TowerLayer> h((size_t)n);
     for (int i = 0; i < n; i++) {
         const TcConv *c = descs[i].conv;
-        if (!c || !c->pair_ok || c->bn != 256 || (c->epi != EPI_LN && c->epi != EPI_LN_SE)) {
+        if (!c || c->bn != 256 || (c->epi != EPI_LN && c->epi != EPI_LN_SE)) {
             set_error("tc_tower_create: layer is not a 256-wide tower convolution");
             return SC_E_INVAL;
         }
         memset(&h[i], 0, sizeof(TowerLayer));
-        if (TcCfg<256, true, true>::AREUSE)
-            SCB_CHECK(tc_make_act_map_hbw(descs[i].in, boards_alloc, c->k_per_tap, &h[i].map_a));
-        else
-            SCB_CHECK(make_act_map_4d(descs[i].in, boards_alloc, c->k_per_tap, &h[i].map_a));
-        h[i].map_w = c->map_w_half;
+        SCB_CHECK(tc_make_act_map_hbw(descs[i].in, boards_alloc, c->k_per_tap, &h[i].map_a));
+        h[i].map_w = c->map_w;
         h[i].out = descs[i].out;
         h[i].resid = descs[i].resid;
         h[i].bias = c->bias;
@@ -1509,21 +1422,18 @@ int tc_conv_launch(TcConv *c, const __nv_bfloat16 *in, int rows_alloc, int n_uni
 {
     if (n_units <= 0) return SC_OK;
     const bool a4d = c->epi != EPI_RAW;
-    // CTA-pair (cta_group::2) path for the 256-wide tower convolutions: clusters of two CTAs, each pair
-    // owns a 256-row tile (4 boards).  SCB200_CTA_PAIR=0 selects the single-CTA kernel.
-    static const bool pair_enabled = !(getenv("SCB200_CTA_PAIR") && getenv("SCB200_CTA_PAIR")[0] == '0');
-    const bool use_pair = pair_enabled && c->pair_ok;  // also for a single tile: the arithmetic must not depend on the batch size
-    const bool hbw = use_pair && TcCfg<256, true>::AREUSE;
+    // CTA-pair (cta_group::2) kernels for every 256-wide convolution: clusters of two CTAs, each pair owns a 256-row
+    // tile (4 boards) -- also for a single tile: the arithmetic must not depend on the batch size
+    const bool pair = c->bn == 256;
     const CUtensorMap *ma = nullptr;
     for (auto &m : c->act_maps)
-        if (m.ptr == in && m.rows == rows_alloc && m.c == c->k_per_tap && m.hbw == hbw) ma = &m.map;
+        if (m.ptr == in && m.rows == rows_alloc && m.c == c->k_per_tap) ma = &m.map;
     if (!ma) {
         ActMap am;
         am.ptr = in;
         am.rows = rows_alloc;
         am.c = c->k_per_tap;
-        am.hbw = hbw;
-        if (hbw)
+        if (pair)
             SCB_CHECK(tc_make_act_map_hbw(in, rows_alloc, c->k_per_tap, &am.map));
         else if (a4d)
             SCB_CHECK(make_act_map_4d(in, rows_alloc, c->k_per_tap, &am.map));
@@ -1571,7 +1481,7 @@ int tc_conv_launch(TcConv *c, const __nv_bfloat16 *in, int rows_alloc, int n_uni
     }
     const int n_work = a4d ? a.n_tiles : a.n_tiles * a.n_splits;
     const int grid = n_work < num_sms ? n_work : num_sms;
-    if (use_pair) {
+    if (pair) {
         const int n_pairs = (a.n_tiles + 1) / 2;
         int g2 = 2 * n_pairs;
         if (g2 > (num_sms & ~1)) g2 = num_sms & ~1;
@@ -1587,49 +1497,36 @@ int tc_conv_launch(TcConv *c, const __nv_bfloat16 *in, int rows_alloc, int n_uni
         attr[0].val.clusterDim.z = 1;
         cfg.attrs = attr;
         cfg.numAttrs = 1;
-        if (c->epi == EPI_F32) {
-            SCB_CUDA(cudaLaunchKernelEx(&cfg, tc_gemm_kernel<256, EPI_F32, true, true>, *ma, c->map_w_half, a));
-            goto launched;
-        }
-        if (c->epi == EPI_LN)
-            SCB_CUDA(cudaLaunchKernelEx(&cfg, tc_gemm_kernel<256, EPI_LN, true, true>, *ma, c->map_w_half, a));
+        if (c->epi == EPI_F32)
+            SCB_CUDA(cudaLaunchKernelEx(&cfg, tc_gemm_kernel<256, EPI_F32, true, true>, *ma, c->map_w, a));
+        else if (c->epi == EPI_LN)
+            SCB_CUDA(cudaLaunchKernelEx(&cfg, tc_gemm_kernel<256, EPI_LN, true, true>, *ma, c->map_w, a));
         else {
             if (!resid) {
                 set_error("tc_conv_launch: residual epilogue without block input");
                 return SC_E_INVAL;
             }
-            SCB_CUDA(cudaLaunchKernelEx(&cfg, tc_gemm_kernel<256, EPI_LN_SE, true, true>, *ma, c->map_w_half, a));
+            SCB_CUDA(cudaLaunchKernelEx(&cfg, tc_gemm_kernel<256, EPI_LN_SE, true, true>, *ma, c->map_w, a));
         }
-        goto launched;
-    }
-    switch (c->epi) {
-    case EPI_LN:
-        tc_gemm_kernel<256, EPI_LN, true><<<grid, TC_THREADS, TcCfg<256>::SMEM_BYTES, st>>>(*ma, c->map_w, a);
-        break;
-    case EPI_LN_SE:
-        if (!resid) {
-            set_error("tc_conv_launch: residual epilogue without block input");
+    } else {
+        switch (c->epi) {
+        case EPI_LN73:
+            if (gather) {
+                a.gather = *gather;
+                tc_gemm_kernel<LD_POLICY, EPI_LN73_GATHER, true><<<grid, TC_THREADS, TcCfg<LD_POLICY>::SMEM_BYTES, st>>>(*ma, c->map_w, a);
+            } else
+                tc_gemm_kernel<LD_POLICY, EPI_LN73, true><<<grid, TC_THREADS, TcCfg<LD_POLICY>::SMEM_BYTES, st>>>(*ma, c->map_w, a);
+            break;
+        case EPI_RAW:
+            if (finish) a.vfin = *finish;
+            tc_gemm_kernel<N_VALUE_HIDDEN, EPI_RAW, false><<<grid, TC_THREADS, TcCfg<N_VALUE_HIDDEN>::SMEM_BYTES, st>>>(
+                *ma, c->map_w, a);
+            break;
+        default:
+            set_error("tc_conv_launch: bad epilogue");
             return SC_E_INVAL;
         }
-        tc_gemm_kernel<256, EPI_LN_SE, true><<<grid, TC_THREADS, TcCfg<256>::SMEM_BYTES, st>>>(*ma, c->map_w, a);
-        break;
-    case EPI_LN73:
-        if (gather) {
-            a.gather = *gather;
-            tc_gemm_kernel<LD_POLICY, EPI_LN73_GATHER, true><<<grid, TC_THREADS, TcCfg<LD_POLICY>::SMEM_BYTES, st>>>(*ma, c->map_w, a);
-        } else
-            tc_gemm_kernel<LD_POLICY, EPI_LN73, true><<<grid, TC_THREADS, TcCfg<LD_POLICY>::SMEM_BYTES, st>>>(*ma, c->map_w, a);
-        break;
-    case EPI_RAW:
-        if (finish) a.vfin = *finish;
-        tc_gemm_kernel<N_VALUE_HIDDEN, EPI_RAW, false><<<grid, TC_THREADS, TcCfg<N_VALUE_HIDDEN>::SMEM_BYTES, st>>>(
-            *ma, c->map_w, a);
-        break;
-    default:
-        set_error("tc_conv_launch: bad epilogue");
-        return SC_E_INVAL;
     }
-launched:
     SCB_CUDA(cudaGetLastError());
     if (want_prof) {
         // debugging aid: per-phase SM-cycle counters of this launch, averaged over CTAs (synchronous!)

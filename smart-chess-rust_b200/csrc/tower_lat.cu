@@ -45,7 +45,6 @@ struct alignas(64) LatLayer {
     CUtensorMap map_a1;  // the same tensor, box of one board
     CUtensorMap map_w;  // weights {cin, cout, dx, dy}, box {64, NC, 1, 3 | 1}
     CUtensorMap map_o, map_o1;  // output {C, file, board, rank}, box {NC, 8, 2 | 1, 8}, no swizzle (TMA store hand-over)
-    void *out;
     const __nv_bfloat16 *resid;
     const float *bias, *gamma, *beta;
     const uint4 *se_w1s, *se_w2s;  // per cluster rank: fc1 columns [NC / 8][128] x 8 bf16, fc2 rows [16][NC] x 8 bf16
@@ -58,7 +57,6 @@ struct LatArgs {
     int n_layers;
     int n_tiles;
     long long *prof;  // optional [grid][16] cycle counters (SCB200_PHASE_PROFILE=1)
-    int tma_store;    // hand-over: stage the CTA's output slice in shared memory, ONE thread stores it with the TMA
 };
 
 template <int CL, int NB = 2> struct LatCfg {
@@ -440,11 +438,9 @@ __global__ void __launch_bounds__(LAT_THREADS, 1) lat_tower_kernel(const LatArgs
             }
 #pragma unroll
             for (int j = 0; j < NC; j++) a[j] = ln_apply(a[j], mean, rstd, s_gamma[j], s_beta[j]);
-            __nv_bfloat16 *og = static_cast<__nv_bfloat16 *>(L.out) + grow * 256 + c0;
-            // TMA-store hand-over: the row goes to the staging tile [row][NC] instead (row = accumulator row = the box's
-            // (rank, board, file) order, so the tile is exactly the store box)
-            uint4 *so = reinterpret_cast<uint4 *>(smem + Cfg::OFF_OUT + row * NC * 2);
-            uint4 *odst = args.tma_store ? so : reinterpret_cast<uint4 *>(og);
+            // the row goes to the output staging tile [row][NC] (row = accumulator row = the store box's (rank, board, file)
+            // order, so the tile is exactly the store box)
+            uint4 *odst = reinterpret_cast<uint4 *>(smem + Cfg::OFF_OUT + row * NC * 2);
             if (!L.se) {
                 // ---- bias + LayerNorm (+ReLU) -> bf16 ----
                 if (active) {
@@ -573,18 +569,15 @@ __global__ void __launch_bounds__(LAT_THREADS, 1) lat_tower_kernel(const LatArgs
                     }
                 }
             }
-            // ---- hand the layer's output to the TMA loads of the whole cluster: every thread makes its stores visible
-            //      to the async proxy (this fence waits for them at GPU scope), block barrier, then ONE warp signals the
-            //      `ready` barrier of every CTA (release is cumulative over the barrier) ----
+            // ---- hand the layer's output to the TMA loads of the whole cluster: every thread makes its staging-tile
+            //      stores visible to the async proxy, block barrier, then ONE warp stores the CTA's slice and signals
+            //      the `ready` barrier of every CTA ----
             const long long tf0 = prof ? clock64() : 0;
-            if (args.tma_store)
-                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // staging tile -> visible to the TMA
-            else
-                asm volatile("fence.proxy.async;" ::: "memory");
+            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
             const long long tf1 = prof ? clock64() : 0;
             lat_epi_sync();
             const long long tf2 = prof ? clock64() : 0;
-            if (args.tma_store && quad == 0) {
+            if (quad == 0) {
                 // one thread stores the CTA's slice and waits until the write is complete, then the warp signals
                 if (elect_one()) {
                     asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];" ::"l"(
@@ -701,7 +694,6 @@ int lat_tower_create(LatTower **out, const LatLayerDesc *descs, int n, int board
                 lat_tower_destroy(t);
                 return rc;
             }
-            L.out = d.out;
             L.resid = d.resid;
             L.bias = d.bias;
             L.gamma = d.gamma;
@@ -761,9 +753,6 @@ template <int CL, int NB> static int lat_launch(const LatTower *t, int v, int n_
     a.n_layers = max_layers > 0 && max_layers < t->n_layers ? max_layers : t->n_layers;
     a.n_tiles = n_tiles;
     a.prof = nullptr;
-    // SCB200_LAT_TMA_STORE=0: per-thread global stores + async-proxy fence instead (A/B: 519 k vs 503 k cycles at n = 1)
-    static const bool tma_store = !(getenv("SCB200_LAT_TMA_STORE") && getenv("SCB200_LAT_TMA_STORE")[0] == '0');
-    a.tma_store = tma_store ? 1 : 0;
     static const bool want_prof = getenv("SCB200_PHASE_PROFILE") != nullptr;
     if (want_prof) {
         SCB_CUDA(cudaMalloc(&a.prof, (size_t)n_tiles * CL * 16 * sizeof(long long)));
@@ -795,7 +784,7 @@ template <int CL, int NB> static int lat_launch(const LatTower *t, int v, int n_
         fprintf(stderr,
                 "[lat CL=%d NB=%d tiles=%d layers=%d] A-producer: wait_ready %.0f wait_empty %.0f | mma: total %.0f wait_A(first box) %.0f "
                 "wait(rest) %.0f (%.0f) | epilogue: wait_tmem_full %.0f work %.0f (tmem load %.0f, stat exchange %.0f, SE %.0f, "
-                "proxy fence %.0f, block barrier %.0f, gpu fence + signal %.0f)\n",
+                "proxy fence %.0f, block barrier %.0f, TMA store + signal %.0f)\n",
                 CL, NB, n_tiles, a.n_layers, acc[0], acc[1], acc[5], acc[2], acc[3], acc[4], acc[6], acc[9], acc[10], acc[7], acc[8],
                 acc[11], acc[12], acc[13]);
     }
