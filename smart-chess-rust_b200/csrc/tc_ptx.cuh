@@ -268,46 +268,51 @@ __device__ __forceinline__ float2 warp_transpose_reduce_2boards(float (&v)[32], 
 // ---- LayerNorm arithmetic shared by both kernels -------------------------------------------------------------
 // Written with explicit round-to-nearest intrinsics so that the compiler cannot contract / reassociate it
 // differently in different kernels: the latency kernel must produce the bits of the throughput kernel.
-// Statistics: per 32-channel chunk k the sums (s_k, q_k) of a = acc + bias and a * a (ln_chunk_stats: two 16-channel
-// halves, each four interleaved chains and a tree); combined as
+// Statistics: per group of channels the pair (s, M2) = (sum of a = acc + bias, sum of squares of a about the group's own
+// mean).  A 32-channel chunk computes both from its registers (ln_chunk_stats); chunks are merged with the pairwise
+// formula of ln_combine, in a fixed tree:
 //   half0 = (p0 + p1) + (p2 + p3), half1 = (p4 + p5) + (p6 + p7), total = half0 + half1
-// -- a fixed tree, so the chunks may be computed by different threads / CTAs.
-// half a chunk: 16 channels as four interleaved sequential chains (j mod 4) and a fixed tree
-__device__ __forceinline__ void ln_half_chunk_stats(const float *a /*[16]*/, float &s, float &q)
+// so the chunks may be computed by different threads / CTAs.  The variance is M2 / 256: unlike the one-pass
+// E[a^2] - mean^2 it does not cancel when the channel mean of a square is large next to its spread (a checkpoint whose
+// conv biases share a common offset), because no sum of squares is taken about a point far from the values.
+// A chunk: the deviations d = a - a[0] from its first channel as eight interleaved sequential chains (j mod 8) of sums
+// and of squares and a fixed tree, then s = sum d + 32 a[0] and M2 = sum d^2 - (sum d)^2 / 32.  a[0] lies within
+// sqrt(31) standard deviations of the chunk's mean, so that subtraction loses at most five bits; shifting by a[0]
+// rather than by the chunk's mean keeps the two chains independent (one pass, as short as unshifted sums).
+__device__ __forceinline__ void ln_chunk_stats(const float (&a)[32], float &s, float &m2)
 {
-    float s4[4] = {0.f, 0.f, 0.f, 0.f}, q4[4] = {0.f, 0.f, 0.f, 0.f};
+    float s8[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f}, q8[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+    const float k = a[0];
 #pragma unroll
-    for (int j = 0; j < 16; j++) {
-        s4[j & 3] = __fadd_rn(s4[j & 3], a[j]);
-        q4[j & 3] = __fmaf_rn(a[j], a[j], q4[j & 3]);
+    for (int j = 1; j < 32; j++) {
+        const float d = __fsub_rn(a[j], k);
+        s8[j & 7] = __fadd_rn(s8[j & 7], d);
+        q8[j & 7] = __fmaf_rn(d, d, q8[j & 7]);
     }
-    s = __fadd_rn(__fadd_rn(s4[0], s4[1]), __fadd_rn(s4[2], s4[3]));
-    q = __fadd_rn(__fadd_rn(q4[0], q4[1]), __fadd_rn(q4[2], q4[3]));
+    const float sd = __fadd_rn(__fadd_rn(__fadd_rn(s8[0], s8[1]), __fadd_rn(s8[2], s8[3])),
+                               __fadd_rn(__fadd_rn(s8[4], s8[5]), __fadd_rn(s8[6], s8[7])));
+    const float qd = __fadd_rn(__fadd_rn(__fadd_rn(q8[0], q8[1]), __fadd_rn(q8[2], q8[3])),
+                               __fadd_rn(__fadd_rn(q8[4], q8[5]), __fadd_rn(q8[6], q8[7])));
+    s = __fmaf_rn(32.f, k, sd);
+    m2 = fmaxf(__fmaf_rn(__fmul_rn(sd, -1.f / 32.f), sd, qd), 0.f);
 }
-// a 32-channel chunk = its two halves added (the latency kernel computes the halves in two threads)
-__device__ __forceinline__ float2 ln_join_halves(const float2 h0, const float2 h1)
+// (s, M2) of two groups of n channels each -> the union: M2 = M2a + M2b + (sa - sb)^2 / (2n), inv_2n = 1 / (2n)
+__device__ __forceinline__ float2 ln_combine(const float2 p, const float2 q, float inv_2n)
 {
-    return make_float2(__fadd_rn(h0.x, h1.x), __fadd_rn(h0.y, h1.y));
+    const float d = __fsub_rn(p.x, q.x);
+    return make_float2(__fadd_rn(p.x, q.x), __fmaf_rn(__fmul_rn(d, d), inv_2n, __fadd_rn(p.y, q.y)));
 }
-__device__ __forceinline__ void ln_chunk_stats(const float (&a)[32], float &s, float &q)
-{
-    float2 h0, h1;
-    ln_half_chunk_stats(a, h0.x, h0.y);
-    ln_half_chunk_stats(a + 16, h1.x, h1.y);
-    const float2 c = ln_join_halves(h0, h1);
-    s = c.x;
-    q = c.y;
-}
+// four 32-channel chunks -> 128 channels
 __device__ __forceinline__ float2 ln_half(const float2 p0, const float2 p1, const float2 p2, const float2 p3)
 {
-    return make_float2(__fadd_rn(__fadd_rn(p0.x, p1.x), __fadd_rn(p2.x, p3.x)),
-                       __fadd_rn(__fadd_rn(p0.y, p1.y), __fadd_rn(p2.y, p3.y)));
+    return ln_combine(ln_combine(p0, p1, 1.f / 64.f), ln_combine(p2, p3, 1.f / 64.f), 1.f / 128.f);
 }
+// two 128-channel halves -> mean and 1 / sqrt(var + eps) of all 256
 __device__ __forceinline__ void ln_finish(const float2 h0, const float2 h1, float eps, float &mean, float &rstd)
 {
-    mean = __fmul_rn(__fadd_rn(h0.x, h1.x), 1.f / 256.f);
-    const float var = fmaxf(__fsub_rn(__fmul_rn(__fadd_rn(h0.y, h1.y), 1.f / 256.f), __fmul_rn(mean, mean)), 0.f);
-    rstd = rsqrtf(__fadd_rn(var, eps));
+    const float2 t = ln_combine(h0, h1, 1.f / 256.f);
+    mean = __fmul_rn(t.x, 1.f / 256.f);
+    rstd = rsqrtf(__fadd_rn(__fmul_rn(t.y, 1.f / 256.f), eps));
 }
 // (a - mean) * rstd * gamma + beta with a = acc + bias already formed
 __device__ __forceinline__ float ln_apply(float a, float mean, float rstd, float gamma, float beta)

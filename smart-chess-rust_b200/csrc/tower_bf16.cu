@@ -808,8 +808,8 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                 uint32_t r[32];
                 float mean, rstd;
                 if (P.ln) {
-                    // one TMEM pass: per 32-channel chunk the sums of (acc + bias) and its square, combined in the
-                    // fixed tree of tc_ptx.cuh (the latency kernel computes the same chunks in other CTAs)
+                    // one TMEM pass: per 32-channel chunk the sum of a = acc + bias and its centred sum of squares,
+                    // combined in the fixed tree of tc_ptx.cuh (the latency kernel computes the same chunks in other CTAs)
                     uint32_t r2[32];
                     float2 p0, p1, p2, p3;
                     auto chunk_pair = [&](int ch, float2 &pa, float2 &pb) {
