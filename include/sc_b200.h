@@ -33,6 +33,10 @@ extern "C" {
                           cores as bf16x3 split operands (6 bf16 products per fp32 product) with fp32 accumulate  */
 #define SC_MODE_BF16 1 /* throughput mode: tcgen05 bf16 operands, fp32 accumulate      */
 #define SC_MODE_FP32_FFMA 2 /* FP32 on the CUDA cores only (FFMA): the referee of the parity mode                */
+#define SC_MODE_FP16 3 /* tensor cores with fp16 operands, fp32 accumulate: the kernels and launch structure of
+                          SC_MODE_BF16, rounding where it rounds but to fp16 (11 significant bits instead of 8).  A
+                          parked value (a layer output, the SE input) beyond +-65504 becomes +-inf, as in the reference's
+                          fp16 autocast; a weight beyond that range fails sc_create with SC_E_IO                  */
 
 #define SC_LOOKBACK 8       /* src/chess.rs:23 */
 #define SC_N_PLANES 112     /* 8 x 14, py/module.py:118-121 */
@@ -243,9 +247,9 @@ int sc_arena_create(sc_engine *white, sc_engine *black, const sc_selfplay_config
 int sc_random_positions(int n, uint64_t seed, int max_ply, sc_position *pos_out, sc_move *moves_out,
                         int32_t *move_off /* n+1 */, int max_moves_total);
 
-/* Test hook (bf16 engines): encodes n leaves and runs only the first n_layers (0 = all 41: stem, 19 x (conv1, conv2),
+/* Test hook (bf16 and fp16 engines): encodes n leaves and runs only the first n_layers (0 = all 41: stem, 19 x (conv1, conv2),
  * the two 256-wide head 1x1 convolutions) of the convolution tower with the throughput kernel (which = 0) or the
- * small-batch latency kernel (which = 1); copies the three activation buffers (bf16 bit patterns, [n][64][256]:
+ * small-batch latency kernel (which = 1); copies the three activation buffers (bf16 / fp16 bit patterns, [n][64][256]:
  * x = block input / output, t = conv1 output / policy head input, y = value head input) to the host.  Lets the tests
  * compare the two kernels layer by layer. */
 int sc_debug_tower(sc_engine *e, int n, const sc_position *pos, int n_layers, int which, uint16_t *x_out,

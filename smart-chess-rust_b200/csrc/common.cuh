@@ -2,6 +2,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <stdint.h>
 #include <string>
 
@@ -42,9 +43,12 @@ int launch_encode_f32(const sc_position *d_pos, int n, float *out /*[n][64][112]
                       cudaStream_t st);
 int launch_encode_bf16(const sc_position *d_pos, int n, __nv_bfloat16 *out /*[n][64][128]*/,
                        float *meta_out /*[n][8]*/, cudaStream_t st);
+int launch_encode_fp16(const sc_position *d_pos, int n, __half *out /*[n][64][128]*/, float *meta_out /*[n][8]*/,
+                       cudaStream_t st);
 // NCHW float planes (sc_forward_only input) -> NHWC
 int launch_nchw_to_nhwc_f32(const float *in, int n, float *out, cudaStream_t st);
 int launch_nchw_to_nhwc_bf16(const float *in, int n, __nv_bfloat16 *out, cudaStream_t st);
+int launch_nchw_to_nhwc_fp16(const float *in, int n, __half *out, cudaStream_t st);
 
 // ---- policy.cu ----------------------------------------------------------------------------
 // logits [n][64][LD_POLICY] fp32 (square-major) -> per-leaf log-sum-exp, legal-move gather,
@@ -75,16 +79,18 @@ int launch_value_finish(const float *hidden_pre, int n_split, int n, const float
                         const float *b1, const float *w2, const float *b2, float *value_out, cudaStream_t st);
 
 // ---- tower_bf16.cu (tcgen05) --------------------------------------------------------------
+// The 16-bit tensor-core modes share these kernels and interfaces: `fp16` selects fp16 operands instead of bf16, and
+// then every 16-bit buffer below (weights, activations; typed __nv_bfloat16) holds fp16 bit patterns.
 struct TcConv;  // opaque per-layer state (tensor maps)
 enum { TC_EPI_LN = 0, TC_EPI_LN_SE = 1, TC_EPI_LN73 = 2, TC_EPI_RAW = 3 };
 // w: bf16 [taps][bn][k_per_tap] (K-major B operand); bn = 256 (tower / head 1x1 convs),
 // 80 (policy 256->73, rows 73..79 zero) or 128 (value FC, taps = 1, k_per_tap = 16384)
 int tc_conv_create(TcConv **out, const __nv_bfloat16 *w, int taps, int k_per_tap, int bn, int epi, const float *bias,
-                   const float *gamma, const float *beta);
+                   const float *gamma, const float *beta, bool fp16);
 // FP32 parity mode: conv to 256 channels as a bf16x3 split GEMM on the tensor cores, fp32 [boards * 64][256] out (+ bias).
 // w3 = bf16 [taps][256][3 * cin_pad] (three planes side by side along K), activations bf16 [boards][64][a_planes * cin_pad]
 int tc_split_conv_create(TcConv **out, const __nv_bfloat16 *w3, int taps, int cin_pad, int a_planes, const float *bias);
-// squeeze-excitation weights for TC_EPI_LN_SE: fc1 packed [32][128][8] bf16, fc2 packed [16][256][8] bf16
+// squeeze-excitation weights for TC_EPI_LN_SE: fc1 packed [32][128][8], fc2 packed [16][256][8], in the operand type
 void tc_conv_set_se(TcConv *c, const void *w1p, const float *b1, const void *w2p, const float *b2);
 void tc_conv_destroy(TcConv *c);
 // convs: in = bf16 NHWC [rows_alloc boards][64][k_per_tap], n_units = boards.
@@ -121,7 +127,7 @@ struct TcTowerLayerDesc {
     const __nv_bfloat16 *resid;  // SE layers: block input (may alias out)
     int relu;
 };
-int tc_tower_create(TcTower **out, const TcTowerLayerDesc *descs, int n, int boards_alloc);
+int tc_tower_create(TcTower **out, const TcTowerLayerDesc *descs, int n, int boards_alloc, bool fp16);
 // group = tiles per CTA carried through all layers together (0 = all of the CTA's tiles)
 // max_layers > 0: only the first max_layers layers (sc_debug_tower's layer-by-layer comparison)
 int tc_tower_launch(TcTower *t, int n_boards, int num_sms, int group, cudaStream_t st, int max_layers = 0);
@@ -142,7 +148,7 @@ struct LatLayerDesc {
     const void *se_w1s8, *se_w2s8, *se_w1s4, *se_w2s4;
     const float *se_b1, *se_b2;
 };
-int lat_tower_create(LatTower **out, const LatLayerDesc *descs, int n, int boards_alloc);
+int lat_tower_create(LatTower **out, const LatLayerDesc *descs, int n, int boards_alloc, bool fp16);
 // largest batch the latency kernel takes (one wave of clusters); 0 if it cannot run on this device
 int lat_tower_max_boards(const LatTower *t);
 // SC_E_STATE (no message) when the batch does not fit: run the throughput kernel instead

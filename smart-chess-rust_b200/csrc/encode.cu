@@ -108,12 +108,14 @@ __global__ void __launch_bounds__(ENC_WARPS * 32) encode_f32_kernel(const sc_pos
     if (lane < 8) meta_out[b * 8 + lane] = lane < SC_N_META ? (float)pos[b].meta[lane] : 0.f;
 }
 
-// bf16 form (the network's own input): FOUR warps per position, 16 squares each.  The kernel is short (34 MB at 2048
-// leaves) and ends in a store stream, so it is bound by how many bytes are in flight when it starts: with one warp per
-// position the 32 store instructions of a position were issued one after another by a single warp.
-__global__ void __launch_bounds__(ENC_WARPS * 32) encode_bf16_kernel(const sc_position *__restrict__ pos, int n,
-                                                                     __nv_bfloat16 *__restrict__ out,
-                                                                     float *__restrict__ meta_out)
+// 16-bit form (the network's own input, ONE = the bit pattern of 1.0: 0x3F80 bf16, 0x3C00 fp16): FOUR warps per
+// position, 16 squares each.  The kernel is short (34 MB at 2048 leaves) and ends in a store stream, so it is bound by
+// how many bytes are in flight when it starts: with one warp per position the 32 store instructions of a position were
+// issued one after another by a single warp.
+template <uint32_t ONE>
+__global__ void __launch_bounds__(ENC_WARPS * 32) encode_16bit_kernel(const sc_position *__restrict__ pos, int n,
+                                                                      uint16_t *__restrict__ out,
+                                                                      float *__restrict__ meta_out)
 {
     __shared__ uint64_t s_slots[64];
     __shared__ uint64_t s_masks[128];
@@ -135,8 +137,8 @@ __global__ void __launch_bounds__(ENC_WARPS * 32) encode_bf16_kernel(const sc_po
         uint32_t w[4];
 #pragma unroll
         for (int j = 0; j < 4; j++) {
-            uint32_t lo = (uint32_t)((m[2 * j] >> s) & 1ULL) * 0x3F80u;      // bf16 1.0
-            uint32_t hi = (uint32_t)((m[2 * j + 1] >> s) & 1ULL) * 0x3F80u;
+            uint32_t lo = (uint32_t)((m[2 * j] >> s) & 1ULL) * ONE;
+            uint32_t hi = (uint32_t)((m[2 * j + 1] >> s) & 1ULL) * ONE;
             w[j] = lo | (hi << 16);
         }
         dst[it * 32 + lane] = make_uint4(w[0], w[1], w[2], w[3]);
@@ -163,7 +165,15 @@ int launch_encode_f32(const sc_position *d_pos, int n, float *out, float *meta_o
 int launch_encode_bf16(const sc_position *d_pos, int n, __nv_bfloat16 *out, float *meta_out, cudaStream_t st)
 {
     if (n <= 0) return SC_OK;
-    encode_bf16_kernel<<<n, ENC_WARPS * 32, 0, st>>>(d_pos, n, out, meta_out);
+    encode_16bit_kernel<0x3F80u><<<n, ENC_WARPS * 32, 0, st>>>(d_pos, n, reinterpret_cast<uint16_t *>(out), meta_out);
+    SCB_CUDA(cudaGetLastError());
+    return SC_OK;
+}
+
+int launch_encode_fp16(const sc_position *d_pos, int n, __half *out, float *meta_out, cudaStream_t st)
+{
+    if (n <= 0) return SC_OK;
+    encode_16bit_kernel<0x3C00u><<<n, ENC_WARPS * 32, 0, st>>>(d_pos, n, reinterpret_cast<uint16_t *>(out), meta_out);
     SCB_CUDA(cudaGetLastError());
     return SC_OK;
 }
@@ -172,6 +182,7 @@ int launch_encode_bf16(const sc_position *d_pos, int n, __nv_bfloat16 *out, floa
 template <typename T> __device__ __forceinline__ T cvt(float v);
 template <> __device__ __forceinline__ float cvt<float>(float v) { return v; }
 template <> __device__ __forceinline__ __nv_bfloat16 cvt<__nv_bfloat16>(float v) { return __float2bfloat16(v); }
+template <> __device__ __forceinline__ __half cvt<__half>(float v) { return __float2half_rn(v); }
 
 template <typename T, int LD>
 __global__ void __launch_bounds__(256) nchw_to_nhwc_kernel(const float *__restrict__ in, int n, T *__restrict__ out)
@@ -203,6 +214,14 @@ int launch_nchw_to_nhwc_bf16(const float *in, int n, __nv_bfloat16 *out, cudaStr
 {
     if (n <= 0) return SC_OK;
     nchw_to_nhwc_kernel<__nv_bfloat16, C_IN_PAD><<<n, 256, 0, st>>>(in, n, out);
+    SCB_CUDA(cudaGetLastError());
+    return SC_OK;
+}
+
+int launch_nchw_to_nhwc_fp16(const float *in, int n, __half *out, cudaStream_t st)
+{
+    if (n <= 0) return SC_OK;
+    nchw_to_nhwc_kernel<__half, C_IN_PAD><<<n, 256, 0, st>>>(in, n, out);
     SCB_CUDA(cudaGetLastError());
     return SC_OK;
 }

@@ -4,6 +4,7 @@
 // for n leaves at once: H2D of the packed positions and legal moves, plane encode, the
 // policy/value network, move-index gather + renormalisation, D2H of priors and values.
 // There is no CPU fallback: without an sm_100 device sc_create() fails with SC_E_NOGPU.
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -110,17 +111,46 @@ static uint16_t f2bf(float f)
     return (uint16_t)(u >> 16);
 }
 
+// float -> fp16 bits, round to nearest even (subnormals kept, beyond the range +-inf)
+static uint16_t f2h(float f)
+{
+    const __half h = __float2half_rn(f);
+    uint16_t r;
+    memcpy(&r, &h, 2);
+    return r;
+}
+
+// The weights of a 16-bit tensor-core engine that become MMA / SE operands, rounded to its operand type.  An fp16 engine
+// cannot represent a weight beyond +-65504: `bad` records one, and the load then fails naming the tensor (a bf16 engine
+// has the fp32 exponent range and takes every finite weight).
+struct Op16Weights {
+    bool fp16;
+    bool bad = false;
+    uint16_t operator()(float f)
+    {
+        if (!fp16) return f2bf(f);
+        if (fabsf(f) > 65504.f) bad = true;
+        return f2h(f);
+    }
+    int check(const std::string &tensor) const
+    {
+        if (!bad) return SC_OK;
+        set_error("weight blob: " + tensor + " has a weight beyond the fp16 range (|w| > 65504)");
+        return SC_E_IO;
+    }
+};
+
 struct ConvW {
     int taps = 1, cin = 0, cin_pad = 0, cout = 0, ldw = 0;
     float *w_f32 = nullptr;          // [taps][cin][ldw]        (fp32 mode)
-    __nv_bfloat16 *w_bf16 = nullptr; // [taps][cout][cin_pad]   (bf16 mode, K-major B operand)
+    __nv_bfloat16 *w_bf16 = nullptr; // [taps][cout][cin_pad]   (16-bit modes, K-major B operand; fp16 bits in fp16 mode)
     float *bias = nullptr, *gamma = nullptr, *beta = nullptr;
     TcConv *tc = nullptr;
 };
 
 struct SeW {
     float *w1t = nullptr, *b1 = nullptr, *w2t = nullptr, *b2 = nullptr;  // fp32 mode
-    uint16_t *w1p = nullptr, *w2p = nullptr;                            // bf16 mode, packed for the fused epilogue
+    uint16_t *w1p = nullptr, *w2p = nullptr;                            // 16-bit modes, packed for the fused epilogue
     uint16_t *w1s[2] = {nullptr, nullptr}, *w2s[2] = {nullptr, nullptr};  // latency kernel: sliced per cluster rank (CL = 8, 4)
 };
 
@@ -131,6 +161,8 @@ using namespace scb;
 struct sc_engine {
     int device = 0, mode = 0, max_batch = 0, n_blocks = 0, num_sms = 148;
     int mode_requested = 0;
+    // SC_MODE_BF16 / SC_MODE_FP16: the same tensor-core kernels with bf16 / fp16 operands (tc16() below)
+    bool fp16 = false;
     // FP32 parity mode: the 256-wide convolutions as bf16x3 split GEMMs on the tensor cores (fp32 accumulate), LayerNorm /
     // SE / the narrow head layers in fp32 on the CUDA cores.  SC_MODE_FP32_FFMA = everything FFMA.
     bool fp32_tc = false;
@@ -160,7 +192,7 @@ struct sc_engine {
     int max_moves_total = 0;
     // activations
     float *f_planes = nullptr, *f_x = nullptr, *f_t = nullptr, *f_y = nullptr;
-    __nv_bfloat16 *h_planes = nullptr, *h_x = nullptr, *h_t = nullptr, *h_y = nullptr;
+    __nv_bfloat16 *h_planes = nullptr, *h_x = nullptr, *h_t = nullptr, *h_y = nullptr;  // fp16 bits in fp16 mode
     float *logits = nullptr, *vpre = nullptr;
     int vsplit = 1;
     // gates
@@ -211,6 +243,9 @@ struct sc_engine {
 namespace scb {
 
 constexpr int SC_SMALL_N = 128;
+
+// a 16-bit tensor-core mode (bf16 or fp16 operands): the tower, latency and head kernels of tower_bf16.cu / tower_lat.cu
+static bool tc16(const sc_engine *e) { return e->mode == SC_MODE_BF16 || e->mode == SC_MODE_FP16; }
 
 template <typename T> static int dev_alloc(sc_engine *e, T **p, size_t count)
 {
@@ -306,14 +341,16 @@ static int load_conv(sc_engine *e, const Blob &b, const std::string &wname, cons
         // B operand, K-major: [tap][bn rows][cin_pad]; bn = 256, or 80 for the 73-wide policy conv
         const int bn = cout == C_TOWER ? C_TOWER : LD_POLICY;
         std::vector<uint16_t> h((size_t)taps * bn * c.cin_pad, 0);
+        Op16Weights cv{e->fp16};
         for (int co = 0; co < cout; co++)
             for (int ci = 0; ci < cin; ci++)
                 for (int t = 0; t < taps; t++)
-                    h[((size_t)t * bn + co) * c.cin_pad + ci] = f2bf(w->data[((size_t)co * cin + ci) * taps + t]);
+                    h[((size_t)t * bn + co) * c.cin_pad + ci] = cv(w->data[((size_t)co * cin + ci) * taps + t]);
+        SCB_CHECK(cv.check(wname + ".weight"));
         uint16_t *d = nullptr;
         SCB_CHECK(upload(e, &d, h));
         c.w_bf16 = reinterpret_cast<__nv_bfloat16 *>(d);
-        SCB_CHECK(tc_conv_create(&c.tc, c.w_bf16, taps, c.cin_pad, bn, epi, c.bias, c.gamma, c.beta));
+        SCB_CHECK(tc_conv_create(&c.tc, c.w_bf16, taps, c.cin_pad, bn, epi, c.bias, c.gamma, c.beta, e->fp16));
     }
     return SC_OK;
 }
@@ -351,14 +388,17 @@ static int load_weights(sc_engine *e, const Blob &b)
             // packed so that epilogue thread j (fc1) / channel c (fc2) reads 8 consecutive inputs
             // with one coalesced 16-byte load: w1p[q][j][i] = fc1[j][8q+i], w2p[q][c][i] = fc2[c][8q+i]
             std::vector<uint16_t> w1p((size_t)C_TOWER * C_SE), w2p((size_t)C_SE * C_TOWER);
+            Op16Weights cv1{e->fp16}, cv2{e->fp16};
             for (int q = 0; q < C_TOWER / 8; q++)
                 for (int j = 0; j < C_SE; j++)
                     for (int k = 0; k < 8; k++)
-                        w1p[((size_t)q * C_SE + j) * 8 + k] = f2bf(f1->data[(size_t)j * C_TOWER + 8 * q + k]);
+                        w1p[((size_t)q * C_SE + j) * 8 + k] = cv1(f1->data[(size_t)j * C_TOWER + 8 * q + k]);
             for (int q = 0; q < C_SE / 8; q++)
                 for (int c = 0; c < C_TOWER; c++)
                     for (int k = 0; k < 8; k++)
-                        w2p[((size_t)q * C_TOWER + c) * 8 + k] = f2bf(f2->data[(size_t)c * C_SE + 8 * q + k]);
+                        w2p[((size_t)q * C_TOWER + c) * 8 + k] = cv2(f2->data[(size_t)c * C_SE + 8 * q + k]);
+            SCB_CHECK(cv1.check(p + "se.fc1.weight"));
+            SCB_CHECK(cv2.check(p + "se.fc2.weight"));
             SCB_CHECK(upload(e, &e->se[i].w1p, w1p));
             SCB_CHECK(upload(e, &e->se[i].w2p, w2p));
             // latency kernel: the same numbers sliced per cluster rank r -- fc1 COLUMNS (input channels) [r * NC, +NC)
@@ -371,12 +411,12 @@ static int load_weights(sc_engine *e, const Blob &b)
                         for (int j = 0; j < C_SE; j++)
                             for (int k = 0; k < 8; k++)
                                 a[(((size_t)r * (NC / 8) + q) * C_SE + j) * 8 + k] =
-                                    f2bf(f1->data[(size_t)j * C_TOWER + r * NC + 8 * q + k]);
+                                    cv1(f1->data[(size_t)j * C_TOWER + r * NC + 8 * q + k]);
                     for (int q = 0; q < C_SE / 8; q++)
                         for (int c = 0; c < NC; c++)
                             for (int k = 0; k < 8; k++)
                                 b[(((size_t)r * (C_SE / 8) + q) * NC + c) * 8 + k] =
-                                    f2bf(f2->data[(size_t)(r * NC + c) * C_SE + 8 * q + k]);
+                                    cv2(f2->data[(size_t)(r * NC + c) * C_SE + 8 * q + k]);
                 }
                 SCB_CHECK(upload(e, &e->se[i].w1s[v], a));
                 SCB_CHECK(upload(e, &e->se[i].w2s[v], b));
@@ -410,15 +450,18 @@ static int load_weights(sc_engine *e, const Blob &b)
             SCB_CHECK(upload(e, &e->vfc_w_f32, h));
         } else {
             // B operand of the value FC GEMM, K-major: [128][16384] with k' = s*256 + c
+            // (the meta columns stay fp32: the fused value tail applies them)
             std::vector<uint16_t> h((size_t)N_VALUE_HIDDEN * KV);
+            Op16Weights cv{e->fp16};
             for (int j = 0; j < N_VALUE_HIDDEN; j++)
                 for (int c = 0; c < C_TOWER; c++)
                     for (int s = 0; s < 64; s++)
-                        h[(size_t)j * KV + (size_t)s * C_TOWER + c] = f2bf(fc->data[(size_t)j * KT + c * 64 + s]);
+                        h[(size_t)j * KV + (size_t)s * C_TOWER + c] = cv(fc->data[(size_t)j * KT + c * 64 + s]);
+            SCB_CHECK(cv.check("value_head.ffn.0.weight"));
             uint16_t *d = nullptr;
             SCB_CHECK(upload(e, &d, h));
             SCB_CHECK(tc_conv_create(&e->vfc_tc, reinterpret_cast<__nv_bfloat16 *>(d), 1, KV, N_VALUE_HIDDEN, TC_EPI_RAW,
-                                     nullptr, nullptr, nullptr));
+                                     nullptr, nullptr, nullptr, e->fp16));
         }
     }
     SCB_CHECK(upload_vec(e, b, "value_head.ffn.0.bias", N_VALUE_HIDDEN, &e->v_b1));
@@ -489,7 +532,7 @@ static int kev_mark(sc_engine *e, cudaStream_t st)
 }
 
 // the network on n boards; planes already in f_planes / h_planes, meta in d_meta.
-// `gather` (bf16 mode only): the policy head's epilogue turns the logits into legal-move priors itself; the caller
+// `gather` (16-bit modes only): the policy head's epilogue turns the logits into legal-move priors itself; the caller
 // then skips launch_policy_gather.  Returns through *fused whether that happened.
 static int run_network(sc_engine *e, int n, cudaStream_t st, const TcGather *gather = nullptr)
 {
@@ -649,6 +692,7 @@ static int encode_for_mode(sc_engine *e, const sc_position *d_pos, int n, cudaSt
     NvtxRange nv("scb200: encode planes");
     e->launches += 1;
     if (e->mode == SC_MODE_FP32 && !e->fp32_tc) return launch_encode_f32(d_pos, n, e->f_planes, e->d_meta, st);
+    if (e->fp16) return launch_encode_fp16(d_pos, n, reinterpret_cast<__half *>(e->h_planes), e->d_meta, st);
     return launch_encode_bf16(d_pos, n, e->h_planes, e->d_meta, st);
 }
 
@@ -681,7 +725,7 @@ const char *sc_last_error(void) { return g_err.c_str(); }
 int sc_create(const char *weights_blob_path, int device, int mode, int max_batch, sc_engine **out)
 {
     if (!out || !weights_blob_path || max_batch <= 0 ||
-        (mode != SC_MODE_FP32 && mode != SC_MODE_BF16 && mode != SC_MODE_FP32_FFMA)) {
+        (mode != SC_MODE_FP32 && mode != SC_MODE_BF16 && mode != SC_MODE_FP32_FFMA && mode != SC_MODE_FP16)) {
         set_error("sc_create: bad argument");
         return SC_E_INVAL;
     }
@@ -705,6 +749,7 @@ int sc_create(const char *weights_blob_path, int device, int mode, int max_batch
     e->mode_requested = mode;
     e->mode = mode == SC_MODE_FP32_FFMA ? SC_MODE_FP32 : mode;
     e->fp32_tc = mode == SC_MODE_FP32;
+    e->fp16 = mode == SC_MODE_FP16;
     e->max_batch = max_batch;
     e->num_sms = prop.multiProcessorCount;
     int rc = SC_OK;
@@ -715,7 +760,7 @@ int sc_create(const char *weights_blob_path, int device, int mode, int max_batch
         if (rc) break;
         if ((rc = load_weights(e, blob)) != SC_OK) break;
         if ((rc = alloc_buffers(e)) != SC_OK) break;
-        if (mode == SC_MODE_BF16) {
+        if (tc16(e)) {
             std::vector<TcTowerLayerDesc> d;
             d.push_back(TcTowerLayerDesc{e->stem.tc, e->h_planes, e->h_x, nullptr, 1});
             for (int i = 0; i < e->n_blocks; i++) {
@@ -725,7 +770,7 @@ int sc_create(const char *weights_blob_path, int device, int mode, int max_batch
             // the two 256-wide 1x1 head convolutions read the tower output tile by tile as well
             d.push_back(TcTowerLayerDesc{e->pol1.tc, e->h_x, e->h_t, nullptr, 0});
             d.push_back(TcTowerLayerDesc{e->val1.tc, e->h_x, e->h_y, nullptr, 1});
-            if ((rc = tc_tower_create(&e->tower, d.data(), (int)d.size(), e->alloc_boards)) != SC_OK) break;
+            if ((rc = tc_tower_create(&e->tower, d.data(), (int)d.size(), e->alloc_boards, e->fp16)) != SC_OK) break;
             // the same layers for the latency kernel
             std::vector<LatLayerDesc> ld;
             auto lat_layer = [&](const ConvW &c, const __nv_bfloat16 *in, void *out, const __nv_bfloat16 *resid, int relu,
@@ -761,7 +806,7 @@ int sc_create(const char *weights_blob_path, int device, int mode, int max_batch
             }
             lat_layer(e->pol1, e->h_x, e->h_t, nullptr, 0, 0, nullptr);
             lat_layer(e->val1, e->h_x, e->h_y, nullptr, 1, 0, nullptr);
-            if ((rc = lat_tower_create(&e->lat, ld.data(), (int)ld.size(), e->alloc_boards)) != SC_OK) break;
+            if ((rc = lat_tower_create(&e->lat, ld.data(), (int)ld.size(), e->alloc_boards, e->fp16)) != SC_OK) break;
             e->lat_max_boards = lat_tower_max_boards(e->lat);
         }
         if (cudaDeviceSynchronize() != cudaSuccess) { rc = SC_E_CUDA; set_error("sync after weight upload failed"); break; }
@@ -845,7 +890,7 @@ int sc_eval_device(sc_engine *e, int n, const void *d_pos, const void *d_moves, 
     e->d_value = static_cast<float *>(d_value_out);
     const TcGather g{pos, static_cast<const sc_move *>(d_moves), static_cast<const int32_t *>(d_move_off), nullptr,
                      static_cast<float *>(d_priors_out), n};
-    const bool fused = e->mode == SC_MODE_BF16 && e->fuse_gather;
+    const bool fused = tc16(e) && e->fuse_gather;
     int rc = run_network(e, n, st, fused ? &g : nullptr);
     e->d_value = saved;
     SCB_CHECK(rc);
@@ -956,7 +1001,7 @@ int sc_eval_submit(sc_engine *e, int n, const sc_position *pos, const sc_move *m
         const int saved_timing = e->timing;
         e->timing = 0;  // asynchronous path never synchronises
         const TcGather g{io.pos, io.moves, nullptr, io.cnt, io.priors, n};
-        const bool fused = e->mode == SC_MODE_BF16 && e->fuse_gather;
+        const bool fused = tc16(e) && e->fuse_gather;
         float *saved_value = e->d_value;
         e->d_value = io.value;
         int rc = run_network(e, n, st, fused ? &g : nullptr);
@@ -1181,6 +1226,8 @@ int sc_forward_only(sc_engine *e, int n, const float *planes, const float *meta,
     SCB_CUDA(cudaMemcpy2DAsync(e->d_meta, 8 * 4, meta, SC_N_META * 4, SC_N_META * 4, (size_t)n, cudaMemcpyHostToDevice, st));
     if (e->mode == SC_MODE_FP32 && !e->fp32_tc)
         SCB_CHECK(launch_nchw_to_nhwc_f32(d_nchw, n, e->f_planes, st));
+    else if (e->fp16)
+        SCB_CHECK(launch_nchw_to_nhwc_fp16(d_nchw, n, reinterpret_cast<__half *>(e->h_planes), st));
     else
         SCB_CHECK(launch_nchw_to_nhwc_bf16(d_nchw, n, e->h_planes, st));
     e->launches += 1;
@@ -1198,8 +1245,8 @@ int sc_forward_only(sc_engine *e, int n, const float *planes, const float *meta,
 int sc_debug_tower(sc_engine *e, int n, const sc_position *pos, int n_layers, int which, uint16_t *x_out, uint16_t *t_out,
                    uint16_t *y_out)
 {
-    if (!e || e->mode != SC_MODE_BF16 || n <= 0 || n > e->max_batch || !pos || !e->tower) {
-        set_error("sc_debug_tower: bad argument (bf16 engines only)");
+    if (!e || !tc16(e) || n <= 0 || n > e->max_batch || !pos || !e->tower) {
+        set_error("sc_debug_tower: bad argument (bf16 / fp16 engines only)");
         return SC_E_INVAL;
     }
     cudaStream_t st = e->stream;

@@ -4,6 +4,7 @@
 #pragma once
 #include <cuda.h>
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <stdint.h>
 
 namespace scb {
@@ -193,6 +194,59 @@ __host__ __device__ constexpr uint32_t umma_idesc_bf16(int M, int N)
 {
     return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
+
+// Tensor-core operand types of the 16-bit modes (kind::f16, fp32 accumulate): the kernels are templates on one of these,
+// so each type is its own instantiation and the bf16 code is unchanged by the fp16 one.  Both types are 2 bytes, so TMA
+// boxes, swizzle, descriptors and shared-memory layouts are the same.
+//   IDESC_AB  a_format / b_format bits of the instruction descriptor (bits 7-9 / 10-12: 0 = F16, 1 = BF16)
+//   TMAP      tensor-map element type
+//   pack2     two floats -> two operands, round to nearest even, first argument in the low half
+//   lo, hi    the inverse: the low / high operand of a packed pair as float (exact)
+//   round     a float rounded to the operand type and back: a value the kernels park in that type
+//   unpack8   eight packed operands -> floats (the SE weights)
+__device__ __forceinline__ void bf16x8_to_float(const uint4 &u, float (&f)[8]);
+struct OpBf16 {
+    static constexpr uint32_t IDESC_AB = (1u << 7) | (1u << 10);
+    static constexpr CUtensorMapDataType TMAP = CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+    __device__ __forceinline__ static uint32_t pack2(float lo, float hi)
+    {
+        __nv_bfloat162 h = __floats2bfloat162_rn(lo, hi);
+        return *reinterpret_cast<uint32_t *>(&h);
+    }
+    __device__ __forceinline__ static float lo(uint32_t w) { return __uint_as_float(w << 16); }
+    __device__ __forceinline__ static float hi(uint32_t w) { return __uint_as_float(w & 0xffff0000u); }
+    __device__ __forceinline__ static float round(float x) { return __bfloat162float(__float2bfloat16_rn(x)); }
+    __device__ __forceinline__ static void unpack8(const uint4 &u, float (&f)[8]) { bf16x8_to_float(u, f); }
+};
+// fp16: 11 significant bits against bf16's 8; a value beyond +-65504 becomes +-inf, as in fp16 autocast
+struct OpFp16 {
+    static constexpr uint32_t IDESC_AB = 0u;
+    static constexpr CUtensorMapDataType TMAP = CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
+    __device__ __forceinline__ static uint32_t pack2(float lo, float hi)
+    {
+        __half2 h = __floats2half2_rn(lo, hi);
+        return *reinterpret_cast<uint32_t *>(&h);
+    }
+    __device__ __forceinline__ static float lo(uint32_t w) { return __half2float(__ushort_as_half((unsigned short)(w & 0xffffu))); }
+    __device__ __forceinline__ static float hi(uint32_t w) { return __half2float(__ushort_as_half((unsigned short)(w >> 16))); }
+    __device__ __forceinline__ static float round(float x) { return __half2float(__float2half_rn(x)); }
+    __device__ __forceinline__ static void unpack8(const uint4 &u, float (&f)[8])
+    {
+        const uint32_t w[4] = {u.x, u.y, u.z, u.w};
+#pragma unroll
+        for (int i = 0; i < 4; i++) {
+            const float2 p = __half22float2(*reinterpret_cast<const __half2 *>(&w[i]));
+            f[2 * i] = p.x;
+            f[2 * i + 1] = p.y;
+        }
+    }
+};
+// instruction descriptor of operand type OT (umma_idesc_bf16 for OpBf16)
+template <class OT> __host__ __device__ constexpr uint32_t umma_idesc(int M, int N)
+{
+    return (1u << 4) | OT::IDESC_AB | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
+}
+static_assert(umma_idesc<OpBf16>(256, 256) == umma_idesc_bf16(256, 256), "bf16 instruction descriptor");
 
 __device__ __forceinline__ void tmem_ld32_nowait(uint32_t taddr, uint32_t (&r)[32])
 {

@@ -17,7 +17,9 @@
 //   B (weights, bf16 [tap][cout][cin]) is a plain 2-D box.
 //   D accumulates in TMEM (128 lanes x 256 fp32 columns per tile, two tiles = all 512
 //   columns, so the epilogue of tile i overlaps the MMAs of tile i+1).
-// One kernel template, tc_gemm_kernel<BN, EPI, A4D, CTA2, TOWER>:
+// One kernel template, tc_gemm_kernel<BN, EPI, A4D, CTA2, TOWER, OT>:
+//   * OT: the operand type, OpBf16 or OpFp16 (tc_ptx.cuh).  Activations, weights, the parked SE tile and the stored
+//     layer outputs are all of that type; the accumulator, LayerNorm, SE arithmetic and the head tails are fp32;
 //   * CTA2: every 256-wide convolution; clusters of two CTAs issue tcgen05.mma.cta_group::2 (256-row
 //     tiles, each CTA stages its own rows of A and half of the weight rows);
 //   * TOWER: the stem, all residual blocks and the two 256-wide head 1x1 convolutions run
@@ -40,6 +42,7 @@
 #include <cstring>
 #include <map>
 #include <mutex>
+#include <type_traits>
 #include <vector>
 
 #include "common.cuh"
@@ -179,7 +182,7 @@ template <int BN, bool CTA2 = false, bool YSMEM = false> struct TcCfg {
 
 constexpr int TC_MAX_SLOTS = 32;  // TOWER: tiles per CTA whose layer-to-layer hand-over is tracked
 
-template <int BN, int EPI, bool A4D, bool CTA2 = false, bool TOWER = false>
+template <int BN, int EPI, bool A4D, bool CTA2 = false, bool TOWER = false, class OT = OpBf16>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_w,
                const TcArgs args)
@@ -189,6 +192,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     // produced: the hand-over is a per-tile mbarrier inside the CTA, there is no grid-wide barrier, no
     // per-layer launch gap and no per-layer tail.
     static_assert(!TOWER || (CTA2 && EPI == EPI_LN_SE), "tower kernel = pair mode with both epilogues compiled in");
+    static_assert(EPI != EPI_F32 || std::is_same<OT, OpBf16>::value, "the bf16x3 split of the FP32 parity mode is bf16");
     constexpr bool YSMEM = EPI == EPI_LN_SE;
     using Cfg = TcCfg<BN, CTA2, YSMEM>;
     constexpr int STAGE_BYTES = Cfg::STAGE_BYTES;
@@ -411,7 +415,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
         }
     } else if (warp == 1) {
         if (cta_rank == 0) {
-            constexpr uint32_t idesc = umma_idesc_bf16(CTA2 ? 2 * TC_BM : TC_BM, BN);
+            constexpr uint32_t idesc = umma_idesc<OT>(CTA2 ? 2 * TC_BM : TC_BM, BN);
             int stage = 0, ra = 0, rb = 0;
             uint32_t phase = 0, rap = 0, rbp = 0;
             int it = 0;
@@ -865,16 +869,13 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                             y[j] = ln_apply(__fadd_rn(__uint_as_float(cur[j]), s_bias[c]), mean, rstd, s_gamma[c], s_beta[c]);
                         }
                         if constexpr (YSMEM) {
-                            // keep LN(acc) as bf16 in shared memory: the final pass then needs neither TMEM nor
-                            // the LayerNorm arithmetic again, and the accumulator can be handed back early
+                            // keep LN(acc) in the operand type in shared memory: the final pass then needs neither
+                            // TMEM nor the LayerNorm arithmetic again, and the accumulator can be handed back early
 #pragma unroll
                             for (int q = 0; q < 4; q++) {
                                 uint32_t pw[4];
 #pragma unroll
-                                for (int i = 0; i < 4; i++) {
-                                    __nv_bfloat162 h = __floats2bfloat162_rn(y[8 * q + 2 * i], y[8 * q + 2 * i + 1]);
-                                    pw[i] = *reinterpret_cast<uint32_t *>(&h);
-                                }
+                                for (int i = 0; i < 4; i++) pw[i] = OT::pack2(y[8 * q + 2 * i], y[8 * q + 2 * i + 1]);
                                 const int chunk = (c0 + ch * 32) / 8 + q;
                                 *reinterpret_cast<uint4 *>(s_y + orow * 512 + ((chunk ^ (orow & 7)) << 4)) =
                                     make_uint4(pw[0], pw[1], pw[2], pw[3]);
@@ -924,7 +925,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                             for (int uu = 0; uu < 4; uu++) {
                                 const int u = 4 * k + uu, q = hc * 16 + u;
                                 float wf[8];
-                                bf16x8_to_float(w1v[u], wf);
+                                OT::unpack8(w1v[u], wf);
                                 a0 = se_chain8(wf, *reinterpret_cast<const float4 *>(s_mean + q * 8),
                                                *reinterpret_cast<const float4 *>(s_mean + q * 8 + 4), a0);
                                 a1 = se_chain8(wf, *reinterpret_cast<const float4 *>(s_mean + 256 + q * 8),
@@ -960,7 +961,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                             for (int qq = 0; qq < 4; qq++) {
                                 const int q = 4 * k + qq;
                                 float wf[8];
-                                bf16x8_to_float(w2v[q], wf);
+                                OT::unpack8(w2v[q], wf);
                                 a0 = se_chain8(wf, *reinterpret_cast<const float4 *>(s_hid + q * 8),
                                                *reinterpret_cast<const float4 *>(s_hid + q * 8 + 4), a0);
                                 a1 = se_chain8(wf, *reinterpret_cast<const float4 *>(s_hid + 128 + q * 8),
@@ -1004,7 +1005,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                     }
                     const size_t tile_row0 = (size_t)tile * TC_BM;
                     const uint4 *xg = reinterpret_cast<const uint4 *>(P.resid + tile_row0 * BN) + chunk;
-                    uint4 *og = reinterpret_cast<uint4 *>(static_cast<__nv_bfloat16 *>(P.out) + tile_row0 * BN) + chunk;
+                    uint4 *og = reinterpret_cast<uint4 *>(static_cast<uint16_t *>(P.out) + tile_row0 * BN) + chunk;
 #pragma unroll
                     for (int i0 = 0; i0 < 16; i0 += 8) {
                         uint4 xv[8];
@@ -1020,11 +1021,9 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                             uint32_t ow[4];
 #pragma unroll
                             for (int k = 0; k < 4; k++) {
-                                const float o0 = fmaxf(fmaf(g[2 * k], __uint_as_float(yw[k] << 16), __uint_as_float(xw[k] << 16)), 0.f);
-                                const float o1 = fmaxf(fmaf(g[2 * k + 1], __uint_as_float(yw[k] & 0xffff0000u),
-                                                            __uint_as_float(xw[k] & 0xffff0000u)), 0.f);
-                                __nv_bfloat162 h = __floats2bfloat162_rn(o0, o1);
-                                ow[k] = *reinterpret_cast<uint32_t *>(&h);
+                                const float o0 = fmaxf(fmaf(g[2 * k], OT::lo(yw[k]), OT::lo(xw[k])), 0.f);
+                                const float o1 = fmaxf(fmaf(g[2 * k + 1], OT::hi(yw[k]), OT::hi(xw[k])), 0.f);
+                                ow[k] = OT::pack2(o0, o1);
                             }
                             og[(size_t)rr * (BN / 8)] = make_uint4(ow[0], ow[1], ow[2], ow[3]);
                         }
@@ -1033,8 +1032,8 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                     tile_done(slot);
                     continue;  // the accumulator was released after the pooling pass
                 }
-                // ---- final pass of the LayerNorm-only layers: y (recomputed from TMEM), ReLU, bf16 store ------
-                uint8_t *gtile = reinterpret_cast<uint8_t *>(static_cast<__nv_bfloat16 *>(P.out) + (size_t)tile * TC_BM * BN + c0);
+                // ---- final pass of the LayerNorm-only layers: y (recomputed from TMEM), ReLU, 16-bit store ------
+                uint8_t *gtile = reinterpret_cast<uint8_t *>(static_cast<uint16_t *>(P.out) + (size_t)tile * TC_BM * BN + c0);
                 uint32_t rm[32];
                 tmem_ld32(tcol, r);
 #pragma unroll
@@ -1052,8 +1051,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                             y0 = fmaxf(y0, 0.f);
                             y1 = fmaxf(y1, 0.f);
                         }
-                        __nv_bfloat162 h = __floats2bfloat162_rn(y0, y1);
-                        const uint32_t hv = *reinterpret_cast<uint32_t *>(&h);
+                        const uint32_t hv = OT::pack2(y0, y1);
                         if ((j & 3) == 0) pk[j >> 2].x = hv;
                         else if ((j & 3) == 1) pk[j >> 2].y = hv;
                         else if ((j & 3) == 2) pk[j >> 2].z = hv;
@@ -1122,6 +1120,7 @@ struct ActMap {
 struct TcConv {
     CUtensorMap map_w;
     int taps, k_per_tap, bn, epi;
+    bool fp16 = false;                     // operand type: OpFp16 instead of OpBf16
     int split_pairs = 0, split_kreal = 0;  // FP32 parity mode: (A plane, B plane) pairs of the bf16x3 split
     uint8_t split_ap[8] = {0}, split_bp[8] = {0};
     const float *bias, *gamma, *beta;
@@ -1130,8 +1129,8 @@ struct TcConv {
     std::vector<ActMap> act_maps;
 };
 
-int tc_encode_map(CUtensorMap *m, const void *ptr, int rank, const cuuint64_t *dims, const cuuint64_t *strides,
-                  const cuuint32_t *box, const char *what, bool swizzle128)
+int tc_encode_map(CUtensorMap *m, CUtensorMapDataType dt, const void *ptr, int rank, const cuuint64_t *dims,
+                  const cuuint64_t *strides, const cuuint32_t *box, const char *what, bool swizzle128)
 {
     EncodeTiledFn enc = get_encode();
     if (!enc) {
@@ -1139,7 +1138,7 @@ int tc_encode_map(CUtensorMap *m, const void *ptr, int rank, const cuuint64_t *d
         return SC_E_CUDA;
     }
     cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, (cuuint32_t)rank, const_cast<void *>(ptr), dims, strides, box,
+    CUresult r = enc(m, dt, (cuuint32_t)rank, const_cast<void *>(ptr), dims, strides, box,
                      estr, CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_NONE,
                      CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
@@ -1151,44 +1150,60 @@ int tc_encode_map(CUtensorMap *m, const void *ptr, int rank, const cuuint64_t *d
 }
 
 // activations as a 4-D tensor {C, file, rank, board}, box = 64 channels of two whole boards
-static int make_act_map_4d(const void *ptr, int boards, int c, CUtensorMap *m)
+static int make_act_map_4d(CUtensorMapDataType dt, const void *ptr, int boards, int c, CUtensorMap *m)
 {
     cuuint64_t dims[4] = {(cuuint64_t)c, 8, 8, (cuuint64_t)boards};
     cuuint64_t strides[3] = {(cuuint64_t)c * 2, (cuuint64_t)c * 16, (cuuint64_t)c * 128};
     cuuint32_t box[4] = {TC_BK, 8, 8, 2};
-    return tc_encode_map(m, ptr, 4, dims, strides, box, "activations 4d");
+    return tc_encode_map(m, dt, ptr, 4, dims, strides, box, "activations 4d");
 }
 
 // the same activations as {C, file, board, rank}: a box of 64 channels x 8 files x 2 boards x 10 ranks lands in
 // shared memory with rows ordered (rank, board, file), so the three dy taps are 2 KB apart in ONE box
-int tc_make_act_map_hbw(const void *ptr, int boards, int c, CUtensorMap *m)
+int tc_make_act_map_hbw(CUtensorMapDataType dt, const void *ptr, int boards, int c, CUtensorMap *m)
 {
     cuuint64_t dims[4] = {(cuuint64_t)c, 8, (cuuint64_t)boards, 8};
     cuuint64_t strides[3] = {(cuuint64_t)c * 2, (cuuint64_t)c * 128, (cuuint64_t)c * 16};
     cuuint32_t box[4] = {TC_BK, 8, 2, 10};
-    return tc_encode_map(m, ptr, 4, dims, strides, box, "activations (rank, board, file)");
+    return tc_encode_map(m, dt, ptr, 4, dims, strides, box, "activations (rank, board, file)");
 }
 
 // plain row-major [rows][k] matrix, box = 64 k x 128 rows
-static int make_act_map_2d(const void *ptr, int rows, int k, CUtensorMap *m)
+static int make_act_map_2d(CUtensorMapDataType dt, const void *ptr, int rows, int k, CUtensorMap *m)
 {
     cuuint64_t dims[2] = {(cuuint64_t)k, (cuuint64_t)rows};
     cuuint64_t strides[1] = {(cuuint64_t)k * 2};
     cuuint32_t box[2] = {TC_BK, TC_BM};
-    return tc_encode_map(m, ptr, 2, dims, strides, box, "activations 2d");
+    return tc_encode_map(m, dt, ptr, 2, dims, strides, box, "activations 2d");
 }
 
-template <int BN, int EPI, bool A4D> static int set_smem_attr()
+template <int BN, int EPI, bool A4D, class OT> static int set_smem_attr()
 {
-    SCB_CUDA(cudaFuncSetAttribute(tc_gemm_kernel<BN, EPI, A4D>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    SCB_CUDA(cudaFuncSetAttribute(tc_gemm_kernel<BN, EPI, A4D, false, false, OT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   TcCfg<BN>::SMEM_BYTES));
     return SC_OK;
 }
 
+// the dynamic shared-memory sizes of the non-split kernels of one operand type
+template <class OT> static int set_conv_attrs()
+{
+    SCB_CUDA(cudaFuncSetAttribute(tc_gemm_kernel<256, EPI_LN, true, true, false, OT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  TcCfg<256, true>::SMEM_BYTES));
+    SCB_CUDA(cudaFuncSetAttribute(tc_gemm_kernel<256, EPI_LN_SE, true, true, false, OT>,
+                                  cudaFuncAttributeMaxDynamicSharedMemorySize, TcCfg<256, true, true>::SMEM_BYTES));
+    SCB_CHECK((set_smem_attr<LD_POLICY, EPI_LN73, true, OT>()));
+    SCB_CHECK((set_smem_attr<LD_POLICY, EPI_LN73_GATHER, true, OT>()));
+    SCB_CHECK((set_smem_attr<N_VALUE_HIDDEN, EPI_RAW, false, OT>()));
+    return SC_OK;
+}
+
+static CUtensorMapDataType tmap_type(bool fp16) { return fp16 ? OpFp16::TMAP : OpBf16::TMAP; }
+
 int tc_conv_create(TcConv **out, const __nv_bfloat16 *w, int taps, int k_per_tap, int bn, int epi, const float *bias,
-                   const float *gamma, const float *beta)
+                   const float *gamma, const float *beta, bool fp16)
 {
     TcConv *c = new TcConv();
+    c->fp16 = fp16;
     c->taps = taps;
     c->k_per_tap = k_per_tap;
     c->bn = bn;
@@ -1200,26 +1215,20 @@ int tc_conv_create(TcConv **out, const __nv_bfloat16 *w, int taps, int k_per_tap
     cuuint64_t dims[2] = {(cuuint64_t)k_per_tap, (cuuint64_t)taps * bn};
     cuuint64_t strides[1] = {(cuuint64_t)k_per_tap * 2};
     cuuint32_t box[2] = {TC_BK, (cuuint32_t)(bn == 256 ? bn / 2 : bn)};
-    int rc = tc_encode_map(&c->map_w, w, 2, dims, strides, box, "weights");
+    int rc = tc_encode_map(&c->map_w, tmap_type(fp16), w, 2, dims, strides, box, "weights");
     if (rc != SC_OK) {
         delete c;
         return rc;
     }
     // function attributes belong to the device (context): set them once per device, not once per process
     static std::mutex attr_mu;
-    static std::map<int, bool> attr_done;
+    static std::map<std::pair<int, bool>, bool> attr_done;
     int dev = 0;
     SCB_CUDA(cudaGetDevice(&dev));
     std::lock_guard<std::mutex> lk(attr_mu);
-    bool &attr_set = attr_done[dev];
+    bool &attr_set = attr_done[{dev, fp16}];
     if (!attr_set) {
-        SCB_CUDA(cudaFuncSetAttribute(tc_gemm_kernel<256, EPI_LN, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      TcCfg<256, true>::SMEM_BYTES));
-        SCB_CUDA(cudaFuncSetAttribute(tc_gemm_kernel<256, EPI_LN_SE, true, true>,
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, TcCfg<256, true, true>::SMEM_BYTES));
-        SCB_CHECK((set_smem_attr<LD_POLICY, EPI_LN73, true>()));
-        SCB_CHECK((set_smem_attr<LD_POLICY, EPI_LN73_GATHER, true>()));
-        SCB_CHECK((set_smem_attr<N_VALUE_HIDDEN, EPI_RAW, false>()));
+        SCB_CHECK(fp16 ? set_conv_attrs<OpFp16>() : set_conv_attrs<OpBf16>());
         attr_set = true;
     }
     *out = c;
@@ -1247,7 +1256,7 @@ int tc_split_conv_create(TcConv **out, const __nv_bfloat16 *w3, int taps, int ci
     cuuint64_t dims[2] = {(cuuint64_t)3 * cin_pad, (cuuint64_t)taps * 256};
     cuuint64_t strides[1] = {(cuuint64_t)3 * cin_pad * 2};
     cuuint32_t box2[2] = {TC_BK, 128};
-    int rc = tc_encode_map(&c->map_w, w3, 2, dims, strides, box2, "split weights (pair half)");
+    int rc = tc_encode_map(&c->map_w, OpBf16::TMAP, w3, 2, dims, strides, box2, "split weights (pair half)");
     if (rc != SC_OK) {
         delete c;
         return rc;
@@ -1307,9 +1316,10 @@ static int prof_buffer(int num_sms, cudaStream_t st, long long **out)
 struct TcTower {
     TowerLayer *d_layers = nullptr;
     int n_layers = 0;
+    bool fp16 = false;
 };
 
-int tc_tower_create(TcTower **out, const TcTowerLayerDesc *descs, int n, int boards_alloc)
+int tc_tower_create(TcTower **out, const TcTowerLayerDesc *descs, int n, int boards_alloc, bool fp16)
 {
     std::vector<TowerLayer> h((size_t)n);
     for (int i = 0; i < n; i++) {
@@ -1318,8 +1328,12 @@ int tc_tower_create(TcTower **out, const TcTowerLayerDesc *descs, int n, int boa
             set_error("tc_tower_create: layer is not a 256-wide tower convolution");
             return SC_E_INVAL;
         }
+        if (c->fp16 != fp16) {
+            set_error("tc_tower_create: layer of another operand type");
+            return SC_E_INVAL;
+        }
         memset(&h[i], 0, sizeof(TowerLayer));
-        SCB_CHECK(tc_make_act_map_hbw(descs[i].in, boards_alloc, c->k_per_tap, &h[i].map_a));
+        SCB_CHECK(tc_make_act_map_hbw(tmap_type(fp16), descs[i].in, boards_alloc, c->k_per_tap, &h[i].map_a));
         h[i].map_w = c->map_w;
         h[i].out = descs[i].out;
         h[i].resid = descs[i].resid;
@@ -1343,14 +1357,19 @@ int tc_tower_create(TcTower **out, const TcTowerLayerDesc *descs, int n, int boa
     }
     TcTower *t = new TcTower();
     t->n_layers = n;
+    t->fp16 = fp16;
     if (cudaMalloc(&t->d_layers, sizeof(TowerLayer) * (size_t)n) != cudaSuccess ||
         cudaMemcpy(t->d_layers, h.data(), sizeof(TowerLayer) * (size_t)n, cudaMemcpyHostToDevice) != cudaSuccess) {
         delete t;
         set_error("tc_tower_create: device allocation failed");
         return SC_E_CUDA;
     }
-    SCB_CUDA(cudaFuncSetAttribute(tc_gemm_kernel<256, EPI_LN_SE, true, true, true>,
-                                  cudaFuncAttributeMaxDynamicSharedMemorySize, TcCfg<256, true, true>::SMEM_BYTES));
+    if (fp16)
+        SCB_CUDA(cudaFuncSetAttribute(tc_gemm_kernel<256, EPI_LN_SE, true, true, true, OpFp16>,
+                                      cudaFuncAttributeMaxDynamicSharedMemorySize, TcCfg<256, true, true>::SMEM_BYTES));
+    else
+        SCB_CUDA(cudaFuncSetAttribute(tc_gemm_kernel<256, EPI_LN_SE, true, true, true>,
+                                      cudaFuncAttributeMaxDynamicSharedMemorySize, TcCfg<256, true, true>::SMEM_BYTES));
     *out = t;
     return SC_OK;
 }
@@ -1399,7 +1418,10 @@ int tc_tower_launch(TcTower *t, int n_boards, int num_sms, int group, cudaStream
         SCB_CHECK(prof_buffer(num_sms, st, &d_prof));
         a.prof = d_prof;
     }
-    SCB_CUDA(cudaLaunchKernelEx(&cfg, tc_gemm_kernel<256, EPI_LN_SE, true, true, true>, dummy, dummy, a));
+    if (t->fp16)
+        SCB_CUDA(cudaLaunchKernelEx(&cfg, tc_gemm_kernel<256, EPI_LN_SE, true, true, true, OpFp16>, dummy, dummy, a));
+    else
+        SCB_CUDA(cudaLaunchKernelEx(&cfg, tc_gemm_kernel<256, EPI_LN_SE, true, true, true>, dummy, dummy, a));
     SCB_CUDA(cudaGetLastError());
     if (want_prof) {
         std::vector<long long> h((size_t)num_sms * 16);
@@ -1412,6 +1434,66 @@ int tc_tower_launch(TcTower *t, int n_boards, int num_sms, int group, cudaStream
                 "[tower layers=%d grid=%d] tiles/cta %.2f | producer wait_empty %.0f | mma: total %.0f wait_tmem_empty %.0f "
                 "wait_full %.0f | epilogue: wait_tmem_full %.0f work %.0f (stats %.0f pool %.0f fc %.0f final %.0f)\n",
                 t->n_layers, g2, acc[4], acc[0], acc[3], acc[1], acc[2], acc[5], acc[6], acc[7], acc[8], acc[9], acc[10]);
+    }
+    return SC_OK;
+}
+
+// the launch of one convolution / head GEMM with operand type OT (a: everything but the pair / gather / finish choice)
+template <class OT>
+static int conv_launch_kernel(const TcConv *c, const CUtensorMap &ma, TcArgs &a, int grid, int num_sms, cudaStream_t st,
+                              const __nv_bfloat16 *resid, const TcGather *gather, const TcValueFinish *finish)
+{
+    const bool pair = c->bn == 256;
+    if (pair) {
+        const int n_pairs = (a.n_tiles + 1) / 2;
+        int g2 = 2 * n_pairs;
+        if (g2 > (num_sms & ~1)) g2 = num_sms & ~1;
+        cudaLaunchConfig_t cfg{};
+        cfg.gridDim = dim3(g2);
+        cfg.blockDim = dim3(TC_THREADS);
+        cfg.dynamicSmemBytes = c->epi == EPI_LN_SE ? TcCfg<256, true, true>::SMEM_BYTES : TcCfg<256, true>::SMEM_BYTES;
+        cfg.stream = st;
+        cudaLaunchAttribute attr[1];
+        attr[0].id = cudaLaunchAttributeClusterDimension;
+        attr[0].val.clusterDim.x = 2;
+        attr[0].val.clusterDim.y = 1;
+        attr[0].val.clusterDim.z = 1;
+        cfg.attrs = attr;
+        cfg.numAttrs = 1;
+        if (c->epi == EPI_F32) {
+            if constexpr (std::is_same<OT, OpBf16>::value) {
+                SCB_CUDA(cudaLaunchKernelEx(&cfg, tc_gemm_kernel<256, EPI_F32, true, true>, ma, c->map_w, a));
+            } else {
+                set_error("tc_conv_launch: the split fp32 epilogue has bf16 operands only");
+                return SC_E_INVAL;
+            }
+        } else if (c->epi == EPI_LN)
+            SCB_CUDA(cudaLaunchKernelEx(&cfg, tc_gemm_kernel<256, EPI_LN, true, true, false, OT>, ma, c->map_w, a));
+        else {
+            if (!resid) {
+                set_error("tc_conv_launch: residual epilogue without block input");
+                return SC_E_INVAL;
+            }
+            SCB_CUDA(cudaLaunchKernelEx(&cfg, tc_gemm_kernel<256, EPI_LN_SE, true, true, false, OT>, ma, c->map_w, a));
+        }
+    } else {
+        switch (c->epi) {
+        case EPI_LN73:
+            if (gather) {
+                a.gather = *gather;
+                tc_gemm_kernel<LD_POLICY, EPI_LN73_GATHER, true, false, false, OT><<<grid, TC_THREADS, TcCfg<LD_POLICY>::SMEM_BYTES, st>>>(ma, c->map_w, a);
+            } else
+                tc_gemm_kernel<LD_POLICY, EPI_LN73, true, false, false, OT><<<grid, TC_THREADS, TcCfg<LD_POLICY>::SMEM_BYTES, st>>>(ma, c->map_w, a);
+            break;
+        case EPI_RAW:
+            if (finish) a.vfin = *finish;
+            tc_gemm_kernel<N_VALUE_HIDDEN, EPI_RAW, false, false, false, OT><<<grid, TC_THREADS, TcCfg<N_VALUE_HIDDEN>::SMEM_BYTES, st>>>(
+                ma, c->map_w, a);
+            break;
+        default:
+            set_error("tc_conv_launch: bad epilogue");
+            return SC_E_INVAL;
+        }
     }
     return SC_OK;
 }
@@ -1433,12 +1515,14 @@ int tc_conv_launch(TcConv *c, const __nv_bfloat16 *in, int rows_alloc, int n_uni
         am.ptr = in;
         am.rows = rows_alloc;
         am.c = c->k_per_tap;
+        // (the split kernel of the FP32 parity mode is created with fp16 = false)
+        const CUtensorMapDataType dt = tmap_type(c->fp16);
         if (pair)
-            SCB_CHECK(tc_make_act_map_hbw(in, rows_alloc, c->k_per_tap, &am.map));
+            SCB_CHECK(tc_make_act_map_hbw(dt, in, rows_alloc, c->k_per_tap, &am.map));
         else if (a4d)
-            SCB_CHECK(make_act_map_4d(in, rows_alloc, c->k_per_tap, &am.map));
+            SCB_CHECK(make_act_map_4d(dt, in, rows_alloc, c->k_per_tap, &am.map));
         else
-            SCB_CHECK(make_act_map_2d(in, rows_alloc, c->k_per_tap, &am.map));
+            SCB_CHECK(make_act_map_2d(dt, in, rows_alloc, c->k_per_tap, &am.map));
         c->act_maps.push_back(am);
         ma = &c->act_maps.back().map;
     }
@@ -1481,52 +1565,10 @@ int tc_conv_launch(TcConv *c, const __nv_bfloat16 *in, int rows_alloc, int n_uni
     }
     const int n_work = a4d ? a.n_tiles : a.n_tiles * a.n_splits;
     const int grid = n_work < num_sms ? n_work : num_sms;
-    if (pair) {
-        const int n_pairs = (a.n_tiles + 1) / 2;
-        int g2 = 2 * n_pairs;
-        if (g2 > (num_sms & ~1)) g2 = num_sms & ~1;
-        cudaLaunchConfig_t cfg{};
-        cfg.gridDim = dim3(g2);
-        cfg.blockDim = dim3(TC_THREADS);
-        cfg.dynamicSmemBytes = c->epi == EPI_LN_SE ? TcCfg<256, true, true>::SMEM_BYTES : TcCfg<256, true>::SMEM_BYTES;
-        cfg.stream = st;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeClusterDimension;
-        attr[0].val.clusterDim.x = 2;
-        attr[0].val.clusterDim.y = 1;
-        attr[0].val.clusterDim.z = 1;
-        cfg.attrs = attr;
-        cfg.numAttrs = 1;
-        if (c->epi == EPI_F32)
-            SCB_CUDA(cudaLaunchKernelEx(&cfg, tc_gemm_kernel<256, EPI_F32, true, true>, *ma, c->map_w, a));
-        else if (c->epi == EPI_LN)
-            SCB_CUDA(cudaLaunchKernelEx(&cfg, tc_gemm_kernel<256, EPI_LN, true, true>, *ma, c->map_w, a));
-        else {
-            if (!resid) {
-                set_error("tc_conv_launch: residual epilogue without block input");
-                return SC_E_INVAL;
-            }
-            SCB_CUDA(cudaLaunchKernelEx(&cfg, tc_gemm_kernel<256, EPI_LN_SE, true, true>, *ma, c->map_w, a));
-        }
-    } else {
-        switch (c->epi) {
-        case EPI_LN73:
-            if (gather) {
-                a.gather = *gather;
-                tc_gemm_kernel<LD_POLICY, EPI_LN73_GATHER, true><<<grid, TC_THREADS, TcCfg<LD_POLICY>::SMEM_BYTES, st>>>(*ma, c->map_w, a);
-            } else
-                tc_gemm_kernel<LD_POLICY, EPI_LN73, true><<<grid, TC_THREADS, TcCfg<LD_POLICY>::SMEM_BYTES, st>>>(*ma, c->map_w, a);
-            break;
-        case EPI_RAW:
-            if (finish) a.vfin = *finish;
-            tc_gemm_kernel<N_VALUE_HIDDEN, EPI_RAW, false><<<grid, TC_THREADS, TcCfg<N_VALUE_HIDDEN>::SMEM_BYTES, st>>>(
-                *ma, c->map_w, a);
-            break;
-        default:
-            set_error("tc_conv_launch: bad epilogue");
-            return SC_E_INVAL;
-        }
-    }
+    if (c->fp16)
+        SCB_CHECK(conv_launch_kernel<OpFp16>(c, *ma, a, grid, num_sms, st, resid, gather, finish));
+    else
+        SCB_CHECK(conv_launch_kernel<OpBf16>(c, *ma, a, grid, num_sms, st, resid, gather, finish));
     SCB_CUDA(cudaGetLastError());
     if (want_prof) {
         // debugging aid: per-phase SM-cycle counters of this launch, averaged over CTAs (synchronous!)

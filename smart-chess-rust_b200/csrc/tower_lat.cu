@@ -169,7 +169,8 @@ __device__ __forceinline__ float2 warp_transpose_reduce_16(float (&v)[32], int l
 __device__ __forceinline__ void lat_epi_sync() { asm volatile("bar.sync 1, 128;" ::: "memory"); }
 
 
-template <int CL, int NB>
+// OT: the operand type (OpBf16 / OpFp16, tc_ptx.cuh), the same as the throughput kernel's for the same engine
+template <int CL, int NB, class OT = OpBf16>
 __global__ void __launch_bounds__(LAT_THREADS, 1) lat_tower_kernel(const LatArgs args)
 {
     using Cfg = LatCfg<CL, NB>;
@@ -297,7 +298,7 @@ __global__ void __launch_bounds__(LAT_THREADS, 1) lat_tower_kernel(const LatArgs
         }
     } else if (warp == 2) {
         // ---- MMA issuer: k order (channel chunk, dx, dy, 16-element step) as in tower_bf16.cu ----
-        constexpr uint32_t idesc = umma_idesc_bf16(64 * NB, NC);
+        constexpr uint32_t idesc = umma_idesc<OT>(64 * NB, NC);
         int rs = 0;
         uint32_t rph = 0;
         long long pm_a = 0, pm_a0 = 0, pm_total = args.prof ? clock64() : 0;
@@ -442,7 +443,7 @@ __global__ void __launch_bounds__(LAT_THREADS, 1) lat_tower_kernel(const LatArgs
             // order, so the tile is exactly the store box)
             uint4 *odst = reinterpret_cast<uint4 *>(smem + Cfg::OFF_OUT + row * NC * 2);
             if (!L.se) {
-                // ---- bias + LayerNorm (+ReLU) -> bf16 ----
+                // ---- bias + LayerNorm (+ReLU) -> operand type ----
                 if (active) {
 #pragma unroll
                     for (int i = 0; i < NC / 8; i++) {
@@ -454,8 +455,7 @@ __global__ void __launch_bounds__(LAT_THREADS, 1) lat_tower_kernel(const LatArgs
                                 y0 = fmaxf(y0, 0.f);
                                 y1 = fmaxf(y1, 0.f);
                             }
-                            __nv_bfloat162 h = __floats2bfloat162_rn(y0, y1);
-                            pw[k] = *reinterpret_cast<uint32_t *>(&h);
+                            pw[k] = OT::pack2(y0, y1);
                         }
                         odst[i] = make_uint4(pw[0], pw[1], pw[2], pw[3]);
                     }
@@ -492,7 +492,7 @@ __global__ void __launch_bounds__(LAT_THREADS, 1) lat_tower_kernel(const LatArgs
 #pragma unroll
                             for (int uu = 0; uu < 4; uu++) {
                                 float wf[8];
-                                bf16x8_to_float(s_w1s[(ch * 4 + uu) * 128 + j], wf);
+                                OT::unpack8(s_w1s[(ch * 4 + uu) * 128 + j], wf);
                                 const float *m = s_mean + ch * 32 + uu * 8;
                                 p0 = se_chain8(wf, *reinterpret_cast<const float4 *>(m), *reinterpret_cast<const float4 *>(m + 4), p0);
                                 if (NB == 2)
@@ -530,7 +530,7 @@ __global__ void __launch_bounds__(LAT_THREADS, 1) lat_tower_kernel(const LatArgs
                         for (int qq = 0; qq < 4; qq++) {
                             const int q = 4 * k + qq;
                             float wf[8];
-                            bf16x8_to_float(s_w2s[q * NC + c], wf);
+                            OT::unpack8(s_w2s[q * NC + c], wf);
                             acc = se_chain8(wf, *reinterpret_cast<const float4 *>(s_hid + b * 128 + q * 8),
                                             *reinterpret_cast<const float4 *>(s_hid + b * 128 + q * 8 + 4), acc);
                         }
@@ -547,7 +547,8 @@ __global__ void __launch_bounds__(LAT_THREADS, 1) lat_tower_kernel(const LatArgs
                     n_se++;
                 }
                 if (prof) pe_se += clock64() - tq0;
-                // ---- out = relu(gate * bf16(y) + x), in place over the block input ----
+                // ---- out = relu(gate * OT(y) + x), in place over the block input (y parked in the operand type, as the
+                //      throughput kernel parks it in shared memory) ----
                 if (active) {
                     const float *gate = s_gate + board * NC;
 #pragma unroll
@@ -557,13 +558,12 @@ __global__ void __launch_bounds__(LAT_THREADS, 1) lat_tower_kernel(const LatArgs
 #pragma unroll
                         for (int k = 0; k < 4; k++) {
                             const int c = 8 * i + 2 * k;
-                            const float yb0 = __bfloat162float(__float2bfloat16_rn(a[c]));
-                            const float yb1 = __bfloat162float(__float2bfloat16_rn(a[c + 1]));
+                            const float yb0 = OT::round(a[c]);
+                            const float yb1 = OT::round(a[c + 1]);
                             const float g0 = L.se == 1 ? gate[c] : 1.f, g1 = L.se == 1 ? gate[c + 1] : 1.f;
-                            const float o0 = fmaxf(fmaf(g0, yb0, __uint_as_float(xw[k] << 16)), 0.f);
-                            const float o1 = fmaxf(fmaf(g1, yb1, __uint_as_float(xw[k] & 0xffff0000u)), 0.f);
-                            __nv_bfloat162 h = __floats2bfloat162_rn(o0, o1);
-                            pw[k] = *reinterpret_cast<uint32_t *>(&h);
+                            const float o0 = fmaxf(fmaf(g0, yb0, OT::lo(xw[k])), 0.f);
+                            const float o1 = fmaxf(fmaf(g1, yb1, OT::hi(xw[k])), 0.f);
+                            pw[k] = OT::pack2(o0, o1);
                         }
                         odst[i] = make_uint4(pw[0], pw[1], pw[2], pw[3]);
                     }
@@ -629,14 +629,15 @@ template <int CL> constexpr int lat_smem_bytes()
 struct LatTower {
     LatLayer *d_layers[2] = {nullptr, nullptr};  // [0]: CL = 8, [1]: CL = 4
     int n_layers = 0;
+    bool fp16 = false;                           // operand type OpFp16 instead of OpBf16
     int max_tiles[2] = {0, 0};                   // co-resident clusters of 8 / 4 CTAs
     bool one_board = true;                       // one-board tiles (M64) while there are clusters for them
 };
 
-template <int CL> static int lat_max_clusters(int *out)
+template <int CL, class OT> static int lat_max_clusters(int *out)
 {
-    SCB_CUDA(cudaFuncSetAttribute(lat_tower_kernel<CL, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, lat_smem_bytes<CL>()));
-    SCB_CUDA(cudaFuncSetAttribute(lat_tower_kernel<CL, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, lat_smem_bytes<CL>()));
+    SCB_CUDA(cudaFuncSetAttribute(lat_tower_kernel<CL, 2, OT>, cudaFuncAttributeMaxDynamicSharedMemorySize, lat_smem_bytes<CL>()));
+    SCB_CUDA(cudaFuncSetAttribute(lat_tower_kernel<CL, 1, OT>, cudaFuncAttributeMaxDynamicSharedMemorySize, lat_smem_bytes<CL>()));
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = dim3(CL * 64);
     cfg.blockDim = dim3(LAT_THREADS);
@@ -649,15 +650,17 @@ template <int CL> static int lat_max_clusters(int *out)
     cfg.attrs = attr;
     cfg.numAttrs = 1;
     int n = 0;
-    SCB_CUDA(cudaOccupancyMaxActiveClusters(&n, lat_tower_kernel<CL, 2>, &cfg));
+    SCB_CUDA(cudaOccupancyMaxActiveClusters(&n, lat_tower_kernel<CL, 2, OT>, &cfg));
     *out = n;
     return SC_OK;
 }
 
-int lat_tower_create(LatTower **out, const LatLayerDesc *descs, int n, int boards_alloc)
+int lat_tower_create(LatTower **out, const LatLayerDesc *descs, int n, int boards_alloc, bool fp16)
 {
     LatTower *t = new LatTower();
     t->n_layers = n;
+    t->fp16 = fp16;
+    const CUtensorMapDataType dt = fp16 ? OpFp16::TMAP : OpBf16::TMAP;
     for (int v = 0; v < 2; v++) {
         const int CL = v == 0 ? 8 : 4, NC = 256 / CL;
         std::vector<LatLayer> h((size_t)n);
@@ -665,21 +668,21 @@ int lat_tower_create(LatTower **out, const LatLayerDesc *descs, int n, int board
             const LatLayerDesc &d = descs[i];
             LatLayer &L = h[i];
             memset(&L, 0, sizeof(L));
-            int rc = tc_make_act_map_hbw(d.in, boards_alloc, d.cin_pad, &L.map_a);
+            int rc = tc_make_act_map_hbw(dt, d.in, boards_alloc, d.cin_pad, &L.map_a);
             if (rc == SC_OK) {
                 // the same tensor {C, file, board, rank} with a box of ONE board: 80 rows ordered (rank, file)
                 cuuint64_t dims[4] = {(cuuint64_t)d.cin_pad, 8, (cuuint64_t)boards_alloc, 8};
                 cuuint64_t strides[3] = {(cuuint64_t)d.cin_pad * 2, (cuuint64_t)d.cin_pad * 128, (cuuint64_t)d.cin_pad * 16};
                 cuuint32_t box[4] = {TC_BK, 8, 1, 10};
-                rc = tc_encode_map(&L.map_a1, d.in, 4, dims, strides, box, "activations (rank, file), one board");
+                rc = tc_encode_map(&L.map_a1, dt, d.in, 4, dims, strides, box, "activations (rank, file), one board");
             }
             if (rc == SC_OK) {
                 // output {C, file, board, rank}: box of this CTA's NC channels of the tile's boards, unswizzled
                 cuuint64_t dims[4] = {256, 8, (cuuint64_t)boards_alloc, 8};
                 cuuint64_t strides[3] = {256 * 2, 256 * 128, 256 * 16};
                 cuuint32_t box2[4] = {(cuuint32_t)NC, 8, 2, 8}, box1[4] = {(cuuint32_t)NC, 8, 1, 8};
-                rc = tc_encode_map(&L.map_o, d.out, 4, dims, strides, box2, "output slice, two boards", false);
-                if (rc == SC_OK) rc = tc_encode_map(&L.map_o1, d.out, 4, dims, strides, box1, "output slice, one board", false);
+                rc = tc_encode_map(&L.map_o, dt, d.out, 4, dims, strides, box2, "output slice, two boards", false);
+                if (rc == SC_OK) rc = tc_encode_map(&L.map_o1, dt, d.out, 4, dims, strides, box1, "output slice, one board", false);
             }
             if (rc == SC_OK) {
                 // weights [tap = dy * 3 + dx][256][cin_pad] as {cin, cout, dx, dy}
@@ -688,7 +691,7 @@ int lat_tower_create(LatTower **out, const LatLayerDesc *descs, int n, int board
                 cuuint64_t strides[3] = {(cuuint64_t)d.cin_pad * 2, (cuuint64_t)d.cin_pad * 2 * 256,
                                          (cuuint64_t)d.cin_pad * 2 * 256 * 3};
                 cuuint32_t box[4] = {TC_BK, (cuuint32_t)NC, 1, (cuuint32_t)nd};
-                rc = tc_encode_map(&L.map_w, d.w, 4, dims, strides, box, "weights (cluster slice)");
+                rc = tc_encode_map(&L.map_w, dt, d.w, 4, dims, strides, box, "weights (cluster slice)");
             }
             if (rc != SC_OK) {
                 lat_tower_destroy(t);
@@ -720,8 +723,8 @@ int lat_tower_create(LatTower **out, const LatLayerDesc *descs, int n, int board
             return SC_E_CUDA;
         }
     }
-    int rc = lat_max_clusters<8>(&t->max_tiles[0]);
-    if (rc == SC_OK) rc = lat_max_clusters<4>(&t->max_tiles[1]);
+    int rc = fp16 ? lat_max_clusters<8, OpFp16>(&t->max_tiles[0]) : lat_max_clusters<8, OpBf16>(&t->max_tiles[0]);
+    if (rc == SC_OK) rc = fp16 ? lat_max_clusters<4, OpFp16>(&t->max_tiles[1]) : lat_max_clusters<4, OpBf16>(&t->max_tiles[1]);
     if (rc != SC_OK) {
         lat_tower_destroy(t);
         return rc;
@@ -746,7 +749,7 @@ void lat_tower_destroy(LatTower *t)
 
 int lat_tower_max_boards(const LatTower *t) { return t ? 2 * (t->max_tiles[0] > t->max_tiles[1] ? t->max_tiles[0] : t->max_tiles[1]) : 0; }
 
-template <int CL, int NB> static int lat_launch(const LatTower *t, int v, int n_tiles, cudaStream_t st, int max_layers)
+template <int CL, int NB, class OT> static int lat_launch(const LatTower *t, int v, int n_tiles, cudaStream_t st, int max_layers)
 {
     LatArgs a;
     a.layers = t->d_layers[v];
@@ -770,7 +773,7 @@ template <int CL, int NB> static int lat_launch(const LatTower *t, int v, int n_
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    SCB_CUDA(cudaLaunchKernelEx(&cfg, lat_tower_kernel<CL, NB>, a));
+    SCB_CUDA(cudaLaunchKernelEx(&cfg, lat_tower_kernel<CL, NB, OT>, a));
     SCB_CUDA(cudaGetLastError());
     if (want_prof) {
         // debugging aid (synchronous): SM cycles per phase, summed over the layers, averaged over the CTAs
@@ -791,18 +794,23 @@ template <int CL, int NB> static int lat_launch(const LatTower *t, int v, int n_
     return SC_OK;
 }
 
+template <class OT> static int lat_dispatch(const LatTower *t, int n_boards, cudaStream_t st, int max_layers)
+{
+    const int n_tiles = (n_boards + 1) / 2;
+    if (t->one_board && n_boards <= t->max_tiles[0]) return lat_launch<8, 1, OT>(t, 0, n_boards, st, max_layers);
+    if (t->one_board && n_boards <= t->max_tiles[1]) return lat_launch<4, 1, OT>(t, 1, n_boards, st, max_layers);
+    if (n_tiles <= t->max_tiles[0]) return lat_launch<8, 2, OT>(t, 0, n_tiles, st, max_layers);
+    if (n_tiles <= t->max_tiles[1]) return lat_launch<4, 2, OT>(t, 1, n_tiles, st, max_layers);
+    return SC_E_STATE;
+}
+
 // SC_E_STATE (no message): the batch does not fit one wave of clusters; the caller runs the throughput kernel
 int lat_tower_launch(LatTower *t, int n_boards, cudaStream_t st, int max_layers)
 {
     if (n_boards <= 0) return SC_OK;
     // one-board tiles (half the operand traffic per CTA) while every board can have a cluster -- 8 CTAs per board, then 4
     // (measured, n = 16: 0.418 ms against 0.433 ms for two boards per 8-CTA cluster) -- then two-board tiles
-    const int n_tiles = (n_boards + 1) / 2;
-    if (t->one_board && n_boards <= t->max_tiles[0]) return lat_launch<8, 1>(t, 0, n_boards, st, max_layers);
-    if (t->one_board && n_boards <= t->max_tiles[1]) return lat_launch<4, 1>(t, 1, n_boards, st, max_layers);
-    if (n_tiles <= t->max_tiles[0]) return lat_launch<8, 2>(t, 0, n_tiles, st, max_layers);
-    if (n_tiles <= t->max_tiles[1]) return lat_launch<4, 2>(t, 1, n_tiles, st, max_layers);
-    return SC_E_STATE;
+    return t->fp16 ? lat_dispatch<OpFp16>(t, n_boards, st, max_layers) : lat_dispatch<OpBf16>(t, n_boards, st, max_layers);
 }
 
 }  // namespace scb

@@ -17,6 +17,7 @@ from .binding import (  # noqa: F401
     SC_MODE_BF16,
     SC_MODE_FP32,
     SC_MODE_FP32_FFMA,
+    SC_MODE_FP16,
     POSITION_DTYPE,
     MOVE_DTYPE,
     lib_path,

@@ -14,7 +14,7 @@ import os
 
 
 def main(argv=None):
-    from . import Engine, SelfPlay, SC_MODE_BF16, SC_MODE_FP32
+    from . import Engine, SelfPlay, SC_MODE_BF16, SC_MODE_FP16, SC_MODE_FP32
     from .shard import game_ids_for_rank, rank_seed
 
     ap = argparse.ArgumentParser(description=__doc__.splitlines()[0])
@@ -28,7 +28,10 @@ def main(argv=None):
     ap.add_argument("--cpuct", type=float, default=1.0)
     ap.add_argument("--temperature-switch", type=int, default=30)
     ap.add_argument("--epsilon", type=float, default=0.15)
-    ap.add_argument("--fp32", action="store_true", help="parity mode (FP32 FFMA) instead of bf16 tensor cores")
+    prec = ap.add_mutually_exclusive_group()
+    prec.add_argument("--fp32", action="store_true", help="parity mode (FP32 FFMA) instead of bf16 tensor cores")
+    prec.add_argument("--fp16", action="store_true",
+                      help="fp16 tensor-core operands instead of bf16 (the precision of a 16-mixed trained net)")
     ap.add_argument("--leaves-per-tree", type=int, default=1,
                     help="1 = the reference's sequential search; K > 1 = K leaves per tree per batch (virtual loss); "
                          "-1 = 1 until games run out, then the remaining games share the batch")
@@ -43,7 +46,7 @@ def main(argv=None):
         return 0
     trees = max(1, min(a.trees, len(mine)))
     kl = max(1, a.leaves_per_tree)
-    eng = Engine(a.checkpoint, local, SC_MODE_FP32 if a.fp32 else SC_MODE_BF16, trees * kl)
+    eng = Engine(a.checkpoint, local, SC_MODE_FP32 if a.fp32 else SC_MODE_FP16 if a.fp16 else SC_MODE_BF16, trees * kl)
     sp = SelfPlay(eng, n_trees=trees, rollout_num=a.rollout_num, num_steps=a.num_steps, cpuct=a.cpuct, epsilon=a.epsilon,
                   with_noise=True, temperature_switch=a.temperature_switch, temperature=a.temperature,
                   seed=rank_seed(a.seed, rank), n_threads=a.threads or max(1, (os.cpu_count() or 8) // world),
