@@ -95,6 +95,19 @@ int sc_eval(sc_engine *e, int n, const sc_position *pos, const sc_move *moves, c
 int sc_eval_device(sc_engine *e, int n, const void *d_pos, const void *d_moves, const void *d_move_off,
                    int n_moves_total, void *d_priors_out, void *d_value_out, void *stream);
 
+/* Game::predict for n leaves in one call (src/game.rs:3-15, src/backends/torch.rs:89-146): legal moves generated on the
+ * device in python-chess order (the generator of the native rules), then the network.
+ * ep_square[i] = python-chess `ep_square` (the skipped square after any double push) or -1; NULL = -1 for all.  Any
+ * other value, or n > max_batch, fails with SC_E_INVAL.
+ * moves_out / priors_out strided by SC_MAX_MOVES (as sc_eval_submit): leaf i owns [i*SC_MAX_MOVES, +move_cnt_out[i]);
+ * the call copies back the whole stride, and the entries past move_cnt_out[i] are unspecified.  A leaf with
+ * move_cnt_out[i] == 0 is terminal and value_out[i] is torch.rs:98-106's rule in White's perspective (the checkmated
+ * side loses, stalemate 0).  A leaf with more than SC_MAX_MOVES pseudo-legal moves (not a legal position; a legal one
+ * has at most 218 legal moves) fails the call with SC_E_INVAL; the outputs are still written, at most SC_MAX_MOVES
+ * moves per leaf.  Host pointers, synchronous, all modes; staging and kernels as sc_eval. */
+int sc_predict(sc_engine *e, int n, const sc_position *pos, const int8_t *ep_square, sc_move *moves_out,
+               int32_t *move_cnt_out, float *priors_out, float *value_out, void *stream);
+
 /* asynchronous form of sc_eval for double-buffered callers: submit returns as soon as the work is
  * queued on `stream` (host buffers must be pinned and stay untouched until the wait returns);
  * moves and priors are STRIDED: leaf i owns moves[i*SC_MAX_MOVES .. +move_cnt[i]) and the same
@@ -150,6 +163,8 @@ int sc_set_timing(sc_engine *e, int enabled);
  * leaf those launches cover together */
 int sc_kernel_timing(sc_engine *e, float *conv3x3_avg_ms, int *n_launches);
 double sc_timed_flops_per_leaf(const sc_engine *e);
+/* level >= 1: device time (ms) of the legal-move kernel of the most recent sc_predict call (CUDA events on its stream) */
+int sc_predict_timing(sc_engine *e, float *movegen_ms);
 
 /* ===================== batched self-play driver (host side, C++) ================================
  * Replaces the single-tree loop of the `selfplay` binary (src/main.rs:153-238) and `mcts::mcts` /

@@ -64,6 +64,17 @@ int launch_dist_scatter(const sc_position *d_pos, const sc_move *d_moves, const 
                         const int32_t *d_off, int n, float *d_dist /*[n][4672]*/, cudaStream_t st);
 int launch_policy_logp_full(const float *logits, int n, float *d_logp /*[n][4672]*/, cudaStream_t st);
 
+// ---- movegen.cu ---------------------------------------------------------------------------
+// the attack tables of host/chess_rules.hpp to the device (once per engine, before the first launch)
+int upload_move_tables(cudaStream_t st);
+// one thread per leaf: the legal moves of pos[i] (en-passant square d_ep[i], or -1 for all when d_ep == nullptr) in
+// python-chess order into d_moves[i * SC_MAX_MOVES ..], their number into d_cnt[i], and into d_term[i] 0, a
+// termination code of chess_rules.hpp (T_CHECKMATE / T_STALEMATE) when there is none, or PREDICT_OVERFLOW when the
+// position has more than SC_MAX_MOVES pseudo-legal moves (then at most SC_MAX_MOVES are written)
+constexpr int PREDICT_OVERFLOW = -1;
+int launch_legal_moves(const sc_position *d_pos, const int8_t *d_ep, int n, sc_move *d_moves, int32_t *d_cnt,
+                       int32_t *d_term, cudaStream_t st);
+
 // ---- tower_f32.cu -------------------------------------------------------------------------
 // C[M][N] = gather_taps(A)[M][TAPS*K] * W[TAPS*K][ldw] + bias ; A is [rows][lda] fp32
 // n_splits > 1 (taps == 1, no bias): split-K over gridDim.z, partial sums to out[split][M][ldo]

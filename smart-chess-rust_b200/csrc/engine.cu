@@ -238,6 +238,15 @@ struct sc_engine {
     int kev_used = 0;
     float last_conv_avg_ms = 0.f;
     int last_conv_n = 0;
+    // sc_predict, set up by its first call: the legal-move kernel runs on gen_stream next to the encoder and the tower;
+    // d_pred_out = [moves n x SC_MAX_MOVES | move counts n | termination codes n] for a call of n leaves, copied back
+    // to h_pred_out in one piece
+    cudaStream_t gen_stream = nullptr;
+    cudaEvent_t ev_gen_fork = nullptr, ev_gen_done = nullptr;
+    cudaEvent_t ev_gen_t[2] = {nullptr, nullptr};  // timing: around the legal-move kernel
+    int8_t *d_pred_ep = nullptr;
+    uint8_t *d_pred_out = nullptr, *h_pred_out = nullptr;
+    float last_movegen_ms = 0.f;
 };
 
 namespace scb {
@@ -534,7 +543,9 @@ static int kev_mark(sc_engine *e, cudaStream_t st)
 // the network on n boards; planes already in f_planes / h_planes, meta in d_meta.
 // `gather` (16-bit modes only): the policy head's epilogue turns the logits into legal-move priors itself; the caller
 // then skips launch_policy_gather.  Returns through *fused whether that happened.
-static int run_network(sc_engine *e, int n, cudaStream_t st, const TcGather *gather = nullptr)
+// `gather_ready` (with `gather`): the policy head waits for this event first (sc_predict's legal moves)
+static int run_network(sc_engine *e, int n, cudaStream_t st, const TcGather *gather = nullptr,
+                       cudaEvent_t gather_ready = nullptr)
 {
     NvtxRange nv_net("scb200: network (tower + heads)");
     const int rows = n * 64;
@@ -672,11 +683,13 @@ static int run_network(sc_engine *e, int n, cudaStream_t st, const TcGather *gat
             SCB_CUDA(cudaStreamWaitEvent(e->head_stream, e->ev_fork, 0));
             SCB_CHECK(tc_conv_launch(e->vfc_tc, e->h_y, nb, n, e->vpre, nullptr, 0, e->vsplit, e->num_sms, e->head_stream, nullptr, &vf));
             SCB_CUDA(cudaEventRecord(e->ev_join, e->head_stream));
+            if (gather_ready) SCB_CUDA(cudaStreamWaitEvent(st, gather_ready, 0));
             SCB_CHECK(tc_conv_launch(e->pol2.tc, e->h_t, nb, n, e->logits, nullptr, 0, 1, e->num_sms, st, gather));
             SCB_CUDA(cudaStreamWaitEvent(st, e->ev_join, 0));
             e->launches += 2;
             return SC_OK;
         }
+        if (gather_ready) SCB_CUDA(cudaStreamWaitEvent(st, gather_ready, 0));
         SCB_CHECK(tc_conv_launch(e->pol2.tc, e->h_t, nb, n, e->logits, nullptr, 0, 1, e->num_sms, st, gather));
         SCB_CHECK(tc_conv_launch(e->vfc_tc, e->h_y, nb, n, e->vpre, nullptr, 0, e->vsplit, e->num_sms, st));
         e->launches += 2;
@@ -694,6 +707,22 @@ static int encode_for_mode(sc_engine *e, const sc_position *d_pos, int n, cudaSt
     if (e->mode == SC_MODE_FP32 && !e->fp32_tc) return launch_encode_f32(d_pos, n, e->f_planes, e->d_meta, st);
     if (e->fp16) return launch_encode_fp16(d_pos, n, reinterpret_cast<__half *>(e->h_planes), e->d_meta, st);
     return launch_encode_bf16(d_pos, n, e->h_planes, e->d_meta, st);
+}
+
+// sc_predict's buffers, stream and events (first call)
+static int predict_setup(sc_engine *e)
+{
+    if (e->gen_stream) return SC_OK;
+    const size_t out_b = (size_t)e->max_batch * (SC_MAX_MOVES * sizeof(sc_move) + 2 * sizeof(int32_t));
+    SCB_CHECK(dev_alloc(e, &e->d_pred_ep, (size_t)e->max_batch));
+    SCB_CHECK(dev_alloc(e, &e->d_pred_out, out_b));
+    if (!e->h_pred_out) SCB_CUDA(cudaMallocHost(&e->h_pred_out, out_b));
+    if (!e->ev_gen_fork) SCB_CUDA(cudaEventCreateWithFlags(&e->ev_gen_fork, cudaEventDisableTiming));
+    if (!e->ev_gen_done) SCB_CUDA(cudaEventCreateWithFlags(&e->ev_gen_done, cudaEventDisableTiming));
+    for (cudaEvent_t &ev : e->ev_gen_t)
+        if (!ev) SCB_CUDA(cudaEventCreate(&ev));
+    SCB_CUDA(cudaStreamCreateWithFlags(&e->gen_stream, cudaStreamNonBlocking));
+    return SC_OK;
 }
 
 static int finish_timing(sc_engine *e, cudaStream_t st)
@@ -760,6 +789,7 @@ int sc_create(const char *weights_blob_path, int device, int mode, int max_batch
         if (rc) break;
         if ((rc = load_weights(e, blob)) != SC_OK) break;
         if ((rc = alloc_buffers(e)) != SC_OK) break;
+        if ((rc = upload_move_tables(e->stream)) != SC_OK) break;
         if (tc16(e)) {
             std::vector<TcTowerLayerDesc> d;
             d.push_back(TcTowerLayerDesc{e->stem.tc, e->h_planes, e->h_x, nullptr, 1});
@@ -844,6 +874,10 @@ int sc_destroy(sc_engine *e)
         if (s.compute_done) cudaEventDestroy(s.compute_done);
         if (s.out_done) cudaEventDestroy(s.out_done);
     }
+    if (e->h_pred_out) cudaFreeHost(e->h_pred_out);
+    for (cudaEvent_t ev : {e->ev_gen_fork, e->ev_gen_done, e->ev_gen_t[0], e->ev_gen_t[1]})
+        if (ev) cudaEventDestroy(ev);
+    if (e->gen_stream) cudaStreamDestroy(e->gen_stream);
     if (e->head_stream) cudaStreamDestroy(e->head_stream);
     if (e->ev_fork) cudaEventDestroy(e->ev_fork);
     if (e->ev_join) cudaEventDestroy(e->ev_join);
@@ -948,6 +982,113 @@ int sc_eval(sc_engine *e, int n, const sc_position *pos, const sc_move *moves, c
     if (total) SCB_CUDA(cudaMemcpyAsync(priors_out, e->d_priors, sizeof(float) * (size_t)total, cudaMemcpyDeviceToHost, st));
     SCB_CUDA(cudaMemcpyAsync(value_out, e->d_value, sizeof(float) * (size_t)n, cudaMemcpyDeviceToHost, st));
     SCB_CUDA(cudaStreamSynchronize(st));
+    return SC_OK;
+}
+
+int sc_predict(sc_engine *e, int n, const sc_position *pos, const int8_t *ep_square, sc_move *moves_out,
+               int32_t *move_cnt_out, float *priors_out, float *value_out, void *stream)
+{
+    if (!e || n < 0 || n > e->max_batch ||
+        (n > 0 && (!pos || !moves_out || !move_cnt_out || !priors_out || !value_out))) {
+        set_error("sc_predict: bad argument");
+        return SC_E_INVAL;
+    }
+    for (int i = 0; ep_square && i < n; i++) {
+        const int s = ep_square[i];
+        if (s != -1 && !(s >= 16 && s < 24) && !(s >= 40 && s < 48)) {
+            set_error("sc_predict: ep_square[" + std::to_string(i) + "] = " + std::to_string(s) +
+                      " is neither -1 nor a square of rank 3 or 6");
+            return SC_E_INVAL;
+        }
+    }
+    if (n == 0) return SC_OK;
+    NvtxRange nv_call("sc_predict");
+    cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
+    SCB_CUDA(cudaSetDevice(e->device));
+    SCB_CHECK(predict_setup(e));
+    const size_t pos_b = sizeof(sc_position) * (size_t)n, mv_b = sizeof(sc_move) * (size_t)n * SC_MAX_MOVES;
+    const size_t cnt_b = sizeof(int32_t) * (size_t)n;
+    const sc_position *d_pos;
+    const int8_t *d_ep = nullptr;
+    float *d_priors, *d_value;
+    const bool small = n <= SC_SMALL_N;
+    if (small) {
+        // sc_eval's staging: [positions | ep squares] in one pinned buffer, read in place by the kernels for up to 16
+        // leaves, else one copy; values and strided priors written straight into the pinned output buffer
+        memcpy(e->h_small_in, pos, pos_b);
+        if (ep_square) memcpy(e->h_small_in + pos_b, ep_square, (size_t)n);
+        const uint8_t *in_dev = e->d_small_in;
+        if (n <= 16)
+            in_dev = e->h_small_in;
+        else
+            SCB_CUDA(cudaMemcpyAsync(e->d_small_in, e->h_small_in, pos_b + (ep_square ? n : 0), cudaMemcpyHostToDevice, st));
+        d_pos = reinterpret_cast<const sc_position *>(in_dev);
+        if (ep_square) d_ep = reinterpret_cast<const int8_t *>(in_dev + pos_b);
+        d_value = e->h_small_out;
+        d_priors = e->h_small_out + n;
+    } else {
+        SCB_CUDA(cudaMemcpyAsync(e->d_pos, pos, pos_b, cudaMemcpyHostToDevice, st));
+        if (ep_square) {
+            SCB_CUDA(cudaMemcpyAsync(e->d_pred_ep, ep_square, (size_t)n, cudaMemcpyHostToDevice, st));
+            d_ep = e->d_pred_ep;
+        }
+        d_pos = e->d_pos;
+        d_value = e->d_value;
+        d_priors = e->d_priors;
+    }
+    if (e->timing) SCB_CUDA(cudaEventRecord(e->ev[0], st));
+    // the legal moves on their own stream next to the encoder and the tower (they do not depend on the network); the
+    // policy head's gather waits for them
+    sc_move *d_moves = reinterpret_cast<sc_move *>(e->d_pred_out);
+    int32_t *d_cnt = reinterpret_cast<int32_t *>(e->d_pred_out + mv_b), *d_term = d_cnt + n;
+    SCB_CUDA(cudaEventRecord(e->ev_gen_fork, st));
+    SCB_CUDA(cudaStreamWaitEvent(e->gen_stream, e->ev_gen_fork, 0));
+    if (e->timing) SCB_CUDA(cudaEventRecord(e->ev_gen_t[0], e->gen_stream));
+    SCB_CHECK(launch_legal_moves(d_pos, d_ep, n, d_moves, d_cnt, d_term, e->gen_stream));
+    if (e->timing) SCB_CUDA(cudaEventRecord(e->ev_gen_t[1], e->gen_stream));
+    SCB_CUDA(cudaEventRecord(e->ev_gen_done, e->gen_stream));
+    e->launches += 1;
+    SCB_CHECK(encode_for_mode(e, d_pos, n, st));
+    const TcGather g{d_pos, d_moves, nullptr, d_cnt, d_priors, n};
+    const bool fused = tc16(e) && e->fuse_gather;
+    float *saved_value = e->d_value;
+    e->d_value = d_value;
+    int rc = run_network(e, n, st, fused ? &g : nullptr, fused ? e->ev_gen_done : nullptr);
+    e->d_value = saved_value;
+    SCB_CHECK(rc);
+    if (!fused) {
+        SCB_CUDA(cudaStreamWaitEvent(st, e->ev_gen_done, 0));
+        SCB_CHECK(launch_policy_gather(e->logits, d_pos, d_moves, nullptr, d_cnt, n, d_priors, st));
+        e->launches += 1;
+    }
+    // results: moves, counts and termination codes in one copy, the full SC_MAX_MOVES stride of every leaf
+    SCB_CUDA(cudaMemcpyAsync(e->h_pred_out, e->d_pred_out, mv_b + 2 * cnt_b, cudaMemcpyDeviceToHost, st));
+    if (!small) {
+        SCB_CUDA(cudaMemcpyAsync(priors_out, d_priors, sizeof(float) * (size_t)n * SC_MAX_MOVES, cudaMemcpyDeviceToHost, st));
+        SCB_CUDA(cudaMemcpyAsync(value_out, d_value, sizeof(float) * (size_t)n, cudaMemcpyDeviceToHost, st));
+    }
+    SCB_CHECK(finish_timing(e, st));
+    SCB_CUDA(cudaStreamSynchronize(st));
+    if (e->timing) SCB_CUDA(cudaEventElapsedTime(&e->last_movegen_ms, e->ev_gen_t[0], e->ev_gen_t[1]));
+    memcpy(moves_out, e->h_pred_out, mv_b);
+    memcpy(move_cnt_out, e->h_pred_out + mv_b, cnt_b);
+    if (small) {
+        memcpy(value_out, e->h_small_out, sizeof(float) * (size_t)n);
+        memcpy(priors_out, e->h_small_out + n, sizeof(float) * (size_t)n * SC_MAX_MOVES);
+    }
+    // a leaf without legal moves is terminal: torch.rs:98-106's value in White's perspective replaces the network's
+    const int32_t *term = reinterpret_cast<const int32_t *>(e->h_pred_out + mv_b + cnt_b);
+    int bad = -1;
+    for (int i = 0; i < n; i++) {
+        if (term[i] == PREDICT_OVERFLOW && bad < 0) bad = i;
+        if (term[i] == chess::T_CHECKMATE) value_out[i] = pos[i].meta[0] ? -1.f : 1.f;
+        if (term[i] == chess::T_STALEMATE) value_out[i] = 0.f;
+    }
+    if (bad >= 0) {
+        set_error("sc_predict: leaf " + std::to_string(bad) + " has more than " + std::to_string(SC_MAX_MOVES) +
+                  " pseudo-legal moves (not a legal position)");
+        return SC_E_INVAL;
+    }
     return SC_OK;
 }
 
@@ -1291,6 +1432,13 @@ int sc_kernel_timing(sc_engine *e, float *conv3x3_avg_ms, int *n_launches)
     if (!e) return SC_E_INVAL;
     if (conv3x3_avg_ms) *conv3x3_avg_ms = e->last_conv_avg_ms;
     if (n_launches) *n_launches = e->last_conv_n;
+    return SC_OK;
+}
+
+int sc_predict_timing(sc_engine *e, float *movegen_ms)
+{
+    if (!e) return SC_E_INVAL;
+    if (movegen_ms) *movegen_ms = e->last_movegen_ms;
     return SC_OK;
 }
 

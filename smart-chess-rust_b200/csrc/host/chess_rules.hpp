@@ -9,11 +9,24 @@
 //
 // Board representation: piece bitboards + colour occupancy, a1 = bit 0 ... h8 = bit 63;
 // sliding attacks by directional rays and bit scans (classical ray attacks).
+//
+// The legal-move generator (attack tables, Position::gen_*, is_safe, gen_legal) also compiles for the device under
+// nvcc: movegen.cu runs it one thread per leaf for sc_predict.  Generation order is defined here only, for both targets.
+// The generator writes through a sink (anything with add(from, to, promo)): the host collects into a MoveList, a device
+// thread writes straight into its leaf's output slot.
 #pragma once
 #include <cstdint>
 #include <cstdio>
 #include <cstring>
 #include <vector>
+
+#include "../../../include/sc_b200.h"
+
+#ifdef __CUDACC__
+#define SCB_HD __host__ __device__ inline
+#else
+#define SCB_HD inline
+#endif
 
 namespace scb {
 namespace chess {
@@ -32,7 +45,7 @@ struct Move {
 struct MoveList {
     Move m[256];
     int n = 0;
-    void add(int f, int t, int p = 0)
+    SCB_HD void add(int f, int t, int p = 0)
     {
         m[n].from = (uint8_t)f;
         m[n].to = (uint8_t)t;
@@ -41,22 +54,29 @@ struct MoveList {
     }
 };
 
-inline u64 bit(int s) { return 1ULL << s; }
+SCB_HD u64 bit(int s) { return 1ULL << s; }
+#ifdef __CUDA_ARCH__
+SCB_HD int lsb(u64 b) { return __ffsll((long long)b) - 1; }
+SCB_HD int msb(u64 b) { return 63 - __clzll((long long)b); }
+SCB_HD int popcnt(u64 b) { return __popcll(b); }
+#else
 inline int lsb(u64 b) { return __builtin_ctzll(b); }
 inline int msb(u64 b) { return 63 - __builtin_clzll(b); }
 inline int popcnt(u64 b) { return __builtin_popcountll(b); }
-inline int rank_of(int s) { return s >> 3; }
-inline int file_of(int s) { return s & 7; }
-const u64 RANK1 = 0xFFULL, RANK8 = 0xFFULL << 56, FILE_A = 0x0101010101010101ULL;
-inline u64 rank_mask(int r) { return RANK1 << (8 * r); }
+#endif
+SCB_HD int rank_of(int s) { return s >> 3; }
+SCB_HD int file_of(int s) { return s & 7; }
+constexpr u64 RANK1 = 0xFFULL, RANK8 = 0xFFULL << 56, FILE_A = 0x0101010101010101ULL;
+SCB_HD u64 rank_mask(int r) { return RANK1 << (8 * r); }
 
-// direction order: N, S, E, W, NE, NW, SE, SW
+// direction order: N, S, E, W, NE, NW, SE, SW.  Plain data (70 KB): built once on the host, and copied as it is to the
+// device (movegen.cu), where it is too large for constant memory.
 struct Tables {
     u64 ray[8][64];
     u64 knight[64], king[64], pawn_att[2][64];
     u64 line[64][64];     // full line through a and b (edge to edge), 0 if not aligned
     u64 between[64][64];  // squares strictly between
-    Tables()
+    void build()
     {
         static const int dr[8] = {1, -1, 0, 0, 1, 1, -1, -1};
         static const int df[8] = {0, 0, 1, -1, 1, -1, 1, -1};
@@ -107,13 +127,31 @@ struct Tables {
     }
 };
 
-inline const Tables &T()
+#ifdef __CUDACC__
+// the device copy of the tables; defined by movegen.cu, the translation unit that generates moves on the device
+__device__ const Tables &device_tables();
+#endif
+
+inline const Tables &host_tables()
 {
-    static const Tables t;
+    static const Tables t = [] {
+        Tables x;
+        x.build();
+        return x;
+    }();
     return t;
 }
 
-inline u64 ray_attack(int d, int s, u64 occ)
+SCB_HD const Tables &T()
+{
+#ifdef __CUDA_ARCH__
+    return device_tables();
+#else
+    return host_tables();
+#endif
+}
+
+SCB_HD u64 ray_attack(int d, int s, u64 occ)
 {
     const Tables &t = T();
     u64 r = t.ray[d][s];
@@ -125,9 +163,9 @@ inline u64 ray_attack(int d, int s, u64 occ)
     }
     return r;
 }
-inline u64 rook_attacks(int s, u64 occ) { return ray_attack(0, s, occ) | ray_attack(1, s, occ) | ray_attack(2, s, occ) | ray_attack(3, s, occ); }
-inline u64 bishop_attacks(int s, u64 occ) { return ray_attack(4, s, occ) | ray_attack(5, s, occ) | ray_attack(6, s, occ) | ray_attack(7, s, occ); }
-inline u64 rank_attacks(int s, u64 occ) { return ray_attack(2, s, occ) | ray_attack(3, s, occ); }
+SCB_HD u64 rook_attacks(int s, u64 occ) { return ray_attack(0, s, occ) | ray_attack(1, s, occ) | ray_attack(2, s, occ) | ray_attack(3, s, occ); }
+SCB_HD u64 bishop_attacks(int s, u64 occ) { return ray_attack(4, s, occ) | ray_attack(5, s, occ) | ray_attack(6, s, occ) | ray_attack(7, s, occ); }
+SCB_HD u64 rank_attacks(int s, u64 occ) { return ray_attack(2, s, occ) | ray_attack(3, s, occ); }
 
 struct Position {
     u64 pt[7];  // [1..6] piece-type bitboards, both colours
@@ -138,6 +176,28 @@ struct Position {
     int ep;  // en-passant square or -1
     int halfmove, fullmove;
 
+    // the current board of a packed leaf: pieces and colour from slot[0] (white-oriented, unrotated), the side to move
+    // from meta[0], castling rights from meta[2..5] (side to move K / Q, opponent K / Q) on the standard rook squares,
+    // the en-passant square from `ep_square` (python-chess `ep_square`: -1, or the square a double push skipped)
+    SCB_HD void set_packed(const sc_position &p, int ep_square)
+    {
+        all = 0;
+        pt[NONE] = 0;
+        for (int i = 0; i < 6; i++) {
+            pt[PAWN + i] = p.slot[0][i];
+            all |= p.slot[0][i];
+        }
+        occ[WHITE] = p.slot[0][6] & all;
+        occ[BLACK] = all & ~occ[WHITE];
+        turn = p.meta[0] ? WHITE : BLACK;
+        const int us = turn, them = !us;
+        const u64 k_rook[2] = {bit(63), bit(7)}, q_rook[2] = {bit(56), bit(0)};
+        castling = (p.meta[2] ? k_rook[us] : 0) | (p.meta[3] ? q_rook[us] : 0) | (p.meta[4] ? k_rook[them] : 0) |
+                   (p.meta[5] ? q_rook[them] : 0);
+        ep = ep_square;
+        halfmove = p.meta[6];
+        fullmove = p.meta[1];
+    }
     void set_start()
     {
         memset(this, 0, sizeof(*this));
@@ -240,12 +300,12 @@ struct Position {
         occ[color] |= m;
         all |= m;
     }
-    int king_sq(int color) const
+    SCB_HD int king_sq(int color) const
     {
         u64 k = pt[KING] & occ[color];
         return k ? msb(k) : -1;
     }
-    u64 attackers(int color, int s, u64 occupied) const
+    SCB_HD u64 attackers(int color, int s, u64 occupied) const
     {
         const Tables &t = T();
         u64 rq = pt[ROOK] | pt[QUEEN], bq = pt[BISHOP] | pt[QUEEN];
@@ -253,13 +313,13 @@ struct Position {
                 (bishop_attacks(s, occupied) & bq) | (t.pawn_att[!color][s] & pt[PAWN]);
         return a & occ[color];
     }
-    bool in_check() const
+    SCB_HD bool in_check() const
     {
         int k = king_sq(turn);
         return k >= 0 && attackers(!turn, k, all) != 0;
     }
     // python-chess clean_castling_rights (standard chess)
-    u64 clean_castling() const
+    SCB_HD u64 clean_castling() const
     {
         u64 c = castling & pt[ROOK];
         u64 w = c & occ[WHITE] & (bit(0) | bit(7));
@@ -285,13 +345,13 @@ struct Position {
         u64 touched = bit(m.from) ^ bit(m.to);
         return (touched & pt[PAWN]) || (touched & occ[!turn]);
     }
-    bool is_en_passant(const Move &m) const
+    SCB_HD bool is_en_passant(const Move &m) const
     {
         int d = (int)m.to - (int)m.from;
         if (d < 0) d = -d;
         return ep == m.to && (pt[PAWN] & bit(m.from)) && (d == 7 || d == 9) && !(all & bit(m.to));
     }
-    bool is_castling(const Move &m) const
+    SCB_HD bool is_castling(const Move &m) const
     {
         if (!(pt[KING] & bit(m.from))) return false;
         int d = file_of(m.from) - file_of(m.to);
@@ -339,7 +399,7 @@ struct Position {
     }
 
     // ---- legal move generation in python-chess order ---------------------------------------
-    u64 attacks_from(int s) const
+    SCB_HD u64 attacks_from(int s) const
     {
         const Tables &t = T();
         u64 m = bit(s);
@@ -351,7 +411,7 @@ struct Position {
         if ((pt[ROOK] | pt[QUEEN]) & m) a |= rook_attacks(s, all);
         return a;
     }
-    static void add_pawn(MoveList &l, int from, int to)
+    template <class Sink> SCB_HD static void add_pawn(Sink &l, int from, int to)
     {
         int r = rank_of(to);
         if (r == 0 || r == 7) {
@@ -360,19 +420,19 @@ struct Position {
             l.add(from, to, BISHOP);
             l.add(from, to, KNIGHT);
         } else
-            l.add(from, to);
+            l.add(from, to, 0);
     }
-    void gen_ep(u64 from_mask, u64 to_mask, MoveList &l) const
+    template <class Sink> SCB_HD void gen_ep(u64 from_mask, u64 to_mask, Sink &l) const
     {
         if (ep < 0 || !(bit(ep) & to_mask) || (bit(ep) & all)) return;
         u64 c = pt[PAWN] & occ[turn] & from_mask & T().pawn_att[!turn][ep] & rank_mask(turn == WHITE ? 4 : 3);
         while (c) {
             int s = msb(c);
             c ^= bit(s);
-            l.add(s, ep);
+            l.add(s, ep, 0);
         }
     }
-    bool any_attacked(u64 squares, u64 occupied) const
+    SCB_HD bool any_attacked(u64 squares, u64 occupied) const
     {
         while (squares) {
             int s = msb(squares);
@@ -381,7 +441,7 @@ struct Position {
         }
         return false;
     }
-    void gen_castling(u64 from_mask, u64 to_mask, MoveList &l) const
+    template <class Sink> SCB_HD void gen_castling(u64 from_mask, u64 to_mask, Sink &l) const
     {
         const Tables &t = T();
         u64 back = turn == WHITE ? RANK1 : RANK8;
@@ -401,10 +461,10 @@ struct Position {
             if ((all ^ king ^ rook) & (kpath | rpath | bit(kto) | bit(rto))) continue;
             if (any_attacked(kpath | king, all ^ king)) continue;
             if (any_attacked(bit(kto), all ^ king ^ rook ^ bit(rto))) continue;
-            l.add(ks, kto);
+            l.add(ks, kto, 0);
         }
     }
-    void gen_pseudo(u64 from_mask, u64 to_mask, MoveList &l) const
+    template <class Sink> SCB_HD void gen_pseudo(u64 from_mask, u64 to_mask, Sink &l) const
     {
         const Tables &t = T();
         u64 ours = occ[turn];
@@ -416,7 +476,7 @@ struct Position {
             while (mv) {
                 int d = msb(mv);
                 mv ^= bit(d);
-                l.add(s, d);
+                l.add(s, d, 0);
             }
         }
         if (from_mask & pt[KING]) gen_castling(from_mask, to_mask, l);
@@ -452,11 +512,11 @@ struct Position {
         while (dbl) {
             int d = msb(dbl);
             dbl ^= bit(d);
-            l.add(d + 2 * back1, d);
+            l.add(d + 2 * back1, d, 0);
         }
         if (ep >= 0) gen_ep(from_mask, to_mask, l);
     }
-    u64 slider_blockers(int king) const
+    SCB_HD u64 slider_blockers(int king) const
     {
         const Tables &t = T();
         u64 rq = pt[ROOK] | pt[QUEEN], bq = pt[BISHOP] | pt[QUEEN];
@@ -470,7 +530,7 @@ struct Position {
         }
         return blockers & occ[turn];
     }
-    u64 pin_mask(int color, int s) const
+    SCB_HD u64 pin_mask(int color, int s) const
     {
         const Tables &t = T();
         int king = king_sq(color);
@@ -491,7 +551,7 @@ struct Position {
             }
         return ~0ULL;
     }
-    bool ep_skewered(int king, int capturer) const
+    SCB_HD bool ep_skewered(int king, int capturer) const
     {
         int last_double = ep + (turn == WHITE ? -8 : 8);
         u64 o = (all & ~bit(last_double) & ~bit(capturer)) | bit(ep);
@@ -499,7 +559,7 @@ struct Position {
         if (bishop_attacks(king, o) & occ[!turn] & (pt[BISHOP] | pt[QUEEN])) return true;
         return false;
     }
-    bool is_safe(int king, u64 blockers, const Move &m) const
+    SCB_HD bool is_safe(int king, u64 blockers, const Move &m) const
     {
         if (m.from == king) {
             if (is_castling(m)) return true;
@@ -508,7 +568,7 @@ struct Position {
         if (is_en_passant(m)) return (pin_mask(turn, m.from) & bit(m.to)) && !ep_skewered(king, m.from);
         return !(blockers & bit(m.from)) || (T().line[m.from][m.to] & bit(king));
     }
-    void gen_evasions(int king, u64 checkers, MoveList &l) const
+    template <class Sink> SCB_HD void gen_evasions(int king, u64 checkers, Sink &l) const
     {
         const Tables &t = T();
         u64 sliders = checkers & (pt[BISHOP] | pt[ROOK] | pt[QUEEN]);
@@ -522,7 +582,7 @@ struct Position {
         while (mv) {
             int d = msb(mv);
             mv ^= bit(d);
-            l.add(king, d);
+            l.add(king, d, 0);
         }
         int checker = msb(checkers);
         if (bit(checker) == checkers) {
@@ -534,23 +594,42 @@ struct Position {
             }
         }
     }
+    // passes the pseudo-legal candidates that is_safe accepts on to `out`, in generation order (without a king to keep
+    // safe, king < 0, every candidate)
+    template <class Sink> struct SafeFilter {
+        const Position &p;
+        int king;
+        u64 blockers;
+        Sink &out;
+        int seen;  // pseudo-legal candidates generated
+        SCB_HD void add(int f, int t, int pr)
+        {
+            seen++;
+            const Move m{(uint8_t)f, (uint8_t)t, (uint8_t)pr};
+            if (king < 0 || p.is_safe(king, blockers, m)) out.add(f, t, pr);
+        }
+    };
+    // the legal moves in python-chess order into `out`; returns the number of pseudo-legal candidates they were
+    // filtered from (never fewer than the legal moves)
+    template <class Sink> SCB_HD int gen_legal(Sink &out) const
+    {
+        const int king = king_sq(turn);
+        SafeFilter<Sink> f{*this, king, 0, out, 0};
+        u64 checkers = 0;
+        if (king >= 0) {
+            f.blockers = slider_blockers(king);
+            checkers = attackers(!turn, king, all);
+        }
+        if (checkers)
+            gen_evasions(king, checkers, f);
+        else
+            gen_pseudo(~0ULL, ~0ULL, f);
+        return f.seen;
+    }
     void legal_moves(MoveList &out) const
     {
         out.n = 0;
-        MoveList tmp;
-        int king = king_sq(turn);
-        if (king < 0) {
-            gen_pseudo(~0ULL, ~0ULL, out);
-            return;
-        }
-        u64 blockers = slider_blockers(king);
-        u64 checkers = attackers(!turn, king, all);
-        if (checkers)
-            gen_evasions(king, checkers, tmp);
-        else
-            gen_pseudo(~0ULL, ~0ULL, tmp);
-        for (int i = 0; i < tmp.n; i++)
-            if (is_safe(king, blockers, tmp.m[i])) out.m[out.n++] = tmp.m[i];
+        gen_legal(out);
     }
     bool has_legal_ep() const
     {

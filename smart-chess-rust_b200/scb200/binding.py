@@ -13,6 +13,7 @@ SC_MODE_FP16 = 3
 SC_N_PLANES = 112
 SC_N_META = 7
 SC_N_POLICY = 4672
+SC_MAX_MOVES = 256
 
 # struct sc_position { uint64_t slot[8][8]; int32_t meta[7]; int32_t n_hist; }  (544 bytes)
 POSITION_DTYPE = np.dtype([("slot", np.uint64, (8, 8)), ("meta", np.int32, (7,)), ("n_hist", np.int32)])
@@ -26,7 +27,8 @@ DECLARED_SYMBOLS = [
     "sc_eval_submit", "sc_eval_wait", "sc_selfplay_create", "sc_selfplay_run", "sc_selfplay_trace_json",
     "sc_selfplay_destroy", "sc_rules_probe", "sc_arena_create", "sc_encode_steps", "sc_timed_flops_per_leaf",
     "sc_random_positions", "sc_test_dirichlet", "sc_game_selfplay", "sc_rules_perft", "sc_device_info",
-    "sc_selfplay_run_many", "sc_debug_tower", "sc_rules_probe_fen", "sc_selfplay_trace_game",
+    "sc_selfplay_run_many", "sc_debug_tower", "sc_rules_probe_fen", "sc_selfplay_trace_game", "sc_predict",
+    "sc_predict_timing",
 ]
 
 
@@ -78,6 +80,8 @@ def load_library():
                                            C.POINTER(SelfPlayStats)]
         L.sc_debug_tower.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
         L.sc_eval.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 6
+        L.sc_predict.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 7
+        L.sc_predict_timing.argtypes = [C.c_void_p, C.POINTER(C.c_float)]
         L.sc_eval_device.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,
                                      C.c_void_p, C.c_void_p]
         L.sc_encode_only.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
@@ -193,6 +197,41 @@ class Engine:
         _check(load_library().sc_eval(self._h, n, _ptr(positions), _ptr(moves), _ptr(move_off), _ptr(priors_out),
                                       _ptr(value_out), stream or None), "sc_eval")
         return priors_out[:total], value_out[:n]
+
+    def predict(self, positions: np.ndarray, ep_square=None, out=None, stream: int = 0, check: bool = True):
+        """`Game::predict` for n leaves (sc_predict): legal moves generated on the device, then the network.
+        ep_square: python-chess `ep_square` per leaf (-1 for none), or None for -1 everywhere.  Returns
+        (moves MOVE_DTYPE[n, 256], counts int32[n], priors float32[n, 256], values float32[n]); leaf i's moves and priors
+        are the first counts[i] entries of row i, and a leaf with counts[i] == 0 is terminal (value -1 / +1 for the
+        mated side to move White / Black, 0 for stalemate).  `out`: these four arrays to fill instead of new ones (at
+        least n rows each).  check=False returns the outputs with the status code (rc, moves, counts, priors, values)
+        instead of raising."""
+        n = len(positions)
+        positions = np.ascontiguousarray(positions, dtype=POSITION_DTYPE)
+        if ep_square is not None:
+            ep = np.asarray(ep_square)
+            if len(ep) != n or ep.min(initial=-1) < -128 or ep.max(initial=-1) > 127:
+                raise SCError("predict: ep_square must hold one square (or -1) per leaf")
+            ep_square = np.ascontiguousarray(ep, dtype=np.int8)
+        if out is None:
+            out = (np.zeros((n, SC_MAX_MOVES), dtype=MOVE_DTYPE), np.zeros(n, dtype=np.int32),
+                   np.zeros((n, SC_MAX_MOVES), dtype=np.float32), np.zeros(n, dtype=np.float32))
+        for a, dt, shape in zip(out, (MOVE_DTYPE, np.int32, np.float32, np.float32), ((SC_MAX_MOVES,), (), (SC_MAX_MOVES,), ())):
+            if a.dtype != dt or a.shape[1:] != shape or len(a) < n or not a.flags.c_contiguous:
+                raise SCError("predict: `out` must be (moves, counts, priors, values) arrays as predict() returns them")
+        moves, counts, priors, values = (a[:n] for a in out)
+        rc = load_library().sc_predict(self._h, n, _ptr(positions), _ptr(ep_square), _ptr(moves), _ptr(counts),
+                                       _ptr(priors), _ptr(values), stream or None)
+        if not check:
+            return rc, moves, counts, priors, values
+        _check(rc, "sc_predict")
+        return moves, counts, priors, values
+
+    def predict_timing(self) -> float:
+        """device time (ms) of the legal-move kernel of the last predict() (timing level >= 1)"""
+        ms = C.c_float()
+        _check(load_library().sc_predict_timing(self._h, C.byref(ms)), "sc_predict_timing")
+        return ms.value
 
     def eval_device(self, n, d_pos, d_moves, d_off, n_moves_total, d_priors, d_value, stream: int = 0):
         _check(load_library().sc_eval_device(self._h, n, _ptr(d_pos), _ptr(d_moves), _ptr(d_off), n_moves_total,
