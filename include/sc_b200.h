@@ -108,6 +108,28 @@ int sc_eval_device(sc_engine *e, int n, const void *d_pos, const void *d_moves, 
 int sc_predict(sc_engine *e, int n, const sc_position *pos, const int8_t *ep_square, sc_move *moves_out,
                int32_t *move_cnt_out, float *priors_out, float *value_out, void *stream);
 
+/* sc_predict for n leaves given as move stacks instead of packed positions: the device replays each game with the
+ * native rules and packs the leaf as the batched driver does (src/chess.rs:356-412,553-591,845-877).
+ * Leaf i is the initial position (`chess.Board()`, src/main.rs:155) followed by stack[stack_off[i] .. stack_off[i+1]):
+ * python-chess `board.move_stack`, oldest move first, castling as the king's two-square move.
+ * n_hist[i] = the history slots `_encode` sees: the node and up to 7 ancestors, stopping at the tree root
+ * (src/chess.rs:851-867); 1..8 and at most the stack length + 1 (chess.rs:863).  NULL = min(8, length + 1), the game
+ * root (the batched driver's pack_leaf).  Slots are newest first, each with its is_repetition(2)/(3) flags, then meta
+ * (encode_meta) and python-chess `ep_square`; then the call is sc_predict on those leaves: same moves, priors, values
+ * and terminal rule, all modes, synchronous, host pointers.  pos_out (may be NULL) receives the n packed leaves, for
+ * sc_eval / sc_encode_only.
+ * SC_E_INVAL before any launch: sc_predict's n / NULL checks, stack_off[0] != 0 or decreasing offsets, a stack longer
+ * than SC_MAX_STACK, a move with from/to >= 64 or promo not in {0, 2, 3, 4, 5}, an n_hist out of range.
+ * SC_E_INVAL after the outputs are written (as sc_predict's overflow; the message names the leaf and the ply): a move
+ * whose from-square holds no piece of the side to move, whose to-square holds a piece of the side to move or a king,
+ * that promotes anything but a pawn reaching the last rank, or a pawn reaching the last rank without a promotion; that
+ * leaf is packed from the moves before it.  Legality (pins, moving into check) is not verified, as python-chess
+ * Board.push does not verify it: such a leaf is packed from whatever the replay gives. */
+#define SC_MAX_STACK 1024 /* plies in one leaf's move stack (sc_predict_stack) */
+int sc_predict_stack(sc_engine *e, int n, const sc_move *stack, const int32_t *stack_off, const int8_t *n_hist,
+                     sc_position *pos_out, sc_move *moves_out, int32_t *move_cnt_out, float *priors_out,
+                     float *value_out, void *stream);
+
 /* asynchronous form of sc_eval for double-buffered callers: submit returns as soon as the work is
  * queued on `stream` (host buffers must be pinned and stay untouched until the wait returns);
  * moves and priors are STRIDED: leaf i owns moves[i*SC_MAX_MOVES .. +move_cnt[i]) and the same
@@ -165,6 +187,9 @@ int sc_kernel_timing(sc_engine *e, float *conv3x3_avg_ms, int *n_launches);
 double sc_timed_flops_per_leaf(const sc_engine *e);
 /* level >= 1: device time (ms) of the legal-move kernel of the most recent sc_predict call (CUDA events on its stream) */
 int sc_predict_timing(sc_engine *e, float *movegen_ms);
+/* level >= 1: device time (ms) of the replay kernel of the most recent sc_predict_stack call (CUDA events on its
+ * stream); sc_predict_timing reports that call's legal-move kernel */
+int sc_predict_stack_timing(sc_engine *e, float *replay_ms);
 
 /* ===================== batched self-play driver (host side, C++) ================================
  * Replaces the single-tree loop of the `selfplay` binary (src/main.rs:153-238) and `mcts::mcts` /

@@ -74,6 +74,16 @@ int upload_move_tables(cudaStream_t st);
 constexpr int PREDICT_OVERFLOW = -1;
 int launch_legal_moves(const sc_position *d_pos, const int8_t *d_ep, int n, sc_move *d_moves, int32_t *d_cnt,
                        int32_t *d_term, cudaStream_t st);
+// sc_predict_stack, one thread per leaf: replays leaf i's moves d_stack[d_off[i], d_off[i+1]) from the initial position
+// and packs it as host::pack_position does with d_n_hist[i] history slots (nullptr: min(SC_LOOKBACK, plies + 1)) into
+// d_pos[i], its python-chess ep_square into d_ep[i], and into d_status[i] 0 or REPLAY_STATUS(ply, reason) for the first
+// move it rejects (the leaf is then packed from the moves before that one).  d_scratch: replay_scratch_bytes(d_off[n] + n)
+// bytes, a record of every replayed position
+enum { REPLAY_NOT_OURS = 1, REPLAY_BAD_TARGET, REPLAY_BAD_PROMO, REPLAY_NO_PROMO };
+__host__ __device__ constexpr int32_t REPLAY_STATUS(int ply, int reason) { return ply << 3 | reason; }
+size_t replay_scratch_bytes(int64_t positions);
+int launch_replay(const sc_move *d_stack, const int32_t *d_off, const int8_t *d_n_hist, int n, void *d_scratch,
+                  sc_position *d_pos, int8_t *d_ep, int32_t *d_status, cudaStream_t st);
 
 // ---- tower_f32.cu -------------------------------------------------------------------------
 // C[M][N] = gather_taps(A)[M][TAPS*K] * W[TAPS*K][ldw] + bias ; A is [rows][lda] fp32

@@ -247,11 +247,22 @@ struct sc_engine {
     int8_t *d_pred_ep = nullptr;
     uint8_t *d_pred_out = nullptr, *h_pred_out = nullptr;
     float last_movegen_ms = 0.f;
+    // sc_predict_stack, set up by its first call: stacks / offsets / n_hist of calls that do not fit the small staging
+    // buffer, the replay's per-leaf status (copied back to h_replay_status) and its scratch, grown to the largest call
+    sc_move *d_stack = nullptr;
+    int32_t *d_stack_off = nullptr, *d_replay_status = nullptr, *h_replay_status = nullptr;
+    int8_t *d_stack_nhist = nullptr;
+    void *d_replay_scratch = nullptr;
+    size_t replay_scratch_cap = 0;
+    cudaEvent_t ev_replay_t[2] = {nullptr, nullptr};  // timing: around the replay kernel
+    float last_replay_ms = 0.f;
 };
 
 namespace scb {
 
 constexpr int SC_SMALL_N = 128;
+// the pinned small-batch input buffer: sc_eval's positions, offsets and moves for SC_SMALL_N leaves
+constexpr size_t SMALL_IN_BYTES = (size_t)SC_SMALL_N * (sizeof(sc_position) + 4 + SC_MAX_MOVES * sizeof(sc_move)) + 64;
 
 // a 16-bit tensor-core mode (bf16 or fp16 operands): the tower, latency and head kernels of tower_bf16.cu / tower_lat.cu
 static bool tc16(const sc_engine *e) { return e->mode == SC_MODE_BF16 || e->mode == SC_MODE_FP16; }
@@ -515,7 +526,7 @@ static int alloc_buffers(sc_engine *e)
     }
     SCB_CHECK(dev_alloc(e, &e->vpre, (size_t)e->vsplit * B * N_VALUE_HIDDEN));
     {
-        const size_t in_bytes = (size_t)SC_SMALL_N * (sizeof(sc_position) + 4 + SC_MAX_MOVES * sizeof(sc_move)) + 64;
+        const size_t in_bytes = SMALL_IN_BYTES;
         const size_t out_floats = (size_t)SC_SMALL_N * (1 + SC_MAX_MOVES);
         SCB_CHECK(dev_alloc(e, &e->d_small_in, in_bytes));
         SCB_CUDA(cudaMallocHost(&e->h_small_in, in_bytes));
@@ -725,6 +736,29 @@ static int predict_setup(sc_engine *e)
     return SC_OK;
 }
 
+// sc_predict_stack's buffers and events (first call), and a replay scratch for `positions` replayed positions
+static int predict_stack_setup(sc_engine *e, int64_t positions)
+{
+    SCB_CHECK(predict_setup(e));
+    if (!e->d_stack) {
+        SCB_CHECK(dev_alloc(e, &e->d_stack, (size_t)e->max_batch * SC_MAX_STACK));
+        SCB_CHECK(dev_alloc(e, &e->d_stack_off, (size_t)e->max_batch + 1));
+        SCB_CHECK(dev_alloc(e, &e->d_stack_nhist, (size_t)e->max_batch));
+        SCB_CHECK(dev_alloc(e, &e->d_replay_status, (size_t)e->max_batch));
+        SCB_CUDA(cudaMallocHost(&e->h_replay_status, sizeof(int32_t) * (size_t)e->max_batch));
+        for (cudaEvent_t &ev : e->ev_replay_t) SCB_CUDA(cudaEventCreate(&ev));
+    }
+    const size_t need = replay_scratch_bytes(positions);
+    if (need > e->replay_scratch_cap) {
+        if (e->d_replay_scratch) SCB_CUDA(cudaFree(e->d_replay_scratch));
+        e->d_replay_scratch = nullptr;
+        e->replay_scratch_cap = 0;
+        SCB_CUDA(cudaMalloc(&e->d_replay_scratch, need));
+        e->replay_scratch_cap = need;
+    }
+    return SC_OK;
+}
+
 static int finish_timing(sc_engine *e, cudaStream_t st)
 {
     if (!e->timing) return SC_OK;
@@ -741,6 +775,82 @@ static int finish_timing(sc_engine *e, cudaStream_t st)
         }
         e->last_conv_n = e->kev_used / 2;
         e->last_conv_avg_ms = e->last_conv_n ? tot / e->last_conv_n : 0.f;
+    }
+    return SC_OK;
+}
+
+// sc_predict and sc_predict_stack once the packed leaves are on the device (d_pos / d_ep, as the kernels read them):
+// the legal moves, the encoder, the network and the gather, and the copies back, all queued on `st`.  Up to
+// SC_SMALL_N leaves write values and strided priors straight into the pinned small output buffer.
+static int predict_launch(sc_engine *e, int n, const sc_position *d_pos, const int8_t *d_ep, float *priors_out,
+                          float *value_out, cudaStream_t st)
+{
+    const size_t mv_b = sizeof(sc_move) * (size_t)n * SC_MAX_MOVES;
+    const bool small = n <= SC_SMALL_N;
+    float *d_value = small ? e->h_small_out : e->d_value, *d_priors = small ? e->h_small_out + n : e->d_priors;
+    if (e->timing) SCB_CUDA(cudaEventRecord(e->ev[0], st));
+    // the legal moves on their own stream next to the encoder and the tower (they do not depend on the network); the
+    // policy head's gather waits for them
+    sc_move *d_moves = reinterpret_cast<sc_move *>(e->d_pred_out);
+    int32_t *d_cnt = reinterpret_cast<int32_t *>(e->d_pred_out + mv_b), *d_term = d_cnt + n;
+    SCB_CUDA(cudaEventRecord(e->ev_gen_fork, st));
+    SCB_CUDA(cudaStreamWaitEvent(e->gen_stream, e->ev_gen_fork, 0));
+    if (e->timing) SCB_CUDA(cudaEventRecord(e->ev_gen_t[0], e->gen_stream));
+    SCB_CHECK(launch_legal_moves(d_pos, d_ep, n, d_moves, d_cnt, d_term, e->gen_stream));
+    if (e->timing) SCB_CUDA(cudaEventRecord(e->ev_gen_t[1], e->gen_stream));
+    SCB_CUDA(cudaEventRecord(e->ev_gen_done, e->gen_stream));
+    e->launches += 1;
+    SCB_CHECK(encode_for_mode(e, d_pos, n, st));
+    const TcGather g{d_pos, d_moves, nullptr, d_cnt, d_priors, n};
+    const bool fused = tc16(e) && e->fuse_gather;
+    float *saved_value = e->d_value;
+    e->d_value = d_value;
+    int rc = run_network(e, n, st, fused ? &g : nullptr, fused ? e->ev_gen_done : nullptr);
+    e->d_value = saved_value;
+    SCB_CHECK(rc);
+    if (!fused) {
+        SCB_CUDA(cudaStreamWaitEvent(st, e->ev_gen_done, 0));
+        SCB_CHECK(launch_policy_gather(e->logits, d_pos, d_moves, nullptr, d_cnt, n, d_priors, st));
+        e->launches += 1;
+    }
+    // results: moves, counts and termination codes in one copy, the full SC_MAX_MOVES stride of every leaf
+    SCB_CUDA(cudaMemcpyAsync(e->h_pred_out, e->d_pred_out, mv_b + 2 * sizeof(int32_t) * (size_t)n, cudaMemcpyDeviceToHost, st));
+    if (!small) {
+        SCB_CUDA(cudaMemcpyAsync(priors_out, d_priors, sizeof(float) * (size_t)n * SC_MAX_MOVES, cudaMemcpyDeviceToHost, st));
+        SCB_CUDA(cudaMemcpyAsync(value_out, d_value, sizeof(float) * (size_t)n, cudaMemcpyDeviceToHost, st));
+    }
+    return SC_OK;
+}
+
+// waits for predict_launch's work and hands out its results; white(i): leaf i has White to move (for the terminal
+// values)
+template <class WhiteToMove>
+static int predict_collect(sc_engine *e, const char *what, int n, sc_move *moves_out, int32_t *move_cnt_out,
+                           float *priors_out, float *value_out, cudaStream_t st, WhiteToMove white)
+{
+    const size_t mv_b = sizeof(sc_move) * (size_t)n * SC_MAX_MOVES, cnt_b = sizeof(int32_t) * (size_t)n;
+    const bool small = n <= SC_SMALL_N;
+    SCB_CHECK(finish_timing(e, st));
+    SCB_CUDA(cudaStreamSynchronize(st));
+    if (e->timing) SCB_CUDA(cudaEventElapsedTime(&e->last_movegen_ms, e->ev_gen_t[0], e->ev_gen_t[1]));
+    memcpy(moves_out, e->h_pred_out, mv_b);
+    memcpy(move_cnt_out, e->h_pred_out + mv_b, cnt_b);
+    if (small) {
+        memcpy(value_out, e->h_small_out, sizeof(float) * (size_t)n);
+        memcpy(priors_out, e->h_small_out + n, sizeof(float) * (size_t)n * SC_MAX_MOVES);
+    }
+    // a leaf without legal moves is terminal: torch.rs:98-106's value in White's perspective replaces the network's
+    const int32_t *term = reinterpret_cast<const int32_t *>(e->h_pred_out + mv_b + cnt_b);
+    int bad = -1;
+    for (int i = 0; i < n; i++) {
+        if (term[i] == PREDICT_OVERFLOW && bad < 0) bad = i;
+        if (term[i] == chess::T_CHECKMATE) value_out[i] = white(i) ? -1.f : 1.f;
+        if (term[i] == chess::T_STALEMATE) value_out[i] = 0.f;
+    }
+    if (bad >= 0) {
+        set_error(std::string(what) + ": leaf " + std::to_string(bad) + " has more than " + std::to_string(SC_MAX_MOVES) +
+                  " pseudo-legal moves (not a legal position)");
+        return SC_E_INVAL;
     }
     return SC_OK;
 }
@@ -875,7 +985,9 @@ int sc_destroy(sc_engine *e)
         if (s.out_done) cudaEventDestroy(s.out_done);
     }
     if (e->h_pred_out) cudaFreeHost(e->h_pred_out);
-    for (cudaEvent_t ev : {e->ev_gen_fork, e->ev_gen_done, e->ev_gen_t[0], e->ev_gen_t[1]})
+    if (e->h_replay_status) cudaFreeHost(e->h_replay_status);
+    if (e->d_replay_scratch) cudaFree(e->d_replay_scratch);
+    for (cudaEvent_t ev : {e->ev_gen_fork, e->ev_gen_done, e->ev_gen_t[0], e->ev_gen_t[1], e->ev_replay_t[0], e->ev_replay_t[1]})
         if (ev) cudaEventDestroy(ev);
     if (e->gen_stream) cudaStreamDestroy(e->gen_stream);
     if (e->head_stream) cudaStreamDestroy(e->head_stream);
@@ -1006,15 +1118,12 @@ int sc_predict(sc_engine *e, int n, const sc_position *pos, const int8_t *ep_squ
     cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
     SCB_CUDA(cudaSetDevice(e->device));
     SCB_CHECK(predict_setup(e));
-    const size_t pos_b = sizeof(sc_position) * (size_t)n, mv_b = sizeof(sc_move) * (size_t)n * SC_MAX_MOVES;
-    const size_t cnt_b = sizeof(int32_t) * (size_t)n;
+    const size_t pos_b = sizeof(sc_position) * (size_t)n;
     const sc_position *d_pos;
     const int8_t *d_ep = nullptr;
-    float *d_priors, *d_value;
-    const bool small = n <= SC_SMALL_N;
-    if (small) {
+    if (n <= SC_SMALL_N) {
         // sc_eval's staging: [positions | ep squares] in one pinned buffer, read in place by the kernels for up to 16
-        // leaves, else one copy; values and strided priors written straight into the pinned output buffer
+        // leaves, else one copy
         memcpy(e->h_small_in, pos, pos_b);
         if (ep_square) memcpy(e->h_small_in + pos_b, ep_square, (size_t)n);
         const uint8_t *in_dev = e->d_small_in;
@@ -1024,8 +1133,6 @@ int sc_predict(sc_engine *e, int n, const sc_position *pos, const int8_t *ep_squ
             SCB_CUDA(cudaMemcpyAsync(e->d_small_in, e->h_small_in, pos_b + (ep_square ? n : 0), cudaMemcpyHostToDevice, st));
         d_pos = reinterpret_cast<const sc_position *>(in_dev);
         if (ep_square) d_ep = reinterpret_cast<const int8_t *>(in_dev + pos_b);
-        d_value = e->h_small_out;
-        d_priors = e->h_small_out + n;
     } else {
         SCB_CUDA(cudaMemcpyAsync(e->d_pos, pos, pos_b, cudaMemcpyHostToDevice, st));
         if (ep_square) {
@@ -1033,63 +1140,107 @@ int sc_predict(sc_engine *e, int n, const sc_position *pos, const int8_t *ep_squ
             d_ep = e->d_pred_ep;
         }
         d_pos = e->d_pos;
-        d_value = e->d_value;
-        d_priors = e->d_priors;
     }
-    if (e->timing) SCB_CUDA(cudaEventRecord(e->ev[0], st));
-    // the legal moves on their own stream next to the encoder and the tower (they do not depend on the network); the
-    // policy head's gather waits for them
-    sc_move *d_moves = reinterpret_cast<sc_move *>(e->d_pred_out);
-    int32_t *d_cnt = reinterpret_cast<int32_t *>(e->d_pred_out + mv_b), *d_term = d_cnt + n;
-    SCB_CUDA(cudaEventRecord(e->ev_gen_fork, st));
-    SCB_CUDA(cudaStreamWaitEvent(e->gen_stream, e->ev_gen_fork, 0));
-    if (e->timing) SCB_CUDA(cudaEventRecord(e->ev_gen_t[0], e->gen_stream));
-    SCB_CHECK(launch_legal_moves(d_pos, d_ep, n, d_moves, d_cnt, d_term, e->gen_stream));
-    if (e->timing) SCB_CUDA(cudaEventRecord(e->ev_gen_t[1], e->gen_stream));
-    SCB_CUDA(cudaEventRecord(e->ev_gen_done, e->gen_stream));
-    e->launches += 1;
-    SCB_CHECK(encode_for_mode(e, d_pos, n, st));
-    const TcGather g{d_pos, d_moves, nullptr, d_cnt, d_priors, n};
-    const bool fused = tc16(e) && e->fuse_gather;
-    float *saved_value = e->d_value;
-    e->d_value = d_value;
-    int rc = run_network(e, n, st, fused ? &g : nullptr, fused ? e->ev_gen_done : nullptr);
-    e->d_value = saved_value;
-    SCB_CHECK(rc);
-    if (!fused) {
-        SCB_CUDA(cudaStreamWaitEvent(st, e->ev_gen_done, 0));
-        SCB_CHECK(launch_policy_gather(e->logits, d_pos, d_moves, nullptr, d_cnt, n, d_priors, st));
-        e->launches += 1;
-    }
-    // results: moves, counts and termination codes in one copy, the full SC_MAX_MOVES stride of every leaf
-    SCB_CUDA(cudaMemcpyAsync(e->h_pred_out, e->d_pred_out, mv_b + 2 * cnt_b, cudaMemcpyDeviceToHost, st));
-    if (!small) {
-        SCB_CUDA(cudaMemcpyAsync(priors_out, d_priors, sizeof(float) * (size_t)n * SC_MAX_MOVES, cudaMemcpyDeviceToHost, st));
-        SCB_CUDA(cudaMemcpyAsync(value_out, d_value, sizeof(float) * (size_t)n, cudaMemcpyDeviceToHost, st));
-    }
-    SCB_CHECK(finish_timing(e, st));
-    SCB_CUDA(cudaStreamSynchronize(st));
-    if (e->timing) SCB_CUDA(cudaEventElapsedTime(&e->last_movegen_ms, e->ev_gen_t[0], e->ev_gen_t[1]));
-    memcpy(moves_out, e->h_pred_out, mv_b);
-    memcpy(move_cnt_out, e->h_pred_out + mv_b, cnt_b);
-    if (small) {
-        memcpy(value_out, e->h_small_out, sizeof(float) * (size_t)n);
-        memcpy(priors_out, e->h_small_out + n, sizeof(float) * (size_t)n * SC_MAX_MOVES);
-    }
-    // a leaf without legal moves is terminal: torch.rs:98-106's value in White's perspective replaces the network's
-    const int32_t *term = reinterpret_cast<const int32_t *>(e->h_pred_out + mv_b + cnt_b);
-    int bad = -1;
-    for (int i = 0; i < n; i++) {
-        if (term[i] == PREDICT_OVERFLOW && bad < 0) bad = i;
-        if (term[i] == chess::T_CHECKMATE) value_out[i] = pos[i].meta[0] ? -1.f : 1.f;
-        if (term[i] == chess::T_STALEMATE) value_out[i] = 0.f;
-    }
-    if (bad >= 0) {
-        set_error("sc_predict: leaf " + std::to_string(bad) + " has more than " + std::to_string(SC_MAX_MOVES) +
-                  " pseudo-legal moves (not a legal position)");
+    SCB_CHECK(predict_launch(e, n, d_pos, d_ep, priors_out, value_out, st));
+    return predict_collect(e, "sc_predict", n, moves_out, move_cnt_out, priors_out, value_out, st,
+                           [pos](int i) { return pos[i].meta[0] != 0; });
+}
+
+int sc_predict_stack(sc_engine *e, int n, const sc_move *stack, const int32_t *stack_off, const int8_t *n_hist,
+                     sc_position *pos_out, sc_move *moves_out, int32_t *move_cnt_out, float *priors_out,
+                     float *value_out, void *stream)
+{
+    if (!e || n < 0 || n > e->max_batch ||
+        (n > 0 && (!stack_off || !moves_out || !move_cnt_out || !priors_out || !value_out))) {
+        set_error("sc_predict_stack: bad argument");
         return SC_E_INVAL;
     }
-    return SC_OK;
+    if (n == 0) return SC_OK;
+    if (stack_off[0] != 0) {
+        set_error("sc_predict_stack: stack_off[0] = " + std::to_string(stack_off[0]) + ", not 0");
+        return SC_E_INVAL;
+    }
+    for (int i = 0; i < n; i++) {
+        const int64_t len = (int64_t)stack_off[i + 1] - stack_off[i];
+        if (len < 0) {
+            set_error("sc_predict_stack: stack_off decreases at leaf " + std::to_string(i));
+            return SC_E_INVAL;
+        }
+        if (len > SC_MAX_STACK) {
+            set_error("sc_predict_stack: leaf " + std::to_string(i) + " has " + std::to_string(len) +
+                      " plies, more than SC_MAX_STACK = " + std::to_string(SC_MAX_STACK));
+            return SC_E_INVAL;
+        }
+        if (n_hist && (n_hist[i] < 1 || n_hist[i] > SC_LOOKBACK || n_hist[i] > len + 1)) {
+            set_error("sc_predict_stack: n_hist[" + std::to_string(i) + "] = " + std::to_string(n_hist[i]) +
+                      " is not in 1.." + std::to_string(len + 1 < SC_LOOKBACK ? len + 1 : SC_LOOKBACK));
+            return SC_E_INVAL;
+        }
+    }
+    const int total = stack_off[n];
+    if (total > 0 && !stack) {
+        set_error("sc_predict_stack: bad argument");
+        return SC_E_INVAL;
+    }
+    for (int k = 0; k < total; k++) {
+        const sc_move m = stack[k];
+        if (m.from >= 64 || m.to >= 64 || m.promo == 1 || m.promo > 5) {
+            set_error("sc_predict_stack: stack[" + std::to_string(k) + "] = (" + std::to_string(m.from) + ", " +
+                      std::to_string(m.to) + ", " + std::to_string(m.promo) +
+                      "): from/to must be below 64 and promo one of 0, 2, 3, 4, 5");
+            return SC_E_INVAL;
+        }
+    }
+    NvtxRange nv_call("sc_predict_stack");
+    cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
+    SCB_CUDA(cudaSetDevice(e->device));
+    SCB_CHECK(predict_stack_setup(e, (int64_t)total + n));
+    const size_t off_b = sizeof(int32_t) * ((size_t)n + 1), stk_b = sizeof(sc_move) * (size_t)total;
+    const size_t nh_b = n_hist ? (size_t)n : 0;
+    const int32_t *d_off = e->d_stack_off;
+    const sc_move *d_stk = e->d_stack;
+    const int8_t *d_nh = n_hist ? e->d_stack_nhist : nullptr;
+    if (n <= SC_SMALL_N && off_b + stk_b + nh_b <= SMALL_IN_BYTES) {
+        // [offsets | moves | n_hist] through the pinned staging buffer in one copy.  Not read in place: the replay
+        // reads its moves one dependent ply at a time, each read a round trip over PCIe from pinned memory
+        memcpy(e->h_small_in, stack_off, off_b);
+        if (total) memcpy(e->h_small_in + off_b, stack, stk_b);
+        if (n_hist) memcpy(e->h_small_in + off_b + stk_b, n_hist, nh_b);
+        SCB_CUDA(cudaMemcpyAsync(e->d_small_in, e->h_small_in, off_b + stk_b + nh_b, cudaMemcpyHostToDevice, st));
+        d_off = reinterpret_cast<const int32_t *>(e->d_small_in);
+        d_stk = reinterpret_cast<const sc_move *>(e->d_small_in + off_b);
+        if (n_hist) d_nh = reinterpret_cast<const int8_t *>(e->d_small_in + off_b + stk_b);
+    } else {
+        SCB_CUDA(cudaMemcpyAsync(e->d_stack_off, stack_off, off_b, cudaMemcpyHostToDevice, st));
+        if (total) SCB_CUDA(cudaMemcpyAsync(e->d_stack, stack, stk_b, cudaMemcpyHostToDevice, st));
+        if (n_hist) SCB_CUDA(cudaMemcpyAsync(e->d_stack_nhist, n_hist, nh_b, cudaMemcpyHostToDevice, st));
+    }
+    // the packed leaves and their ep squares go where sc_predict's kernels read them on the device
+    if (e->timing) SCB_CUDA(cudaEventRecord(e->ev_replay_t[0], st));
+    SCB_CHECK(launch_replay(d_stk, d_off, d_nh, n, e->d_replay_scratch, e->d_pos, e->d_pred_ep, e->d_replay_status, st));
+    if (e->timing) SCB_CUDA(cudaEventRecord(e->ev_replay_t[1], st));
+    e->launches += 1;
+    SCB_CHECK(predict_launch(e, n, e->d_pos, e->d_pred_ep, priors_out, value_out, st));
+    SCB_CUDA(cudaMemcpyAsync(e->h_replay_status, e->d_replay_status, sizeof(int32_t) * (size_t)n, cudaMemcpyDeviceToHost, st));
+    if (pos_out) SCB_CUDA(cudaMemcpyAsync(pos_out, e->d_pos, sizeof(sc_position) * (size_t)n, cudaMemcpyDeviceToHost, st));
+    // the side to move of a leaf replayed from the initial position: White after an even number of plies
+    const int32_t *status = e->h_replay_status;
+    auto plies = [&](int i) { return status[i] ? status[i] >> 3 : stack_off[i + 1] - stack_off[i]; };
+    const int rc = predict_collect(e, "sc_predict_stack", n, moves_out, move_cnt_out, priors_out, value_out, st,
+                                   [&](int i) { return plies(i) % 2 == 0; });
+    if (rc != SC_OK && rc != SC_E_INVAL) return rc;
+    if (e->timing) SCB_CUDA(cudaEventElapsedTime(&e->last_replay_ms, e->ev_replay_t[0], e->ev_replay_t[1]));
+    for (int i = 0; i < n; i++) {
+        if (!status[i]) continue;
+        static const char *why[] = {"", "its from-square holds no piece of the side to move",
+                                    "its to-square holds a piece of the side to move or a king",
+                                    "it promotes a piece that is not a pawn reaching the last rank",
+                                    "a pawn reaches the last rank without a promotion"};
+        set_error("sc_predict_stack: leaf " + std::to_string(i) + ", ply " + std::to_string(plies(i)) +
+                  ": move rejected, " + why[status[i] & 7]);
+        return SC_E_INVAL;
+    }
+    return rc;
 }
 
 int sc_eval_submit(sc_engine *e, int n, const sc_position *pos, const sc_move *moves_strided, const int32_t *move_cnt,
@@ -1439,6 +1590,13 @@ int sc_predict_timing(sc_engine *e, float *movegen_ms)
 {
     if (!e) return SC_E_INVAL;
     if (movegen_ms) *movegen_ms = e->last_movegen_ms;
+    return SC_OK;
+}
+
+int sc_predict_stack_timing(sc_engine *e, float *replay_ms)
+{
+    if (!e) return SC_E_INVAL;
+    if (replay_ms) *replay_ms = e->last_replay_ms;
     return SC_OK;
 }
 

@@ -198,7 +198,7 @@ struct Position {
         halfmove = p.meta[6];
         fullmove = p.meta[1];
     }
-    void set_start()
+    SCB_HD void set_start()
     {
         memset(this, 0, sizeof(*this));
         pt[PAWN] = rank_mask(1) | rank_mask(6);
@@ -272,7 +272,7 @@ struct Position {
         }
         return (pt[KING] & occ[WHITE]) && (pt[KING] & occ[BLACK]);
     }
-    int piece_at(int s) const
+    SCB_HD int piece_at(int s) const
     {
         u64 m = bit(s);
         if (!(all & m)) return NONE;
@@ -280,7 +280,7 @@ struct Position {
             if (pt[p] & m) return p;
         return NONE;
     }
-    int take(int s)
+    SCB_HD int take(int s)
     {
         int p = piece_at(s);
         if (p) {
@@ -292,7 +292,7 @@ struct Position {
         }
         return p;
     }
-    void put(int s, int p, int color)
+    SCB_HD void put(int s, int p, int color)
     {
         take(s);
         u64 m = bit(s);
@@ -328,19 +328,19 @@ struct Position {
         if (!(occ[BLACK] & pt[KING] & bit(60))) b = 0;
         return w | b;
     }
-    bool has_kingside(int color) const
+    SCB_HD bool has_kingside(int color) const
     {
         u64 back = color == WHITE ? RANK1 : RANK8;
         if (!(pt[KING] & occ[color] & back)) return false;
         return (clean_castling() & back & bit(color == WHITE ? 7 : 63)) != 0;
     }
-    bool has_queenside(int color) const
+    SCB_HD bool has_queenside(int color) const
     {
         u64 back = color == WHITE ? RANK1 : RANK8;
         if (!(pt[KING] & occ[color] & back)) return false;
         return (clean_castling() & back & bit(color == WHITE ? 0 : 56)) != 0;
     }
-    bool is_zeroing(const Move &m) const
+    SCB_HD bool is_zeroing(const Move &m) const
     {
         u64 touched = bit(m.from) ^ bit(m.to);
         return (touched & pt[PAWN]) || (touched & occ[!turn]);
@@ -359,7 +359,7 @@ struct Position {
     }
 
     // ---- python-chess Board.push ---------------------------------------------------------
-    void push(const Move &m)
+    SCB_HD void push(const Move &m)
     {
         castling = clean_castling();
         const int old_ep = ep;
@@ -631,26 +631,34 @@ struct Position {
         out.n = 0;
         gen_legal(out);
     }
-    bool has_legal_ep() const
+    // sinks of has_legal_ep: whether any move is generated, whether an en-passant capture is
+    struct AnySink {
+        bool any;
+        SCB_HD void add(int, int, int) { any = true; }
+    };
+    struct EpSink {
+        const Position &p;
+        bool any;
+        SCB_HD void add(int f, int t, int pr) { any = any || p.is_en_passant(Move{(uint8_t)f, (uint8_t)t, (uint8_t)pr}); }
+    };
+    SCB_HD bool has_legal_ep() const
     {
         if (ep < 0) return false;
-        MoveList c;
+        AnySink c{false};
         gen_ep(~0ULL, ~0ULL, c);
-        if (!c.n) return false;
-        MoveList l;
-        legal_moves(l);
-        for (int i = 0; i < l.n; i++)
-            if (is_en_passant(l.m[i])) return true;
-        return false;
+        if (!c.any) return false;
+        EpSink l{*this, false};
+        gen_legal(l);
+        return l.any;
     }
-    bool reduces_castling(const Move &m) const
+    SCB_HD bool reduces_castling(const Move &m) const
     {
         u64 cr = clean_castling();
         u64 touched = bit(m.from) ^ bit(m.to);
         return (touched & cr) || ((cr & RANK1) && (touched & pt[KING] & occ[WHITE])) ||
                ((cr & RANK8) && (touched & pt[KING] & occ[BLACK]));
     }
-    bool is_irreversible(const Move &m) const { return is_zeroing(m) || reduces_castling(m) || has_legal_ep(); }
+    SCB_HD bool is_irreversible(const Move &m) const { return is_zeroing(m) || reduces_castling(m) || has_legal_ep(); }
     bool insufficient(int color) const
     {
         u64 own = occ[color];
@@ -669,12 +677,14 @@ struct Position {
 struct TKey {
     u64 pt[6], w, b, cr;
     int turn, ep;
-    bool operator==(const TKey &o) const
+    SCB_HD bool operator==(const TKey &o) const
     {
-        return memcmp(pt, o.pt, sizeof(pt)) == 0 && w == o.w && b == o.b && cr == o.cr && turn == o.turn && ep == o.ep;
+        for (int i = 0; i < 6; i++)
+            if (pt[i] != o.pt[i]) return false;
+        return w == o.w && b == o.b && cr == o.cr && turn == o.turn && ep == o.ep;
     }
 };
-inline TKey tkey(const Position &p)
+SCB_HD TKey tkey(const Position &p)
 {
     TKey k;
     for (int i = 0; i < 6; i++) k.pt[i] = p.pt[i + 1];
@@ -684,6 +694,57 @@ inline TKey tkey(const Position &p)
     k.turn = p.turn;
     k.ep = p.has_legal_ep() ? p.ep : -1;
     return k;
+}
+
+// The packed form of a leaf (`_encode`'s inputs, src/chess.rs:845-877): one history slot, the piece-type boards
+// pieces[0..5] (pawn .. king) and White's occupancy of a position with its repetition flags `rep` (bit 0
+// is_repetition(2), bit 1 is_repetition(3)), and the meta vector of the current position (`encode_meta`,
+// src/chess.rs:652-662).  host::pack_position and the device replay of sc_predict_stack both write them.
+SCB_HD void pack_slot(const u64 *pieces, u64 white, u64 rep, uint64_t *s)
+{
+    for (int i = 0; i < 6; i++) s[i] = pieces[i];
+    s[6] = white;
+    s[7] = rep;
+}
+SCB_HD void pack_meta(const Position &c, int32_t *meta)
+{
+    meta[0] = c.turn;
+    meta[1] = c.fullmove;
+    meta[2] = c.has_kingside(c.turn);
+    meta[3] = c.has_queenside(c.turn);
+    meta[4] = c.has_kingside(!c.turn);
+    meta[5] = c.has_queenside(!c.turn);
+    meta[6] = c.halfmove;
+}
+
+// python-chess Board.is_repetition(count) of the position after `ply` moves, whose halfmove clock is `halfmove`, over a
+// history with h.occupancy(k) / h.key(k) = the occupied squares / tkey of the position after k moves (k <= ply) and
+// h.irreversible(k) = whether move k is irreversible (k < ply).  The host Game and the device replay of
+// sc_predict_stack (movegen.cu) both call it, so the repetition flags of a packed leaf are defined in one place.
+#ifdef __CUDACC__
+#pragma nv_exec_check_disable  // the host Game's accessor is host code; the device instantiation has a device one
+#endif
+template <class History> SCB_HD bool is_repetition(const History &h, int ply, int halfmove, int count)
+{
+    // python-chess pre-filters on equal occupancy over the whole stack; the exact walk below stops at
+    // the first irreversible move, and every zeroing move is irreversible, so only the last
+    // `halfmove` plies can hold a real repetition -- scanning just those gives the same answer
+    int maybe = 1;
+    const u64 all = h.occupancy(ply);
+    const int lo = ply - halfmove > 0 ? ply - halfmove : 0;
+    for (int k = ply - 1; k >= lo; k--)
+        if (h.occupancy(k) == all && ++maybe >= count) break;
+    if (maybe < count) return false;
+    const TKey key = h.key(ply);
+    int len = ply;
+    for (;;) {
+        if (count <= 1) return true;
+        if (len < count - 1) break;
+        len--;
+        if (h.irreversible(len)) break;
+        if (h.key(len) == key) count--;
+    }
+    return false;
 }
 
 // A game = python-chess Board with its move stack (`BoardState`, src/chess.rs:107-109).  Every
@@ -705,27 +766,11 @@ struct Game {
     const Position &pos_at(int k) const { return k == ply() ? cur : stack[k].pos; }
     uint8_t rep_at(int k) const { return k == ply() ? cur_rep : stack[k].rep; }
 
-    bool is_repetition(int count) const
-    {
-        // python-chess pre-filters on equal occupancy over the whole stack; the exact walk below stops at
-        // the first irreversible move, and every zeroing move is irreversible, so only the last
-        // `halfmove` plies can hold a real repetition -- scanning just those gives the same answer
-        int maybe = 1;
-        const int lo = ply() - cur.halfmove > 0 ? ply() - cur.halfmove : 0;
-        for (int k = ply() - 1; k >= lo; k--)
-            if (stack[k].pos.all == cur.all && ++maybe >= count) break;
-        if (maybe < count) return false;
-        const TKey key = tkey(cur);
-        int len = ply();
-        for (;;) {
-            if (count <= 1) return true;
-            if (len < count - 1) break;
-            len--;
-            if (stack[len].pos.is_irreversible(moves[len])) break;
-            if (tkey(stack[len].pos) == key) count--;
-        }
-        return false;
-    }
+    // the history accessor of chess::is_repetition
+    u64 occupancy(int k) const { return pos_at(k).all; }
+    TKey key(int k) const { return tkey(pos_at(k)); }
+    bool irreversible(int k) const { return stack[k].pos.is_irreversible(moves[k]); }
+    bool is_repetition(int count) const { return chess::is_repetition(*this, ply(), cur.halfmove, count); }
     void push(const Move &m)
     {
         stack.push_back(Entry{cur, cur_rep});

@@ -209,19 +209,9 @@ inline void pack_position(const Game &g, int n_hist, sc_position *out)
     for (int k = 0; k < n_hist; k++) {
         const int ply = g.ply() - k;
         const Position &p = g.pos_at(ply);
-        uint64_t *s = out->slot[k];
-        for (int i = 0; i < 6; i++) s[i] = p.pt[i + 1];
-        s[6] = p.occ[WHITE];
-        s[7] = g.rep_at(ply);
+        pack_slot(p.pt + 1, p.occ[WHITE], g.rep_at(ply), out->slot[k]);
     }
-    const Position &c = g.cur;
-    out->meta[0] = c.turn;
-    out->meta[1] = c.fullmove;
-    out->meta[2] = c.has_kingside(c.turn);
-    out->meta[3] = c.has_queenside(c.turn);
-    out->meta[4] = c.has_kingside(!c.turn);
-    out->meta[5] = c.has_queenside(!c.turn);
-    out->meta[6] = c.halfmove;
+    pack_meta(g.cur, out->meta);
     out->n_hist = n_hist;
 }
 

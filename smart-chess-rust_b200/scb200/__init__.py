@@ -19,6 +19,7 @@ from .binding import (  # noqa: F401
     SC_MODE_FP32_FFMA,
     SC_MODE_FP16,
     SC_MAX_MOVES,
+    SC_MAX_STACK,
     POSITION_DTYPE,
     MOVE_DTYPE,
     lib_path,

@@ -14,6 +14,7 @@ SC_N_PLANES = 112
 SC_N_META = 7
 SC_N_POLICY = 4672
 SC_MAX_MOVES = 256
+SC_MAX_STACK = 1024
 
 # struct sc_position { uint64_t slot[8][8]; int32_t meta[7]; int32_t n_hist; }  (544 bytes)
 POSITION_DTYPE = np.dtype([("slot", np.uint64, (8, 8)), ("meta", np.int32, (7,)), ("n_hist", np.int32)])
@@ -28,7 +29,7 @@ DECLARED_SYMBOLS = [
     "sc_selfplay_destroy", "sc_rules_probe", "sc_arena_create", "sc_encode_steps", "sc_timed_flops_per_leaf",
     "sc_random_positions", "sc_test_dirichlet", "sc_game_selfplay", "sc_rules_perft", "sc_device_info",
     "sc_selfplay_run_many", "sc_debug_tower", "sc_rules_probe_fen", "sc_selfplay_trace_game", "sc_predict",
-    "sc_predict_timing",
+    "sc_predict_timing", "sc_predict_stack", "sc_predict_stack_timing",
 ]
 
 
@@ -82,6 +83,8 @@ def load_library():
         L.sc_eval.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 6
         L.sc_predict.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 7
         L.sc_predict_timing.argtypes = [C.c_void_p, C.POINTER(C.c_float)]
+        L.sc_predict_stack.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 9
+        L.sc_predict_stack_timing.argtypes = [C.c_void_p, C.POINTER(C.c_float)]
         L.sc_eval_device.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,
                                      C.c_void_p, C.c_void_p]
         L.sc_encode_only.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
@@ -226,6 +229,62 @@ class Engine:
             return rc, moves, counts, priors, values
         _check(rc, "sc_predict")
         return moves, counts, priors, values
+
+    def predict_stack(self, stacks, n_hist=None, out=None, positions: bool = False, stream: int = 0, check: bool = True):
+        """predict() for leaves given as move stacks (sc_predict_stack): the device replays each game from the initial
+        position and packs the leaf itself.  stacks: a list of per-leaf move lists ((from, to, promo) tuples or
+        MOVE_DTYPE arrays; python-chess `board.move_stack`, oldest first, castling as the king's two-square move), or
+        (flat MOVE_DTYPE array, int32 offsets[n + 1]).  n_hist: per-leaf history slots (1..8, at most plies + 1), or
+        None for min(8, plies + 1).  Returns predict()'s (moves, counts, priors, values), then the packed leaves
+        (POSITION_DTYPE[n]) when `positions`; check=False puts the status code first instead of raising."""
+        if isinstance(stacks, tuple):
+            flat, off = stacks
+            flat = np.ascontiguousarray(flat, dtype=MOVE_DTYPE)
+            off = np.ascontiguousarray(off, dtype=np.int32)
+        else:
+            lens = [len(st) for st in stacks]
+            off = np.zeros(len(stacks) + 1, dtype=np.int32)
+            off[1:] = np.cumsum(lens)
+            flat = np.zeros(int(off[-1]), dtype=MOVE_DTYPE)
+            for st, b, ln in zip(stacks, off[:-1], lens):
+                if ln:
+                    a = np.asarray(st)
+                    if a.dtype == MOVE_DTYPE:
+                        flat[b : b + ln] = a
+                    else:
+                        a = a.reshape(ln, -1)
+                        for k, f in enumerate(("from", "to", "promo")):
+                            flat[f][b : b + ln] = a[:, k]
+        n = len(off) - 1
+        if n < 0:
+            raise SCError("predict_stack: offsets must hold n + 1 entries")
+        if n_hist is not None:
+            nh = np.asarray(n_hist)
+            if len(nh) != n or nh.min(initial=1) < -128 or nh.max(initial=1) > 127:
+                raise SCError("predict_stack: n_hist must hold one history length per leaf")
+            n_hist = np.ascontiguousarray(nh, dtype=np.int8)
+        if out is None:
+            out = (np.zeros((n, SC_MAX_MOVES), dtype=MOVE_DTYPE), np.zeros(n, dtype=np.int32),
+                   np.zeros((n, SC_MAX_MOVES), dtype=np.float32), np.zeros(n, dtype=np.float32))
+        for a, dt, shape in zip(out, (MOVE_DTYPE, np.int32, np.float32, np.float32), ((SC_MAX_MOVES,), (), (SC_MAX_MOVES,), ())):
+            if a.dtype != dt or a.shape[1:] != shape or len(a) < n or not a.flags.c_contiguous:
+                raise SCError("predict_stack: `out` must be (moves, counts, priors, values) arrays as predict() returns them")
+        moves, counts, priors, values = (a[:n] for a in out)
+        pos = np.zeros(n, dtype=POSITION_DTYPE) if positions else None
+        rc = load_library().sc_predict_stack(self._h, n, _ptr(flat) if len(flat) else None, _ptr(off), _ptr(n_hist),
+                                             _ptr(pos), _ptr(moves), _ptr(counts), _ptr(priors), _ptr(values),
+                                             stream or None)
+        res = (moves, counts, priors, values) + ((pos,) if positions else ())
+        if not check:
+            return (rc,) + res
+        _check(rc, "sc_predict_stack")
+        return res
+
+    def predict_stack_timing(self) -> float:
+        """device time (ms) of the replay kernel of the last predict_stack() (timing level >= 1)"""
+        ms = C.c_float()
+        _check(load_library().sc_predict_stack_timing(self._h, C.byref(ms)), "sc_predict_stack_timing")
+        return ms.value
 
     def predict_timing(self) -> float:
         """device time (ms) of the legal-move kernel of the last predict() (timing level >= 1)"""
