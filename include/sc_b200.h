@@ -130,6 +130,25 @@ int sc_predict_stack(sc_engine *e, int n, const sc_move *stack, const int32_t *s
                      sc_position *pos_out, sc_move *moves_out, int32_t *move_cnt_out, float *priors_out,
                      float *value_out, void *stream);
 
+/* Stored game roots, so that a search replays its game once per real move instead of once per leaf.
+ * sc_set_roots replays n_roots games (stack / stack_off as sc_predict_stack's) on the device and keeps, per root, what
+ * a later sc_predict_path needs to continue it: the final position (its ep square included) and the per-ply replay
+ * records.  The table replaces the previous one and lives until the next sc_set_roots or sc_destroy; n_roots = 0 clears
+ * it.  0 <= n_roots <= max_batch.  Host-side argument errors as sc_predict_stack's, before any launch and with the table
+ * left as it was.  A replay-time rejection returns SC_E_INVAL naming the root and the ply, and leaves the engine without
+ * roots.  Synchronous, on the engine's stream; sc_predict, sc_predict_stack and sc_eval* do not touch the table. */
+int sc_set_roots(sc_engine *e, int n_roots, const sc_move *stack, const int32_t *stack_off);
+
+/* Leaf i is root[i]'s game followed by path[path_off[i] .. path_off[i+1]).  Every output (pos_out, moves, counts,
+ * priors, values, terminal rule, status, error messages) is what sc_predict_stack returns for the concatenated stack
+ * root ++ path, with the same n_hist meaning and limits (NULL = min(8, total length + 1)).  Plies in messages count
+ * from the initial position.  SC_E_STATE if no roots are set (also for n = 0); SC_E_INVAL if root[i] is outside
+ * [0, n_roots) or the total length exceeds SC_MAX_STACK, and for path_off / path / n_hist as sc_predict_stack's
+ * stack_off / stack / n_hist. */
+int sc_predict_path(sc_engine *e, int n, const int32_t *root, const sc_move *path, const int32_t *path_off,
+                    const int8_t *n_hist, sc_position *pos_out, sc_move *moves_out, int32_t *move_cnt_out,
+                    float *priors_out, float *value_out, void *stream);
+
 /* asynchronous form of sc_eval for double-buffered callers: submit returns as soon as the work is
  * queued on `stream` (host buffers must be pinned and stay untouched until the wait returns);
  * moves and priors are STRIDED: leaf i owns moves[i*SC_MAX_MOVES .. +move_cnt[i]) and the same
@@ -190,6 +209,8 @@ int sc_predict_timing(sc_engine *e, float *movegen_ms);
 /* level >= 1: device time (ms) of the replay kernel of the most recent sc_predict_stack call (CUDA events on its
  * stream); sc_predict_timing reports that call's legal-move kernel */
 int sc_predict_stack_timing(sc_engine *e, float *replay_ms);
+/* level >= 1: device time (ms) of the path-replay kernel of the most recent sc_predict_path call */
+int sc_predict_path_timing(sc_engine *e, float *replay_ms);
 
 /* ===================== batched self-play driver (host side, C++) ================================
  * Replaces the single-tree loop of the `selfplay` binary (src/main.rs:153-238) and `mcts::mcts` /

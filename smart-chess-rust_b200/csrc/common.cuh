@@ -84,6 +84,18 @@ __host__ __device__ constexpr int32_t REPLAY_STATUS(int ply, int reason) { retur
 size_t replay_scratch_bytes(int64_t positions);
 int launch_replay(const sc_move *d_stack, const int32_t *d_off, const int8_t *d_n_hist, int n, void *d_scratch,
                   sc_position *d_pos, int8_t *d_ep, int32_t *d_status, cudaStream_t st);
+// sc_set_roots, one thread per root: replays root r's moves d_stack[d_off[r], d_off[r+1]) as launch_replay does and keeps
+// its records (replay_scratch_bytes(d_off[n] + n) bytes of d_rec in all), its final position in d_root_pos[r] and its
+// status in d_status[r]
+namespace chess { struct Position; }
+int launch_root_replay(const sc_move *d_stack, const int32_t *d_off, int n, void *d_rec, chess::Position *d_root_pos,
+                       int32_t *d_status, cudaStream_t st);
+// sc_predict_path, one thread per leaf: leaf i continues root d_root[i] of the table above (d_root_off = the d_off it
+// was built from) with d_path[d_off[i], d_off[i+1]) and is packed as launch_replay packs the whole game; statuses name
+// plies from the game start.  d_scratch: replay_scratch_bytes(d_off[n] + n) bytes, the path's records
+int launch_path_replay(const void *d_root_rec, const int32_t *d_root_off, const chess::Position *d_root_pos,
+                       const int32_t *d_root, const sc_move *d_path, const int32_t *d_off, const int8_t *d_n_hist, int n,
+                       void *d_scratch, sc_position *d_pos, int8_t *d_ep, int32_t *d_status, cudaStream_t st);
 
 // ---- tower_f32.cu -------------------------------------------------------------------------
 // C[M][N] = gather_taps(A)[M][TAPS*K] * W[TAPS*K][ldw] + bias ; A is [rows][lda] fp32

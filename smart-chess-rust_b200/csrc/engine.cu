@@ -8,6 +8,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <initializer_list>
 #include <map>
 #include <mutex>
 #include <string>
@@ -256,6 +257,16 @@ struct sc_engine {
     size_t replay_scratch_cap = 0;
     cudaEvent_t ev_replay_t[2] = {nullptr, nullptr};  // timing: around the replay kernel
     float last_replay_ms = 0.f;
+    // sc_set_roots' table, set up by its first call: per root its final position and the offsets of its moves (device,
+    // and a host copy in root_off), every root's replay records (grown to the largest call); n_roots == 0: no roots.
+    // d_path_root: sc_predict_path's root indices of calls that do not fit the small staging buffer
+    chess::Position *d_root_pos = nullptr;
+    int32_t *d_root_off = nullptr, *d_path_root = nullptr;
+    void *d_root_rec = nullptr;
+    size_t root_rec_cap = 0;
+    std::vector<int32_t> root_off;
+    int n_roots = 0;
+    float last_path_ms = 0.f;  // timing: the path-replay kernel (between ev_replay_t)
 };
 
 namespace scb {
@@ -736,6 +747,20 @@ static int predict_setup(sc_engine *e)
     return SC_OK;
 }
 
+// grows *buf (*cap bytes) to hold the replay records of `positions` replayed positions; its contents are not kept
+static int grow_records(void **buf, size_t *cap, int64_t positions)
+{
+    const size_t need = replay_scratch_bytes(positions);
+    if (need > *cap) {
+        if (*buf) SCB_CUDA(cudaFree(*buf));
+        *buf = nullptr;
+        *cap = 0;
+        SCB_CUDA(cudaMalloc(buf, need));
+        *cap = need;
+    }
+    return SC_OK;
+}
+
 // sc_predict_stack's buffers and events (first call), and a replay scratch for `positions` replayed positions
 static int predict_stack_setup(sc_engine *e, int64_t positions)
 {
@@ -748,15 +773,101 @@ static int predict_stack_setup(sc_engine *e, int64_t positions)
         SCB_CUDA(cudaMallocHost(&e->h_replay_status, sizeof(int32_t) * (size_t)e->max_batch));
         for (cudaEvent_t &ev : e->ev_replay_t) SCB_CUDA(cudaEventCreate(&ev));
     }
-    const size_t need = replay_scratch_bytes(positions);
-    if (need > e->replay_scratch_cap) {
-        if (e->d_replay_scratch) SCB_CUDA(cudaFree(e->d_replay_scratch));
-        e->d_replay_scratch = nullptr;
-        e->replay_scratch_cap = 0;
-        SCB_CUDA(cudaMalloc(&e->d_replay_scratch, need));
-        e->replay_scratch_cap = need;
+    return grow_records(&e->d_replay_scratch, &e->replay_scratch_cap, positions);
+}
+
+// sc_set_roots' table (first call), with room for the records of `positions` replayed positions
+static int roots_setup(sc_engine *e, int64_t positions)
+{
+    SCB_CHECK(predict_stack_setup(e, 0));
+    if (!e->d_root_pos) {
+        SCB_CHECK(dev_alloc(e, &e->d_root_pos, (size_t)e->max_batch));
+        SCB_CHECK(dev_alloc(e, &e->d_root_off, (size_t)e->max_batch + 1));
+        SCB_CHECK(dev_alloc(e, &e->d_path_root, (size_t)e->max_batch));
+    }
+    return grow_records(&e->d_root_rec, &e->root_rec_cap, positions);
+}
+
+// copies host arrays to the device on `st` and puts the address each is read from in dev[]: through the pinned small
+// staging buffer in one copy when n <= SC_SMALL_N and they fit it, else each into its own device buffer.  Not read in
+// place from pinned memory: the replay kernels read their moves one dependent ply at a time, each read a round trip
+// over PCIe.  An input with no host array gets nullptr.
+struct StagedInput {
+    const void *src;
+    size_t bytes;
+    void *dev;  // its device buffer
+};
+static int stage_inputs(sc_engine *e, int n, std::initializer_list<StagedInput> in, const void **dev, cudaStream_t st)
+{
+    size_t total = 0;
+    for (const StagedInput &a : in) total += a.bytes;
+    const bool small = n <= SC_SMALL_N && total <= SMALL_IN_BYTES;
+    size_t o = 0;
+    for (const StagedInput &a : in) {
+        if (small && a.bytes) memcpy(e->h_small_in + o, a.src, a.bytes);
+        if (!small && a.bytes) SCB_CUDA(cudaMemcpyAsync(a.dev, a.src, a.bytes, cudaMemcpyHostToDevice, st));
+        *dev++ = !a.src ? nullptr : small ? static_cast<const void *>(e->d_small_in + o) : a.dev;
+        o += a.bytes;
+    }
+    if (small) SCB_CUDA(cudaMemcpyAsync(e->d_small_in, e->h_small_in, total, cudaMemcpyHostToDevice, st));
+    return SC_OK;
+}
+
+// the host-side checks of n move lists (sc_predict_stack's stacks, sc_set_roots' roots, sc_predict_path's paths), before
+// any launch: offsets off[0..n] from 0 and not decreasing, the game of list i -- base(i) plies stored before it, then its
+// own -- at most SC_MAX_STACK plies, n_hist[i] (if given) in 1..min(SC_LOOKBACK, game plies + 1), every move's fields.
+// `unit` names a list in the messages, `off_name` / `mv_name` the two arrays
+template <class Base>
+static int check_move_lists(const char *what, const char *unit, const char *off_name, const char *mv_name, int n,
+                            const sc_move *mv, const int32_t *off, const int8_t *n_hist, Base base)
+{
+    const std::string w = std::string(what) + ": ";
+    if (off[0] != 0) {
+        set_error(w + off_name + "[0] = " + std::to_string(off[0]) + ", not 0");
+        return SC_E_INVAL;
+    }
+    for (int i = 0; i < n; i++) {
+        const int64_t own = (int64_t)off[i + 1] - off[i], len = base(i) + own;
+        if (own < 0) {
+            set_error(w + off_name + " decreases at " + unit + " " + std::to_string(i));
+            return SC_E_INVAL;
+        }
+        if (len > SC_MAX_STACK) {
+            set_error(w + unit + " " + std::to_string(i) + " has " + std::to_string(len) +
+                      " plies, more than SC_MAX_STACK = " + std::to_string(SC_MAX_STACK));
+            return SC_E_INVAL;
+        }
+        if (n_hist && (n_hist[i] < 1 || n_hist[i] > SC_LOOKBACK || n_hist[i] > len + 1)) {
+            set_error(w + "n_hist[" + std::to_string(i) + "] = " + std::to_string(n_hist[i]) + " is not in 1.." +
+                      std::to_string(len + 1 < SC_LOOKBACK ? len + 1 : SC_LOOKBACK));
+            return SC_E_INVAL;
+        }
+    }
+    const int total = off[n];
+    if (total > 0 && !mv) {
+        set_error(w + "bad argument");
+        return SC_E_INVAL;
+    }
+    for (int k = 0; k < total; k++) {
+        const sc_move m = mv[k];
+        if (m.from >= 64 || m.to >= 64 || m.promo == 1 || m.promo > 5) {
+            set_error(w + mv_name + "[" + std::to_string(k) + "] = (" + std::to_string(m.from) + ", " +
+                      std::to_string(m.to) + ", " + std::to_string(m.promo) +
+                      "): from/to must be below 64 and promo one of 0, 2, 3, 4, 5");
+            return SC_E_INVAL;
+        }
     }
     return SC_OK;
+}
+
+// the message of a replay status (REPLAY_STATUS)
+static const char *replay_reason(int32_t status)
+{
+    static const char *why[] = {"", "its from-square holds no piece of the side to move",
+                                "its to-square holds a piece of the side to move or a king",
+                                "it promotes a piece that is not a pawn reaching the last rank",
+                                "a pawn reaches the last rank without a promotion"};
+    return why[status & 7];
 }
 
 static int finish_timing(sc_engine *e, cudaStream_t st)
@@ -853,6 +964,33 @@ static int predict_collect(sc_engine *e, const char *what, int n, sc_move *moves
         return SC_E_INVAL;
     }
     return SC_OK;
+}
+
+// sc_predict_stack and sc_predict_path once their replay kernel is queued on `st` (packed leaves in d_pos / d_pred_ep,
+// statuses in d_replay_status, timing events ev_replay_t around it): sc_predict's launches and the results.
+// game_plies(i): leaf i's moves from the initial position; replay_ms: where timing puts the replay kernel's time
+template <class GamePlies>
+static int predict_replayed(sc_engine *e, const char *what, int n, GamePlies game_plies, sc_position *pos_out,
+                            sc_move *moves_out, int32_t *move_cnt_out, float *priors_out, float *value_out,
+                            float *replay_ms, cudaStream_t st)
+{
+    SCB_CHECK(predict_launch(e, n, e->d_pos, e->d_pred_ep, priors_out, value_out, st));
+    SCB_CUDA(cudaMemcpyAsync(e->h_replay_status, e->d_replay_status, sizeof(int32_t) * (size_t)n, cudaMemcpyDeviceToHost, st));
+    if (pos_out) SCB_CUDA(cudaMemcpyAsync(pos_out, e->d_pos, sizeof(sc_position) * (size_t)n, cudaMemcpyDeviceToHost, st));
+    // the side to move of a leaf replayed from the initial position: White after an even number of plies
+    const int32_t *status = e->h_replay_status;
+    auto plies = [&](int i) { return status[i] ? status[i] >> 3 : game_plies(i); };
+    const int rc = predict_collect(e, what, n, moves_out, move_cnt_out, priors_out, value_out, st,
+                                   [&](int i) { return plies(i) % 2 == 0; });
+    if (rc != SC_OK && rc != SC_E_INVAL) return rc;
+    if (e->timing) SCB_CUDA(cudaEventElapsedTime(replay_ms, e->ev_replay_t[0], e->ev_replay_t[1]));
+    for (int i = 0; i < n; i++) {
+        if (!status[i]) continue;
+        set_error(std::string(what) + ": leaf " + std::to_string(i) + ", ply " + std::to_string(plies(i)) +
+                  ": move rejected, " + replay_reason(status[i]));
+        return SC_E_INVAL;
+    }
+    return rc;
 }
 
 }  // namespace scb
@@ -987,6 +1125,7 @@ int sc_destroy(sc_engine *e)
     if (e->h_pred_out) cudaFreeHost(e->h_pred_out);
     if (e->h_replay_status) cudaFreeHost(e->h_replay_status);
     if (e->d_replay_scratch) cudaFree(e->d_replay_scratch);
+    if (e->d_root_rec) cudaFree(e->d_root_rec);
     for (cudaEvent_t ev : {e->ev_gen_fork, e->ev_gen_done, e->ev_gen_t[0], e->ev_gen_t[1], e->ev_replay_t[0], e->ev_replay_t[1]})
         if (ev) cudaEventDestroy(ev);
     if (e->gen_stream) cudaStreamDestroy(e->gen_stream);
@@ -1156,91 +1295,111 @@ int sc_predict_stack(sc_engine *e, int n, const sc_move *stack, const int32_t *s
         return SC_E_INVAL;
     }
     if (n == 0) return SC_OK;
-    if (stack_off[0] != 0) {
-        set_error("sc_predict_stack: stack_off[0] = " + std::to_string(stack_off[0]) + ", not 0");
-        return SC_E_INVAL;
-    }
-    for (int i = 0; i < n; i++) {
-        const int64_t len = (int64_t)stack_off[i + 1] - stack_off[i];
-        if (len < 0) {
-            set_error("sc_predict_stack: stack_off decreases at leaf " + std::to_string(i));
-            return SC_E_INVAL;
-        }
-        if (len > SC_MAX_STACK) {
-            set_error("sc_predict_stack: leaf " + std::to_string(i) + " has " + std::to_string(len) +
-                      " plies, more than SC_MAX_STACK = " + std::to_string(SC_MAX_STACK));
-            return SC_E_INVAL;
-        }
-        if (n_hist && (n_hist[i] < 1 || n_hist[i] > SC_LOOKBACK || n_hist[i] > len + 1)) {
-            set_error("sc_predict_stack: n_hist[" + std::to_string(i) + "] = " + std::to_string(n_hist[i]) +
-                      " is not in 1.." + std::to_string(len + 1 < SC_LOOKBACK ? len + 1 : SC_LOOKBACK));
-            return SC_E_INVAL;
-        }
-    }
-    const int total = stack_off[n];
-    if (total > 0 && !stack) {
-        set_error("sc_predict_stack: bad argument");
-        return SC_E_INVAL;
-    }
-    for (int k = 0; k < total; k++) {
-        const sc_move m = stack[k];
-        if (m.from >= 64 || m.to >= 64 || m.promo == 1 || m.promo > 5) {
-            set_error("sc_predict_stack: stack[" + std::to_string(k) + "] = (" + std::to_string(m.from) + ", " +
-                      std::to_string(m.to) + ", " + std::to_string(m.promo) +
-                      "): from/to must be below 64 and promo one of 0, 2, 3, 4, 5");
-            return SC_E_INVAL;
-        }
-    }
+    SCB_CHECK(check_move_lists("sc_predict_stack", "leaf", "stack_off", "stack", n, stack, stack_off, n_hist,
+                               [](int) { return 0; }));
     NvtxRange nv_call("sc_predict_stack");
     cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
     SCB_CUDA(cudaSetDevice(e->device));
+    const int total = stack_off[n];
     SCB_CHECK(predict_stack_setup(e, (int64_t)total + n));
-    const size_t off_b = sizeof(int32_t) * ((size_t)n + 1), stk_b = sizeof(sc_move) * (size_t)total;
-    const size_t nh_b = n_hist ? (size_t)n : 0;
-    const int32_t *d_off = e->d_stack_off;
-    const sc_move *d_stk = e->d_stack;
-    const int8_t *d_nh = n_hist ? e->d_stack_nhist : nullptr;
-    if (n <= SC_SMALL_N && off_b + stk_b + nh_b <= SMALL_IN_BYTES) {
-        // [offsets | moves | n_hist] through the pinned staging buffer in one copy.  Not read in place: the replay
-        // reads its moves one dependent ply at a time, each read a round trip over PCIe from pinned memory
-        memcpy(e->h_small_in, stack_off, off_b);
-        if (total) memcpy(e->h_small_in + off_b, stack, stk_b);
-        if (n_hist) memcpy(e->h_small_in + off_b + stk_b, n_hist, nh_b);
-        SCB_CUDA(cudaMemcpyAsync(e->d_small_in, e->h_small_in, off_b + stk_b + nh_b, cudaMemcpyHostToDevice, st));
-        d_off = reinterpret_cast<const int32_t *>(e->d_small_in);
-        d_stk = reinterpret_cast<const sc_move *>(e->d_small_in + off_b);
-        if (n_hist) d_nh = reinterpret_cast<const int8_t *>(e->d_small_in + off_b + stk_b);
-    } else {
-        SCB_CUDA(cudaMemcpyAsync(e->d_stack_off, stack_off, off_b, cudaMemcpyHostToDevice, st));
-        if (total) SCB_CUDA(cudaMemcpyAsync(e->d_stack, stack, stk_b, cudaMemcpyHostToDevice, st));
-        if (n_hist) SCB_CUDA(cudaMemcpyAsync(e->d_stack_nhist, n_hist, nh_b, cudaMemcpyHostToDevice, st));
-    }
+    const void *d[3];
+    SCB_CHECK(stage_inputs(e, n,
+                           {{stack_off, sizeof(int32_t) * ((size_t)n + 1), e->d_stack_off},
+                            {stack, sizeof(sc_move) * (size_t)total, e->d_stack},
+                            {n_hist, n_hist ? (size_t)n : 0, e->d_stack_nhist}},
+                           d, st));
     // the packed leaves and their ep squares go where sc_predict's kernels read them on the device
     if (e->timing) SCB_CUDA(cudaEventRecord(e->ev_replay_t[0], st));
-    SCB_CHECK(launch_replay(d_stk, d_off, d_nh, n, e->d_replay_scratch, e->d_pos, e->d_pred_ep, e->d_replay_status, st));
+    SCB_CHECK(launch_replay(static_cast<const sc_move *>(d[1]), static_cast<const int32_t *>(d[0]),
+                            static_cast<const int8_t *>(d[2]), n, e->d_replay_scratch, e->d_pos, e->d_pred_ep,
+                            e->d_replay_status, st));
     if (e->timing) SCB_CUDA(cudaEventRecord(e->ev_replay_t[1], st));
     e->launches += 1;
-    SCB_CHECK(predict_launch(e, n, e->d_pos, e->d_pred_ep, priors_out, value_out, st));
-    SCB_CUDA(cudaMemcpyAsync(e->h_replay_status, e->d_replay_status, sizeof(int32_t) * (size_t)n, cudaMemcpyDeviceToHost, st));
-    if (pos_out) SCB_CUDA(cudaMemcpyAsync(pos_out, e->d_pos, sizeof(sc_position) * (size_t)n, cudaMemcpyDeviceToHost, st));
-    // the side to move of a leaf replayed from the initial position: White after an even number of plies
-    const int32_t *status = e->h_replay_status;
-    auto plies = [&](int i) { return status[i] ? status[i] >> 3 : stack_off[i + 1] - stack_off[i]; };
-    const int rc = predict_collect(e, "sc_predict_stack", n, moves_out, move_cnt_out, priors_out, value_out, st,
-                                   [&](int i) { return plies(i) % 2 == 0; });
-    if (rc != SC_OK && rc != SC_E_INVAL) return rc;
-    if (e->timing) SCB_CUDA(cudaEventElapsedTime(&e->last_replay_ms, e->ev_replay_t[0], e->ev_replay_t[1]));
-    for (int i = 0; i < n; i++) {
-        if (!status[i]) continue;
-        static const char *why[] = {"", "its from-square holds no piece of the side to move",
-                                    "its to-square holds a piece of the side to move or a king",
-                                    "it promotes a piece that is not a pawn reaching the last rank",
-                                    "a pawn reaches the last rank without a promotion"};
-        set_error("sc_predict_stack: leaf " + std::to_string(i) + ", ply " + std::to_string(plies(i)) +
-                  ": move rejected, " + why[status[i] & 7]);
+    return predict_replayed(e, "sc_predict_stack", n, [&](int i) { return stack_off[i + 1] - stack_off[i]; }, pos_out,
+                            moves_out, move_cnt_out, priors_out, value_out, &e->last_replay_ms, st);
+}
+
+int sc_set_roots(sc_engine *e, int n_roots, const sc_move *stack, const int32_t *stack_off)
+{
+    if (!e || n_roots < 0 || n_roots > e->max_batch || (n_roots > 0 && !stack_off)) {
+        set_error("sc_set_roots: bad argument");
         return SC_E_INVAL;
     }
-    return rc;
+    if (n_roots > 0)
+        SCB_CHECK(check_move_lists("sc_set_roots", "root", "stack_off", "stack", n_roots, stack, stack_off, nullptr,
+                                   [](int) { return 0; }));
+    NvtxRange nv_call("sc_set_roots");
+    e->n_roots = 0;
+    if (n_roots == 0) return SC_OK;
+    cudaStream_t st = e->stream;
+    SCB_CUDA(cudaSetDevice(e->device));
+    const int total = stack_off[n_roots];
+    SCB_CHECK(roots_setup(e, (int64_t)total + n_roots));
+    // the offsets stay on the device with the table: sc_predict_path finds each root's records through them
+    SCB_CUDA(cudaMemcpyAsync(e->d_root_off, stack_off, sizeof(int32_t) * ((size_t)n_roots + 1), cudaMemcpyHostToDevice, st));
+    if (total) SCB_CUDA(cudaMemcpyAsync(e->d_stack, stack, sizeof(sc_move) * (size_t)total, cudaMemcpyHostToDevice, st));
+    SCB_CHECK(launch_root_replay(e->d_stack, e->d_root_off, n_roots, e->d_root_rec, e->d_root_pos, e->d_replay_status, st));
+    e->launches += 1;
+    SCB_CUDA(cudaMemcpyAsync(e->h_replay_status, e->d_replay_status, sizeof(int32_t) * (size_t)n_roots,
+                             cudaMemcpyDeviceToHost, st));
+    SCB_CUDA(cudaStreamSynchronize(st));
+    for (int r = 0; r < n_roots; r++) {
+        const int32_t status = e->h_replay_status[r];
+        if (!status) continue;
+        set_error("sc_set_roots: root " + std::to_string(r) + ", ply " + std::to_string(status >> 3) +
+                  ": move rejected, " + replay_reason(status));
+        return SC_E_INVAL;
+    }
+    e->root_off.assign(stack_off, stack_off + n_roots + 1);
+    e->n_roots = n_roots;
+    return SC_OK;
+}
+
+int sc_predict_path(sc_engine *e, int n, const int32_t *root, const sc_move *path, const int32_t *path_off,
+                    const int8_t *n_hist, sc_position *pos_out, sc_move *moves_out, int32_t *move_cnt_out,
+                    float *priors_out, float *value_out, void *stream)
+{
+    if (!e || n < 0 || n > e->max_batch ||
+        (n > 0 && (!root || !path_off || !moves_out || !move_cnt_out || !priors_out || !value_out))) {
+        set_error("sc_predict_path: bad argument");
+        return SC_E_INVAL;
+    }
+    if (e->n_roots == 0) {
+        set_error("sc_predict_path: no roots are set (sc_set_roots)");
+        return SC_E_STATE;
+    }
+    if (n == 0) return SC_OK;
+    for (int i = 0; i < n; i++) {
+        if (root[i] < 0 || root[i] >= e->n_roots) {
+            set_error("sc_predict_path: root[" + std::to_string(i) + "] = " + std::to_string(root[i]) + " is not in 0.." +
+                      std::to_string(e->n_roots - 1));
+            return SC_E_INVAL;
+        }
+    }
+    const int32_t *ro = e->root_off.data();
+    auto root_plies = [&](int i) { return ro[root[i] + 1] - ro[root[i]]; };
+    SCB_CHECK(check_move_lists("sc_predict_path", "leaf", "path_off", "path", n, path, path_off, n_hist, root_plies));
+    NvtxRange nv_call("sc_predict_path");
+    cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
+    SCB_CUDA(cudaSetDevice(e->device));
+    const int total = path_off[n];
+    SCB_CHECK(predict_stack_setup(e, (int64_t)total + n));
+    const void *d[4];
+    SCB_CHECK(stage_inputs(e, n,
+                           {{path_off, sizeof(int32_t) * ((size_t)n + 1), e->d_stack_off},
+                            {root, sizeof(int32_t) * (size_t)n, e->d_path_root},
+                            {path, sizeof(sc_move) * (size_t)total, e->d_stack},
+                            {n_hist, n_hist ? (size_t)n : 0, e->d_stack_nhist}},
+                           d, st));
+    if (e->timing) SCB_CUDA(cudaEventRecord(e->ev_replay_t[0], st));
+    SCB_CHECK(launch_path_replay(e->d_root_rec, e->d_root_off, e->d_root_pos, static_cast<const int32_t *>(d[1]),
+                                 static_cast<const sc_move *>(d[2]), static_cast<const int32_t *>(d[0]),
+                                 static_cast<const int8_t *>(d[3]), n, e->d_replay_scratch, e->d_pos, e->d_pred_ep,
+                                 e->d_replay_status, st));
+    if (e->timing) SCB_CUDA(cudaEventRecord(e->ev_replay_t[1], st));
+    e->launches += 1;
+    return predict_replayed(e, "sc_predict_path", n, [&](int i) { return root_plies(i) + path_off[i + 1] - path_off[i]; },
+                            pos_out, moves_out, move_cnt_out, priors_out, value_out, &e->last_path_ms, st);
 }
 
 int sc_eval_submit(sc_engine *e, int n, const sc_position *pos, const sc_move *moves_strided, const int32_t *move_cnt,
@@ -1597,6 +1756,13 @@ int sc_predict_stack_timing(sc_engine *e, float *replay_ms)
 {
     if (!e) return SC_E_INVAL;
     if (replay_ms) *replay_ms = e->last_replay_ms;
+    return SC_OK;
+}
+
+int sc_predict_path_timing(sc_engine *e, float *replay_ms)
+{
+    if (!e) return SC_E_INVAL;
+    if (replay_ms) *replay_ms = e->last_path_ms;
     return SC_OK;
 }
 

@@ -27,6 +27,12 @@
 #else
 #define SCB_HD inline
 #endif
+// SCB_HD, always inlined in device code (the host build is left to the compiler)
+#ifdef __CUDA_ARCH__
+#define SCB_HD_DEVICE_INLINE __host__ __device__ __forceinline__
+#else
+#define SCB_HD_DEVICE_INLINE SCB_HD
+#endif
 
 namespace scb {
 namespace chess {
@@ -611,7 +617,9 @@ struct Position {
     };
     // the legal moves in python-chess order into `out`; returns the number of pseudo-legal candidates they were
     // filtered from (never fewer than the legal moves)
-    template <class Sink> SCB_HD int gen_legal(Sink &out) const
+    // always inlined on the device: has_legal_ep's instance is reached from the three replay kernels of movegen.cu
+    // (through tkey), and left a call it caps each of them at 96 registers with spills
+    template <class Sink> SCB_HD_DEVICE_INLINE int gen_legal(Sink &out) const
     {
         const int king = king_sq(turn);
         SafeFilter<Sink> f{*this, king, 0, out, 0};

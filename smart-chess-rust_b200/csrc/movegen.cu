@@ -1,6 +1,6 @@
 // Legal moves of every leaf on the device, for sc_predict (the `state.legal_moves()` half of `Game::predict`,
 // src/game.rs:3-15, src/backends/torch.rs:96-106), and the replay that packs each leaf from its move stack for
-// sc_predict_stack.
+// sc_predict_stack, or from a stored root and its path for sc_set_roots / sc_predict_path.
 //
 // One thread per leaf runs host/chess_rules.hpp's generator -- the same code as the host driver, so python-chess's
 // generation order is defined in one place -- and writes each legal move straight into the leaf's strided output slot
@@ -57,10 +57,12 @@ __global__ void __launch_bounds__(MOVEGEN_THREADS) legal_moves_kernel(const sc_p
     term[i] = code;
 }
 
-// ---- sc_predict_stack: replay and pack ------------------------------------------------------------------------------
+// ---- sc_predict_stack / sc_set_roots / sc_predict_path: replay and pack ---------------------------------------------
 // Serial per leaf: each ply depends on the last.  What the repetition walk needs of every replayed position goes to a
 // global scratch rather than a per-thread array (local memory is reserved for every resident thread), and
-// chess::is_repetition walks it exactly as the host Game walks its stack.
+// chess::is_repetition walks it exactly as the host Game walks its stack.  sc_set_roots keeps these records of each
+// root game in a persistent table; sc_predict_path continues a stored root's final position with the leaf's path and
+// walks the root's records, then the path's.
 
 namespace {
 
@@ -70,13 +72,28 @@ struct ReplayPly {
     int32_t halfmove, irreversible;
 };
 
-// chess::is_repetition's history over one leaf's replay: ply[k] = the position after k moves
-struct ReplayHistory {
-    const ReplayPly *ply;
-    __device__ chess::u64 occupancy(int k) const { return ply[k].key.w | ply[k].key.b; }
-    __device__ chess::TKey key(int k) const { return ply[k].key; }
-    __device__ bool irreversible(int k) const { return ply[k].irreversible != 0; }
+// chess::is_repetition's history over replay records; Records::at(k) = the record of the position after k moves
+template <class Records> struct PlyHistory : Records {
+    __device__ chess::u64 occupancy(int k) const { return this->at(k).key.w | this->at(k).key.b; }
+    __device__ chess::TKey key(int k) const { return this->at(k).key; }
+    __device__ bool irreversible(int k) const { return this->at(k).irreversible != 0; }
 };
+
+// one game replayed from the initial position: ply[k] = the position after k moves
+struct GameRecords {
+    const ReplayPly *ply;
+    __device__ const ReplayPly &at(int k) const { return ply[k]; }
+};
+using ReplayHistory = PlyHistory<GameRecords>;
+
+// a stored root of `root_plies` moves, then the leaf's path: the root's records up to its last move, the path's
+// (path[0] = the root's final position, recorded again by the path replay) from there on
+struct RootPathRecords {
+    const ReplayPly *root, *path;
+    int root_plies;
+    __device__ const ReplayPly &at(int k) const { return k < root_plies ? root[k] : path[k - root_plies]; }
+};
+using PathHistory = PlyHistory<RootPathRecords>;
 
 // the replay's checks (Board.push verifies no legality either; from/to < 64 and promo are checked on the host)
 __device__ int replay_reject(const chess::Position &p, const sc_move &m)
@@ -89,6 +106,49 @@ __device__ int replay_reject(const chess::Position &p, const sc_move &m)
     if (m.promo && !last_rank) return REPLAY_BAD_PROMO;
     if (!m.promo && last_rank) return REPLAY_NO_PROMO;
     return 0;
+}
+
+// plays mv[0, len) on p, ply by ply: the record h[k] of the position before move k (h[len]: the final position), the
+// move's checks, then Position::push.  A rejected move k ends the replay with len = k and returns
+// REPLAY_STATUS(ply0 + k, why) (ply0: the plies played before p); 0 when every move is played
+__device__ __forceinline__ int replay_moves(chess::Position &p, const sc_move *mv, int &len, ReplayPly *h, int ply0)
+{
+    for (int k = 0;; k++) {
+        const chess::TKey key = chess::tkey(p);
+        h[k].key = key;
+        h[k].halfmove = p.halfmove;
+        if (k == len) return 0;
+        const sc_move m = mv[k];
+        const int why = replay_reject(p, m);
+        if (why) {
+            len = k;
+            return REPLAY_STATUS(ply0 + k, why);
+        }
+        const chess::Move cm{m.from, m.to, m.promo};
+        // Position::is_irreversible, with its has_legal_ep() read off the key (key.ep is the ep square only if legal)
+        h[k].irreversible = p.is_zeroing(cm) || p.reduces_castling(cm) || key.ep >= 0;
+        p.push(cm);
+    }
+}
+
+// host::pack_position of the position p reached after `plies` moves, with min(nh, plies + 1) history slots read off h
+template <class History>
+__device__ __forceinline__ void pack_replayed(const History &h, const chess::Position &p, int plies, int nh,
+                                              sc_position &o)
+{
+    if (nh > plies + 1) nh = plies + 1;
+    chess::pack_meta(p, o.meta);
+    o.n_hist = nh;
+    for (int s = 0; s < SC_LOOKBACK; s++) {
+        if (s < nh) {
+            const int ply = plies - s, hm = h.at(ply).halfmove;
+            uint64_t rep = 0;
+            if (chess::is_repetition(h, ply, hm, 2)) rep = 1 | (chess::is_repetition(h, ply, hm, 3) ? 2 : 0);
+            chess::pack_slot(h.at(ply).key.pt, h.at(ply).key.w, rep, o.slot[s]);
+        } else {
+            for (int j = 0; j < 8; j++) o.slot[s][j] = 0;
+        }
+    }
 }
 
 }  // namespace
@@ -105,46 +165,52 @@ __global__ void __launch_bounds__(REPLAY_THREADS) replay_kernel(const sc_move *_
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     const int base = off[i];
-    const sc_move *mv = stack + base;
     ReplayPly *h = scratch + base + i;  // plies + 1 positions per leaf
-    int len = off[i + 1] - base, st = 0;
+    int len = off[i + 1] - base;
     chess::Position p;
     p.set_start();
-    for (int k = 0;; k++) {
-        const chess::TKey key = chess::tkey(p);
-        h[k].key = key;
-        h[k].halfmove = p.halfmove;
-        if (k == len) break;
-        const sc_move m = mv[k];
-        const int why = replay_reject(p, m);
-        if (why) {
-            st = REPLAY_STATUS(k, why);
-            len = k;
-            break;
-        }
-        const chess::Move cm{m.from, m.to, m.promo};
-        // Position::is_irreversible, with its has_legal_ep() read off the key (key.ep is the ep square only if legal)
-        h[k].irreversible = p.is_zeroing(cm) || p.reduces_castling(cm) || key.ep >= 0;
-        p.push(cm);
-    }
-    int nh = n_hist ? n_hist[i] : SC_LOOKBACK;
-    if (nh > len + 1) nh = len + 1;
-    sc_position &o = pos[i];
-    chess::pack_meta(p, o.meta);
-    o.n_hist = nh;
+    const int st = replay_moves(p, stack + base, len, h, 0);
+    pack_replayed(ReplayHistory{{h}}, p, len, n_hist ? n_hist[i] : SC_LOOKBACK, pos[i]);
     ep[i] = (int8_t)p.ep;
     status[i] = st;
-    const ReplayHistory rh{h};
-    for (int s = 0; s < SC_LOOKBACK; s++) {
-        if (s < nh) {
-            const int ply = len - s, hm = h[ply].halfmove;
-            uint64_t rep = 0;
-            if (chess::is_repetition(rh, ply, hm, 2)) rep = 1 | (chess::is_repetition(rh, ply, hm, 3) ? 2 : 0);
-            chess::pack_slot(h[ply].key.pt, h[ply].key.w, rep, o.slot[s]);
-        } else {
-            for (int j = 0; j < 8; j++) o.slot[s][j] = 0;
-        }
-    }
+}
+
+// sc_set_roots, one thread per root: root r's records (plies + 1) at rec + off[r] + r, its final position and status
+__global__ void __launch_bounds__(REPLAY_THREADS) root_replay_kernel(const sc_move *__restrict__ stack,
+                                                                     const int32_t *__restrict__ off, int n,
+                                                                     ReplayPly *__restrict__ rec,
+                                                                     chess::Position *__restrict__ root_pos,
+                                                                     int32_t *__restrict__ status)
+{
+    const int r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= n) return;
+    const int base = off[r];
+    int len = off[r + 1] - base;
+    chess::Position p;
+    p.set_start();
+    status[r] = replay_moves(p, stack + base, len, rec + base + r, 0);
+    root_pos[r] = p;
+}
+
+// sc_predict_path, one thread per leaf: root[i]'s stored position continued with path[off[i], off[i+1]) (records in
+// the per-call scratch), packed over the root's records and the path's
+__global__ void __launch_bounds__(REPLAY_THREADS) path_replay_kernel(
+    const ReplayPly *__restrict__ root_rec, const int32_t *__restrict__ root_off,
+    const chess::Position *__restrict__ root_pos, const int32_t *__restrict__ root, const sc_move *__restrict__ path,
+    const int32_t *__restrict__ off, const int8_t *__restrict__ n_hist, int n, ReplayPly *__restrict__ scratch,
+    sc_position *__restrict__ pos, int8_t *__restrict__ ep, int32_t *__restrict__ status)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int r = root[i], root_base = root_off[r], root_plies = root_off[r + 1] - root_base;
+    const int base = off[i];
+    ReplayPly *h = scratch + base + i;
+    int len = off[i + 1] - base;
+    chess::Position p = root_pos[r];
+    status[i] = replay_moves(p, path + base, len, h, root_plies);
+    ep[i] = (int8_t)p.ep;
+    const PathHistory ph{{root_rec + root_base + r, h, root_plies}};
+    pack_replayed(ph, p, root_plies + len, n_hist ? n_hist[i] : SC_LOOKBACK, pos[i]);
 }
 
 size_t replay_scratch_bytes(int64_t positions) { return sizeof(ReplayPly) * (size_t)positions; }
@@ -155,6 +221,28 @@ int launch_replay(const sc_move *d_stack, const int32_t *d_off, const int8_t *d_
     if (n <= 0) return SC_OK;
     replay_kernel<<<(n + REPLAY_THREADS - 1) / REPLAY_THREADS, REPLAY_THREADS, 0, st>>>(
         d_stack, d_off, d_n_hist, n, static_cast<ReplayPly *>(d_scratch), d_pos, d_ep, d_status);
+    SCB_CUDA(cudaGetLastError());
+    return SC_OK;
+}
+
+int launch_root_replay(const sc_move *d_stack, const int32_t *d_off, int n, void *d_rec, chess::Position *d_root_pos,
+                       int32_t *d_status, cudaStream_t st)
+{
+    if (n <= 0) return SC_OK;
+    root_replay_kernel<<<(n + REPLAY_THREADS - 1) / REPLAY_THREADS, REPLAY_THREADS, 0, st>>>(
+        d_stack, d_off, n, static_cast<ReplayPly *>(d_rec), d_root_pos, d_status);
+    SCB_CUDA(cudaGetLastError());
+    return SC_OK;
+}
+
+int launch_path_replay(const void *d_root_rec, const int32_t *d_root_off, const chess::Position *d_root_pos,
+                       const int32_t *d_root, const sc_move *d_path, const int32_t *d_off, const int8_t *d_n_hist, int n,
+                       void *d_scratch, sc_position *d_pos, int8_t *d_ep, int32_t *d_status, cudaStream_t st)
+{
+    if (n <= 0) return SC_OK;
+    path_replay_kernel<<<(n + REPLAY_THREADS - 1) / REPLAY_THREADS, REPLAY_THREADS, 0, st>>>(
+        static_cast<const ReplayPly *>(d_root_rec), d_root_off, d_root_pos, d_root, d_path, d_off, d_n_hist, n,
+        static_cast<ReplayPly *>(d_scratch), d_pos, d_ep, d_status);
     SCB_CUDA(cudaGetLastError());
     return SC_OK;
 }

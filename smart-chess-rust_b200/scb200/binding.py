@@ -29,7 +29,8 @@ DECLARED_SYMBOLS = [
     "sc_selfplay_destroy", "sc_rules_probe", "sc_arena_create", "sc_encode_steps", "sc_timed_flops_per_leaf",
     "sc_random_positions", "sc_test_dirichlet", "sc_game_selfplay", "sc_rules_perft", "sc_device_info",
     "sc_selfplay_run_many", "sc_debug_tower", "sc_rules_probe_fen", "sc_selfplay_trace_game", "sc_predict",
-    "sc_predict_timing", "sc_predict_stack", "sc_predict_stack_timing",
+    "sc_predict_timing", "sc_predict_stack", "sc_predict_stack_timing", "sc_set_roots", "sc_predict_path",
+    "sc_predict_path_timing",
 ]
 
 
@@ -85,6 +86,9 @@ def load_library():
         L.sc_predict_timing.argtypes = [C.c_void_p, C.POINTER(C.c_float)]
         L.sc_predict_stack.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 9
         L.sc_predict_stack_timing.argtypes = [C.c_void_p, C.POINTER(C.c_float)]
+        L.sc_set_roots.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
+        L.sc_predict_path.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 10
+        L.sc_predict_path_timing.argtypes = [C.c_void_p, C.POINTER(C.c_float)]
         L.sc_eval_device.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,
                                      C.c_void_p, C.c_void_p]
         L.sc_encode_only.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
@@ -144,6 +148,52 @@ def _ptr(a):
     if hasattr(a, "data_ptr"):  # torch tensor (device or pinned host)
         return a.data_ptr()
     return a.ctypes.data
+
+
+def _move_lists(lists, what):
+    """(flat MOVE_DTYPE array, int32 offsets[n + 1]) of per-leaf move lists ((from, to, promo) tuples or MOVE_DTYPE
+    arrays), or of such a pair given as it is"""
+    if isinstance(lists, tuple):
+        flat, off = lists
+        flat = np.ascontiguousarray(flat, dtype=MOVE_DTYPE)
+        off = np.ascontiguousarray(off, dtype=np.int32)
+    else:
+        lens = [len(st) for st in lists]
+        off = np.zeros(len(lists) + 1, dtype=np.int32)
+        off[1:] = np.cumsum(lens)
+        flat = np.zeros(int(off[-1]), dtype=MOVE_DTYPE)
+        for st, b, ln in zip(lists, off[:-1], lens):
+            if ln:
+                a = np.asarray(st)
+                if a.dtype == MOVE_DTYPE:
+                    flat[b : b + ln] = a
+                else:
+                    a = a.reshape(ln, -1)
+                    for k, f in enumerate(("from", "to", "promo")):
+                        flat[f][b : b + ln] = a[:, k]
+    if len(off) < 1:
+        raise SCError(f"{what}: offsets must hold n + 1 entries")
+    return flat, off
+
+
+def _n_hist_arg(n_hist, n, what):
+    if n_hist is None:
+        return None
+    nh = np.asarray(n_hist)
+    if len(nh) != n or nh.min(initial=1) < -128 or nh.max(initial=1) > 127:
+        raise SCError(f"{what}: n_hist must hold one history length per leaf")
+    return np.ascontiguousarray(nh, dtype=np.int8)
+
+
+def _predict_out(out, n, what):
+    """predict()'s (moves, counts, priors, values) for n leaves: new arrays, or the first n rows of `out`'s"""
+    if out is None:
+        out = (np.zeros((n, SC_MAX_MOVES), dtype=MOVE_DTYPE), np.zeros(n, dtype=np.int32),
+               np.zeros((n, SC_MAX_MOVES), dtype=np.float32), np.zeros(n, dtype=np.float32))
+    for a, dt, shape in zip(out, (MOVE_DTYPE, np.int32, np.float32, np.float32), ((SC_MAX_MOVES,), (), (SC_MAX_MOVES,), ())):
+        if a.dtype != dt or a.shape[1:] != shape or len(a) < n or not a.flags.c_contiguous:
+            raise SCError(f"{what}: `out` must be (moves, counts, priors, values) arrays as predict() returns them")
+    return tuple(a[:n] for a in out)
 
 
 class Engine:
@@ -237,39 +287,10 @@ class Engine:
         (flat MOVE_DTYPE array, int32 offsets[n + 1]).  n_hist: per-leaf history slots (1..8, at most plies + 1), or
         None for min(8, plies + 1).  Returns predict()'s (moves, counts, priors, values), then the packed leaves
         (POSITION_DTYPE[n]) when `positions`; check=False puts the status code first instead of raising."""
-        if isinstance(stacks, tuple):
-            flat, off = stacks
-            flat = np.ascontiguousarray(flat, dtype=MOVE_DTYPE)
-            off = np.ascontiguousarray(off, dtype=np.int32)
-        else:
-            lens = [len(st) for st in stacks]
-            off = np.zeros(len(stacks) + 1, dtype=np.int32)
-            off[1:] = np.cumsum(lens)
-            flat = np.zeros(int(off[-1]), dtype=MOVE_DTYPE)
-            for st, b, ln in zip(stacks, off[:-1], lens):
-                if ln:
-                    a = np.asarray(st)
-                    if a.dtype == MOVE_DTYPE:
-                        flat[b : b + ln] = a
-                    else:
-                        a = a.reshape(ln, -1)
-                        for k, f in enumerate(("from", "to", "promo")):
-                            flat[f][b : b + ln] = a[:, k]
+        flat, off = _move_lists(stacks, "predict_stack")
         n = len(off) - 1
-        if n < 0:
-            raise SCError("predict_stack: offsets must hold n + 1 entries")
-        if n_hist is not None:
-            nh = np.asarray(n_hist)
-            if len(nh) != n or nh.min(initial=1) < -128 or nh.max(initial=1) > 127:
-                raise SCError("predict_stack: n_hist must hold one history length per leaf")
-            n_hist = np.ascontiguousarray(nh, dtype=np.int8)
-        if out is None:
-            out = (np.zeros((n, SC_MAX_MOVES), dtype=MOVE_DTYPE), np.zeros(n, dtype=np.int32),
-                   np.zeros((n, SC_MAX_MOVES), dtype=np.float32), np.zeros(n, dtype=np.float32))
-        for a, dt, shape in zip(out, (MOVE_DTYPE, np.int32, np.float32, np.float32), ((SC_MAX_MOVES,), (), (SC_MAX_MOVES,), ())):
-            if a.dtype != dt or a.shape[1:] != shape or len(a) < n or not a.flags.c_contiguous:
-                raise SCError("predict_stack: `out` must be (moves, counts, priors, values) arrays as predict() returns them")
-        moves, counts, priors, values = (a[:n] for a in out)
+        n_hist = _n_hist_arg(n_hist, n, "predict_stack")
+        moves, counts, priors, values = _predict_out(out, n, "predict_stack")
         pos = np.zeros(n, dtype=POSITION_DTYPE) if positions else None
         rc = load_library().sc_predict_stack(self._h, n, _ptr(flat) if len(flat) else None, _ptr(off), _ptr(n_hist),
                                              _ptr(pos), _ptr(moves), _ptr(counts), _ptr(priors), _ptr(values),
@@ -279,6 +300,42 @@ class Engine:
             return (rc,) + res
         _check(rc, "sc_predict_stack")
         return res
+
+    def set_roots(self, stacks):
+        """Stores root games on the device for predict_path() (sc_set_roots): stacks as predict_stack()'s.  Replaces
+        the previous roots; an empty list clears them."""
+        flat, off = _move_lists(stacks, "set_roots")
+        _check(load_library().sc_set_roots(self._h, len(off) - 1, _ptr(flat) if len(flat) else None, _ptr(off)),
+               "sc_set_roots")
+
+    def predict_path(self, root, paths, n_hist=None, out=None, positions: bool = False, stream: int = 0,
+                     check: bool = True):
+        """predict_stack() for leaves given as a stored root (an index into set_roots()' list) and the moves played
+        after it (sc_predict_path): leaf i is root[i]'s game followed by paths[i].  paths as predict_stack()'s stacks;
+        n_hist and the result as predict_stack()'s for the whole game."""
+        flat, off = _move_lists(paths, "predict_path")
+        n = len(off) - 1
+        r = np.asarray(root)
+        if r.shape != (n,) or r.min(initial=0) < -2**31 or r.max(initial=0) >= 2**31:
+            raise SCError("predict_path: root must hold one root index per leaf")
+        root = np.ascontiguousarray(r, dtype=np.int32)
+        n_hist = _n_hist_arg(n_hist, n, "predict_path")
+        moves, counts, priors, values = _predict_out(out, n, "predict_path")
+        pos = np.zeros(n, dtype=POSITION_DTYPE) if positions else None
+        rc = load_library().sc_predict_path(self._h, n, _ptr(root), _ptr(flat) if len(flat) else None, _ptr(off),
+                                            _ptr(n_hist), _ptr(pos), _ptr(moves), _ptr(counts), _ptr(priors),
+                                            _ptr(values), stream or None)
+        res = (moves, counts, priors, values) + ((pos,) if positions else ())
+        if not check:
+            return (rc,) + res
+        _check(rc, "sc_predict_path")
+        return res
+
+    def predict_path_timing(self) -> float:
+        """device time (ms) of the path-replay kernel of the last predict_path() (timing level >= 1)"""
+        ms = C.c_float()
+        _check(load_library().sc_predict_path_timing(self._h, C.byref(ms)), "sc_predict_path_timing")
+        return ms.value
 
     def predict_stack_timing(self) -> float:
         """device time (ms) of the replay kernel of the last predict_stack() (timing level >= 1)"""
