@@ -74,25 +74,22 @@ int upload_move_tables(cudaStream_t st);
 constexpr int PREDICT_OVERFLOW = -1;
 int launch_legal_moves(const sc_position *d_pos, const int8_t *d_ep, int n, sc_move *d_moves, int32_t *d_cnt,
                        int32_t *d_term, cudaStream_t st);
-// sc_predict_stack, one thread per leaf: replays leaf i's moves d_stack[d_off[i], d_off[i+1]) from the initial position
-// and packs it as host::pack_position does with d_n_hist[i] history slots (nullptr: min(SC_LOOKBACK, plies + 1)) into
-// d_pos[i], its python-chess ep_square into d_ep[i], and into d_status[i] 0 or REPLAY_STATUS(ply, reason) for the first
-// move it rejects (the leaf is then packed from the moves before that one).  d_scratch: replay_scratch_bytes(d_off[n] + n)
-// bytes, a record of every replayed position
+// the replay's statuses: 0, or REPLAY_STATUS(ply, reason) for the first move it rejects, ply counted from the game start
 enum { REPLAY_NOT_OURS = 1, REPLAY_BAD_TARGET, REPLAY_BAD_PROMO, REPLAY_NO_PROMO };
 __host__ __device__ constexpr int32_t REPLAY_STATUS(int ply, int reason) { return ply << 3 | reason; }
 size_t replay_scratch_bytes(int64_t positions);
-int launch_replay(const sc_move *d_stack, const int32_t *d_off, const int8_t *d_n_hist, int n, void *d_scratch,
-                  sc_position *d_pos, int8_t *d_ep, int32_t *d_status, cudaStream_t st);
-// sc_set_roots, one thread per root: replays root r's moves d_stack[d_off[r], d_off[r+1]) as launch_replay does and keeps
-// its records (replay_scratch_bytes(d_off[n] + n) bytes of d_rec in all), its final position in d_root_pos[r] and its
-// status in d_status[r]
+// sc_set_roots, one thread per root: replays root r's moves d_stack[d_off[r], d_off[r+1]) from the initial position and
+// keeps its records (replay_scratch_bytes(d_off[n] + n) bytes of d_rec in all), its final position in d_root_pos[r] and
+// its status in d_status[r]
 namespace chess { struct Position; }
 int launch_root_replay(const sc_move *d_stack, const int32_t *d_off, int n, void *d_rec, chess::Position *d_root_pos,
                        int32_t *d_status, cudaStream_t st);
-// sc_predict_path, one thread per leaf: leaf i continues root d_root[i] of the table above (d_root_off = the d_off it
-// was built from) with d_path[d_off[i], d_off[i+1]) and is packed as launch_replay packs the whole game; statuses name
-// plies from the game start.  d_scratch: replay_scratch_bytes(d_off[n] + n) bytes, the path's records
+// sc_predict_stack / sc_predict_path, one thread per leaf: leaf i starts from root d_root[i] of the table above
+// (d_root_off = the d_off it was built from), or from the initial position when d_root == nullptr (the table is then
+// not read), replays d_path[d_off[i], d_off[i+1]) and packs the game as host::pack_position does with d_n_hist[i]
+// history slots (nullptr: min(SC_LOOKBACK, plies + 1)) into d_pos[i], its python-chess ep_square into d_ep[i], and its
+// status into d_status[i] (after a rejected move the leaf is packed from the moves before it).  d_scratch:
+// replay_scratch_bytes(d_off[n] + n) bytes, the path's records
 int launch_path_replay(const void *d_root_rec, const int32_t *d_root_off, const chess::Position *d_root_pos,
                        const int32_t *d_root, const sc_move *d_path, const int32_t *d_off, const int8_t *d_n_hist, int n,
                        void *d_scratch, sc_position *d_pos, int8_t *d_ep, int32_t *d_status, cudaStream_t st);

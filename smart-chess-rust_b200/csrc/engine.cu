@@ -18,6 +18,7 @@
 
 #include "common.cuh"
 #include "host/chess_rules.hpp"
+#include "host/host_util.hpp"
 
 namespace scb {
 
@@ -966,20 +967,43 @@ static int predict_collect(sc_engine *e, const char *what, int n, sc_move *moves
     return SC_OK;
 }
 
-// sc_predict_stack and sc_predict_path once their replay kernel is queued on `st` (packed leaves in d_pos / d_pred_ep,
-// statuses in d_replay_status, timing events ev_replay_t around it): sc_predict's launches and the results.
-// game_plies(i): leaf i's moves from the initial position; replay_ms: where timing puts the replay kernel's time
-template <class GamePlies>
-static int predict_replayed(sc_engine *e, const char *what, int n, GamePlies game_plies, sc_position *pos_out,
-                            sc_move *moves_out, int32_t *move_cnt_out, float *priors_out, float *value_out,
-                            float *replay_ms, cudaStream_t st)
+// sc_predict_stack and sc_predict_path after their own argument checks: leaf i is stored root root[i] (root ==
+// nullptr: the initial position) followed by mv[off[i], off[i+1]).  The move lists' checks, the replay into d_pos /
+// d_pred_ep, sc_predict's launches and the results.  off_name / mv_name: the two arrays in messages; replay_ms: where
+// timing puts the replay kernel's time
+static int predict_replay(sc_engine *e, const char *what, int n, const int32_t *root, const sc_move *mv,
+                          const int32_t *off, const char *off_name, const char *mv_name, const int8_t *n_hist,
+                          sc_position *pos_out, sc_move *moves_out, int32_t *move_cnt_out, float *priors_out,
+                          float *value_out, float *replay_ms, void *stream)
 {
+    const int32_t *ro = e->root_off.data();
+    auto root_plies = [&](int i) { return root ? ro[root[i] + 1] - ro[root[i]] : 0; };
+    SCB_CHECK(check_move_lists(what, "leaf", off_name, mv_name, n, mv, off, n_hist, root_plies));
+    cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
+    SCB_CUDA(cudaSetDevice(e->device));
+    const int total = off[n];
+    SCB_CHECK(predict_stack_setup(e, (int64_t)total + n));
+    const void *d[4];
+    SCB_CHECK(stage_inputs(e, n,
+                           {{off, sizeof(int32_t) * ((size_t)n + 1), e->d_stack_off},
+                            {root, root ? sizeof(int32_t) * (size_t)n : 0, e->d_path_root},
+                            {mv, sizeof(sc_move) * (size_t)total, e->d_stack},
+                            {n_hist, n_hist ? (size_t)n : 0, e->d_stack_nhist}},
+                           d, st));
+    // the packed leaves and their ep squares go where sc_predict's kernels read them on the device
+    if (e->timing) SCB_CUDA(cudaEventRecord(e->ev_replay_t[0], st));
+    SCB_CHECK(launch_path_replay(e->d_root_rec, e->d_root_off, e->d_root_pos, static_cast<const int32_t *>(d[1]),
+                                 static_cast<const sc_move *>(d[2]), static_cast<const int32_t *>(d[0]),
+                                 static_cast<const int8_t *>(d[3]), n, e->d_replay_scratch, e->d_pos, e->d_pred_ep,
+                                 e->d_replay_status, st));
+    if (e->timing) SCB_CUDA(cudaEventRecord(e->ev_replay_t[1], st));
+    e->launches += 1;
     SCB_CHECK(predict_launch(e, n, e->d_pos, e->d_pred_ep, priors_out, value_out, st));
     SCB_CUDA(cudaMemcpyAsync(e->h_replay_status, e->d_replay_status, sizeof(int32_t) * (size_t)n, cudaMemcpyDeviceToHost, st));
     if (pos_out) SCB_CUDA(cudaMemcpyAsync(pos_out, e->d_pos, sizeof(sc_position) * (size_t)n, cudaMemcpyDeviceToHost, st));
     // the side to move of a leaf replayed from the initial position: White after an even number of plies
     const int32_t *status = e->h_replay_status;
-    auto plies = [&](int i) { return status[i] ? status[i] >> 3 : game_plies(i); };
+    auto plies = [&](int i) { return status[i] ? status[i] >> 3 : root_plies(i) + off[i + 1] - off[i]; };
     const int rc = predict_collect(e, what, n, moves_out, move_cnt_out, priors_out, value_out, st,
                                    [&](int i) { return plies(i) % 2 == 0; });
     if (rc != SC_OK && rc != SC_E_INVAL) return rc;
@@ -1295,28 +1319,9 @@ int sc_predict_stack(sc_engine *e, int n, const sc_move *stack, const int32_t *s
         return SC_E_INVAL;
     }
     if (n == 0) return SC_OK;
-    SCB_CHECK(check_move_lists("sc_predict_stack", "leaf", "stack_off", "stack", n, stack, stack_off, n_hist,
-                               [](int) { return 0; }));
     NvtxRange nv_call("sc_predict_stack");
-    cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
-    SCB_CUDA(cudaSetDevice(e->device));
-    const int total = stack_off[n];
-    SCB_CHECK(predict_stack_setup(e, (int64_t)total + n));
-    const void *d[3];
-    SCB_CHECK(stage_inputs(e, n,
-                           {{stack_off, sizeof(int32_t) * ((size_t)n + 1), e->d_stack_off},
-                            {stack, sizeof(sc_move) * (size_t)total, e->d_stack},
-                            {n_hist, n_hist ? (size_t)n : 0, e->d_stack_nhist}},
-                           d, st));
-    // the packed leaves and their ep squares go where sc_predict's kernels read them on the device
-    if (e->timing) SCB_CUDA(cudaEventRecord(e->ev_replay_t[0], st));
-    SCB_CHECK(launch_replay(static_cast<const sc_move *>(d[1]), static_cast<const int32_t *>(d[0]),
-                            static_cast<const int8_t *>(d[2]), n, e->d_replay_scratch, e->d_pos, e->d_pred_ep,
-                            e->d_replay_status, st));
-    if (e->timing) SCB_CUDA(cudaEventRecord(e->ev_replay_t[1], st));
-    e->launches += 1;
-    return predict_replayed(e, "sc_predict_stack", n, [&](int i) { return stack_off[i + 1] - stack_off[i]; }, pos_out,
-                            moves_out, move_cnt_out, priors_out, value_out, &e->last_replay_ms, st);
+    return predict_replay(e, "sc_predict_stack", n, nullptr, stack, stack_off, "stack_off", "stack", n_hist, pos_out,
+                          moves_out, move_cnt_out, priors_out, value_out, &e->last_replay_ms, stream);
 }
 
 int sc_set_roots(sc_engine *e, int n_roots, const sc_move *stack, const int32_t *stack_off)
@@ -1376,30 +1381,9 @@ int sc_predict_path(sc_engine *e, int n, const int32_t *root, const sc_move *pat
             return SC_E_INVAL;
         }
     }
-    const int32_t *ro = e->root_off.data();
-    auto root_plies = [&](int i) { return ro[root[i] + 1] - ro[root[i]]; };
-    SCB_CHECK(check_move_lists("sc_predict_path", "leaf", "path_off", "path", n, path, path_off, n_hist, root_plies));
     NvtxRange nv_call("sc_predict_path");
-    cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
-    SCB_CUDA(cudaSetDevice(e->device));
-    const int total = path_off[n];
-    SCB_CHECK(predict_stack_setup(e, (int64_t)total + n));
-    const void *d[4];
-    SCB_CHECK(stage_inputs(e, n,
-                           {{path_off, sizeof(int32_t) * ((size_t)n + 1), e->d_stack_off},
-                            {root, sizeof(int32_t) * (size_t)n, e->d_path_root},
-                            {path, sizeof(sc_move) * (size_t)total, e->d_stack},
-                            {n_hist, n_hist ? (size_t)n : 0, e->d_stack_nhist}},
-                           d, st));
-    if (e->timing) SCB_CUDA(cudaEventRecord(e->ev_replay_t[0], st));
-    SCB_CHECK(launch_path_replay(e->d_root_rec, e->d_root_off, e->d_root_pos, static_cast<const int32_t *>(d[1]),
-                                 static_cast<const sc_move *>(d[2]), static_cast<const int32_t *>(d[0]),
-                                 static_cast<const int8_t *>(d[3]), n, e->d_replay_scratch, e->d_pos, e->d_pred_ep,
-                                 e->d_replay_status, st));
-    if (e->timing) SCB_CUDA(cudaEventRecord(e->ev_replay_t[1], st));
-    e->launches += 1;
-    return predict_replayed(e, "sc_predict_path", n, [&](int i) { return root_plies(i) + path_off[i + 1] - path_off[i]; },
-                            pos_out, moves_out, move_cnt_out, priors_out, value_out, &e->last_path_ms, st);
+    return predict_replay(e, "sc_predict_path", n, root, path, path_off, "path_off", "path", n_hist, pos_out,
+                          moves_out, move_cnt_out, priors_out, value_out, &e->last_path_ms, stream);
 }
 
 int sc_eval_submit(sc_engine *e, int n, const sc_position *pos, const sc_move *moves_strided, const int32_t *move_cnt,
@@ -1592,24 +1576,7 @@ int sc_encode_steps(sc_engine *e, int n, const sc_move *played, const sc_move *c
             return SC_E_INVAL;
         }
         // the packed leaf of ply i: full history back to the start (BoardHistory of lib.rs:52, capacity 8)
-        sc_position &p = pos[i];
-        memset(&p, 0, sizeof(p));
-        int nh = std::min(SC_LOOKBACK, g.ply() + 1);
-        for (int t = 0; t < nh; t++) {
-            const chess::Position &q = g.pos_at(g.ply() - t);
-            for (int c = 0; c < 6; c++) p.slot[t][c] = q.pt[c + 1];
-            p.slot[t][6] = q.occ[chess::WHITE];
-            p.slot[t][7] = g.rep_at(g.ply() - t);
-        }
-        const chess::Position &c = g.cur;
-        p.meta[0] = c.turn;
-        p.meta[1] = c.fullmove;
-        p.meta[2] = c.has_kingside(c.turn);
-        p.meta[3] = c.has_queenside(c.turn);
-        p.meta[4] = c.has_kingside(!c.turn);
-        p.meta[5] = c.has_queenside(!c.turn);
-        p.meta[6] = c.halfmove;
-        p.n_hist = nh;
+        host::pack_position(g, SC_LOOKBACK, &pos[i]);
         for (int j = 0; j < l.n; j++) legal.push_back(sc_move{l.m[j].from, l.m[j].to, l.m[j].promo, 0});
         loff[i + 1] = (int32_t)legal.size();
         g.push(mv);

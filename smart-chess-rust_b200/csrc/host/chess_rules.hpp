@@ -617,8 +617,8 @@ struct Position {
     };
     // the legal moves in python-chess order into `out`; returns the number of pseudo-legal candidates they were
     // filtered from (never fewer than the legal moves)
-    // always inlined on the device: has_legal_ep's instance is reached from the three replay kernels of movegen.cu
-    // (through tkey), and left a call it caps each of them at 96 registers with spills
+    // always inlined on the device: has_legal_ep's instance is reached from both replay kernels of movegen.cu (through
+    // tkey), and left a call it costs the leaf replay kernel 64 B of spill stores
     template <class Sink> SCB_HD_DEVICE_INLINE int gen_legal(Sink &out) const
     {
         const int king = king_sq(turn);

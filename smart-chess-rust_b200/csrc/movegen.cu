@@ -79,15 +79,9 @@ template <class Records> struct PlyHistory : Records {
     __device__ bool irreversible(int k) const { return this->at(k).irreversible != 0; }
 };
 
-// one game replayed from the initial position: ply[k] = the position after k moves
-struct GameRecords {
-    const ReplayPly *ply;
-    __device__ const ReplayPly &at(int k) const { return ply[k]; }
-};
-using ReplayHistory = PlyHistory<GameRecords>;
-
 // a stored root of `root_plies` moves, then the leaf's path: the root's records up to its last move, the path's
-// (path[0] = the root's final position, recorded again by the path replay) from there on
+// (path[0] = the root's final position, recorded again by the path replay) from there on.  A path from the initial
+// position has root_plies = 0 and reads path[] alone
 struct RootPathRecords {
     const ReplayPly *root, *path;
     int root_plies;
@@ -155,26 +149,6 @@ __device__ __forceinline__ void pack_replayed(const History &h, const chess::Pos
 
 constexpr int REPLAY_THREADS = 32;
 
-__global__ void __launch_bounds__(REPLAY_THREADS) replay_kernel(const sc_move *__restrict__ stack,
-                                                                const int32_t *__restrict__ off,
-                                                                const int8_t *__restrict__ n_hist, int n,
-                                                                ReplayPly *__restrict__ scratch,
-                                                                sc_position *__restrict__ pos, int8_t *__restrict__ ep,
-                                                                int32_t *__restrict__ status)
-{
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    const int base = off[i];
-    ReplayPly *h = scratch + base + i;  // plies + 1 positions per leaf
-    int len = off[i + 1] - base;
-    chess::Position p;
-    p.set_start();
-    const int st = replay_moves(p, stack + base, len, h, 0);
-    pack_replayed(ReplayHistory{{h}}, p, len, n_hist ? n_hist[i] : SC_LOOKBACK, pos[i]);
-    ep[i] = (int8_t)p.ep;
-    status[i] = st;
-}
-
 // sc_set_roots, one thread per root: root r's records (plies + 1) at rec + off[r] + r, its final position and status
 __global__ void __launch_bounds__(REPLAY_THREADS) root_replay_kernel(const sc_move *__restrict__ stack,
                                                                      const int32_t *__restrict__ off, int n,
@@ -192,8 +166,9 @@ __global__ void __launch_bounds__(REPLAY_THREADS) root_replay_kernel(const sc_mo
     root_pos[r] = p;
 }
 
-// sc_predict_path, one thread per leaf: root[i]'s stored position continued with path[off[i], off[i+1]) (records in
-// the per-call scratch), packed over the root's records and the path's
+// sc_predict_stack / sc_predict_path, one thread per leaf: root[i]'s stored position (root == nullptr: the initial
+// position) continued with path[off[i], off[i+1]) (records in the per-call scratch), packed over the root's records
+// and the path's
 __global__ void __launch_bounds__(REPLAY_THREADS) path_replay_kernel(
     const ReplayPly *__restrict__ root_rec, const int32_t *__restrict__ root_off,
     const chess::Position *__restrict__ root_pos, const int32_t *__restrict__ root, const sc_move *__restrict__ path,
@@ -202,28 +177,27 @@ __global__ void __launch_bounds__(REPLAY_THREADS) path_replay_kernel(
 {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    const int r = root[i], root_base = root_off[r], root_plies = root_off[r + 1] - root_base;
     const int base = off[i];
-    ReplayPly *h = scratch + base + i;
+    ReplayPly *h = scratch + base + i;  // plies + 1 positions per leaf
     int len = off[i + 1] - base;
-    chess::Position p = root_pos[r];
+    chess::Position p;
+    const ReplayPly *rh = nullptr;
+    int root_plies = 0;
+    if (root) {
+        const int r = root[i], root_base = root_off[r];
+        root_plies = root_off[r + 1] - root_base;
+        rh = root_rec + root_base + r;
+        p = root_pos[r];
+    } else {
+        p.set_start();
+    }
     status[i] = replay_moves(p, path + base, len, h, root_plies);
     ep[i] = (int8_t)p.ep;
-    const PathHistory ph{{root_rec + root_base + r, h, root_plies}};
+    const PathHistory ph{{rh, h, root_plies}};
     pack_replayed(ph, p, root_plies + len, n_hist ? n_hist[i] : SC_LOOKBACK, pos[i]);
 }
 
 size_t replay_scratch_bytes(int64_t positions) { return sizeof(ReplayPly) * (size_t)positions; }
-
-int launch_replay(const sc_move *d_stack, const int32_t *d_off, const int8_t *d_n_hist, int n, void *d_scratch,
-                  sc_position *d_pos, int8_t *d_ep, int32_t *d_status, cudaStream_t st)
-{
-    if (n <= 0) return SC_OK;
-    replay_kernel<<<(n + REPLAY_THREADS - 1) / REPLAY_THREADS, REPLAY_THREADS, 0, st>>>(
-        d_stack, d_off, d_n_hist, n, static_cast<ReplayPly *>(d_scratch), d_pos, d_ep, d_status);
-    SCB_CUDA(cudaGetLastError());
-    return SC_OK;
-}
 
 int launch_root_replay(const sc_move *d_stack, const int32_t *d_off, int n, void *d_rec, chess::Position *d_root_pos,
                        int32_t *d_status, cudaStream_t st)

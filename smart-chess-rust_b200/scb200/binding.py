@@ -266,13 +266,7 @@ class Engine:
             if len(ep) != n or ep.min(initial=-1) < -128 or ep.max(initial=-1) > 127:
                 raise SCError("predict: ep_square must hold one square (or -1) per leaf")
             ep_square = np.ascontiguousarray(ep, dtype=np.int8)
-        if out is None:
-            out = (np.zeros((n, SC_MAX_MOVES), dtype=MOVE_DTYPE), np.zeros(n, dtype=np.int32),
-                   np.zeros((n, SC_MAX_MOVES), dtype=np.float32), np.zeros(n, dtype=np.float32))
-        for a, dt, shape in zip(out, (MOVE_DTYPE, np.int32, np.float32, np.float32), ((SC_MAX_MOVES,), (), (SC_MAX_MOVES,), ())):
-            if a.dtype != dt or a.shape[1:] != shape or len(a) < n or not a.flags.c_contiguous:
-                raise SCError("predict: `out` must be (moves, counts, priors, values) arrays as predict() returns them")
-        moves, counts, priors, values = (a[:n] for a in out)
+        moves, counts, priors, values = _predict_out(out, n, "predict")
         rc = load_library().sc_predict(self._h, n, _ptr(positions), _ptr(ep_square), _ptr(moves), _ptr(counts),
                                        _ptr(priors), _ptr(values), stream or None)
         if not check:
@@ -287,19 +281,7 @@ class Engine:
         (flat MOVE_DTYPE array, int32 offsets[n + 1]).  n_hist: per-leaf history slots (1..8, at most plies + 1), or
         None for min(8, plies + 1).  Returns predict()'s (moves, counts, priors, values), then the packed leaves
         (POSITION_DTYPE[n]) when `positions`; check=False puts the status code first instead of raising."""
-        flat, off = _move_lists(stacks, "predict_stack")
-        n = len(off) - 1
-        n_hist = _n_hist_arg(n_hist, n, "predict_stack")
-        moves, counts, priors, values = _predict_out(out, n, "predict_stack")
-        pos = np.zeros(n, dtype=POSITION_DTYPE) if positions else None
-        rc = load_library().sc_predict_stack(self._h, n, _ptr(flat) if len(flat) else None, _ptr(off), _ptr(n_hist),
-                                             _ptr(pos), _ptr(moves), _ptr(counts), _ptr(priors), _ptr(values),
-                                             stream or None)
-        res = (moves, counts, priors, values) + ((pos,) if positions else ())
-        if not check:
-            return (rc,) + res
-        _check(rc, "sc_predict_stack")
-        return res
+        return self._predict_moves(None, stacks, n_hist, out, positions, stream, check)
 
     def set_roots(self, stacks):
         """Stores root games on the device for predict_path() (sc_set_roots): stacks as predict_stack()'s.  Replaces
@@ -313,22 +295,28 @@ class Engine:
         """predict_stack() for leaves given as a stored root (an index into set_roots()' list) and the moves played
         after it (sc_predict_path): leaf i is root[i]'s game followed by paths[i].  paths as predict_stack()'s stacks;
         n_hist and the result as predict_stack()'s for the whole game."""
-        flat, off = _move_lists(paths, "predict_path")
+        return self._predict_moves(np.asarray(root), paths, n_hist, out, positions, stream, check)
+
+    def _predict_moves(self, root, lists, n_hist, out, positions, stream, check):
+        """predict_stack() (root None) and predict_path() (root: its root argument as an array)"""
+        what = "predict_stack" if root is None else "predict_path"
+        flat, off = _move_lists(lists, what)
         n = len(off) - 1
-        r = np.asarray(root)
-        if r.shape != (n,) or r.min(initial=0) < -2**31 or r.max(initial=0) >= 2**31:
-            raise SCError("predict_path: root must hold one root index per leaf")
-        root = np.ascontiguousarray(r, dtype=np.int32)
-        n_hist = _n_hist_arg(n_hist, n, "predict_path")
-        moves, counts, priors, values = _predict_out(out, n, "predict_path")
+        fn, lead = load_library().sc_predict_stack, ()
+        if root is not None:
+            if root.shape != (n,) or root.min(initial=0) < -2**31 or root.max(initial=0) >= 2**31:
+                raise SCError("predict_path: root must hold one root index per leaf")
+            root = np.ascontiguousarray(root, dtype=np.int32)
+            fn, lead = load_library().sc_predict_path, (_ptr(root),)
+        n_hist = _n_hist_arg(n_hist, n, what)
+        moves, counts, priors, values = _predict_out(out, n, what)
         pos = np.zeros(n, dtype=POSITION_DTYPE) if positions else None
-        rc = load_library().sc_predict_path(self._h, n, _ptr(root), _ptr(flat) if len(flat) else None, _ptr(off),
-                                            _ptr(n_hist), _ptr(pos), _ptr(moves), _ptr(counts), _ptr(priors),
-                                            _ptr(values), stream or None)
+        rc = fn(self._h, n, *lead, _ptr(flat) if len(flat) else None, _ptr(off), _ptr(n_hist), _ptr(pos), _ptr(moves),
+                _ptr(counts), _ptr(priors), _ptr(values), stream or None)
         res = (moves, counts, priors, values) + ((pos,) if positions else ())
         if not check:
             return (rc,) + res
-        _check(rc, "sc_predict_path")
+        _check(rc, "sc_" + what)
         return res
 
     def predict_path_timing(self) -> float:
