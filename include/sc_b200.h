@@ -10,7 +10,8 @@
  *
  * Threading: a handle is single-threaded like the reference backends (src/game.rs takes
  * &self but every backend is !Sync in practice: RefCell at src/backends/onnx.rs:9-11).
- * Use one handle per worker thread / per GPU.
+ * Use one handle per worker thread / per GPU, or share one engine between many game threads through the
+ * batching evaluator below, whose calls may come from any thread.
  */
 #ifndef SC_B200_H
 #define SC_B200_H
@@ -148,6 +149,49 @@ int sc_set_roots(sc_engine *e, int n_roots, const sc_move *stack, const int32_t 
 int sc_predict_path(sc_engine *e, int n, const int32_t *root, const sc_move *path, const int32_t *path_off,
                     const int8_t *n_hist, sc_position *pos_out, sc_move *moves_out, int32_t *move_cnt_out,
                     float *priors_out, float *value_out, void *stream);
+
+/* -------- batching evaluator: many host threads, each running one game's sequential search through the one-leaf
+ * interface (src/game.rs:3-15), share one engine.  Each call carries one leaf or one root update and blocks until it is
+ * done; one dispatcher thread takes every request pending when the device becomes free (up to max_batch leaves),
+ * applies the pending root updates in one launch, then evaluates the leaves as one sc_predict_path-style pass and wakes
+ * the callers.  Requests that arrive during a pass wait for the next one, so a lone caller sees about the latency of
+ * one sc_predict_path(n = 1) call and the batches grow with the number of callers.  There is no timer and no setting.
+ * Every game keeps its own root slot, 0 <= slot < n_slots, in a device table of its own: sc_set_roots' table is not
+ * touched.  The evaluator is the only user of the engine's stream while it lives: every other call on the engine
+ * that uses the device (sc_eval*, sc_predict*, sc_set_roots, sc_encode_*, sc_forward_only, sc_debug_tower,
+ * sc_set_timing, sc_destroy) returns SC_E_STATE until sc_evaluator_destroy.  All evaluator calls but create and
+ * destroy may come from any thread; error messages go to the calling thread's sc_last_error. */
+typedef struct sc_evaluator sc_evaluator;
+/* 1 <= n_slots <= max_batch; every slot starts empty.  SC_E_STATE if the engine already has an evaluator */
+int sc_evaluator_create(sc_engine *e, int n_slots, sc_evaluator **out);
+/* Fails the requests still waiting with SC_E_STATE (a pass already running completes), waits until their callers have
+ * returned and gives the engine back.  Not concurrent with other calls on `ev` made after it started. */
+int sc_evaluator_destroy(sc_evaluator *ev);
+/* Stores stack[0, len) (a game from the initial position, as sc_predict_stack's stacks) as slot's root, replayed on
+ * the device; extend_root appends moves[0, len) to the slot's stored game and replays only those, from the stored
+ * position.  Returns once the slot is updated; the update is ordered before every later predict on the slot.  Updates
+ * of several slots pending at once share one launch, and other slots are left untouched.  SC_E_INVAL before any
+ * launch and with the slot left as it was: a bad slot, len < 0, a NULL array with len > 0, a game longer than
+ * SC_MAX_STACK in all, bad move fields (sc_set_roots' checks).  SC_E_STATE: extend_root of an empty slot.  A replay-time
+ * rejection returns SC_E_INVAL naming the slot and the ply (counted from the initial position) and leaves the slot
+ * empty. */
+int sc_evaluator_set_root(sc_evaluator *ev, int slot, const sc_move *stack, int len);
+int sc_evaluator_extend_root(sc_evaluator *ev, int slot, const sc_move *moves, int len);
+/* One leaf: slot's root followed by path[0, len), with n_hist history slots (0 = min(8, total length + 1)).  Outputs,
+ * status and messages are those of sc_predict_path for that leaf against the slot's root (moves_out / priors_out hold
+ * SC_MAX_MOVES entries, the first *move_cnt_out of them valid; pos_out may be NULL), whichever other leaves share its
+ * pass; the messages name the slot instead of a leaf index.  A rejected leaf fails its own call only.  SC_E_STATE: the
+ * slot is empty, or the evaluator is being destroyed. */
+int sc_evaluator_predict(sc_evaluator *ev, int slot, const sc_move *path, int len, int n_hist, sc_position *pos_out,
+                         sc_move *moves_out, int32_t *move_cnt_out, float *priors_out, float *value_out);
+typedef struct sc_evaluator_counts {
+    int64_t passes;        /* dispatcher passes that evaluated leaves */
+    int64_t leaves;        /* leaves evaluated (rejected ones included) */
+    int64_t largest_batch; /* most leaves in one pass */
+    int64_t root_updates;  /* set_root / extend_root calls applied */
+    double wait_seconds;   /* summed over predict calls: time from submission to the result */
+} sc_evaluator_counts;
+int sc_evaluator_stats(sc_evaluator *ev, sc_evaluator_counts *out);
 
 /* asynchronous form of sc_eval for double-buffered callers: submit returns as soon as the work is
  * queued on `stream` (host buffers must be pinned and stay untouched until the wait returns);
@@ -290,6 +334,15 @@ int sc_selfplay_destroy(sc_selfplay *sp);
  * temperature_switch, temperature, seed, evaluator of `cfg`.  Writes the trace (format above) to `buf`;
  * returns the bytes needed including the NUL, or -1 (sc_last_error). */
 int64_t sc_game_selfplay(sc_engine *e, const sc_selfplay_config *cfg, char *buf, int64_t cap);
+
+/* sc_game_selfplay for n_games games at once, game i with seed seeds[i], each on its own host thread, all predicting
+ * through one evaluator of n_games slots on `e` (cfg->evaluator = 0; n_games <= max_batch) or through the position-hash
+ * stand-in (cfg->evaluator = 1, e unused).  Each game owns one slot: before every search it extends the slot by the
+ * moves played since, and its leaves pass only the moves below the search root.  Game i's trace goes to
+ * buf + i * cap (at most cap bytes with the NUL; buf may be NULL), the bytes it needs to sizes[i].  counts_out (may be
+ * NULL): the evaluator's sc_evaluator_stats at the end.  Returns SC_OK, or the first game's error (sc_last_error). */
+int sc_game_selfplay_many(sc_engine *e, const sc_selfplay_config *cfg, int n_games, const uint64_t *seeds, char *buf,
+                          int64_t cap, int64_t *sizes, sc_evaluator_counts *counts_out);
 
 /* ---- arena: two networks play each other (the `play` binary with --black-type nn, src/play.rs:241-343,
  * and scripts/leader-board).  Both players share one configuration, as the reference's CLI does

@@ -84,15 +84,24 @@ size_t replay_scratch_bytes(int64_t positions);
 namespace chess { struct Position; }
 int launch_root_replay(const sc_move *d_stack, const int32_t *d_off, int n, void *d_rec, chess::Position *d_root_pos,
                        int32_t *d_status, cudaStream_t st);
-// sc_predict_stack / sc_predict_path, one thread per leaf: leaf i starts from root d_root[i] of the table above
-// (d_root_off = the d_off it was built from), or from the initial position when d_root == nullptr (the table is then
-// not read), replays d_path[d_off[i], d_off[i+1]) and packs the game as host::pack_position does with d_n_hist[i]
+// an evaluator's slot table: slot g's records at d_rec + replay_scratch_bytes(g * (SC_MAX_STACK + 1)), its final
+// position in d_slot_pos[g] and its plies in d_slot_plies[g].  One thread per update u: replays d_stack[d_off[u],
+// d_off[u+1]) into slot d_slot[u], from the initial position or (d_append[u] != 0) from the slot's stored position,
+// appending to its records; the status into d_status[u].  The caller keeps the plies within SC_MAX_STACK
+int launch_slot_replay(const sc_move *d_stack, const int32_t *d_off, const int32_t *d_slot, const int8_t *d_append,
+                       int n, void *d_rec, chess::Position *d_slot_pos, int32_t *d_slot_plies, int32_t *d_status,
+                       cudaStream_t st);
+// sc_predict_stack / sc_predict_path / an evaluator's leaves, one thread per leaf: leaf i starts from root d_root[i] of
+// the sc_set_roots table above (d_root_off = the d_off it was built from), or of a slot table when d_slot_plies is
+// given (d_root_rec / d_root_pos: its records and positions), or from the initial position when d_root == nullptr (no
+// table is then read), replays d_path[d_off[i], d_off[i+1]) and packs the game as host::pack_position does with d_n_hist[i]
 // history slots (nullptr: min(SC_LOOKBACK, plies + 1)) into d_pos[i], its python-chess ep_square into d_ep[i], and its
 // status into d_status[i] (after a rejected move the leaf is packed from the moves before it).  d_scratch:
 // replay_scratch_bytes(d_off[n] + n) bytes, the path's records
-int launch_path_replay(const void *d_root_rec, const int32_t *d_root_off, const chess::Position *d_root_pos,
-                       const int32_t *d_root, const sc_move *d_path, const int32_t *d_off, const int8_t *d_n_hist, int n,
-                       void *d_scratch, sc_position *d_pos, int8_t *d_ep, int32_t *d_status, cudaStream_t st);
+int launch_path_replay(const void *d_root_rec, const int32_t *d_root_off, const int32_t *d_slot_plies,
+                       const chess::Position *d_root_pos, const int32_t *d_root, const sc_move *d_path,
+                       const int32_t *d_off, const int8_t *d_n_hist, int n, void *d_scratch, sc_position *d_pos,
+                       int8_t *d_ep, int32_t *d_status, cudaStream_t st);
 
 // ---- tower_f32.cu -------------------------------------------------------------------------
 // C[M][N] = gather_taps(A)[M][TAPS*K] * W[TAPS*K][ldw] + bias ; A is [rows][lda] fp32

@@ -4,6 +4,7 @@
 // for n leaves at once: H2D of the packed positions and legal moves, plane encode, the
 // policy/value network, move-index gather + renormalisation, D2H of priors and values.
 // There is no CPU fallback: without an sm_100 device sc_create() fails with SC_E_NOGPU.
+#include <atomic>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -18,6 +19,7 @@
 
 #include "common.cuh"
 #include "host/chess_rules.hpp"
+#include "host/evaluator.hpp"
 #include "host/host_util.hpp"
 
 namespace scb {
@@ -268,6 +270,8 @@ struct sc_engine {
     std::vector<int32_t> root_off;
     int n_roots = 0;
     float last_path_ms = 0.f;  // timing: the path-replay kernel (between ev_replay_t)
+    // an sc_evaluator owns the stream: every other call that uses the device returns SC_E_STATE
+    std::atomic<bool> evaluator{false};
 };
 
 namespace scb {
@@ -817,10 +821,10 @@ static int stage_inputs(sc_engine *e, int n, std::initializer_list<StagedInput> 
 // the host-side checks of n move lists (sc_predict_stack's stacks, sc_set_roots' roots, sc_predict_path's paths), before
 // any launch: offsets off[0..n] from 0 and not decreasing, the game of list i -- base(i) plies stored before it, then its
 // own -- at most SC_MAX_STACK plies, n_hist[i] (if given) in 1..min(SC_LOOKBACK, game plies + 1), every move's fields.
-// `unit` names a list in the messages, `off_name` / `mv_name` the two arrays
+// `unit` names a list in the messages (list i as number first + i), `off_name` / `mv_name` the two arrays
 template <class Base>
 static int check_move_lists(const char *what, const char *unit, const char *off_name, const char *mv_name, int n,
-                            const sc_move *mv, const int32_t *off, const int8_t *n_hist, Base base)
+                            const sc_move *mv, const int32_t *off, const int8_t *n_hist, Base base, int first = 0)
 {
     const std::string w = std::string(what) + ": ";
     if (off[0] != 0) {
@@ -830,11 +834,11 @@ static int check_move_lists(const char *what, const char *unit, const char *off_
     for (int i = 0; i < n; i++) {
         const int64_t own = (int64_t)off[i + 1] - off[i], len = base(i) + own;
         if (own < 0) {
-            set_error(w + off_name + " decreases at " + unit + " " + std::to_string(i));
+            set_error(w + off_name + " decreases at " + unit + " " + std::to_string(first + i));
             return SC_E_INVAL;
         }
         if (len > SC_MAX_STACK) {
-            set_error(w + unit + " " + std::to_string(i) + " has " + std::to_string(len) +
+            set_error(w + unit + " " + std::to_string(first + i) + " has " + std::to_string(len) +
                       " plies, more than SC_MAX_STACK = " + std::to_string(SC_MAX_STACK));
             return SC_E_INVAL;
         }
@@ -869,6 +873,30 @@ static const char *replay_reason(int32_t status)
                                 "it promotes a piece that is not a pawn reaching the last rank",
                                 "a pawn reaches the last rank without a promotion"};
     return why[status & 7];
+}
+
+// the message of a rejected replay: "<what>: <unit> <index>, ply <ply>: move rejected, <reason>"
+static std::string replay_error(const char *what, const char *unit, int index, int ply, int32_t status)
+{
+    return std::string(what) + ": " + unit + " " + std::to_string(index) + ", ply " + std::to_string(ply) +
+           ": move rejected, " + replay_reason(status);
+}
+
+// an evaluator's root slots (engine_backend_create): per slot SC_MAX_STACK + 1 replay records, the final position and
+// the plies on the device, and the plies on the host (-1: the slot has no root)
+struct SlotTable {
+    void *d_rec = nullptr;
+    chess::Position *d_pos = nullptr;
+    int32_t *d_plies = nullptr;
+    std::vector<int32_t> plies;
+};
+
+// SC_E_STATE while an evaluator owns the engine
+static int check_owner(const sc_engine *e, const char *what)
+{
+    if (!e || !e->evaluator) return SC_OK;
+    set_error(std::string(what) + ": the engine belongs to an evaluator until sc_evaluator_destroy");
+    return SC_E_STATE;
 }
 
 static int finish_timing(sc_engine *e, cudaStream_t st)
@@ -967,17 +995,20 @@ static int predict_collect(sc_engine *e, const char *what, int n, sc_move *moves
     return SC_OK;
 }
 
-// sc_predict_stack and sc_predict_path after their own argument checks: leaf i is stored root root[i] (root ==
-// nullptr: the initial position) followed by mv[off[i], off[i+1]).  The move lists' checks, the replay into d_pos /
+// sc_predict_stack, sc_predict_path and an evaluator's pass after their own argument checks: leaf i is root root[i]
+// of sc_set_roots' table or, with `slots`, of that slot table (root == nullptr: the initial position) followed by
+// mv[off[i], off[i+1]).  The move lists' checks, the replay into d_pos /
 // d_pred_ep, sc_predict's launches and the results.  off_name / mv_name: the two arrays in messages; replay_ms: where
 // timing puts the replay kernel's time
-static int predict_replay(sc_engine *e, const char *what, int n, const int32_t *root, const sc_move *mv,
-                          const int32_t *off, const char *off_name, const char *mv_name, const int8_t *n_hist,
-                          sc_position *pos_out, sc_move *moves_out, int32_t *move_cnt_out, float *priors_out,
-                          float *value_out, float *replay_ms, void *stream)
+static int predict_replay(sc_engine *e, const char *what, int n, const int32_t *root, const SlotTable *slots,
+                          const sc_move *mv, const int32_t *off, const char *off_name, const char *mv_name,
+                          const int8_t *n_hist, sc_position *pos_out, sc_move *moves_out, int32_t *move_cnt_out,
+                          float *priors_out, float *value_out, float *replay_ms, void *stream)
 {
     const int32_t *ro = e->root_off.data();
-    auto root_plies = [&](int i) { return root ? ro[root[i] + 1] - ro[root[i]] : 0; };
+    auto root_plies = [&](int i) {
+        return !root ? 0 : slots ? slots->plies[root[i]] : ro[root[i] + 1] - ro[root[i]];
+    };
     SCB_CHECK(check_move_lists(what, "leaf", off_name, mv_name, n, mv, off, n_hist, root_plies));
     cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
     SCB_CUDA(cudaSetDevice(e->device));
@@ -992,7 +1023,8 @@ static int predict_replay(sc_engine *e, const char *what, int n, const int32_t *
                            d, st));
     // the packed leaves and their ep squares go where sc_predict's kernels read them on the device
     if (e->timing) SCB_CUDA(cudaEventRecord(e->ev_replay_t[0], st));
-    SCB_CHECK(launch_path_replay(e->d_root_rec, e->d_root_off, e->d_root_pos, static_cast<const int32_t *>(d[1]),
+    SCB_CHECK(launch_path_replay(slots ? slots->d_rec : e->d_root_rec, e->d_root_off, slots ? slots->d_plies : nullptr,
+                                 slots ? slots->d_pos : e->d_root_pos, static_cast<const int32_t *>(d[1]),
                                  static_cast<const sc_move *>(d[2]), static_cast<const int32_t *>(d[0]),
                                  static_cast<const int8_t *>(d[3]), n, e->d_replay_scratch, e->d_pos, e->d_pred_ep,
                                  e->d_replay_status, st));
@@ -1010,11 +1042,218 @@ static int predict_replay(sc_engine *e, const char *what, int n, const int32_t *
     if (e->timing) SCB_CUDA(cudaEventElapsedTime(replay_ms, e->ev_replay_t[0], e->ev_replay_t[1]));
     for (int i = 0; i < n; i++) {
         if (!status[i]) continue;
-        set_error(std::string(what) + ": leaf " + std::to_string(i) + ", ply " + std::to_string(plies(i)) +
-                  ": move rejected, " + replay_reason(status[i]));
+        set_error(replay_error(what, "leaf", i, plies(i), status[i]));
         return SC_E_INVAL;
     }
     return rc;
+}
+
+// the engine behind an sc_evaluator (host/evaluator.hpp): its slot table, the root updates' launch, and each pass of
+// leaves through predict_replay.  The dispatcher thread is the only caller
+class EngineBackend : public EvalBackend {
+    sc_engine *e_;
+    SlotTable t_;
+    // one pass: the requests that passed their checks, as predict_replay / launch_slot_replay take them
+    std::vector<int32_t> root_, off_;
+    std::vector<sc_move> mv_;
+    std::vector<int8_t> flag_;  // update: append; leaf: n_hist
+    std::vector<sc_position> pos_;
+    std::vector<sc_move> moves_;
+    std::vector<int32_t> cnt_;
+    std::vector<float> priors_, value_;
+
+    void clear()
+    {
+        root_.clear();
+        off_.assign(1, 0);
+        mv_.clear();
+        flag_.clear();
+    }
+    void add(int slot, const sc_move *mv, int len, int8_t flag)
+    {
+        root_.push_back(slot);
+        mv_.insert(mv_.end(), mv, mv + len);
+        off_.push_back((int32_t)mv_.size());
+        flag_.push_back(flag);
+    }
+    // the updates' one launch; statuses in e_->h_replay_status
+    int launch_updates(int n)
+    {
+        cudaStream_t st = e_->stream;
+        SCB_CUDA(cudaSetDevice(e_->device));
+        const void *d[4];
+        SCB_CHECK(stage_inputs(e_, n,
+                               {{off_.data(), sizeof(int32_t) * ((size_t)n + 1), e_->d_stack_off},
+                                {root_.data(), sizeof(int32_t) * (size_t)n, e_->d_path_root},
+                                {flag_.data(), (size_t)n, e_->d_stack_nhist},
+                                {mv_.data(), sizeof(sc_move) * mv_.size(), e_->d_stack}},
+                               d, st));
+        SCB_CHECK(launch_slot_replay(static_cast<const sc_move *>(d[3]), static_cast<const int32_t *>(d[0]),
+                                     static_cast<const int32_t *>(d[1]), static_cast<const int8_t *>(d[2]), n, t_.d_rec,
+                                     t_.d_pos, t_.d_plies, e_->d_replay_status, st));
+        e_->launches += 1;
+        SCB_CUDA(cudaMemcpyAsync(e_->h_replay_status, e_->d_replay_status, sizeof(int32_t) * (size_t)n,
+                                 cudaMemcpyDeviceToHost, st));
+        SCB_CUDA(cudaStreamSynchronize(st));
+        return SC_OK;
+    }
+
+public:
+    explicit EngineBackend(sc_engine *e) : e_(e) {}
+    ~EngineBackend() override
+    {
+        cudaSetDevice(e_->device);
+        cudaStreamSynchronize(e_->stream);
+        if (t_.d_rec) cudaFree(t_.d_rec);
+        if (t_.d_pos) cudaFree(t_.d_pos);
+        if (t_.d_plies) cudaFree(t_.d_plies);
+        e_->evaluator = false;
+    }
+    int setup(int n_slots)
+    {
+        SCB_CUDA(cudaSetDevice(e_->device));
+        SCB_CHECK(roots_setup(e_, 0));  // the staging buffers of sc_set_roots / sc_predict_path
+        SCB_CUDA(cudaMalloc(&t_.d_rec, replay_scratch_bytes((int64_t)n_slots * (SC_MAX_STACK + 1))));
+        SCB_CUDA(cudaMalloc(&t_.d_pos, sizeof(chess::Position) * (size_t)n_slots));
+        SCB_CUDA(cudaMalloc(&t_.d_plies, sizeof(int32_t) * (size_t)n_slots));
+        t_.plies.assign((size_t)n_slots, -1);
+        return SC_OK;
+    }
+
+    void update_roots(const std::vector<RootUpdate *> &u) override
+    {
+        std::vector<RootUpdate *> run;
+        clear();
+        for (RootUpdate *r : u) {
+            const char *what = r->append ? "sc_evaluator_extend_root" : "sc_evaluator_set_root";
+            const int ply0 = r->append ? t_.plies[r->slot] : 0;
+            if (ply0 < 0) {
+                r->rc = SC_E_STATE;
+                r->err = std::string(what) + ": slot " + std::to_string(r->slot) + " has no root";
+                continue;
+            }
+            const int32_t off[2] = {0, r->len};
+            r->rc = check_move_lists(what, "slot", "len", r->append ? "moves" : "stack", 1, r->moves, off, nullptr,
+                                     [&](int) { return ply0; }, r->slot);
+            if (r->rc != SC_OK) {
+                r->err = g_err;
+                continue;
+            }
+            run.push_back(r);
+            add(r->slot, r->moves, r->len, r->append);
+        }
+        if (run.empty()) return;
+        const int rc = launch_updates((int)run.size());
+        for (size_t i = 0; i < run.size(); i++) {
+            RootUpdate *r = run[i];
+            const int32_t status = e_->h_replay_status[i];
+            const int ply0 = r->append ? t_.plies[r->slot] : 0;
+            if (rc != SC_OK || status) {
+                r->rc = rc != SC_OK ? rc : SC_E_INVAL;
+                r->err = rc != SC_OK ? g_err
+                                     : replay_error(r->append ? "sc_evaluator_extend_root" : "sc_evaluator_set_root",
+                                                    "slot", r->slot, status >> 3, status);
+                t_.plies[r->slot] = -1;
+            } else {
+                t_.plies[r->slot] = ply0 + r->len;
+            }
+        }
+    }
+
+    void predict(const std::vector<LeafRequest *> &req) override
+    {
+        const char *what = "sc_evaluator_predict";
+        std::vector<LeafRequest *> run;
+        bool want_pos = false;
+        clear();
+        for (LeafRequest *q : req) {
+            const int plies = t_.plies[q->slot];
+            if (plies < 0) {
+                q->rc = SC_E_STATE;
+                q->err = std::string(what) + ": slot " + std::to_string(q->slot) + " has no root (sc_evaluator_set_root)";
+                continue;
+            }
+            if (q->n_hist < 0 || q->n_hist > SC_LOOKBACK) {
+                q->rc = SC_E_INVAL;
+                q->err = std::string(what) + ": n_hist = " + std::to_string(q->n_hist) + " is not in 0..8";
+                continue;
+            }
+            const int32_t off[2] = {0, q->len};
+            const int8_t nh = (int8_t)q->n_hist;
+            q->rc = check_move_lists(what, "slot", "len", "path", 1, q->path, off, nh ? &nh : nullptr,
+                                     [&](int) { return plies; }, q->slot);
+            if (q->rc != SC_OK) {
+                q->err = g_err;
+                continue;
+            }
+            const int total = plies + q->len;
+            run.push_back(q);
+            add(q->slot, q->path, q->len, nh ? nh : (int8_t)(total + 1 < SC_LOOKBACK ? total + 1 : SC_LOOKBACK));
+            want_pos |= q->pos_out != nullptr;
+        }
+        if (run.empty()) return;
+        const size_t n = run.size();
+        if (moves_.size() < n * SC_MAX_MOVES) {
+            pos_.resize(n);
+            moves_.resize(n * SC_MAX_MOVES);
+            cnt_.resize(n);
+            priors_.resize(n * SC_MAX_MOVES);
+            value_.resize(n);
+        }
+        float replay_ms = 0.f;
+        const int rc = predict_replay(e_, what, (int)n, root_.data(), &t_, mv_.data(), off_.data(), "len", "path",
+                                      flag_.data(), want_pos ? pos_.data() : nullptr, moves_.data(), cnt_.data(),
+                                      priors_.data(), value_.data(), &replay_ms, nullptr);
+        // a rejected leaf fails its own caller (the replay's status, the move generator's termination code)
+        const int32_t *status = e_->h_replay_status;
+        const int32_t *term = reinterpret_cast<const int32_t *>(e_->h_pred_out + (sizeof(sc_move) * SC_MAX_MOVES +
+                                                                                  sizeof(int32_t)) * n);
+        for (size_t i = 0; i < n; i++) {
+            LeafRequest *q = run[i];
+            if (rc != SC_OK && rc != SC_E_INVAL) {
+                q->rc = rc;
+                q->err = g_err;
+                continue;
+            }
+            memcpy(q->moves_out, &moves_[i * SC_MAX_MOVES], sizeof(sc_move) * SC_MAX_MOVES);
+            memcpy(q->priors_out, &priors_[i * SC_MAX_MOVES], sizeof(float) * SC_MAX_MOVES);
+            *q->move_cnt_out = cnt_[i];
+            *q->value_out = value_[i];
+            if (q->pos_out) *q->pos_out = pos_[i];
+            if (status[i]) {
+                q->rc = SC_E_INVAL;
+                q->err = replay_error(what, "slot", q->slot, status[i] >> 3, status[i]);
+            } else if (term[i] == PREDICT_OVERFLOW) {
+                q->rc = SC_E_INVAL;
+                q->err = std::string(what) + ": slot " + std::to_string(q->slot) + " has more than " +
+                         std::to_string(SC_MAX_MOVES) + " pseudo-legal moves (not a legal position)";
+            }
+        }
+    }
+};
+
+int engine_backend_create(sc_engine *e, int n_slots, int *max_batch, EvalBackend **out)
+{
+    if (!e || n_slots < 1 || n_slots > e->max_batch) {
+        set_error("sc_evaluator_create: bad argument (n_slots must be in 1..max_batch)");
+        return SC_E_INVAL;
+    }
+    bool free_engine = false;
+    if (!e->evaluator.compare_exchange_strong(free_engine, true)) {
+        set_error("sc_evaluator_create: the engine already has an evaluator");
+        return SC_E_STATE;
+    }
+    EngineBackend *b = new EngineBackend(e);  // gives the engine back when deleted
+    const int rc = b->setup(n_slots);
+    if (rc != SC_OK) {
+        const std::string msg = g_err;
+        delete b;
+        set_error(msg);
+        return rc;
+    }
+    *max_batch = e->max_batch;
+    *out = b;
+    return SC_OK;
 }
 
 }  // namespace scb
@@ -1124,6 +1363,7 @@ int sc_create(const char *weights_blob_path, int device, int mode, int max_batch
 int sc_destroy(sc_engine *e)
 {
     if (!e) return SC_OK;
+    SCB_CHECK(check_owner(e, "sc_destroy"));
     cudaSetDevice(e->device);
     cudaDeviceSynchronize();
     auto kill = [](ConvW &c) { if (c.tc) tc_conv_destroy(c.tc); c.tc = nullptr; };
@@ -1183,6 +1423,7 @@ int sc_device_info(const sc_engine *e, int *device, int *num_sms)
 int sc_eval_device(sc_engine *e, int n, const void *d_pos, const void *d_moves, const void *d_move_off,
                    int n_moves_total, void *d_priors_out, void *d_value_out, void *stream)
 {
+    SCB_CHECK(check_owner(e, "sc_eval_device"));
     if (!e || n < 0 || n > e->max_batch) {
         set_error("sc_eval_device: bad n");
         return SC_E_INVAL;
@@ -1213,6 +1454,7 @@ int sc_eval_device(sc_engine *e, int n, const void *d_pos, const void *d_moves, 
 int sc_eval(sc_engine *e, int n, const sc_position *pos, const sc_move *moves, const int32_t *move_off,
             float *priors_out, float *value_out, void *stream)
 {
+    SCB_CHECK(check_owner(e, "sc_eval"));
     if (!e || n < 0 || n > e->max_batch || (n > 0 && (!pos || !moves || !move_off || !priors_out || !value_out))) {
         set_error("sc_eval: bad argument");
         return SC_E_INVAL;
@@ -1263,6 +1505,7 @@ int sc_eval(sc_engine *e, int n, const sc_position *pos, const sc_move *moves, c
 int sc_predict(sc_engine *e, int n, const sc_position *pos, const int8_t *ep_square, sc_move *moves_out,
                int32_t *move_cnt_out, float *priors_out, float *value_out, void *stream)
 {
+    SCB_CHECK(check_owner(e, "sc_predict"));
     if (!e || n < 0 || n > e->max_batch ||
         (n > 0 && (!pos || !moves_out || !move_cnt_out || !priors_out || !value_out))) {
         set_error("sc_predict: bad argument");
@@ -1313,6 +1556,7 @@ int sc_predict_stack(sc_engine *e, int n, const sc_move *stack, const int32_t *s
                      sc_position *pos_out, sc_move *moves_out, int32_t *move_cnt_out, float *priors_out,
                      float *value_out, void *stream)
 {
+    SCB_CHECK(check_owner(e, "sc_predict_stack"));
     if (!e || n < 0 || n > e->max_batch ||
         (n > 0 && (!stack_off || !moves_out || !move_cnt_out || !priors_out || !value_out))) {
         set_error("sc_predict_stack: bad argument");
@@ -1320,12 +1564,13 @@ int sc_predict_stack(sc_engine *e, int n, const sc_move *stack, const int32_t *s
     }
     if (n == 0) return SC_OK;
     NvtxRange nv_call("sc_predict_stack");
-    return predict_replay(e, "sc_predict_stack", n, nullptr, stack, stack_off, "stack_off", "stack", n_hist, pos_out,
+    return predict_replay(e, "sc_predict_stack", n, nullptr, nullptr, stack, stack_off, "stack_off", "stack", n_hist, pos_out,
                           moves_out, move_cnt_out, priors_out, value_out, &e->last_replay_ms, stream);
 }
 
 int sc_set_roots(sc_engine *e, int n_roots, const sc_move *stack, const int32_t *stack_off)
 {
+    SCB_CHECK(check_owner(e, "sc_set_roots"));
     if (!e || n_roots < 0 || n_roots > e->max_batch || (n_roots > 0 && !stack_off)) {
         set_error("sc_set_roots: bad argument");
         return SC_E_INVAL;
@@ -1351,8 +1596,7 @@ int sc_set_roots(sc_engine *e, int n_roots, const sc_move *stack, const int32_t 
     for (int r = 0; r < n_roots; r++) {
         const int32_t status = e->h_replay_status[r];
         if (!status) continue;
-        set_error("sc_set_roots: root " + std::to_string(r) + ", ply " + std::to_string(status >> 3) +
-                  ": move rejected, " + replay_reason(status));
+        set_error(replay_error("sc_set_roots", "root", r, status >> 3, status));
         return SC_E_INVAL;
     }
     e->root_off.assign(stack_off, stack_off + n_roots + 1);
@@ -1364,6 +1608,7 @@ int sc_predict_path(sc_engine *e, int n, const int32_t *root, const sc_move *pat
                     const int8_t *n_hist, sc_position *pos_out, sc_move *moves_out, int32_t *move_cnt_out,
                     float *priors_out, float *value_out, void *stream)
 {
+    SCB_CHECK(check_owner(e, "sc_predict_path"));
     if (!e || n < 0 || n > e->max_batch ||
         (n > 0 && (!root || !path_off || !moves_out || !move_cnt_out || !priors_out || !value_out))) {
         set_error("sc_predict_path: bad argument");
@@ -1382,13 +1627,14 @@ int sc_predict_path(sc_engine *e, int n, const int32_t *root, const sc_move *pat
         }
     }
     NvtxRange nv_call("sc_predict_path");
-    return predict_replay(e, "sc_predict_path", n, root, path, path_off, "path_off", "path", n_hist, pos_out,
+    return predict_replay(e, "sc_predict_path", n, root, nullptr, path, path_off, "path_off", "path", n_hist, pos_out,
                           moves_out, move_cnt_out, priors_out, value_out, &e->last_path_ms, stream);
 }
 
 int sc_eval_submit(sc_engine *e, int n, const sc_position *pos, const sc_move *moves_strided, const int32_t *move_cnt,
                    float *priors_out_strided, float *value_out, void *stream, int *ticket)
 {
+    SCB_CHECK(check_owner(e, "sc_eval_submit"));
     if (!e || !ticket || n < 0 || n > e->max_batch ||
         (n > 0 && (!pos || !moves_strided || !move_cnt || !priors_out_strided || !value_out))) {
         set_error("sc_eval_submit: bad argument");
@@ -1467,6 +1713,7 @@ int sc_eval_submit(sc_engine *e, int n, const sc_position *pos, const sc_move *m
 
 int sc_eval_wait(sc_engine *e, int ticket)
 {
+    SCB_CHECK(check_owner(e, "sc_eval_wait"));
     if (!e || ticket < 0 || ticket >= SC_MAX_INFLIGHT || !e->tickets[ticket]) {
         set_error("sc_eval_wait: bad ticket");
         return SC_E_INVAL;
@@ -1478,6 +1725,7 @@ int sc_eval_wait(sc_engine *e, int ticket)
 
 int sc_encode_only(sc_engine *e, int n, const sc_position *pos, int8_t *planes_out, int32_t *meta_out)
 {
+    SCB_CHECK(check_owner(e, "sc_encode_only"));
     if (!e || n < 0 || n > e->max_batch || (n > 0 && (!pos || !planes_out || !meta_out))) {
         set_error("sc_encode_only: bad argument");
         return SC_E_INVAL;
@@ -1499,6 +1747,7 @@ int sc_encode_only(sc_engine *e, int n, const sc_position *pos, int8_t *planes_o
 int sc_move_index_only(sc_engine *e, int n, const sc_position *pos, const sc_move *moves, const int32_t *move_off,
                        int32_t *index_out)
 {
+    SCB_CHECK(check_owner(e, "sc_move_index_only"));
     if (!e || n < 0 || n > e->max_batch || (n > 0 && (!pos || !moves || !move_off || !index_out))) {
         set_error("sc_move_index_only: bad argument");
         return SC_E_INVAL;
@@ -1526,6 +1775,7 @@ int sc_encode_steps(sc_engine *e, int n, const sc_move *played, const sc_move *c
                     const uint32_t *child_counts, const int32_t *child_off, int apply_mirror, int8_t *planes_out,
                     int32_t *meta_out, float *dist_out, int32_t *index_out, int32_t *index_off)
 {
+    SCB_CHECK(check_owner(e, "sc_encode_steps"));
     if (!e || n < 0 || n > e->max_batch ||
         (n > 0 && (!played || !child_moves || !child_counts || !child_off || !planes_out || !meta_out || !dist_out ||
                    !index_out || !index_off))) {
@@ -1629,6 +1879,7 @@ int sc_encode_steps(sc_engine *e, int n, const sc_move *played, const sc_move *c
 
 int sc_forward_only(sc_engine *e, int n, const float *planes, const float *meta, float *logp_out, float *value_out)
 {
+    SCB_CHECK(check_owner(e, "sc_forward_only"));
     if (!e || n < 0 || n > e->max_batch || (n > 0 && (!planes || !meta || !logp_out || !value_out))) {
         set_error("sc_forward_only: bad argument");
         return SC_E_INVAL;
@@ -1663,6 +1914,7 @@ int sc_forward_only(sc_engine *e, int n, const float *planes, const float *meta,
 int sc_debug_tower(sc_engine *e, int n, const sc_position *pos, int n_layers, int which, uint16_t *x_out, uint16_t *t_out,
                    uint16_t *y_out)
 {
+    SCB_CHECK(check_owner(e, "sc_debug_tower"));
     if (!e || !tc16(e) || n <= 0 || n > e->max_batch || !pos || !e->tower) {
         set_error("sc_debug_tower: bad argument (bf16 / fp16 engines only)");
         return SC_E_INVAL;
@@ -1697,6 +1949,7 @@ int64_t sc_launch_count(const sc_engine *e) { return e ? e->launches : 0; }
 
 int sc_set_timing(sc_engine *e, int enabled)
 {
+    SCB_CHECK(check_owner(e, "sc_set_timing"));
     if (!e) return SC_E_INVAL;
     e->timing = enabled < 0 ? 0 : (enabled > 2 ? 2 : enabled);
     return SC_OK;

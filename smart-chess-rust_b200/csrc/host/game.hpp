@@ -186,6 +186,69 @@ public:
     bool reverse_q(const ArcRefNode<Step> &node) const override { return node->step.color == Color::Black; }  // torch.rs:49-52
 };
 
+// ---- the same backend for many games on one engine: one sc_evaluator shared by the game threads, one root slot per
+// game.  The slot follows the real game (set_search_root once per real move) and `predict` passes only the moves below
+// the search root; the device generates the legal moves and applies the terminal rule.
+class ChessB200Slot : public Game<BoardState> {
+    sc_evaluator *ev_;
+    int slot_;
+    size_t root_plies_ = 0;  // moves of the game stored in the slot
+    bool rooted_ = false;
+
+public:
+    ChessB200Slot(sc_evaluator *ev, int slot) : ev_(ev), slot_(slot)
+    {
+        if (!ev) throw std::runtime_error("ChessB200Slot: null evaluator");
+    }
+
+    // the slot follows the game to `state`, the next search root: the moves played since the last call are appended
+    void set_search_root(const BoardState &state)
+    {
+        const std::vector<Move> &ms = state.move_stack();
+        if (ms.size() < root_plies_) throw std::runtime_error("set_search_root: the game is shorter than the slot's");
+        std::vector<sc_move> mv;
+        for (size_t k = root_plies_; k < ms.size(); k++) mv.push_back(sc_move{ms[k].from, ms[k].to, ms[k].promo, 0});
+        const int rc = rooted_ ? sc_evaluator_extend_root(ev_, slot_, mv.data(), (int)mv.size())
+                               : sc_evaluator_set_root(ev_, slot_, mv.data(), (int)mv.size());
+        if (rc != SC_OK) throw std::runtime_error(sc_last_error());
+        root_plies_ = ms.size();
+        rooted_ = true;
+    }
+
+    std::tuple<std::vector<Step>, std::vector<float>, float> predict(const ArcRefNode<Step> &node, const BoardState &state,
+                                                                      bool argmax) const override
+    {
+        if (argmax) throw std::runtime_error("predict: argmax is not used by mcts and not implemented");
+        const std::vector<Move> &ms = state.move_stack();
+        if (!rooted_ || ms.size() < root_plies_) throw std::runtime_error("predict: the state is not below the search root");
+        int n_hist = 0;  // as ChessB200's
+        for (ArcRefNode<Step> n = node; n && n_hist < SC_LOOKBACK;) {
+            n_hist++;
+            if (!n->parent) break;
+            n = n->parent->lock();
+        }
+        if (n_hist > (int)ms.size() + 1) throw std::runtime_error("predict: history longer than the move stack");
+        std::vector<sc_move> path;
+        for (size_t k = root_plies_; k < ms.size(); k++) path.push_back(sc_move{ms[k].from, ms[k].to, ms[k].promo, 0});
+        sc_move moves[SC_MAX_MOVES];
+        float priors[SC_MAX_MOVES];
+        int32_t cnt = 0;
+        float value = 0.f;
+        if (sc_evaluator_predict(ev_, slot_, path.data(), (int)path.size(), n_hist, nullptr, moves, &cnt, priors, &value) !=
+            SC_OK)
+            throw std::runtime_error(sc_last_error());
+        if (cnt == 0) return {{}, {}, value};  // terminal: the device's torch.rs:98-106 value
+        const Color turn = node->step.color;
+        if (turn != state.turn()) throw std::runtime_error("predict: node and state disagree on the side to move");
+        std::vector<Step> steps;
+        steps.reserve((size_t)cnt);
+        for (int i = 0; i < cnt; i++) steps.push_back(Step{Move{moves[i].from, moves[i].to, moves[i].promo}, !turn});
+        return {std::move(steps), std::vector<float>(priors, priors + cnt), value};
+    }
+
+    bool reverse_q(const ArcRefNode<Step> &node) const override { return node->step.color == Color::Black; }
+};
+
 // ---- src/mcts.rs:61-328 ----------------------------------------------------------------------------
 namespace mcts {
 

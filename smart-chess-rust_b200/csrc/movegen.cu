@@ -1,6 +1,6 @@
 // Legal moves of every leaf on the device, for sc_predict (the `state.legal_moves()` half of `Game::predict`,
 // src/game.rs:3-15, src/backends/torch.rs:96-106), and the replay that packs each leaf from its move stack for
-// sc_predict_stack, or from a stored root and its path for sc_set_roots / sc_predict_path.
+// sc_predict_stack, or from a stored root and its path for sc_set_roots / sc_predict_path and an evaluator's slots.
 //
 // One thread per leaf runs host/chess_rules.hpp's generator -- the same code as the host driver, so python-chess's
 // generation order is defined in one place -- and writes each legal move straight into the leaf's strided output slot
@@ -89,6 +89,20 @@ struct RootPathRecords {
 };
 using PathHistory = PlyHistory<RootPathRecords>;
 
+// where path_replay_kernel finds the records and the plies of root r.  sc_set_roots' table: root r's records at
+// off[r] + r, off[r + 1] - off[r] plies
+struct OffsetRoots {
+    const int32_t *off;
+    __device__ int64_t base(int r) const { return off[r] + r; }
+    __device__ int plies(int r) const { return off[r + 1] - off[r]; }
+};
+// an evaluator's slot table: slot r's records at r * (SC_MAX_STACK + 1), n[r] plies
+struct SlotRoots {
+    const int32_t *n;
+    __device__ int64_t base(int r) const { return (int64_t)r * (SC_MAX_STACK + 1); }
+    __device__ int plies(int r) const { return n[r]; }
+};
+
 // the replay's checks (Board.push verifies no legality either; from/to < 64 and promo are checked on the host)
 __device__ int replay_reject(const chess::Position &p, const sc_move &m)
 {
@@ -166,11 +180,40 @@ __global__ void __launch_bounds__(REPLAY_THREADS) root_replay_kernel(const sc_mo
     root_pos[r] = p;
 }
 
-// sc_predict_stack / sc_predict_path, one thread per leaf: root[i]'s stored position (root == nullptr: the initial
-// position) continued with path[off[i], off[i+1]) (records in the per-call scratch), packed over the root's records
-// and the path's
+// an evaluator's root updates, one thread per updated slot: update u replays stack[off[u], off[u+1]) into slot slot[u],
+// from the initial position or (append[u]) from the slot's stored position after its n_plies[slot] moves, and keeps
+// the records from that ply on, the final position, the plies and status[u]
+__global__ void __launch_bounds__(REPLAY_THREADS) slot_replay_kernel(const sc_move *__restrict__ stack,
+                                                                     const int32_t *__restrict__ off,
+                                                                     const int32_t *__restrict__ slot,
+                                                                     const int8_t *__restrict__ append, int n,
+                                                                     ReplayPly *__restrict__ rec,
+                                                                     chess::Position *__restrict__ slot_pos,
+                                                                     int32_t *__restrict__ n_plies,
+                                                                     int32_t *__restrict__ status)
+{
+    const int u = blockIdx.x * blockDim.x + threadIdx.x;
+    if (u >= n) return;
+    const int g = slot[u], base = off[u];
+    int len = off[u + 1] - base, ply0 = 0;
+    chess::Position p;
+    if (append[u]) {
+        p = slot_pos[g];
+        ply0 = n_plies[g];
+    } else {
+        p.set_start();
+    }
+    status[u] = replay_moves(p, stack + base, len, rec + SlotRoots{}.base(g) + ply0, ply0);
+    slot_pos[g] = p;
+    n_plies[g] = ply0 + len;
+}
+
+// sc_predict_stack / sc_predict_path / an evaluator's leaves, one thread per leaf: root[i]'s stored position (root ==
+// nullptr: the initial position) continued with path[off[i], off[i+1]) (records in the per-call scratch), packed over
+// the root's records and the path's
+template <class Roots>
 __global__ void __launch_bounds__(REPLAY_THREADS) path_replay_kernel(
-    const ReplayPly *__restrict__ root_rec, const int32_t *__restrict__ root_off,
+    const ReplayPly *__restrict__ root_rec, Roots roots,
     const chess::Position *__restrict__ root_pos, const int32_t *__restrict__ root, const sc_move *__restrict__ path,
     const int32_t *__restrict__ off, const int8_t *__restrict__ n_hist, int n, ReplayPly *__restrict__ scratch,
     sc_position *__restrict__ pos, int8_t *__restrict__ ep, int32_t *__restrict__ status)
@@ -184,9 +227,9 @@ __global__ void __launch_bounds__(REPLAY_THREADS) path_replay_kernel(
     const ReplayPly *rh = nullptr;
     int root_plies = 0;
     if (root) {
-        const int r = root[i], root_base = root_off[r];
-        root_plies = root_off[r + 1] - root_base;
-        rh = root_rec + root_base + r;
+        const int r = root[i];
+        root_plies = roots.plies(r);
+        rh = root_rec + roots.base(r);
         p = root_pos[r];
     } else {
         p.set_start();
@@ -209,14 +252,32 @@ int launch_root_replay(const sc_move *d_stack, const int32_t *d_off, int n, void
     return SC_OK;
 }
 
-int launch_path_replay(const void *d_root_rec, const int32_t *d_root_off, const chess::Position *d_root_pos,
-                       const int32_t *d_root, const sc_move *d_path, const int32_t *d_off, const int8_t *d_n_hist, int n,
-                       void *d_scratch, sc_position *d_pos, int8_t *d_ep, int32_t *d_status, cudaStream_t st)
+int launch_slot_replay(const sc_move *d_stack, const int32_t *d_off, const int32_t *d_slot, const int8_t *d_append,
+                       int n, void *d_rec, chess::Position *d_slot_pos, int32_t *d_slot_plies, int32_t *d_status,
+                       cudaStream_t st)
 {
     if (n <= 0) return SC_OK;
-    path_replay_kernel<<<(n + REPLAY_THREADS - 1) / REPLAY_THREADS, REPLAY_THREADS, 0, st>>>(
-        static_cast<const ReplayPly *>(d_root_rec), d_root_off, d_root_pos, d_root, d_path, d_off, d_n_hist, n,
-        static_cast<ReplayPly *>(d_scratch), d_pos, d_ep, d_status);
+    slot_replay_kernel<<<(n + REPLAY_THREADS - 1) / REPLAY_THREADS, REPLAY_THREADS, 0, st>>>(
+        d_stack, d_off, d_slot, d_append, n, static_cast<ReplayPly *>(d_rec), d_slot_pos, d_slot_plies, d_status);
+    SCB_CUDA(cudaGetLastError());
+    return SC_OK;
+}
+
+int launch_path_replay(const void *d_root_rec, const int32_t *d_root_off, const int32_t *d_slot_plies,
+                       const chess::Position *d_root_pos, const int32_t *d_root, const sc_move *d_path,
+                       const int32_t *d_off, const int8_t *d_n_hist, int n, void *d_scratch, sc_position *d_pos,
+                       int8_t *d_ep, int32_t *d_status, cudaStream_t st)
+{
+    if (n <= 0) return SC_OK;
+    const dim3 grid((n + REPLAY_THREADS - 1) / REPLAY_THREADS);
+    const ReplayPly *rec = static_cast<const ReplayPly *>(d_root_rec);
+    ReplayPly *scratch = static_cast<ReplayPly *>(d_scratch);
+    if (d_slot_plies)
+        path_replay_kernel<<<grid, REPLAY_THREADS, 0, st>>>(rec, SlotRoots{d_slot_plies}, d_root_pos, d_root, d_path,
+                                                            d_off, d_n_hist, n, scratch, d_pos, d_ep, d_status);
+    else
+        path_replay_kernel<<<grid, REPLAY_THREADS, 0, st>>>(rec, OffsetRoots{d_root_off}, d_root_pos, d_root, d_path,
+                                                            d_off, d_n_hist, n, scratch, d_pos, d_ep, d_status);
     SCB_CUDA(cudaGetLastError());
     return SC_OK;
 }

@@ -6,12 +6,15 @@ CPU box), but creating an Engine without an sm_100 device raises.
 """
 from .binding import (  # noqa: F401
     Engine,
+    Evaluator,
     SelfPlay,
     Arena,
     elo,
     rules_probe,
     rules_perft,
     game_selfplay,
+    game_selfplay_many,
+    last_error,
     random_positions,
     SCError,
     SC_MODE_BF16,

@@ -30,7 +30,8 @@ DECLARED_SYMBOLS = [
     "sc_random_positions", "sc_test_dirichlet", "sc_game_selfplay", "sc_rules_perft", "sc_device_info",
     "sc_selfplay_run_many", "sc_debug_tower", "sc_rules_probe_fen", "sc_selfplay_trace_game", "sc_predict",
     "sc_predict_timing", "sc_predict_stack", "sc_predict_stack_timing", "sc_set_roots", "sc_predict_path",
-    "sc_predict_path_timing",
+    "sc_predict_path_timing", "sc_evaluator_create", "sc_evaluator_destroy", "sc_evaluator_set_root",
+    "sc_evaluator_extend_root", "sc_evaluator_predict", "sc_evaluator_stats", "sc_game_selfplay_many",
 ]
 
 
@@ -41,6 +42,15 @@ class SelfPlayConfig(C.Structure):
                 ("temperature", C.c_float), ("seed", C.c_uint64), ("n_threads", C.c_int32), ("evaluator", C.c_int32),
                 ("pipeline_groups", C.c_int32), ("keep_traces", C.c_int32),
                 ("leaves_per_tree", C.c_int32), ("rollout_factor", C.c_float)]
+
+
+class EvaluatorCounts(C.Structure):
+    """struct sc_evaluator_counts"""
+    _fields_ = [("passes", C.c_int64), ("leaves", C.c_int64), ("largest_batch", C.c_int64),
+                ("root_updates", C.c_int64), ("wait_seconds", C.c_double)]
+
+    def as_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_}
 
 
 class SelfPlayStats(C.Structure):
@@ -89,6 +99,15 @@ def load_library():
         L.sc_set_roots.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
         L.sc_predict_path.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 10
         L.sc_predict_path_timing.argtypes = [C.c_void_p, C.POINTER(C.c_float)]
+        # (ctypes.CDLL releases the GIL around every call: evaluator callers on Python threads overlap)
+        L.sc_evaluator_create.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_void_p)]
+        L.sc_evaluator_destroy.argtypes = [C.c_void_p]
+        L.sc_evaluator_set_root.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int]
+        L.sc_evaluator_extend_root.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int]
+        L.sc_evaluator_predict.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int] + [C.c_void_p] * 5
+        L.sc_evaluator_stats.argtypes = [C.c_void_p, C.POINTER(EvaluatorCounts)]
+        L.sc_game_selfplay_many.argtypes = [C.c_void_p, C.POINTER(SelfPlayConfig), C.c_int, C.c_void_p, C.c_char_p,
+                                            C.c_int64, C.c_void_p, C.POINTER(EvaluatorCounts)]
         L.sc_eval_device.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,
                                      C.c_void_p, C.c_void_p]
         L.sc_encode_only.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
@@ -437,6 +456,108 @@ class Engine:
         a, b = C.c_float(), C.c_float()
         _check(load_library().sc_last_timing(self._h, C.byref(a), C.byref(b)), "sc_last_timing")
         return a.value, b.value
+
+
+def _one_move_list(moves, what):
+    flat, _ = _move_lists([moves], what)
+    return flat
+
+
+class Evaluator:
+    """Batching evaluator (sc_evaluator_*): many threads, each searching one game through the one-leaf interface,
+    share `engine`.  Each game keeps its root in one of n_slots slots.  Every call blocks until its request ran; the
+    engine refuses direct calls while the evaluator exists."""
+
+    def __init__(self, engine, n_slots: int):
+        h = C.c_void_p()
+        _check(load_library().sc_evaluator_create(engine.handle, n_slots, C.byref(h)), "sc_evaluator_create")
+        self._h = h
+        self._engine = engine  # keep alive
+        self.n_slots = n_slots
+
+    def close(self):
+        """sc_evaluator_destroy: callers blocked in predict / set_root / extend_root get SC_E_STATE, and so does every
+        later call on this object"""
+        if getattr(self, "_h", None):
+            h, self._h = self._h, None
+            load_library().sc_evaluator_destroy(h)
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def set_root(self, slot: int, stack, check: bool = True):
+        """stores the game `stack` (moves from the initial position, as predict_stack()'s) as slot's root"""
+        return self._update(load_library().sc_evaluator_set_root, "sc_evaluator_set_root", slot, stack, check)
+
+    def extend_root(self, slot: int, moves, check: bool = True):
+        """appends `moves` to slot's stored game"""
+        return self._update(load_library().sc_evaluator_extend_root, "sc_evaluator_extend_root", slot, moves, check)
+
+    def _update(self, fn, what, slot, moves, check):
+        flat = _one_move_list(moves, what)
+        rc = fn(self._h, slot, _ptr(flat) if len(flat) else None, len(flat))
+        if check:
+            _check(rc, what)
+        return rc
+
+    def predict(self, slot: int, path, n_hist: int = 0, positions: bool = False, check: bool = True):
+        """one leaf: slot's root followed by `path`.  Returns (moves MOVE_DTYPE[256], count, priors float32[256],
+        value) as one row of Engine.predict_path(), then the packed leaf when `positions`; check=False puts the status
+        code first instead of raising (the message is then sc_last_error() of this thread)."""
+        flat = _one_move_list(path, "predict")
+        h = self._h
+        if h is None:
+            if check:
+                raise SCError("sc_evaluator_predict failed (-5): the evaluator is closed")
+            return (-5, None, 0, None, 0.0) + ((None,) if positions else ())
+        moves = np.zeros(SC_MAX_MOVES, dtype=MOVE_DTYPE)
+        priors = np.zeros(SC_MAX_MOVES, dtype=np.float32)
+        cnt, value = np.zeros(1, dtype=np.int32), np.zeros(1, dtype=np.float32)
+        pos = np.zeros(1, dtype=POSITION_DTYPE) if positions else None
+        rc = load_library().sc_evaluator_predict(h, slot, _ptr(flat) if len(flat) else None, len(flat), int(n_hist),
+                                                 _ptr(pos), _ptr(moves), _ptr(cnt), _ptr(priors), _ptr(value))
+        res = (moves, int(cnt[0]), priors, float(value[0])) + ((pos[0],) if positions else ())
+        if not check:
+            return (rc,) + res
+        _check(rc, "sc_evaluator_predict")
+        return res
+
+    def stats(self):
+        """{passes, leaves, largest_batch, root_updates, wait_seconds}"""
+        c = EvaluatorCounts()
+        _check(load_library().sc_evaluator_stats(self._h, C.byref(c)), "sc_evaluator_stats")
+        return c.as_dict()
+
+
+def last_error() -> str:
+    """sc_last_error() of the calling thread"""
+    return load_library().sc_last_error().decode()
+
+
+def game_selfplay_many(engine, seeds, rollout_num=20, num_steps=150, cpuct=2.5, epsilon=0.15, with_noise=False,
+                       temperature_switch=0, temperature=0.0, evaluator="engine", cap=1 << 18):
+    """game_selfplay() for len(seeds) games at once, each on its own host thread, all through one evaluator on
+    `engine` (sc_game_selfplay_many).  Returns (traces, evaluator counts)."""
+    import json
+
+    L = load_library()
+    n = len(seeds)
+    cfg = SelfPlayConfig(1, rollout_num, num_steps, cpuct, epsilon, int(with_noise), temperature_switch, temperature, 0,
+                         1, 0 if evaluator == "engine" else 1, 1, 1, 1, 0.0)
+    sd = np.ascontiguousarray(seeds, dtype=np.uint64)
+    sizes = np.zeros(n, dtype=np.int64)
+    buf = C.create_string_buffer(n * cap)
+    counts = EvaluatorCounts()
+    _check(L.sc_game_selfplay_many(engine.handle if engine is not None else None, C.byref(cfg), n, _ptr(sd), buf, cap,
+                                   _ptr(sizes), C.byref(counts)), "sc_game_selfplay_many")
+    if sizes.max() > cap:
+        raise SCError(f"game_selfplay_many: a trace needs {int(sizes.max())} bytes, more than cap = {cap}")
+    raw = buf.raw
+    traces = [json.loads(raw[g * cap : g * cap + int(sizes[g]) - 1].decode()) for g in range(n)]
+    return traces, counts.as_dict()
 
 
 class SelfPlay:
