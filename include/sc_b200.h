@@ -38,6 +38,11 @@ extern "C" {
                           SC_MODE_BF16, rounding where it rounds but to fp16 (11 significant bits instead of 8).  A
                           parked value (a layer output, the SE input) beyond +-65504 becomes +-inf, as in the reference's
                           fp16 autocast; a weight beyond that range fails sc_create with SC_E_IO                  */
+#define SC_MODE_FP8 4  /* throughput mode with fp8 (e4m3) tensor-core operands, fp32 accumulate: the weights of every
+                          tensor-core layer are e4m3 with a power-of-two scale per output channel, each layer's output
+                          is stored as e4m3 (round to nearest even, saturated to +-448); LayerNorm, SE, the SE weights
+                          and the heads' tails stay as in SC_MODE_BF16.  Every batch size runs the throughput kernels
+                          (there is no latency kernel), so a one-leaf call takes about as long as a 128-leaf one   */
 
 #define SC_LOOKBACK 8       /* src/chess.rs:23 */
 #define SC_N_PLANES 112     /* 8 x 14, py/module.py:118-121 */
@@ -361,9 +366,10 @@ int sc_arena_create(sc_engine *white, sc_engine *black, const sc_selfplay_config
 int sc_random_positions(int n, uint64_t seed, int max_ply, sc_position *pos_out, sc_move *moves_out,
                         int32_t *move_off /* n+1 */, int max_moves_total);
 
-/* Test hook (bf16 and fp16 engines): encodes n leaves and runs only the first n_layers (0 = all 41: stem, 19 x (conv1, conv2),
+/* Test hook (bf16, fp16 and fp8 engines): encodes n leaves and runs only the first n_layers (0 = all 41: stem, 19 x (conv1, conv2),
  * the two 256-wide head 1x1 convolutions) of the convolution tower with the throughput kernel (which = 0) or the
- * small-batch latency kernel (which = 1); copies the three activation buffers (bf16 / fp16 bit patterns, [n][64][256]:
+ * small-batch latency kernel (which = 1, not on fp8 engines); copies the three activation buffers (bf16 / fp16 bit patterns,
+ * an fp8 engine's e4m3 values as the fp16 bit patterns of the same values, [n][64][256]:
  * x = block input / output, t = conv1 output / policy head input, y = value head input) to the host.  Lets the tests
  * compare the two kernels layer by layer. */
 int sc_debug_tower(sc_engine *e, int n, const sc_position *pos, int n_layers, int which, uint16_t *x_out,

@@ -29,7 +29,7 @@ void set_error(const std::string &msg);
 
 constexpr int C_TOWER = 256;     // tower width (py/module.py:120)
 constexpr int C_IN = 112;        // input planes
-constexpr int C_IN_PAD = 128;    // bf16 path: planes padded to two 64-channel K chunks
+constexpr int C_IN_PAD = 128;    // tensor-core modes: planes padded to two 16-bit K chunks (one e4m3 chunk)
 constexpr int C_SE = 128;        // SqueezeExcitation(256, 128) (py/module.py:29-33)
 constexpr int C_POLICY = 73;
 constexpr int LD_POLICY = 80;    // row stride of the policy logits buffer [B][64][80]
@@ -45,10 +45,13 @@ int launch_encode_bf16(const sc_position *d_pos, int n, __nv_bfloat16 *out /*[n]
                        float *meta_out /*[n][8]*/, cudaStream_t st);
 int launch_encode_fp16(const sc_position *d_pos, int n, __half *out /*[n][64][128]*/, float *meta_out /*[n][8]*/,
                        cudaStream_t st);
+int launch_encode_e4m3(const sc_position *d_pos, int n, uint8_t *out /*[n][64][128]*/, float *meta_out /*[n][8]*/,
+                       cudaStream_t st);
 // NCHW float planes (sc_forward_only input) -> NHWC
 int launch_nchw_to_nhwc_f32(const float *in, int n, float *out, cudaStream_t st);
 int launch_nchw_to_nhwc_bf16(const float *in, int n, __nv_bfloat16 *out, cudaStream_t st);
 int launch_nchw_to_nhwc_fp16(const float *in, int n, __half *out, cudaStream_t st);
+int launch_nchw_to_nhwc_e4m3(const float *in, int n, uint8_t *out, cudaStream_t st);
 
 // ---- policy.cu ----------------------------------------------------------------------------
 // logits [n][64][LD_POLICY] fp32 (square-major) -> per-leaf log-sum-exp, legal-move gather,
@@ -114,18 +117,25 @@ int launch_ln_f32(float *x, int rows, int C, int ld, const float *gamma, const f
                   cudaStream_t st, __nv_bfloat16 *planes = nullptr);
 int launch_se_res_f32(const float *y, const float *x, float *out, int n, const float *w1t, const float *b1,
                       const float *w2t, const float *b2, cudaStream_t st, __nv_bfloat16 *planes = nullptr);
+// scale (fp8 mode): the hidden units' weight scales, applied to the split sum
 int launch_value_finish(const float *hidden_pre, int n_split, int n, const float *meta, const float *w_meta,
-                        const float *b1, const float *w2, const float *b2, float *value_out, cudaStream_t st);
+                        const float *b1, const float *w2, const float *b2, float *value_out, cudaStream_t st,
+                        const float *scale = nullptr);
 
 // ---- tower_bf16.cu (tcgen05) --------------------------------------------------------------
-// The 16-bit tensor-core modes share these kernels and interfaces: `fp16` selects fp16 operands instead of bf16, and
-// then every 16-bit buffer below (weights, activations; typed __nv_bfloat16) holds fp16 bit patterns.
+// The tensor-core modes share these kernels and interfaces.  The operand type selects fp16 or e4m3 operands instead of
+// bf16, and then every operand buffer below (weights, activations; typed __nv_bfloat16) holds fp16 bit patterns, or
+// e4m3 bytes ([..][k] with k one byte each).  e4m3 weights come with `scale`: per output channel a power of two that the
+// epilogue multiplies the accumulator by.
+enum TcOp { TC_OP_BF16 = 0, TC_OP_FP16 = 1, TC_OP_E4M3 = 2 };
+// channels per K chunk (one 128-byte swizzle row): 64 16-bit or 128 8-bit elements
+constexpr int tc_op_bk(TcOp op) { return op == TC_OP_E4M3 ? 128 : 64; }
 struct TcConv;  // opaque per-layer state (tensor maps)
 enum { TC_EPI_LN = 0, TC_EPI_LN_SE = 1, TC_EPI_LN73 = 2, TC_EPI_RAW = 3 };
 // w: bf16 [taps][bn][k_per_tap] (K-major B operand); bn = 256 (tower / head 1x1 convs),
 // 80 (policy 256->73, rows 73..79 zero) or 128 (value FC, taps = 1, k_per_tap = 16384)
 int tc_conv_create(TcConv **out, const __nv_bfloat16 *w, int taps, int k_per_tap, int bn, int epi, const float *bias,
-                   const float *gamma, const float *beta, bool fp16);
+                   const float *gamma, const float *beta, TcOp op, const float *scale = nullptr);
 // FP32 parity mode: conv to 256 channels as a bf16x3 split GEMM on the tensor cores, fp32 [boards * 64][256] out (+ bias).
 // w3 = bf16 [taps][256][3 * cin_pad] (three planes side by side along K), activations bf16 [boards][64][a_planes * cin_pad]
 int tc_split_conv_create(TcConv **out, const __nv_bfloat16 *w3, int taps, int cin_pad, int a_planes, const float *bias);
@@ -166,7 +176,7 @@ struct TcTowerLayerDesc {
     const __nv_bfloat16 *resid;  // SE layers: block input (may alias out)
     int relu;
 };
-int tc_tower_create(TcTower **out, const TcTowerLayerDesc *descs, int n, int boards_alloc, bool fp16);
+int tc_tower_create(TcTower **out, const TcTowerLayerDesc *descs, int n, int boards_alloc, TcOp op);
 // group = tiles per CTA carried through all layers together (0 = all of the CTA's tiles)
 // max_layers > 0: only the first max_layers layers (sc_debug_tower's layer-by-layer comparison)
 int tc_tower_launch(TcTower *t, int n_boards, int num_sms, int group, cudaStream_t st, int max_layers = 0);

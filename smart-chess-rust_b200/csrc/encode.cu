@@ -13,6 +13,8 @@
 // "side to move" is that of the CURRENT position for every history slot (src/chess.rs:871).
 #include "common.cuh"
 
+#include <cuda_fp8.h>
+
 namespace scb {
 
 constexpr int ENC_WARPS = 4;
@@ -146,6 +148,35 @@ __global__ void __launch_bounds__(ENC_WARPS * 32) encode_16bit_kernel(const sc_p
     if (warp == 0 && lane < 8) meta_out[b * 8 + lane] = lane < SC_N_META ? (float)pos[b].meta[lane] : 0.f;
 }
 
+// e4m3 form (fp8 mode; 1.0 = 0x38): the 16-bit kernel's work split, 8 bytes per lane and row
+__global__ void __launch_bounds__(ENC_WARPS * 32) encode_e4m3_kernel(const sc_position *__restrict__ pos, int n,
+                                                                     uint8_t *__restrict__ out,
+                                                                     float *__restrict__ meta_out)
+{
+    __shared__ uint64_t s_slots[64];
+    __shared__ uint64_t s_masks[128];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int b = blockIdx.x;
+    if (b >= n) return;
+    if (warp == 0) build_masks(pos + b, s_slots, s_masks, lane);
+    __syncthreads();
+    uint2 *dst = reinterpret_cast<uint2 *>(out + (size_t)b * 64 * C_IN_PAD);
+    const int c0 = (lane & 15) * 8;
+    uint64_t m[8];
+#pragma unroll
+    for (int j = 0; j < 8; j++) m[j] = s_masks[c0 + j];
+#pragma unroll
+    for (int it8 = 0; it8 < 8; it8++) {
+        const int it = warp * 8 + it8;
+        const int s = it * 2 + (lane >> 4);
+        uint32_t w[2] = {0u, 0u};
+#pragma unroll
+        for (int j = 0; j < 8; j++) w[j >> 2] |= (uint32_t)((m[j] >> s) & 1ULL) * 0x38u << (8 * (j & 3));
+        dst[it * 32 + lane] = make_uint2(w[0], w[1]);
+    }
+    if (warp == 0 && lane < 8) meta_out[b * 8 + lane] = lane < SC_N_META ? (float)pos[b].meta[lane] : 0.f;
+}
+
 int launch_encode_i8(const sc_position *d_pos, int n, int8_t *out, int32_t *meta_out, cudaStream_t st)
 {
     if (n <= 0) return SC_OK;
@@ -178,11 +209,21 @@ int launch_encode_fp16(const sc_position *d_pos, int n, __half *out, float *meta
     return SC_OK;
 }
 
+int launch_encode_e4m3(const sc_position *d_pos, int n, uint8_t *out, float *meta_out, cudaStream_t st)
+{
+    if (n <= 0) return SC_OK;
+    encode_e4m3_kernel<<<n, ENC_WARPS * 32, 0, st>>>(d_pos, n, out, meta_out);
+    SCB_CUDA(cudaGetLastError());
+    return SC_OK;
+}
+
 // ---- NCHW float (what the reference backends feed the net) -> NHWC ------------------------
 template <typename T> __device__ __forceinline__ T cvt(float v);
 template <> __device__ __forceinline__ float cvt<float>(float v) { return v; }
 template <> __device__ __forceinline__ __nv_bfloat16 cvt<__nv_bfloat16>(float v) { return __float2bfloat16(v); }
 template <> __device__ __forceinline__ __half cvt<__half>(float v) { return __float2half_rn(v); }
+// e4m3, round to nearest even, satfinite (+-448)
+template <> __device__ __forceinline__ __nv_fp8_e4m3 cvt<__nv_fp8_e4m3>(float v) { return __nv_fp8_e4m3(v); }
 
 template <typename T, int LD>
 __global__ void __launch_bounds__(256) nchw_to_nhwc_kernel(const float *__restrict__ in, int n, T *__restrict__ out)
@@ -222,6 +263,14 @@ int launch_nchw_to_nhwc_fp16(const float *in, int n, __half *out, cudaStream_t s
 {
     if (n <= 0) return SC_OK;
     nchw_to_nhwc_kernel<__half, C_IN_PAD><<<n, 256, 0, st>>>(in, n, out);
+    SCB_CUDA(cudaGetLastError());
+    return SC_OK;
+}
+
+int launch_nchw_to_nhwc_e4m3(const float *in, int n, uint8_t *out, cudaStream_t st)
+{
+    if (n <= 0) return SC_OK;
+    nchw_to_nhwc_kernel<__nv_fp8_e4m3, C_IN_PAD><<<n, 256, 0, st>>>(in, n, reinterpret_cast<__nv_fp8_e4m3 *>(out));
     SCB_CUDA(cudaGetLastError());
     return SC_OK;
 }

@@ -15,6 +15,7 @@
 #include <string>
 #include <vector>
 
+#include <cuda_fp8.h>
 #include <nvtx3/nvToolsExt.h>
 
 #include "common.cuh"
@@ -144,11 +145,38 @@ struct Op16Weights {
     }
 };
 
+// fp8 mode: the e4m3 weights of one output channel whose largest |w| is amax carry the scale s = 2^ceil(log2(amax / 448))
+// (1 for an all-zero channel): w / s is at most 448 and is rounded to e4m3 (round to nearest even).  A power of two
+// makes both w / s and the epilogue's acc * s exact, so the only rounding the scale brings is the operand's own.
+static float e4m3_scale(float amax)
+{
+    if (!(amax > 0.f)) return 1.f;
+    int e;
+    const float f = frexpf(amax, &e);  // amax = f 2^e, f in [0.5, 1); 448 = 0.875 2^9
+    return ldexpf(1.f, f <= 0.875f ? e - 9 : e - 8);
+}
+static uint8_t f2e4m3(float f) { return (uint8_t)__nv_cvt_float_to_fp8(f, __NV_SATFINITE, __NV_E4M3); }
+
+// rows x k fp32 weights (row r at w[r * k], one output channel each) -> e4m3 bytes and the rows' scales
+static void quantize_e4m3(const std::vector<float> &w, int rows, size_t k, std::vector<uint8_t> &q, std::vector<float> &scale)
+{
+    q.assign(w.size(), 0);
+    scale.assign((size_t)rows, 1.f);
+    for (int r = 0; r < rows; r++) {
+        float amax = 0.f;
+        for (size_t i = 0; i < k; i++) amax = fmaxf(amax, fabsf(w[r * k + i]));
+        scale[r] = e4m3_scale(amax);
+        for (size_t i = 0; i < k; i++) q[r * k + i] = f2e4m3(w[r * k + i] / scale[r]);
+    }
+}
+
 struct ConvW {
     int taps = 1, cin = 0, cin_pad = 0, cout = 0, ldw = 0;
     float *w_f32 = nullptr;          // [taps][cin][ldw]        (fp32 mode)
-    __nv_bfloat16 *w_bf16 = nullptr; // [taps][cout][cin_pad]   (16-bit modes, K-major B operand; fp16 bits in fp16 mode)
+    __nv_bfloat16 *w_bf16 = nullptr; // [taps][cout][cin_pad]   (tensor-core modes, K-major B operand; fp16 bits in fp16
+                                     //                          mode, e4m3 bytes in fp8 mode)
     float *bias = nullptr, *gamma = nullptr, *beta = nullptr;
+    float *scale = nullptr;          // fp8 mode: per output channel the weights' scale (e4m3_scale)
     TcConv *tc = nullptr;
 };
 
@@ -165,8 +193,9 @@ using namespace scb;
 struct sc_engine {
     int device = 0, mode = 0, max_batch = 0, n_blocks = 0, num_sms = 148;
     int mode_requested = 0;
-    // SC_MODE_BF16 / SC_MODE_FP16: the same tensor-core kernels with bf16 / fp16 operands (tc16() below)
-    bool fp16 = false;
+    // SC_MODE_BF16 / SC_MODE_FP16 / SC_MODE_FP8: the same tensor-core kernels with bf16 / fp16 / e4m3 operands (tc_mode()
+    // below).  fp8 has no latency kernel: every batch runs the throughput kernels
+    TcOp op = TC_OP_BF16;
     // FP32 parity mode: the 256-wide convolutions as bf16x3 split GEMMs on the tensor cores (fp32 accumulate), LayerNorm /
     // SE / the narrow head layers in fp32 on the CUDA cores.  SC_MODE_FP32_FFMA = everything FFMA.
     bool fp32_tc = false;
@@ -187,6 +216,7 @@ struct sc_engine {
     bool lat_enabled = !(getenv("SCB200_LATENCY") && getenv("SCB200_LATENCY")[0] == '0');
     double timed_flops_per_leaf = 0.0;    // FLOPs per leaf covered by the level-2 timed launches
     float *v_wmeta = nullptr, *v_b1 = nullptr, *v_w2 = nullptr, *v_b2 = nullptr;
+    float *v_scale = nullptr;             // fp8 mode: the value FC's per-hidden-unit weight scales
     // io
     sc_position *d_pos = nullptr;
     sc_move *d_moves = nullptr;
@@ -196,7 +226,7 @@ struct sc_engine {
     int max_moves_total = 0;
     // activations
     float *f_planes = nullptr, *f_x = nullptr, *f_t = nullptr, *f_y = nullptr;
-    __nv_bfloat16 *h_planes = nullptr, *h_x = nullptr, *h_t = nullptr, *h_y = nullptr;  // fp16 bits in fp16 mode
+    __nv_bfloat16 *h_planes = nullptr, *h_x = nullptr, *h_t = nullptr, *h_y = nullptr;  // fp16 bits / e4m3 bytes
     float *logits = nullptr, *vpre = nullptr;
     int vsplit = 1;
     // gates
@@ -280,8 +310,12 @@ constexpr int SC_SMALL_N = 128;
 // the pinned small-batch input buffer: sc_eval's positions, offsets and moves for SC_SMALL_N leaves
 constexpr size_t SMALL_IN_BYTES = (size_t)SC_SMALL_N * (sizeof(sc_position) + 4 + SC_MAX_MOVES * sizeof(sc_move)) + 64;
 
-// a 16-bit tensor-core mode (bf16 or fp16 operands): the tower, latency and head kernels of tower_bf16.cu / tower_lat.cu
-static bool tc16(const sc_engine *e) { return e->mode == SC_MODE_BF16 || e->mode == SC_MODE_FP16; }
+// a tensor-core mode (bf16, fp16 or e4m3 operands): the tower and head kernels of tower_bf16.cu (and for the 16-bit
+// types the latency kernel of tower_lat.cu)
+static bool tc_mode(const sc_engine *e)
+{
+    return e->mode == SC_MODE_BF16 || e->mode == SC_MODE_FP16 || e->mode == SC_MODE_FP8;
+}
 
 template <typename T> static int dev_alloc(sc_engine *e, T **p, size_t count)
 {
@@ -376,8 +410,27 @@ static int load_conv(sc_engine *e, const Blob &b, const std::string &wname, cons
     } else {
         // B operand, K-major: [tap][bn rows][cin_pad]; bn = 256, or 80 for the 73-wide policy conv
         const int bn = cout == C_TOWER ? C_TOWER : LD_POLICY;
+        if (e->op == TC_OP_E4M3) {
+            // per output channel [taps][cin_pad] -> e4m3 with the channel's scale, then [tap][bn][cin_pad]
+            const size_t k = (size_t)taps * c.cin_pad;
+            std::vector<float> wc((size_t)bn * k, 0.f);
+            for (int co = 0; co < cout; co++)
+                for (int ci = 0; ci < cin; ci++)
+                    for (int t = 0; t < taps; t++) wc[co * k + (size_t)t * c.cin_pad + ci] = w->data[((size_t)co * cin + ci) * taps + t];
+            std::vector<uint8_t> q, h(wc.size());
+            std::vector<float> sc;
+            quantize_e4m3(wc, bn, k, q, sc);
+            for (int co = 0; co < bn; co++)
+                for (int t = 0; t < taps; t++)
+                    memcpy(&h[((size_t)t * bn + co) * c.cin_pad], &q[co * k + (size_t)t * c.cin_pad], (size_t)c.cin_pad);
+            uint8_t *d = nullptr;
+            SCB_CHECK(upload(e, &d, h));
+            SCB_CHECK(upload(e, &c.scale, sc));
+            c.w_bf16 = reinterpret_cast<__nv_bfloat16 *>(d);
+            return tc_conv_create(&c.tc, c.w_bf16, taps, c.cin_pad, bn, epi, c.bias, c.gamma, c.beta, TC_OP_E4M3, c.scale);
+        }
         std::vector<uint16_t> h((size_t)taps * bn * c.cin_pad, 0);
-        Op16Weights cv{e->fp16};
+        Op16Weights cv{e->op == TC_OP_FP16};
         for (int co = 0; co < cout; co++)
             for (int ci = 0; ci < cin; ci++)
                 for (int t = 0; t < taps; t++)
@@ -386,7 +439,7 @@ static int load_conv(sc_engine *e, const Blob &b, const std::string &wname, cons
         uint16_t *d = nullptr;
         SCB_CHECK(upload(e, &d, h));
         c.w_bf16 = reinterpret_cast<__nv_bfloat16 *>(d);
-        SCB_CHECK(tc_conv_create(&c.tc, c.w_bf16, taps, c.cin_pad, bn, epi, c.bias, c.gamma, c.beta, e->fp16));
+        SCB_CHECK(tc_conv_create(&c.tc, c.w_bf16, taps, c.cin_pad, bn, epi, c.bias, c.gamma, c.beta, e->op));
     }
     return SC_OK;
 }
@@ -423,8 +476,9 @@ static int load_weights(sc_engine *e, const Blob &b)
         } else {
             // packed so that epilogue thread j (fc1) / channel c (fc2) reads 8 consecutive inputs
             // with one coalesced 16-byte load: w1p[q][j][i] = fc1[j][8q+i], w2p[q][c][i] = fc2[c][8q+i]
+            // (fp8 mode: bf16, the SE runs on the CUDA cores)
             std::vector<uint16_t> w1p((size_t)C_TOWER * C_SE), w2p((size_t)C_SE * C_TOWER);
-            Op16Weights cv1{e->fp16}, cv2{e->fp16};
+            Op16Weights cv1{e->op == TC_OP_FP16}, cv2{e->op == TC_OP_FP16};
             for (int q = 0; q < C_TOWER / 8; q++)
                 for (int j = 0; j < C_SE; j++)
                     for (int k = 0; k < 8; k++)
@@ -484,11 +538,25 @@ static int load_weights(sc_engine *e, const Blob &b)
                     for (int s = 0; s < 64; s++)
                         h[((size_t)s * C_TOWER + c) * N_VALUE_HIDDEN + j] = fc->data[(size_t)j * KT + c * 64 + s];
             SCB_CHECK(upload(e, &e->vfc_w_f32, h));
+        } else if (e->op == TC_OP_E4M3) {
+            // the B operand below in e4m3, with the hidden units' scales
+            std::vector<float> wf((size_t)N_VALUE_HIDDEN * KV);
+            for (int j = 0; j < N_VALUE_HIDDEN; j++)
+                for (int c = 0; c < C_TOWER; c++)
+                    for (int s = 0; s < 64; s++) wf[(size_t)j * KV + (size_t)s * C_TOWER + c] = fc->data[(size_t)j * KT + c * 64 + s];
+            std::vector<uint8_t> q;
+            std::vector<float> sc;
+            quantize_e4m3(wf, N_VALUE_HIDDEN, KV, q, sc);
+            uint8_t *d = nullptr;
+            SCB_CHECK(upload(e, &d, q));
+            SCB_CHECK(upload(e, &e->v_scale, sc));
+            SCB_CHECK(tc_conv_create(&e->vfc_tc, reinterpret_cast<__nv_bfloat16 *>(d), 1, KV, N_VALUE_HIDDEN, TC_EPI_RAW,
+                                     nullptr, nullptr, nullptr, TC_OP_E4M3, e->v_scale));
         } else {
             // B operand of the value FC GEMM, K-major: [128][16384] with k' = s*256 + c
             // (the meta columns stay fp32: the fused value tail applies them)
             std::vector<uint16_t> h((size_t)N_VALUE_HIDDEN * KV);
-            Op16Weights cv{e->fp16};
+            Op16Weights cv{e->op == TC_OP_FP16};
             for (int j = 0; j < N_VALUE_HIDDEN; j++)
                 for (int c = 0; c < C_TOWER; c++)
                     for (int s = 0; s < 64; s++)
@@ -497,7 +565,7 @@ static int load_weights(sc_engine *e, const Blob &b)
             uint16_t *d = nullptr;
             SCB_CHECK(upload(e, &d, h));
             SCB_CHECK(tc_conv_create(&e->vfc_tc, reinterpret_cast<__nv_bfloat16 *>(d), 1, KV, N_VALUE_HIDDEN, TC_EPI_RAW,
-                                     nullptr, nullptr, nullptr, e->fp16));
+                                     nullptr, nullptr, nullptr, e->op));
         }
     }
     SCB_CHECK(upload_vec(e, b, "value_head.ffn.0.bias", N_VALUE_HIDDEN, &e->v_b1));
@@ -722,7 +790,7 @@ static int run_network(sc_engine *e, int n, cudaStream_t st, const TcGather *gat
         e->launches += 2;
     }
     SCB_CHECK(launch_value_finish(e->vpre, e->vsplit, n, e->d_meta, e->v_wmeta, e->v_b1, e->v_w2, e->v_b2,
-                                  e->d_value, st));
+                                  e->d_value, st, e->v_scale));
     e->launches += 1;
     return SC_OK;
 }
@@ -732,7 +800,8 @@ static int encode_for_mode(sc_engine *e, const sc_position *d_pos, int n, cudaSt
     NvtxRange nv("scb200: encode planes");
     e->launches += 1;
     if (e->mode == SC_MODE_FP32 && !e->fp32_tc) return launch_encode_f32(d_pos, n, e->f_planes, e->d_meta, st);
-    if (e->fp16) return launch_encode_fp16(d_pos, n, reinterpret_cast<__half *>(e->h_planes), e->d_meta, st);
+    if (e->op == TC_OP_FP16) return launch_encode_fp16(d_pos, n, reinterpret_cast<__half *>(e->h_planes), e->d_meta, st);
+    if (e->op == TC_OP_E4M3) return launch_encode_e4m3(d_pos, n, reinterpret_cast<uint8_t *>(e->h_planes), e->d_meta, st);
     return launch_encode_bf16(d_pos, n, e->h_planes, e->d_meta, st);
 }
 
@@ -942,7 +1011,7 @@ static int predict_launch(sc_engine *e, int n, const sc_position *d_pos, const i
     e->launches += 1;
     SCB_CHECK(encode_for_mode(e, d_pos, n, st));
     const TcGather g{d_pos, d_moves, nullptr, d_cnt, d_priors, n};
-    const bool fused = tc16(e) && e->fuse_gather;
+    const bool fused = tc_mode(e) && e->fuse_gather;
     float *saved_value = e->d_value;
     e->d_value = d_value;
     int rc = run_network(e, n, st, fused ? &g : nullptr, fused ? e->ev_gen_done : nullptr);
@@ -1265,7 +1334,8 @@ const char *sc_last_error(void) { return g_err.c_str(); }
 int sc_create(const char *weights_blob_path, int device, int mode, int max_batch, sc_engine **out)
 {
     if (!out || !weights_blob_path || max_batch <= 0 ||
-        (mode != SC_MODE_FP32 && mode != SC_MODE_BF16 && mode != SC_MODE_FP32_FFMA && mode != SC_MODE_FP16)) {
+        (mode != SC_MODE_FP32 && mode != SC_MODE_BF16 && mode != SC_MODE_FP32_FFMA && mode != SC_MODE_FP16 &&
+         mode != SC_MODE_FP8)) {
         set_error("sc_create: bad argument");
         return SC_E_INVAL;
     }
@@ -1289,7 +1359,7 @@ int sc_create(const char *weights_blob_path, int device, int mode, int max_batch
     e->mode_requested = mode;
     e->mode = mode == SC_MODE_FP32_FFMA ? SC_MODE_FP32 : mode;
     e->fp32_tc = mode == SC_MODE_FP32;
-    e->fp16 = mode == SC_MODE_FP16;
+    e->op = mode == SC_MODE_FP16 ? TC_OP_FP16 : mode == SC_MODE_FP8 ? TC_OP_E4M3 : TC_OP_BF16;
     e->max_batch = max_batch;
     e->num_sms = prop.multiProcessorCount;
     int rc = SC_OK;
@@ -1301,7 +1371,7 @@ int sc_create(const char *weights_blob_path, int device, int mode, int max_batch
         if ((rc = load_weights(e, blob)) != SC_OK) break;
         if ((rc = alloc_buffers(e)) != SC_OK) break;
         if ((rc = upload_move_tables(e->stream)) != SC_OK) break;
-        if (tc16(e)) {
+        if (tc_mode(e)) {
             std::vector<TcTowerLayerDesc> d;
             d.push_back(TcTowerLayerDesc{e->stem.tc, e->h_planes, e->h_x, nullptr, 1});
             for (int i = 0; i < e->n_blocks; i++) {
@@ -1311,44 +1381,46 @@ int sc_create(const char *weights_blob_path, int device, int mode, int max_batch
             // the two 256-wide 1x1 head convolutions read the tower output tile by tile as well
             d.push_back(TcTowerLayerDesc{e->pol1.tc, e->h_x, e->h_t, nullptr, 0});
             d.push_back(TcTowerLayerDesc{e->val1.tc, e->h_x, e->h_y, nullptr, 1});
-            if ((rc = tc_tower_create(&e->tower, d.data(), (int)d.size(), e->alloc_boards, e->fp16)) != SC_OK) break;
-            // the same layers for the latency kernel
-            std::vector<LatLayerDesc> ld;
-            auto lat_layer = [&](const ConvW &c, const __nv_bfloat16 *in, void *out, const __nv_bfloat16 *resid, int relu,
-                                 int se, const SeW *sw) {
-                LatLayerDesc L{};
-                L.w = c.w_bf16;
-                L.taps = c.taps;
-                L.cin_pad = c.cin_pad;
-                L.in = in;
-                L.out = out;
-                L.resid = resid;
-                L.bias = c.bias;
-                L.gamma = c.gamma;
-                L.beta = c.beta;
-                L.relu = relu;
-                L.ln = c.gamma != nullptr;
-                L.se = se;
-                if (sw) {
-                    L.se_w1s8 = sw->w1s[0];
-                    L.se_w2s8 = sw->w2s[0];
-                    L.se_w1s4 = sw->w1s[1];
-                    L.se_w2s4 = sw->w2s[1];
-                    L.se_b1 = sw->b1;
-                    L.se_b2 = sw->b2;
+            if ((rc = tc_tower_create(&e->tower, d.data(), (int)d.size(), e->alloc_boards, e->op)) != SC_OK) break;
+            // the same layers for the latency kernel (fp8 is a throughput mode: it has none)
+            if (e->op != TC_OP_E4M3) {
+                std::vector<LatLayerDesc> ld;
+                auto lat_layer = [&](const ConvW &c, const __nv_bfloat16 *in, void *out, const __nv_bfloat16 *resid, int relu,
+                                     int se, const SeW *sw) {
+                    LatLayerDesc L{};
+                    L.w = c.w_bf16;
+                    L.taps = c.taps;
+                    L.cin_pad = c.cin_pad;
+                    L.in = in;
+                    L.out = out;
+                    L.resid = resid;
+                    L.bias = c.bias;
+                    L.gamma = c.gamma;
+                    L.beta = c.beta;
+                    L.relu = relu;
+                    L.ln = c.gamma != nullptr;
+                    L.se = se;
+                    if (sw) {
+                        L.se_w1s8 = sw->w1s[0];
+                        L.se_w2s8 = sw->w2s[0];
+                        L.se_w1s4 = sw->w1s[1];
+                        L.se_w2s4 = sw->w2s[1];
+                        L.se_b1 = sw->b1;
+                        L.se_b2 = sw->b2;
+                    }
+                    ld.push_back(L);
+                };
+                lat_layer(e->stem, e->h_planes, e->h_x, nullptr, 1, 0, nullptr);
+                for (int i = 0; i < e->n_blocks; i++) {
+                    lat_layer(e->conv1[i], e->h_x, e->h_t, nullptr, 1, 0, nullptr);
+                    const bool has_se = e->se[i].w1p != nullptr;
+                    lat_layer(e->conv2[i], e->h_t, e->h_x, e->h_x, 0, has_se ? 1 : 2, has_se ? &e->se[i] : nullptr);
                 }
-                ld.push_back(L);
-            };
-            lat_layer(e->stem, e->h_planes, e->h_x, nullptr, 1, 0, nullptr);
-            for (int i = 0; i < e->n_blocks; i++) {
-                lat_layer(e->conv1[i], e->h_x, e->h_t, nullptr, 1, 0, nullptr);
-                const bool has_se = e->se[i].w1p != nullptr;
-                lat_layer(e->conv2[i], e->h_t, e->h_x, e->h_x, 0, has_se ? 1 : 2, has_se ? &e->se[i] : nullptr);
+                lat_layer(e->pol1, e->h_x, e->h_t, nullptr, 0, 0, nullptr);
+                lat_layer(e->val1, e->h_x, e->h_y, nullptr, 1, 0, nullptr);
+                if ((rc = lat_tower_create(&e->lat, ld.data(), (int)ld.size(), e->alloc_boards, e->op == TC_OP_FP16)) != SC_OK) break;
+                e->lat_max_boards = lat_tower_max_boards(e->lat);
             }
-            lat_layer(e->pol1, e->h_x, e->h_t, nullptr, 0, 0, nullptr);
-            lat_layer(e->val1, e->h_x, e->h_y, nullptr, 1, 0, nullptr);
-            if ((rc = lat_tower_create(&e->lat, ld.data(), (int)ld.size(), e->alloc_boards, e->fp16)) != SC_OK) break;
-            e->lat_max_boards = lat_tower_max_boards(e->lat);
         }
         if (cudaDeviceSynchronize() != cudaSuccess) { rc = SC_E_CUDA; set_error("sync after weight upload failed"); break; }
     } while (0);
@@ -1440,7 +1512,7 @@ int sc_eval_device(sc_engine *e, int n, const void *d_pos, const void *d_moves, 
     e->d_value = static_cast<float *>(d_value_out);
     const TcGather g{pos, static_cast<const sc_move *>(d_moves), static_cast<const int32_t *>(d_move_off), nullptr,
                      static_cast<float *>(d_priors_out), n};
-    const bool fused = tc16(e) && e->fuse_gather;
+    const bool fused = tc_mode(e) && e->fuse_gather;
     int rc = run_network(e, n, st, fused ? &g : nullptr);
     e->d_value = saved;
     SCB_CHECK(rc);
@@ -1682,7 +1754,7 @@ int sc_eval_submit(sc_engine *e, int n, const sc_position *pos, const sc_move *m
         const int saved_timing = e->timing;
         e->timing = 0;  // asynchronous path never synchronises
         const TcGather g{io.pos, io.moves, nullptr, io.cnt, io.priors, n};
-        const bool fused = tc16(e) && e->fuse_gather;
+        const bool fused = tc_mode(e) && e->fuse_gather;
         float *saved_value = e->d_value;
         e->d_value = io.value;
         int rc = run_network(e, n, st, fused ? &g : nullptr);
@@ -1895,8 +1967,10 @@ int sc_forward_only(sc_engine *e, int n, const float *planes, const float *meta,
     SCB_CUDA(cudaMemcpy2DAsync(e->d_meta, 8 * 4, meta, SC_N_META * 4, SC_N_META * 4, (size_t)n, cudaMemcpyHostToDevice, st));
     if (e->mode == SC_MODE_FP32 && !e->fp32_tc)
         SCB_CHECK(launch_nchw_to_nhwc_f32(d_nchw, n, e->f_planes, st));
-    else if (e->fp16)
+    else if (e->op == TC_OP_FP16)
         SCB_CHECK(launch_nchw_to_nhwc_fp16(d_nchw, n, reinterpret_cast<__half *>(e->h_planes), st));
+    else if (e->op == TC_OP_E4M3)
+        SCB_CHECK(launch_nchw_to_nhwc_e4m3(d_nchw, n, reinterpret_cast<uint8_t *>(e->h_planes), st));
     else
         SCB_CHECK(launch_nchw_to_nhwc_bf16(d_nchw, n, e->h_planes, st));
     e->launches += 1;
@@ -1915,8 +1989,8 @@ int sc_debug_tower(sc_engine *e, int n, const sc_position *pos, int n_layers, in
                    uint16_t *y_out)
 {
     SCB_CHECK(check_owner(e, "sc_debug_tower"));
-    if (!e || !tc16(e) || n <= 0 || n > e->max_batch || !pos || !e->tower) {
-        set_error("sc_debug_tower: bad argument (bf16 / fp16 engines only)");
+    if (!e || !tc_mode(e) || n <= 0 || n > e->max_batch || !pos || !e->tower) {
+        set_error("sc_debug_tower: bad argument (bf16 / fp16 / fp8 engines only)");
         return SC_E_INVAL;
     }
     cudaStream_t st = e->stream;
@@ -1937,7 +2011,20 @@ int sc_debug_tower(sc_engine *e, int n, const sc_position *pos, int n_layers, in
         SCB_CHECK(rc);
     } else
         SCB_CHECK(tc_tower_launch(e->tower, n, e->num_sms, e->tower_group, st, n_layers));
-    const size_t bytes = (size_t)n * 64 * C_TOWER * 2;
+    const size_t count = (size_t)n * 64 * C_TOWER;
+    if (e->op == TC_OP_E4M3) {
+        // e4m3 bytes, widened to the fp16 bit patterns of the same values (exact)
+        std::vector<uint8_t> h(count);
+        const std::pair<uint16_t *, const void *> bufs[3] = {{x_out, e->h_x}, {t_out, e->h_t}, {y_out, e->h_y}};
+        for (const auto &b : bufs) {
+            if (!b.first) continue;
+            SCB_CUDA(cudaMemcpyAsync(h.data(), b.second, count, cudaMemcpyDeviceToHost, st));
+            SCB_CUDA(cudaStreamSynchronize(st));
+            for (size_t i = 0; i < count; i++) b.first[i] = __nv_cvt_fp8_to_halfraw((__nv_fp8_storage_t)h[i], __NV_E4M3).x;
+        }
+        return SC_OK;
+    }
+    const size_t bytes = count * 2;
     if (x_out) SCB_CUDA(cudaMemcpyAsync(x_out, e->h_x, bytes, cudaMemcpyDeviceToHost, st));
     if (t_out) SCB_CUDA(cudaMemcpyAsync(t_out, e->h_t, bytes, cudaMemcpyDeviceToHost, st));
     if (y_out) SCB_CUDA(cudaMemcpyAsync(y_out, e->h_y, bytes, cudaMemcpyDeviceToHost, st));

@@ -106,6 +106,19 @@ __device__ __forceinline__ void tc2_mma_bf16(uint32_t tmem_d, uint64_t desc_a, u
         "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
         : "memory");
 }
+// the same with 8-bit operands (kind::f8f6f4): K = 32 elements = 32 bytes per instruction, as kind::f16's K = 16
+__device__ __forceinline__ void tc2_mma_f8(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
+                                           uint32_t accumulate)
+{
+    asm volatile(
+        "{\n\t"
+        ".reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::2.kind::f8f6f4 [%0], %1, %2, %3, p;\n\t"
+        "}" ::"r"(tmem_d),
+        "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
+        : "memory");
+}
 // arrives on the barrier at the same shared-memory offset in BOTH CTAs of the pair
 __device__ __forceinline__ void tc2_commit_mc(uint32_t bar)
 {
@@ -155,6 +168,18 @@ __device__ __forceinline__ void tc_mma_bf16(uint32_t tmem_d, uint64_t desc_a, ui
         "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
         : "memory");
 }
+__device__ __forceinline__ void tc_mma_f8(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
+                                          uint32_t accumulate)
+{
+    asm volatile(
+        "{\n\t"
+        ".reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::f8f6f4 [%0], %1, %2, %3, p;\n\t"
+        "}" ::"r"(tmem_d),
+        "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
+        : "memory");
+}
 __device__ __forceinline__ void tc_commit(uint32_t bar)
 {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
@@ -195,18 +220,26 @@ __host__ __device__ constexpr uint32_t umma_idesc_bf16(int M, int N)
     return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
 
-// Tensor-core operand types of the 16-bit modes (kind::f16, fp32 accumulate): the kernels are templates on one of these,
-// so each type is its own instantiation and the bf16 code is unchanged by the fp16 one.  Both types are 2 bytes, so TMA
-// boxes, swizzle, descriptors and shared-memory layouts are the same.
-//   IDESC_AB  a_format / b_format bits of the instruction descriptor (bits 7-9 / 10-12: 0 = F16, 1 = BF16)
+// Tensor-core operand types (fp32 accumulate): the kernels are templates on one of these, so each type is its own
+// instantiation and the bf16 code is unchanged by the others.  A K chunk is one 128-byte swizzle row whatever the type
+// (BK * BYTES == 128), so TMA boxes, swizzle, descriptors and shared-memory layouts are the same in bytes.
+//   IDESC_AB  a_format / b_format bits of the instruction descriptor (bits 7-9 / 10-12; kind::f16: 0 = F16, 1 = BF16;
+//             kind::f8f6f4: 0 = E4M3)
+//   F8        the instruction kind: kind::f8f6f4 instead of kind::f16 (the format bits alone do not tell them apart)
 //   TMAP      tensor-map element type
+//   BYTES     bytes per element; BK = elements per K chunk
+//   SCALED    the weights carry a per-output-channel power-of-two scale that the epilogue applies (acc * s + bias)
+//   Park      the type the kernels keep internal values in (the SE layers' LayerNorm output, parked in shared memory)
 //   pack2     two floats -> two operands, round to nearest even, first argument in the low half
 //   lo, hi    the inverse: the low / high operand of a packed pair as float (exact)
 //   round     a float rounded to the operand type and back: a value the kernels park in that type
-//   unpack8   eight packed operands -> floats (the SE weights)
+//   unpack8   eight packed SE weights -> floats
 __device__ __forceinline__ void bf16x8_to_float(const uint4 &u, float (&f)[8]);
 struct OpBf16 {
     static constexpr uint32_t IDESC_AB = (1u << 7) | (1u << 10);
+    static constexpr bool F8 = false, SCALED = false;
+    static constexpr int BYTES = 2, BK = 64;
+    using Park = OpBf16;
     static constexpr CUtensorMapDataType TMAP = CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
     __device__ __forceinline__ static uint32_t pack2(float lo, float hi)
     {
@@ -221,6 +254,9 @@ struct OpBf16 {
 // fp16: 11 significant bits against bf16's 8; a value beyond +-65504 becomes +-inf, as in fp16 autocast
 struct OpFp16 {
     static constexpr uint32_t IDESC_AB = 0u;
+    static constexpr bool F8 = false, SCALED = false;
+    static constexpr int BYTES = 2, BK = 64;
+    using Park = OpFp16;
     static constexpr CUtensorMapDataType TMAP = CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
     __device__ __forceinline__ static uint32_t pack2(float lo, float hi)
     {
@@ -241,6 +277,53 @@ struct OpFp16 {
         }
     }
 };
+// fp8 e4m3 (SC_MODE_FP8): 4 significant bits, largest finite value 448.  A K chunk is 128 channels.  The weights are
+// e4m3 with a power-of-two scale per output channel (SCALED); a stored activation is e4m3 without a scale, saturated to
+// +-448 (satfinite).  The SE layers' parked LayerNorm output and the SE weights stay bf16.
+struct OpE4m3 {
+    static constexpr uint32_t IDESC_AB = 0u;
+    static constexpr bool F8 = true, SCALED = true;
+    static constexpr int BYTES = 1, BK = 128;
+    using Park = OpBf16;
+    static constexpr CUtensorMapDataType TMAP = CU_TENSOR_MAP_DATA_TYPE_UINT8;
+    // four floats -> four e4m3 (round to nearest even, satfinite), first argument in the lowest byte
+    __device__ __forceinline__ static uint32_t pack4(float a, float b, float c, float d)
+    {
+        uint16_t lo, hi;
+        asm("cvt.rn.satfinite.e4m3x2.f32 %0, %1, %2;" : "=h"(lo) : "f"(b), "f"(a));
+        asm("cvt.rn.satfinite.e4m3x2.f32 %0, %1, %2;" : "=h"(hi) : "f"(d), "f"(c));
+        return (uint32_t)lo | ((uint32_t)hi << 16);
+    }
+    // the inverse (exact: every e4m3 value is an fp16 value)
+    __device__ __forceinline__ static void unpack4(uint32_t w, float (&f)[4])
+    {
+        uint32_t h0, h1;
+        asm("cvt.rn.f16x2.e4m3x2 %0, %1;" : "=r"(h0) : "h"((uint16_t)(w & 0xffffu)));
+        asm("cvt.rn.f16x2.e4m3x2 %0, %1;" : "=r"(h1) : "h"((uint16_t)(w >> 16)));
+        const float2 p = __half22float2(*reinterpret_cast<const __half2 *>(&h0));
+        const float2 q = __half22float2(*reinterpret_cast<const __half2 *>(&h1));
+        f[0] = p.x;
+        f[1] = p.y;
+        f[2] = q.x;
+        f[3] = q.y;
+    }
+    __device__ __forceinline__ static void unpack8(const uint4 &u, float (&f)[8]) { bf16x8_to_float(u, f); }
+};
+static_assert(OpBf16::BK * OpBf16::BYTES == 128 && OpFp16::BK * OpFp16::BYTES == 128 && OpE4m3::BK * OpE4m3::BYTES == 128,
+              "a K chunk is one 128-byte swizzle row");
+// one MMA of operand type OT: 4 instructions cover a 128-byte row of K for every type (K = 16 x 2 B or 32 x 1 B)
+template <class OT>
+__device__ __forceinline__ void tc2_mma(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate)
+{
+    if constexpr (OT::F8) tc2_mma_f8(tmem_d, desc_a, desc_b, idesc, accumulate);
+    else tc2_mma_bf16(tmem_d, desc_a, desc_b, idesc, accumulate);
+}
+template <class OT>
+__device__ __forceinline__ void tc_mma(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate)
+{
+    if constexpr (OT::F8) tc_mma_f8(tmem_d, desc_a, desc_b, idesc, accumulate);
+    else tc_mma_bf16(tmem_d, desc_a, desc_b, idesc, accumulate);
+}
 // instruction descriptor of operand type OT (umma_idesc_bf16 for OpBf16)
 template <class OT> __host__ __device__ constexpr uint32_t umma_idesc(int M, int N)
 {

@@ -18,8 +18,10 @@
 //   D accumulates in TMEM (128 lanes x 256 fp32 columns per tile, two tiles = all 512
 //   columns, so the epilogue of tile i overlaps the MMAs of tile i+1).
 // One kernel template, tc_gemm_kernel<BN, EPI, A4D, CTA2, TOWER, OT>:
-//   * OT: the operand type, OpBf16 or OpFp16 (tc_ptx.cuh).  Activations, weights, the parked SE tile and the stored
-//     layer outputs are all of that type; the accumulator, LayerNorm, SE arithmetic and the head tails are fp32;
+//   * OT: the operand type, OpBf16, OpFp16 or OpE4m3 (tc_ptx.cuh).  Activations, weights and the stored layer outputs
+//     are of that type, the parked SE tile of OT::Park; the accumulator, LayerNorm, SE arithmetic and the head tails are
+//     fp32.  OpE4m3's K chunk is 128 channels (OT::BK), the same 128 bytes as 64 16-bit channels, and its epilogues
+//     apply the per-channel weight scale first (acc * scale + bias);
 //   * CTA2: every 256-wide convolution; clusters of two CTAs issue tcgen05.mma.cta_group::2 (256-row
 //     tiles, each CTA stages its own rows of A and half of the weight rows);
 //   * TOWER: the stem, all residual blocks and the two 256-wide head 1x1 convolutions run
@@ -83,6 +85,7 @@ struct alignas(64) TowerLayer {
     const float *se_b1, *se_b2;
     int taps, kchunks, relu, se;
     int ln;                              // 0: no LayerNorm (BatchNorm folded at export): y = acc + bias
+    const float *scale;                  // scaled operand types (OpE4m3): per-channel weight scales, y = acc * scale + bias
 };
 
 struct TcArgs {
@@ -109,6 +112,8 @@ struct TcArgs {
     int group;                           // TOWER: tiles per CTA carried through all layers together (0 = all)
     TcGather gather;                     // EPI_LN73_GATHER: legal moves in, priors out
     TcValueFinish vfin;                  // EPI_RAW: value head tail fused into the split-K GEMM (counters != nullptr)
+    const float *scale;                  // scaled operand types: per-output-channel weight scales (EPI_RAW: of the
+                                         // hidden units, applied after the split sum)
 };
 
 __device__ __forceinline__ void epi_bar_sync() { asm volatile("bar.sync 1, 256;" ::: "memory"); }
@@ -214,7 +219,8 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     float *s_bias = reinterpret_cast<float *>(smem + Cfg::RING_BYTES);
     float *s_gamma = s_bias + 256;
     float *s_beta = s_gamma + 256;
-    float *s_mean = s_beta + 256 + 1024;  // [2 boards][256] (the 4 KB before it are unused)
+    float *s_scale = s_beta + 256;        // OT::SCALED: the weight scales [256] (the 4 KB up to s_mean are otherwise unused)
+    float *s_mean = s_beta + 256 + 1024;  // [2 boards][256]
     float *s_hid = s_mean + 512;    // [2][128]
     float *s_gate = s_hid + 256;    // [2][256]
     float *s_stat = s_gate + 512;   // [2 column halves][128 rows][sum, sumsq]
@@ -254,17 +260,29 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
         int taps, kchunks, relu;
         bool se, ln;
         bool se_fc;  // se: squeeze-excitation gate (false with se: residual + ReLU only, `use_se=False`)
+        const float *scale;
     };
     auto layer_view = [&](int l) -> LayerView {
         if constexpr (TOWER) {
             const TowerLayer &T = args.layers[l];
             return LayerView{&T.map_a, &T.map_w, T.out, T.resid, T.bias, T.gamma, T.beta, T.se_w1p, T.se_w2p, T.se_b1, T.se_b2,
-                             T.taps, T.kchunks, T.relu, T.se != 0, T.ln != 0, T.se == 1};
+                             T.taps, T.kchunks, T.relu, T.se != 0, T.ln != 0, T.se == 1, OT::SCALED ? T.scale : nullptr};
         } else {
             return LayerView{&map_a, &map_w, args.out, args.resid, args.bias, args.gamma, args.beta, args.se_w1p, args.se_w2p,
                              args.se_b1, args.se_b2, args.taps, args.kchunks, args.relu, EPI == EPI_LN_SE, args.ln != 0,
-                             EPI == EPI_LN_SE && args.se_w1p != nullptr};
+                             EPI == EPI_LN_SE && args.se_w1p != nullptr, OT::SCALED ? args.scale : nullptr};
         }
+    };
+    // a = acc + bias of channel c (scaled types: acc * scale + bias; the scale is a power of two, so the product is exact
+    // and the fma rounds once, like the add)
+    auto acc_bias = [&](uint32_t acc, int c) -> float {
+        if constexpr (OT::SCALED) return __fmaf_rn(__uint_as_float(acc), s_scale[c], s_bias[c]);
+        else return __fadd_rn(__uint_as_float(acc), s_bias[c]);
+    };
+    // the same for the narrow head epilogues, whose unscaled form is a contractible add
+    auto head_a = [&](uint32_t acc, int c) -> float {
+        if constexpr (OT::SCALED) return __fmaf_rn(__uint_as_float(acc), s_scale[c], s_bias[c]);
+        else return __uint_as_float(acc) + s_bias[c];
     };
     const int n_layers = TOWER ? args.n_layers : 1;
 
@@ -274,6 +292,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
             s_bias[i] = i < NV ? args.bias[i] : 0.f;
             s_gamma[i] = i < NV ? (args.ln ? args.gamma[i] : 1.f) : 0.f;
             s_beta[i] = i < NV && args.ln ? args.beta[i] : 0.f;
+            if constexpr (OT::SCALED) s_scale[i] = i < NV ? args.scale[i] : 0.f;
         }
     }
     if (threadIdx.x == 0) {
@@ -356,7 +375,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                                 // both CTAs load into their own shared memory and complete on the LEADER's barrier,
                                 // which the leader alone arms with the bytes of both
                                 if (cta_rank == 0) mbar_expect_tx(afull_bar(astage), 2 * A_BOX);
-                                tma2_load_4d(abox_addr(astage), P.ma, afull_bar(astage), ca * TC_BK, nd == 3 ? dxi - 1 : 0, tile * 2, -1);
+                                tma2_load_4d(abox_addr(astage), P.ma, afull_bar(astage), ca * OT::BK, nd == 3 ? dxi - 1 : 0, tile * 2, -1);
                             }
                             __syncwarp();
                             for (int dyi = 0; dyi < nd; dyi++) {
@@ -366,7 +385,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                                 if (args.prof) pc_wait_empty += clock64() - t1;
                                 if (elect_one()) {
                                     if (cta_rank == 0) mbar_expect_tx(bfull_bar(bstage), 2 * B_TILE);
-                                    tma2_load_2d(btile_addr(bstage), P.mw, bfull_bar(bstage), cb * TC_BK,
+                                    tma2_load_2d(btile_addr(bstage), P.mw, bfull_bar(bstage), cb * OT::BK,
                                                  tap * BN + (int)cta_rank * (BN / 2));
                                 }
                                 __syncwarp();
@@ -395,11 +414,11 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                         if (!elect_one()) {
                         } else if (A4D) {
                             mbar_expect_tx(full_bar(stage), STAGE_BYTES);
-                            tma_load_4d(a_dst, &map_a, full_bar(stage), kc * TC_BK, dx, dy, tile * 2);
-                            tma_load_2d(b_dst, &map_w, full_bar(stage), kc * TC_BK, tap * BN);
+                            tma_load_4d(a_dst, &map_a, full_bar(stage), kc * OT::BK, dx, dy, tile * 2);
+                            tma_load_2d(b_dst, &map_w, full_bar(stage), kc * OT::BK, tap * BN);
                         } else {
                             mbar_expect_tx(full_bar(stage), STAGE_BYTES);
-                            const int k0 = (split * P.kchunks + kc) * TC_BK;
+                            const int k0 = (split * P.kchunks + kc) * OT::BK;
                             tma_load_2d(a_dst, &map_a, full_bar(stage), k0, tile * TC_BM);
                             tma_load_2d(b_dst, &map_w, full_bar(stage), k0, 0);
                         }
@@ -451,7 +470,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                             if (elect_one()) {
 #pragma unroll
                                 for (int k = 0; k < TC_BK / 16; k++)
-                                    tc2_mma_bf16(d_tmem, da + (uint64_t)(k * 2), db + (uint64_t)(k * 2), idesc, (acc | (uint32_t)k) != 0);
+                                    tc2_mma<OT>(d_tmem, da + (uint64_t)(k * 2), db + (uint64_t)(k * 2), idesc, (acc | (uint32_t)k) != 0);
                                 tc2_commit_mc(bempty_bar(rb));
                                 if (dyi == nd - 1) tc2_commit_mc(aempty_bar(ra));
                             }
@@ -481,8 +500,8 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                     const uint64_t db = umma_desc_sw128(a_addr + TC_A_BYTES);
                     if (elect_one()) {
 #pragma unroll
-                        for (int k = 0; k < TC_BK / 16; k++)  // +32 bytes per K=16 slice inside the 128-byte swizzle row
-                            tc_mma_bf16(d_tmem, da + (uint64_t)(k * 2), db + (uint64_t)(k * 2), idesc,
+                        for (int k = 0; k < TC_BK / 16; k++)  // +32 bytes per instruction (K = 16 x 2 B or 32 x 1 B) inside the 128-byte row
+                            tc_mma<OT>(d_tmem, da + (uint64_t)(k * 2), db + (uint64_t)(k * 2), idesc,
                                         (uint32_t)((kb | k) != 0));
                         tc_commit(empty_bar(stage));
                     }
@@ -523,6 +542,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
             s_bias[te] = P.bias[te];
             s_gamma[te] = P.ln ? P.gamma[te] : 1.f;
             s_beta[te] = P.ln ? P.beta[te] : 0.f;
+            if constexpr (OT::SCALED) s_scale[te] = P.scale[te];
             epi_bar_sync();
         }
         // end of a tile in the tower kernel: the tile's output (generic-proxy stores) is handed to the TMA
@@ -618,9 +638,10 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                         __threadfence();
                         const float *pre = static_cast<const float *>(args.out);
                         const int nsp = args.n_splits;
-                        float wm[SC_N_META][4], b1v[4], w2v[4];
+                        float wm[SC_N_META][4], b1v[4], w2v[4], sv[4];
 #pragma unroll
                         for (int i = 0; i < 4; i++) {
+                            if constexpr (OT::SCALED) sv[i] = args.scale[4 * lane + i];
                             b1v[i] = F.b1[4 * lane + i];
                             w2v[i] = F.w2[4 * lane + i];
 #pragma unroll
@@ -664,6 +685,9 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                                 if (grow[u] >= args.m_rows) continue;  // warp-uniform
                                 const float *mt = F.meta + (size_t)grow[u] * 8;
                                 float hv[4] = {h[u].x, h[u].y, h[u].z, h[u].w};
+                                if constexpr (OT::SCALED)  // the hidden unit's weight scale, after the split sum (exact)
+#pragma unroll
+                                    for (int i = 0; i < 4; i++) hv[i] = __fmul_rn(hv[i], sv[i]);
                                 float acc = 0.f;
 #pragma unroll
                                 for (int i = 0; i < 4; i++) {
@@ -695,7 +719,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                     uint32_t r[16];
                     tmem_ld16(taddr + ch * 16, r);
 #pragma unroll
-                    for (int j = 0; j < 16; j++) v[ch * 16 + j] = __uint_as_float(r[j]) + s_bias[ch * 16 + j];
+                    for (int j = 0; j < 16; j++) v[ch * 16 + j] = head_a(r[j], ch * 16 + j);
                 }
                 tc_fence_before();
                 mbar_arrive(tempty_bar(as));  // the accumulator is free for the MMAs of tile it + 2
@@ -770,7 +794,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                     tmem_ld16(taddr + ch * 16, r);
 #pragma unroll
                     for (int j = 0; j < 16; j++)
-                        if (ch * 16 + j < C_POLICY) sum += __uint_as_float(r[j]) + s_bias[ch * 16 + j];
+                        if (ch * 16 + j < C_POLICY) sum += head_a(r[j], ch * 16 + j);
                 }
                 const float mean = args.ln ? sum * (1.f / C_POLICY) : 0.f;
                 float sq = 0.f;
@@ -780,7 +804,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
 #pragma unroll
                     for (int j = 0; j < 16; j++)
                         if (ch * 16 + j < C_POLICY) {
-                            float d = __uint_as_float(r[j]) + s_bias[ch * 16 + j] - mean;
+                            float d = head_a(r[j], ch * 16 + j) - mean;
                             sq = fmaf(d, d, sq);
                         }
                 }
@@ -798,7 +822,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
 #pragma unroll
                         for (int i = 0; i < 4; i++) {
                             const int c = ch * 16 + 4 * q + i;
-                            y[i] = c < C_POLICY ? (__uint_as_float(r[4 * q + i]) + s_bias[c] - mean) * rstd * s_gamma[c] + s_beta[c] : 0.f;
+                            y[i] = c < C_POLICY ? (head_a(r[4 * q + i], c) - mean) * rstd * s_gamma[c] + s_beta[c] : 0.f;
                         }
                         v[q] = make_uint4(__float_as_uint(y[0]), __float_as_uint(y[1]), __float_as_uint(y[2]), __float_as_uint(y[3]));
                     }
@@ -823,8 +847,8 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                         float a0[32], a1[32];
 #pragma unroll
                         for (int j = 0; j < 32; j++) {
-                            a0[j] = __fadd_rn(__uint_as_float(r[j]), s_bias[c0 + ch * 32 + j]);
-                            a1[j] = __fadd_rn(__uint_as_float(r2[j]), s_bias[c0 + ch * 32 + 32 + j]);
+                            a0[j] = acc_bias(r[j], c0 + ch * 32 + j);
+                            a1[j] = acc_bias(r2[j], c0 + ch * 32 + 32 + j);
                         }
                         ln_chunk_stats(a0, pa.x, pa.y);
                         ln_chunk_stats(a1, pb.x, pb.y);
@@ -866,7 +890,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
 #pragma unroll
                         for (int j = 0; j < 32; j++) {
                             const int c = c0 + ch * 32 + j;
-                            y[j] = ln_apply(__fadd_rn(__uint_as_float(cur[j]), s_bias[c]), mean, rstd, s_gamma[c], s_beta[c]);
+                            y[j] = ln_apply(acc_bias(cur[j], c), mean, rstd, s_gamma[c], s_beta[c]);
                         }
                         if constexpr (YSMEM) {
                             // keep LN(acc) in the operand type in shared memory: the final pass then needs neither
@@ -875,7 +899,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                             for (int q = 0; q < 4; q++) {
                                 uint32_t pw[4];
 #pragma unroll
-                                for (int i = 0; i < 4; i++) pw[i] = OT::pack2(y[8 * q + 2 * i], y[8 * q + 2 * i + 1]);
+                                for (int i = 0; i < 4; i++) pw[i] = OT::Park::pack2(y[8 * q + 2 * i], y[8 * q + 2 * i + 1]);
                                 const int chunk = (c0 + ch * 32) / 8 + q;
                                 *reinterpret_cast<uint4 *>(s_y + orow * 512 + ((chunk ^ (orow & 7)) << 4)) =
                                     make_uint4(pw[0], pw[1], pw[2], pw[3]);
@@ -1004,61 +1028,119 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                         g1[0] = b0.x; g1[1] = b0.y; g1[2] = b0.z; g1[3] = b0.w; g1[4] = b1.x; g1[5] = b1.y; g1[6] = b1.z; g1[7] = b1.w;
                     }
                     const size_t tile_row0 = (size_t)tile * TC_BM;
-                    const uint4 *xg = reinterpret_cast<const uint4 *>(P.resid + tile_row0 * BN) + chunk;
-                    uint4 *og = reinterpret_cast<uint4 *>(static_cast<uint16_t *>(P.out) + tile_row0 * BN) + chunk;
+                    if constexpr (OT::BYTES == 2) {
+                        const uint4 *xg = reinterpret_cast<const uint4 *>(P.resid + tile_row0 * BN) + chunk;
+                        uint4 *og = reinterpret_cast<uint4 *>(static_cast<uint16_t *>(P.out) + tile_row0 * BN) + chunk;
 #pragma unroll
-                    for (int i0 = 0; i0 < 16; i0 += 8) {
-                        uint4 xv[8];
+                        for (int i0 = 0; i0 < 16; i0 += 8) {
+                            uint4 xv[8];
 #pragma unroll
-                        for (int u = 0; u < 8; u++) xv[u] = xg[(size_t)(r0 + 8 * (i0 + u)) * (BN / 8)];
+                            for (int u = 0; u < 8; u++) xv[u] = xg[(size_t)(r0 + 8 * (i0 + u)) * (BN / 8)];
 #pragma unroll
-                        for (int u = 0; u < 8; u++) {
-                            const int rr = r0 + 8 * (i0 + u);
-                            const uint4 yv = *reinterpret_cast<const uint4 *>(s_y + rr * 512 + ((chunk ^ (rr & 7)) << 4));
-                            const float *g = (i0 + u) < 8 ? g0 : g1;  // rows 0..63 are the tile's first board
-                            const uint32_t yw[4] = {yv.x, yv.y, yv.z, yv.w};
-                            const uint32_t xw[4] = {xv[u].x, xv[u].y, xv[u].z, xv[u].w};
-                            uint32_t ow[4];
+                            for (int u = 0; u < 8; u++) {
+                                const int rr = r0 + 8 * (i0 + u);
+                                const uint4 yv = *reinterpret_cast<const uint4 *>(s_y + rr * 512 + ((chunk ^ (rr & 7)) << 4));
+                                const float *g = (i0 + u) < 8 ? g0 : g1;  // rows 0..63 are the tile's first board
+                                const uint32_t yw[4] = {yv.x, yv.y, yv.z, yv.w};
+                                const uint32_t xw[4] = {xv[u].x, xv[u].y, xv[u].z, xv[u].w};
+                                uint32_t ow[4];
 #pragma unroll
-                            for (int k = 0; k < 4; k++) {
-                                const float o0 = fmaxf(fmaf(g[2 * k], OT::lo(yw[k]), OT::lo(xw[k])), 0.f);
-                                const float o1 = fmaxf(fmaf(g[2 * k + 1], OT::hi(yw[k]), OT::hi(xw[k])), 0.f);
-                                ow[k] = OT::pack2(o0, o1);
+                                for (int k = 0; k < 4; k++) {
+                                    const float o0 = fmaxf(fmaf(g[2 * k], OT::lo(yw[k]), OT::lo(xw[k])), 0.f);
+                                    const float o1 = fmaxf(fmaf(g[2 * k + 1], OT::hi(yw[k]), OT::hi(xw[k])), 0.f);
+                                    ow[k] = OT::pack2(o0, o1);
+                                }
+                                og[(size_t)rr * (BN / 8)] = make_uint4(ow[0], ow[1], ow[2], ow[3]);
                             }
-                            og[(size_t)rr * (BN / 8)] = make_uint4(ow[0], ow[1], ow[2], ow[3]);
+                        }
+                    } else {
+                        // 1-byte operands: the chunk's 8 channels are 8 bytes of x and of the output; y is parked in
+                        // OT::Park (bf16)
+                        const uint2 *xg = reinterpret_cast<const uint2 *>(reinterpret_cast<const uint8_t *>(P.resid) + tile_row0 * BN) + chunk;
+                        uint2 *og = reinterpret_cast<uint2 *>(static_cast<uint8_t *>(P.out) + tile_row0 * BN) + chunk;
+#pragma unroll
+                        for (int i0 = 0; i0 < 16; i0 += 8) {
+                            uint2 xv[8];
+#pragma unroll
+                            for (int u = 0; u < 8; u++) xv[u] = xg[(size_t)(r0 + 8 * (i0 + u)) * (BN / 8)];
+#pragma unroll
+                            for (int u = 0; u < 8; u++) {
+                                const int rr = r0 + 8 * (i0 + u);
+                                const uint4 yv = *reinterpret_cast<const uint4 *>(s_y + rr * 512 + ((chunk ^ (rr & 7)) << 4));
+                                const float *g = (i0 + u) < 8 ? g0 : g1;
+                                const uint32_t yw[4] = {yv.x, yv.y, yv.z, yv.w};
+                                float x[8], o[8];
+                                OT::unpack4(xv[u].x, *reinterpret_cast<float(*)[4]>(x));
+                                OT::unpack4(xv[u].y, *reinterpret_cast<float(*)[4]>(x + 4));
+#pragma unroll
+                                for (int k = 0; k < 4; k++) {
+                                    o[2 * k] = fmaxf(fmaf(g[2 * k], OT::Park::lo(yw[k]), x[2 * k]), 0.f);
+                                    o[2 * k + 1] = fmaxf(fmaf(g[2 * k + 1], OT::Park::hi(yw[k]), x[2 * k + 1]), 0.f);
+                                }
+                                og[(size_t)rr * (BN / 8)] = make_uint2(OT::pack4(o[0], o[1], o[2], o[3]), OT::pack4(o[4], o[5], o[6], o[7]));
+                            }
                         }
                     }
                     if (prof) pe_final += clock64() - tp2;
                     tile_done(slot);
                     continue;  // the accumulator was released after the pooling pass
                 }
-                // ---- final pass of the LayerNorm-only layers: y (recomputed from TMEM), ReLU, 16-bit store ------
-                uint8_t *gtile = reinterpret_cast<uint8_t *>(static_cast<uint16_t *>(P.out) + (size_t)tile * TC_BM * BN + c0);
-                uint32_t rm[32];
-                tmem_ld32(tcol, r);
-#pragma unroll
-                for (int ch = 0; ch < 4; ch++) {
-                    if (ch < 3) tmem_ld32_nowait(tcol + (ch + 1) * 32, (ch & 1) ? r : rm);
-                    const uint32_t(&cur)[32] = (ch & 1) ? rm : r;
+                // ---- final pass of the LayerNorm-only layers: y (recomputed from TMEM), ReLU, store in the operand type --
+                if constexpr (OT::BYTES == 1) {
+                    // 1-byte operands: two 32-channel chunks make the lane's 64 bytes of the staged store
+                    uint8_t *gtile = static_cast<uint8_t *>(P.out) + (size_t)tile * TC_BM * BN + c0;
+                    uint32_t rm[32];
                     uint4 pk[4];
+                    tmem_ld32(tcol, r);
 #pragma unroll
-                    for (int j = 0; j < 16; j++) {
-                        const int c = c0 + ch * 32 + 2 * j;
-                        float y0 = ln_apply(__fadd_rn(__uint_as_float(cur[2 * j]), s_bias[c]), mean, rstd, s_gamma[c], s_beta[c]);
-                        float y1 = ln_apply(__fadd_rn(__uint_as_float(cur[2 * j + 1]), s_bias[c + 1]), mean, rstd, s_gamma[c + 1],
-                                            s_beta[c + 1]);
-                        if (P.relu) {
-                            y0 = fmaxf(y0, 0.f);
-                            y1 = fmaxf(y1, 0.f);
+                    for (int ch = 0; ch < 4; ch++) {
+                        if (ch < 3) tmem_ld32_nowait(tcol + (ch + 1) * 32, (ch & 1) ? r : rm);
+                        const uint32_t(&cur)[32] = (ch & 1) ? rm : r;
+                        uint32_t w[8];
+#pragma unroll
+                        for (int j = 0; j < 8; j++) {
+                            float y[4];
+#pragma unroll
+                            for (int i = 0; i < 4; i++) {
+                                const int c = c0 + ch * 32 + 4 * j + i;
+                                y[i] = ln_apply(acc_bias(cur[4 * j + i], c), mean, rstd, s_gamma[c], s_beta[c]);
+                                if (P.relu) y[i] = fmaxf(y[i], 0.f);
+                            }
+                            w[j] = OT::pack4(y[0], y[1], y[2], y[3]);
                         }
-                        const uint32_t hv = OT::pack2(y0, y1);
-                        if ((j & 3) == 0) pk[j >> 2].x = hv;
-                        else if ((j & 3) == 1) pk[j >> 2].y = hv;
-                        else if ((j & 3) == 2) pk[j >> 2].z = hv;
-                        else pk[j >> 2].w = hv;
+                        pk[(ch & 1) * 2] = make_uint4(w[0], w[1], w[2], w[3]);
+                        pk[(ch & 1) * 2 + 1] = make_uint4(w[4], w[5], w[6], w[7]);
+                        if (ch & 1) staged_store_64B_hbw(stg, lane, pk, gtile + (ch - 1) * 32, (size_t)BN, quad);
+                        if (ch < 3) tmem_wait_ld();
                     }
-                    staged_store_64B_hbw(stg, lane, pk, gtile + ch * 64, (size_t)BN * 2, quad);
-                    if (ch < 3) tmem_wait_ld();
+                } else {
+                    uint8_t *gtile = reinterpret_cast<uint8_t *>(static_cast<uint16_t *>(P.out) + (size_t)tile * TC_BM * BN + c0);
+                    uint32_t rm[32];
+                    tmem_ld32(tcol, r);
+#pragma unroll
+                    for (int ch = 0; ch < 4; ch++) {
+                        if (ch < 3) tmem_ld32_nowait(tcol + (ch + 1) * 32, (ch & 1) ? r : rm);
+                        const uint32_t(&cur)[32] = (ch & 1) ? rm : r;
+                        uint4 pk[4];
+#pragma unroll
+                        for (int j = 0; j < 16; j++) {
+                            const int c = c0 + ch * 32 + 2 * j;
+                            float y0 = ln_apply(__fadd_rn(__uint_as_float(cur[2 * j]), s_bias[c]), mean, rstd, s_gamma[c], s_beta[c]);
+                            float y1 = ln_apply(__fadd_rn(__uint_as_float(cur[2 * j + 1]), s_bias[c + 1]), mean, rstd, s_gamma[c + 1],
+                                                s_beta[c + 1]);
+                            if (P.relu) {
+                                y0 = fmaxf(y0, 0.f);
+                                y1 = fmaxf(y1, 0.f);
+                            }
+                            const uint32_t hv = OT::pack2(y0, y1);
+                            if ((j & 3) == 0) pk[j >> 2].x = hv;
+                            else if ((j & 3) == 1) pk[j >> 2].y = hv;
+                            else if ((j & 3) == 2) pk[j >> 2].z = hv;
+                            else pk[j >> 2].w = hv;
+                        }
+                        staged_store_64B_hbw(stg, lane, pk, gtile + ch * 64, (size_t)BN * 2, quad);
+                        if (ch < 3) tmem_wait_ld();
+                    }
                 }
                 if (prof) pe_final += clock64() - tp2;
             }
@@ -1120,7 +1202,8 @@ struct ActMap {
 struct TcConv {
     CUtensorMap map_w;
     int taps, k_per_tap, bn, epi;
-    bool fp16 = false;                     // operand type: OpFp16 instead of OpBf16
+    TcOp op = TC_OP_BF16;                  // operand type
+    const float *scale = nullptr;          // TC_OP_E4M3: per-output-channel weight scales
     int split_pairs = 0, split_kreal = 0;  // FP32 parity mode: (A plane, B plane) pairs of the bf16x3 split
     uint8_t split_ap[8] = {0}, split_bp[8] = {0};
     const float *bias, *gamma, *beta;
@@ -1149,12 +1232,17 @@ int tc_encode_map(CUtensorMap *m, CUtensorMapDataType dt, const void *ptr, int r
     return SC_OK;
 }
 
-// activations as a 4-D tensor {C, file, rank, board}, box = 64 channels of two whole boards
+// bytes per element of a tensor-map type, and the channels of one 128-byte K chunk
+static cuuint64_t tmap_bytes(CUtensorMapDataType dt) { return dt == CU_TENSOR_MAP_DATA_TYPE_UINT8 ? 1 : 2; }
+static cuuint32_t tmap_bk(CUtensorMapDataType dt) { return (cuuint32_t)(128 / tmap_bytes(dt)); }
+
+// activations as a 4-D tensor {C, file, rank, board}, box = one K chunk of channels of two whole boards
 static int make_act_map_4d(CUtensorMapDataType dt, const void *ptr, int boards, int c, CUtensorMap *m)
 {
+    const cuuint64_t eb = tmap_bytes(dt);
     cuuint64_t dims[4] = {(cuuint64_t)c, 8, 8, (cuuint64_t)boards};
-    cuuint64_t strides[3] = {(cuuint64_t)c * 2, (cuuint64_t)c * 16, (cuuint64_t)c * 128};
-    cuuint32_t box[4] = {TC_BK, 8, 8, 2};
+    cuuint64_t strides[3] = {(cuuint64_t)c * eb, (cuuint64_t)c * 8 * eb, (cuuint64_t)c * 64 * eb};
+    cuuint32_t box[4] = {tmap_bk(dt), 8, 8, 2};
     return tc_encode_map(m, dt, ptr, 4, dims, strides, box, "activations 4d");
 }
 
@@ -1162,18 +1250,19 @@ static int make_act_map_4d(CUtensorMapDataType dt, const void *ptr, int boards, 
 // shared memory with rows ordered (rank, board, file), so the three dy taps are 2 KB apart in ONE box
 int tc_make_act_map_hbw(CUtensorMapDataType dt, const void *ptr, int boards, int c, CUtensorMap *m)
 {
+    const cuuint64_t eb = tmap_bytes(dt);
     cuuint64_t dims[4] = {(cuuint64_t)c, 8, (cuuint64_t)boards, 8};
-    cuuint64_t strides[3] = {(cuuint64_t)c * 2, (cuuint64_t)c * 128, (cuuint64_t)c * 16};
-    cuuint32_t box[4] = {TC_BK, 8, 2, 10};
+    cuuint64_t strides[3] = {(cuuint64_t)c * eb, (cuuint64_t)c * 64 * eb, (cuuint64_t)c * 8 * eb};
+    cuuint32_t box[4] = {tmap_bk(dt), 8, 2, 10};
     return tc_encode_map(m, dt, ptr, 4, dims, strides, box, "activations (rank, board, file)");
 }
 
-// plain row-major [rows][k] matrix, box = 64 k x 128 rows
+// plain row-major [rows][k] matrix, box = one K chunk x 128 rows
 static int make_act_map_2d(CUtensorMapDataType dt, const void *ptr, int rows, int k, CUtensorMap *m)
 {
     cuuint64_t dims[2] = {(cuuint64_t)k, (cuuint64_t)rows};
-    cuuint64_t strides[1] = {(cuuint64_t)k * 2};
-    cuuint32_t box[2] = {TC_BK, TC_BM};
+    cuuint64_t strides[1] = {(cuuint64_t)k * tmap_bytes(dt)};
+    cuuint32_t box[2] = {tmap_bk(dt), TC_BM};
     return tc_encode_map(m, dt, ptr, 2, dims, strides, box, "activations 2d");
 }
 
@@ -1197,13 +1286,21 @@ template <class OT> static int set_conv_attrs()
     return SC_OK;
 }
 
-static CUtensorMapDataType tmap_type(bool fp16) { return fp16 ? OpFp16::TMAP : OpBf16::TMAP; }
+static CUtensorMapDataType tmap_type(TcOp op)
+{
+    return op == TC_OP_E4M3 ? OpE4m3::TMAP : op == TC_OP_FP16 ? OpFp16::TMAP : OpBf16::TMAP;
+}
 
 int tc_conv_create(TcConv **out, const __nv_bfloat16 *w, int taps, int k_per_tap, int bn, int epi, const float *bias,
-                   const float *gamma, const float *beta, bool fp16)
+                   const float *gamma, const float *beta, TcOp op, const float *scale)
 {
+    if ((op == TC_OP_E4M3) != (scale != nullptr) || k_per_tap % tc_op_bk(op) != 0) {
+        set_error("tc_conv_create: e4m3 weights need their scales (and only they), K a whole number of chunks");
+        return SC_E_INVAL;
+    }
     TcConv *c = new TcConv();
-    c->fp16 = fp16;
+    c->op = op;
+    c->scale = scale;
     c->taps = taps;
     c->k_per_tap = k_per_tap;
     c->bn = bn;
@@ -1212,23 +1309,24 @@ int tc_conv_create(TcConv **out, const __nv_bfloat16 *w, int taps, int k_per_tap
     c->gamma = gamma;
     c->beta = beta;
     // weights [taps * bn rows][k_per_tap], K-major
+    const CUtensorMapDataType dt = tmap_type(op);
     cuuint64_t dims[2] = {(cuuint64_t)k_per_tap, (cuuint64_t)taps * bn};
-    cuuint64_t strides[1] = {(cuuint64_t)k_per_tap * 2};
-    cuuint32_t box[2] = {TC_BK, (cuuint32_t)(bn == 256 ? bn / 2 : bn)};
-    int rc = tc_encode_map(&c->map_w, tmap_type(fp16), w, 2, dims, strides, box, "weights");
+    cuuint64_t strides[1] = {(cuuint64_t)k_per_tap * tmap_bytes(dt)};
+    cuuint32_t box[2] = {tmap_bk(dt), (cuuint32_t)(bn == 256 ? bn / 2 : bn)};
+    int rc = tc_encode_map(&c->map_w, dt, w, 2, dims, strides, box, "weights");
     if (rc != SC_OK) {
         delete c;
         return rc;
     }
     // function attributes belong to the device (context): set them once per device, not once per process
     static std::mutex attr_mu;
-    static std::map<std::pair<int, bool>, bool> attr_done;
+    static std::map<std::pair<int, int>, bool> attr_done;
     int dev = 0;
     SCB_CUDA(cudaGetDevice(&dev));
     std::lock_guard<std::mutex> lk(attr_mu);
-    bool &attr_set = attr_done[{dev, fp16}];
+    bool &attr_set = attr_done[{dev, (int)op}];
     if (!attr_set) {
-        SCB_CHECK(fp16 ? set_conv_attrs<OpFp16>() : set_conv_attrs<OpBf16>());
+        SCB_CHECK(op == TC_OP_E4M3 ? set_conv_attrs<OpE4m3>() : op == TC_OP_FP16 ? set_conv_attrs<OpFp16>() : set_conv_attrs<OpBf16>());
         attr_set = true;
     }
     *out = c;
@@ -1316,10 +1414,10 @@ static int prof_buffer(int num_sms, cudaStream_t st, long long **out)
 struct TcTower {
     TowerLayer *d_layers = nullptr;
     int n_layers = 0;
-    bool fp16 = false;
+    TcOp op = TC_OP_BF16;
 };
 
-int tc_tower_create(TcTower **out, const TcTowerLayerDesc *descs, int n, int boards_alloc, bool fp16)
+int tc_tower_create(TcTower **out, const TcTowerLayerDesc *descs, int n, int boards_alloc, TcOp op)
 {
     std::vector<TowerLayer> h((size_t)n);
     for (int i = 0; i < n; i++) {
@@ -1328,12 +1426,12 @@ int tc_tower_create(TcTower **out, const TcTowerLayerDesc *descs, int n, int boa
             set_error("tc_tower_create: layer is not a 256-wide tower convolution");
             return SC_E_INVAL;
         }
-        if (c->fp16 != fp16) {
+        if (c->op != op) {
             set_error("tc_tower_create: layer of another operand type");
             return SC_E_INVAL;
         }
         memset(&h[i], 0, sizeof(TowerLayer));
-        SCB_CHECK(tc_make_act_map_hbw(tmap_type(fp16), descs[i].in, boards_alloc, c->k_per_tap, &h[i].map_a));
+        SCB_CHECK(tc_make_act_map_hbw(tmap_type(op), descs[i].in, boards_alloc, c->k_per_tap, &h[i].map_a));
         h[i].map_w = c->map_w;
         h[i].out = descs[i].out;
         h[i].resid = descs[i].resid;
@@ -1345,7 +1443,8 @@ int tc_tower_create(TcTower **out, const TcTowerLayerDesc *descs, int n, int boa
         h[i].se_b1 = c->se_b1;
         h[i].se_b2 = c->se_b2;
         h[i].taps = c->taps;
-        h[i].kchunks = c->k_per_tap / TC_BK;
+        h[i].kchunks = c->k_per_tap / tc_op_bk(op);
+        h[i].scale = c->scale;
         h[i].relu = descs[i].relu;
         // se: 1 = squeeze-excitation gate, 2 = residual + ReLU only (`use_se=False`, no SE weights)
         h[i].se = c->epi == EPI_LN_SE ? (c->se_w1p ? 1 : 2) : 0;
@@ -1357,14 +1456,17 @@ int tc_tower_create(TcTower **out, const TcTowerLayerDesc *descs, int n, int boa
     }
     TcTower *t = new TcTower();
     t->n_layers = n;
-    t->fp16 = fp16;
+    t->op = op;
     if (cudaMalloc(&t->d_layers, sizeof(TowerLayer) * (size_t)n) != cudaSuccess ||
         cudaMemcpy(t->d_layers, h.data(), sizeof(TowerLayer) * (size_t)n, cudaMemcpyHostToDevice) != cudaSuccess) {
         delete t;
         set_error("tc_tower_create: device allocation failed");
         return SC_E_CUDA;
     }
-    if (fp16)
+    if (op == TC_OP_E4M3)
+        SCB_CUDA(cudaFuncSetAttribute(tc_gemm_kernel<256, EPI_LN_SE, true, true, true, OpE4m3>,
+                                      cudaFuncAttributeMaxDynamicSharedMemorySize, TcCfg<256, true, true>::SMEM_BYTES));
+    else if (op == TC_OP_FP16)
         SCB_CUDA(cudaFuncSetAttribute(tc_gemm_kernel<256, EPI_LN_SE, true, true, true, OpFp16>,
                                       cudaFuncAttributeMaxDynamicSharedMemorySize, TcCfg<256, true, true>::SMEM_BYTES));
     else
@@ -1418,7 +1520,9 @@ int tc_tower_launch(TcTower *t, int n_boards, int num_sms, int group, cudaStream
         SCB_CHECK(prof_buffer(num_sms, st, &d_prof));
         a.prof = d_prof;
     }
-    if (t->fp16)
+    if (t->op == TC_OP_E4M3)
+        SCB_CUDA(cudaLaunchKernelEx(&cfg, tc_gemm_kernel<256, EPI_LN_SE, true, true, true, OpE4m3>, dummy, dummy, a));
+    else if (t->op == TC_OP_FP16)
         SCB_CUDA(cudaLaunchKernelEx(&cfg, tc_gemm_kernel<256, EPI_LN_SE, true, true, true, OpFp16>, dummy, dummy, a));
     else
         SCB_CUDA(cudaLaunchKernelEx(&cfg, tc_gemm_kernel<256, EPI_LN_SE, true, true, true>, dummy, dummy, a));
@@ -1515,8 +1619,8 @@ int tc_conv_launch(TcConv *c, const __nv_bfloat16 *in, int rows_alloc, int n_uni
         am.ptr = in;
         am.rows = rows_alloc;
         am.c = c->k_per_tap;
-        // (the split kernel of the FP32 parity mode is created with fp16 = false)
-        const CUtensorMapDataType dt = tmap_type(c->fp16);
+        // (the split kernel of the FP32 parity mode is created with the bf16 operand type)
+        const CUtensorMapDataType dt = tmap_type(c->op);
         if (pair)
             SCB_CHECK(tc_make_act_map_hbw(dt, in, rows_alloc, c->k_per_tap, &am.map));
         else if (a4d)
@@ -1545,12 +1649,13 @@ int tc_conv_launch(TcConv *c, const __nv_bfloat16 *in, int rows_alloc, int n_uni
     a.se_b2 = c->se_b2;
     a.relu = relu;
     a.ln = c->gamma != nullptr;
+    a.scale = c->scale;
     a.n_splits = n_splits > 0 ? n_splits : 1;
     a.m_rows = n_units;
     if (a4d) {
         a.n_tiles = (n_units + 1) / 2;  // units = boards, two per tile
         a.taps = c->taps;
-        a.kchunks = c->k_per_tap / TC_BK;
+        a.kchunks = c->k_per_tap / tc_op_bk(c->op);
         if (c->split_pairs > 0) {
             a.split_pairs = c->split_pairs;
             a.split_kreal = c->split_kreal;
@@ -1561,11 +1666,13 @@ int tc_conv_launch(TcConv *c, const __nv_bfloat16 *in, int rows_alloc, int n_uni
     } else {
         a.n_tiles = (n_units + TC_BM - 1) / TC_BM;  // units = rows
         a.taps = 1;
-        a.kchunks = c->k_per_tap / TC_BK / a.n_splits;
+        a.kchunks = c->k_per_tap / tc_op_bk(c->op) / a.n_splits;
     }
     const int n_work = a4d ? a.n_tiles : a.n_tiles * a.n_splits;
     const int grid = n_work < num_sms ? n_work : num_sms;
-    if (c->fp16)
+    if (c->op == TC_OP_E4M3)
+        SCB_CHECK(conv_launch_kernel<OpE4m3>(c, *ma, a, grid, num_sms, st, resid, gather, finish));
+    else if (c->op == TC_OP_FP16)
         SCB_CHECK(conv_launch_kernel<OpFp16>(c, *ma, a, grid, num_sms, st, resid, gather, finish));
     else
         SCB_CHECK(conv_launch_kernel<OpBf16>(c, *ma, a, grid, num_sms, st, resid, gather, finish));

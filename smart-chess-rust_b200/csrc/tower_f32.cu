@@ -257,13 +257,16 @@ int launch_se_res_f32(const float *y, const float *x, float *out, int n, const f
 // Value head tail (py/module.py:95-106, :147-149): hidden = relu(sum_splits pre + W_meta
 // meta + b1); v = tanh(w2 . hidden + b2) * (2*turn - 1).  One warp per leaf.
 // ---------------------------------------------------------------------------------------
+// SCALED (fp8 mode): the split sum is multiplied by the hidden unit's weight scale first, as in the fused tail
+template <bool SCALED>
 __global__ void __launch_bounds__(128) value_finish_kernel(const float *__restrict__ pre, int n_split, int n,
                                                            const float *__restrict__ meta,
                                                            const float *__restrict__ w_meta /*[7][128]*/,
                                                            const float *__restrict__ b1,
                                                            const float *__restrict__ w2,
                                                            const float *__restrict__ b2,
-                                                           float *__restrict__ value_out)
+                                                           float *__restrict__ value_out,
+                                                           const float *__restrict__ scale)
 {
     // lane = hidden units 4 lane .. 4 lane + 3: one coalesced 512-byte row per split.  The arithmetic (split-order sum,
     // meta fma chain, + b1, ReLU, fma with w2 over the lane's four units, xor-shuffle sum) is, operation for operation,
@@ -281,6 +284,9 @@ __global__ void __launch_bounds__(128) value_finish_kernel(const float *__restri
         h.w += p.w;
     }
     float hv[4] = {h.x, h.y, h.z, h.w};
+    if constexpr (SCALED)
+#pragma unroll
+        for (int i = 0; i < 4; i++) hv[i] = __fmul_rn(hv[i], scale[4 * lane + i]);
     float acc = 0.f;
 #pragma unroll
     for (int i = 0; i < 4; i++) {
@@ -295,10 +301,14 @@ __global__ void __launch_bounds__(128) value_finish_kernel(const float *__restri
 }
 
 int launch_value_finish(const float *hidden_pre, int n_split, int n, const float *meta, const float *w_meta,
-                        const float *b1, const float *w2, const float *b2, float *value_out, cudaStream_t st)
+                        const float *b1, const float *w2, const float *b2, float *value_out, cudaStream_t st,
+                        const float *scale)
 {
     if (n <= 0) return SC_OK;
-    value_finish_kernel<<<(n + 3) / 4, 128, 0, st>>>(hidden_pre, n_split, n, meta, w_meta, b1, w2, b2, value_out);
+    if (scale)
+        value_finish_kernel<true><<<(n + 3) / 4, 128, 0, st>>>(hidden_pre, n_split, n, meta, w_meta, b1, w2, b2, value_out, scale);
+    else
+        value_finish_kernel<false><<<(n + 3) / 4, 128, 0, st>>>(hidden_pre, n_split, n, meta, w_meta, b1, w2, b2, value_out, nullptr);
     SCB_CUDA(cudaGetLastError());
     return SC_OK;
 }

@@ -21,6 +21,7 @@ from .binding import (  # noqa: F401
     SC_MODE_FP32,
     SC_MODE_FP32_FFMA,
     SC_MODE_FP16,
+    SC_MODE_FP8,
     SC_MAX_MOVES,
     SC_MAX_STACK,
     POSITION_DTYPE,

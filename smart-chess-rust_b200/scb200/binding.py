@@ -10,6 +10,7 @@ SC_MODE_FP32 = 0
 SC_MODE_BF16 = 1
 SC_MODE_FP32_FFMA = 2
 SC_MODE_FP16 = 3
+SC_MODE_FP8 = 4
 SC_N_PLANES = 112
 SC_N_META = 7
 SC_N_POLICY = 4672
@@ -429,7 +430,7 @@ class Engine:
 
     def debug_tower(self, positions, n_layers: int, which: int):
         """test hook sc_debug_tower: (x, t, y) activation buffers as uint16 [n, 64, 256] after n_layers layers
-        (bf16 bit patterns on a bf16 engine, fp16 on an fp16 engine)"""
+        (bf16 bit patterns on a bf16 engine, fp16 on an fp16 engine, an fp8 engine's e4m3 values as fp16)"""
         n = len(positions)
         positions = np.ascontiguousarray(positions, dtype=POSITION_DTYPE)
         out = [np.zeros((n, 64, 256), dtype=np.uint16) for _ in range(3)]

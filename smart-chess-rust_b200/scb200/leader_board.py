@@ -38,7 +38,7 @@ def play_half(white, black, n_games, prefix, tag, a):
 
 
 def main(argv=None):
-    from . import Engine, SC_MODE_BF16, SC_MODE_FP16, elo
+    from . import Engine, SC_MODE_BF16, SC_MODE_FP16, SC_MODE_FP8, elo
 
     ap = argparse.ArgumentParser(description=__doc__.splitlines()[0])
     ap.add_argument("-W", "--white-checkpoint", required=True)
@@ -54,7 +54,9 @@ def main(argv=None):
     ap.add_argument("--threads", type=int, default=0)
     ap.add_argument("--seed", type=int, default=0)
     ap.add_argument("--device", type=int, default=0)
-    ap.add_argument("--fp16", action="store_true", help="fp16 tensor-core operands instead of bf16 for both engines")
+    prec = ap.add_mutually_exclusive_group()
+    prec.add_argument("--fp16", action="store_true", help="fp16 tensor-core operands instead of bf16 for both engines")
+    prec.add_argument("--fp8", action="store_true", help="fp8 (e4m3) tensor-core operands instead of bf16 for both engines")
     a = ap.parse_args(argv)
 
     # under torchrun every rank plays its share of the games on its own GPU (games are independent: no collective
@@ -72,7 +74,7 @@ def main(argv=None):
     tallies = [0] * 6
     if n_games > 0:
         mb = max(1, min(a.trees, n_games))
-        mode = SC_MODE_FP16 if a.fp16 else SC_MODE_BF16
+        mode = SC_MODE_FP16 if a.fp16 else SC_MODE_FP8 if a.fp8 else SC_MODE_BF16
         ea = Engine(a.white_checkpoint, a.device, mode, mb)
         eb = Engine(a.black_checkpoint, a.device, mode, mb)
         print(f"Results are saved in {a.prefix}")

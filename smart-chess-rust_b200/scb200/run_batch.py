@@ -14,7 +14,7 @@ import os
 
 
 def main(argv=None):
-    from . import Engine, SelfPlay, SC_MODE_BF16, SC_MODE_FP16, SC_MODE_FP32
+    from . import Engine, SelfPlay, SC_MODE_BF16, SC_MODE_FP16, SC_MODE_FP32, SC_MODE_FP8
     from .shard import game_ids_for_rank, rank_seed
 
     ap = argparse.ArgumentParser(description=__doc__.splitlines()[0])
@@ -32,6 +32,8 @@ def main(argv=None):
     prec.add_argument("--fp32", action="store_true", help="parity mode (FP32 FFMA) instead of bf16 tensor cores")
     prec.add_argument("--fp16", action="store_true",
                       help="fp16 tensor-core operands instead of bf16 (the precision of a 16-mixed trained net)")
+    prec.add_argument("--fp8", action="store_true",
+                      help="fp8 (e4m3) tensor-core operands instead of bf16 (throughput mode, lower precision)")
     ap.add_argument("--leaves-per-tree", type=int, default=1,
                     help="1 = the reference's sequential search; K > 1 = K leaves per tree per batch (virtual loss); "
                          "-1 = 1 until games run out, then the remaining games share the batch")
@@ -46,7 +48,8 @@ def main(argv=None):
         return 0
     trees = max(1, min(a.trees, len(mine)))
     kl = max(1, a.leaves_per_tree)
-    eng = Engine(a.checkpoint, local, SC_MODE_FP32 if a.fp32 else SC_MODE_FP16 if a.fp16 else SC_MODE_BF16, trees * kl)
+    mode = SC_MODE_FP32 if a.fp32 else SC_MODE_FP16 if a.fp16 else SC_MODE_FP8 if a.fp8 else SC_MODE_BF16
+    eng = Engine(a.checkpoint, local, mode, trees * kl)
     sp = SelfPlay(eng, n_trees=trees, rollout_num=a.rollout_num, num_steps=a.num_steps, cpuct=a.cpuct, epsilon=a.epsilon,
                   with_noise=True, temperature_switch=a.temperature_switch, temperature=a.temperature,
                   seed=rank_seed(a.seed, rank), n_threads=a.threads or max(1, (os.cpu_count() or 8) // world),

@@ -11,7 +11,7 @@ import torch
 import scb200
 
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 2048
-mode = {"bf16": scb200.SC_MODE_BF16, "fp16": scb200.SC_MODE_FP16, "fp32": scb200.SC_MODE_FP32}[sys.argv[2] if len(sys.argv) > 2 else "bf16"]
+mode = {"bf16": scb200.SC_MODE_BF16, "fp16": scb200.SC_MODE_FP16, "fp8": scb200.SC_MODE_FP8, "fp32": scb200.SC_MODE_FP32}[sys.argv[2] if len(sys.argv) > 2 else "bf16"]
 reps = int(sys.argv[3]) if len(sys.argv) > 3 else 4
 tmp = tempfile.mkdtemp()
 blob = os.path.join(tmp, "w.scw")

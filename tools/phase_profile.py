@@ -8,7 +8,9 @@ import numpy as np, scb200
 tmp = tempfile.mkdtemp()
 sd, blob = bench.make_blob(tmp, int(os.environ.get('BLOCKS', '19')))
 pos, moves, off = bench.make_workload(2048, 1000)
-e = scb200.Engine(blob, 0, scb200.SC_MODE_BF16, 2048)
+# MODE=bf16 (default), fp16 or fp8: the operand type of the tensor-core kernels
+mode = {"bf16": scb200.SC_MODE_BF16, "fp16": scb200.SC_MODE_FP16, "fp8": scb200.SC_MODE_FP8}[os.environ.get("MODE", "bf16")]
+e = scb200.Engine(blob, 0, mode, 2048)
 for i in range(3):
     sys.stderr.write(f"--- eval {i}\n")
     e.eval(pos, moves, off)

@@ -1,13 +1,20 @@
-"""bf16 against fp16 tensor-core mode on the bench.py workload (19 blocks, seed-0 net, seeded random-play leaves).
+"""bf16 against fp16 (or any list of --modes) tensor-core mode on the bench.py workload (19 blocks, seed-0 net,
+seeded random-play leaves).
 
-Alternates a bf16 and an fp16 engine for --rounds rounds each and measures, per round:
+Alternates engines of the --modes (default bf16,fp16) for --rounds rounds each and measures, per round:
   * the device-resident 2048-leaf step (sc_eval_device), CUDA events per step, L2 flushed between timed steps as
     bench.py does, with nvidia-smi SM clock samples during that leg;
   * sc_eval latency (host buffers) at n = 1 / 8 / 64.
 Then both modes' max |d prior| / |d value| against an fp32 engine on the same batch.  Records the card name and power
 limit, prints one JSON line and writes it under profiles/ (--out).
 
+--detail adds, per round, the whole-tower launch time from CUDA events (level-2 timing, after the timed window) and
+the TFLOP/s it achieves; and per mode, against the fp32 engine, the mean prior error, the mean per-leaf total-variation
+distance of the priors, the value error and the rate at which the highest-prior move is the fp32 engine's; and for an
+fp8 engine the share of activation elements saturated at +-448 in each layer's output (sc_debug_tower, 256 leaves).
+
     python tools/precision_ab.py --out profiles/fp16_ab.json
+    python tools/precision_ab.py --modes bf16,fp8 --detail --rounds 3 --out profiles/fp8_precision_ab.json
 """
 import argparse
 import json
@@ -35,7 +42,12 @@ def card():
     return q.stdout.strip()
 
 
-def leg(blob, mode, pos, moves, off, steps, warmup):
+MODES = {"bf16": scb200.SC_MODE_BF16, "fp16": scb200.SC_MODE_FP16, "fp8": scb200.SC_MODE_FP8}
+# data-sheet dense tensor-core rates of one B200 (1000 W), TFLOP/s
+DATASHEET_TFLOPS = {"bf16": 2250.0, "fp16": 2250.0, "fp8": 4500.0}
+
+
+def leg(blob, mode, pos, moves, off, steps, warmup, detail=False):
     B, n_moves = len(pos), int(off[-1])
     eng = scb200.Engine(blob, 0, mode, B)
     dev = "cuda:0"
@@ -74,8 +86,48 @@ def leg(blob, mode, pos, moves, off, steps, warmup):
         out["leaves_per_s"] = B / (out["step_ms_median"] * 1e-3)
         out["sm_mhz_median"] = clocks.get("sm_mhz")
         out["clock_reasons"] = clocks.get("reasons")
+        if detail:
+            # the whole-tower kernel alone: level-2 timing puts an event pair around its launch
+            eng.set_timing(2)
+            tms = []
+            for _ in range(10):
+                flush.zero_()
+                eng.eval(pos, moves, off)
+                tms.append(eng.kernel_timing()[0])
+            eng.set_timing(0)
+            out["tower_launch_ms_median"] = statistics.median(tms)
+            out["tower_tflops"] = eng.timed_flops_per_leaf() * B / (out["tower_launch_ms_median"] * 1e-3) / 1e12
         pri, val = eng.eval(pos, moves, off)
         return out, pri.copy(), val.copy()
+    finally:
+        eng.close()
+
+
+def detail_errors(p, v, p32, v32, off):
+    """mean prior error, mean per-leaf total-variation distance (scripts/validate_*.py's metric), value error, and the
+    rate at which the highest-prior move is the fp32 engine's"""
+    d = np.abs(p - p32)
+    tv, top = [], []
+    for i in range(len(off) - 1):
+        a, b = off[i], off[i + 1]
+        if b > a:
+            tv.append(0.5 * float(d[a:b].sum()))
+            top.append(int(np.argmax(p[a:b]) == np.argmax(p32[a:b])))
+    return {"mean_abs_d_prior": float(d.mean()), "mean_tv_distance": float(np.mean(tv)),
+            "mean_abs_d_value": float(np.abs(v - v32).mean()), "top_move_agreement": float(np.mean(top))}
+
+
+def saturation(blob, pos, n_blocks=19):
+    """fp8 engine: per tower layer, the share of its output elements at +-448 (e4m3 satfinite).  Layer k of the
+    1 + 2 n_blocks + 2 writes x (stem, conv2), t (conv1, policy 1x1) or y (value 1x1)"""
+    eng = scb200.Engine(blob, 0, scb200.SC_MODE_FP8, len(pos))
+    writes = [0] + [1, 0] * n_blocks + [1, 2]
+    try:
+        out = []
+        for k, w in enumerate(writes, start=1):
+            buf = eng.debug_tower(pos, k, 0)[w]
+            out.append(float(((buf & 0x7FFF) == 0x5F00).mean()))  # fp16 bits of 448
+        return out
     finally:
         eng.close()
 
@@ -87,18 +139,20 @@ def main():
     ap.add_argument("--steps", type=int, default=40)
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "fp16_precision_ab.json"))
+    ap.add_argument("--modes", default="bf16,fp16", help="comma-separated tensor-core modes (bf16, fp16, fp8)")
+    ap.add_argument("--detail", action="store_true", help="tower launch times, accuracy metrics, fp8 saturation")
     a = ap.parse_args()
     if not torch.cuda.is_available():
         sys.exit("precision_ab.py needs a CUDA device")
     tmp = tempfile.mkdtemp()
     _, blob = make_blob(tmp)
     pos, moves, off = make_workload(a.leaves, seed=0)
-    modes = {"bf16": scb200.SC_MODE_BF16, "fp16": scb200.SC_MODE_FP16}
+    modes = {k: MODES[k] for k in a.modes.split(",")}
     runs = {k: [] for k in modes}
     outs = {}
     for _ in range(a.rounds):
         for name, mode in modes.items():
-            r, pri, val = leg(blob, mode, pos, moves, off, a.steps, a.warmup)
+            r, pri, val = leg(blob, mode, pos, moves, off, a.steps, a.warmup, a.detail)
             runs[name].append(r)
             outs[name] = (pri, val)
     e = scb200.Engine(blob, 0, scb200.SC_MODE_FP32, a.leaves)
@@ -108,7 +162,16 @@ def main():
         e.close()
     err = {name: {"max_abs_d_prior": float(np.abs(p - p32).max()), "max_abs_d_value": float(np.abs(v - v32).max())}
            for name, (p, v) in outs.items()}
-    res = {"what": "bf16 vs fp16 tensor-core mode, 19 blocks, %d leaves, alternating engines" % a.leaves,
+    if a.detail:
+        for name, (p, v) in outs.items():
+            err[name].update(detail_errors(p, v, p32, v32, off))
+            for r in runs[name]:
+                if "tower_tflops" in r:
+                    r["tower_tflops_of_datasheet_%s" % name] = r["tower_tflops"] / DATASHEET_TFLOPS[name]
+                    r["tower_tflops_of_datasheet_bf16"] = r["tower_tflops"] / DATASHEET_TFLOPS["bf16"]
+            if name == "fp8":
+                err[name]["saturated_share_per_layer"] = saturation(blob, pos[:256])
+    res = {"what": "%s tensor-core mode, 19 blocks, %d leaves, alternating engines" % (" vs ".join(modes), a.leaves),
            "card": card(), "rounds": runs, "error_vs_fp32_engine": err}
     os.makedirs(os.path.dirname(a.out), exist_ok=True)
     with open(a.out, "w") as f:
