@@ -81,30 +81,24 @@ int launch_legal_moves(const sc_position *d_pos, const int8_t *d_ep, int n, sc_m
 enum { REPLAY_NOT_OURS = 1, REPLAY_BAD_TARGET, REPLAY_BAD_PROMO, REPLAY_NO_PROMO };
 __host__ __device__ constexpr int32_t REPLAY_STATUS(int ply, int reason) { return ply << 3 | reason; }
 size_t replay_scratch_bytes(int64_t positions);
-// sc_set_roots, one thread per root: replays root r's moves d_stack[d_off[r], d_off[r+1]) from the initial position and
-// keeps its records (replay_scratch_bytes(d_off[n] + n) bytes of d_rec in all), its final position in d_root_pos[r] and
-// its status in d_status[r]
+// a slot table (sc_set_roots' roots, an evaluator's slots): slot g's records at d_rec + replay_scratch_bytes(g *
+// (SC_MAX_STACK + 1)), its final position in d_slot_pos[g] and its plies in d_slot_plies[g].  One thread per update u:
+// replays d_stack[d_off[u], d_off[u+1]) into slot d_slot[u] (d_slot == nullptr: slot u), from the initial position or
+// (d_append[u] != 0; d_append == nullptr: none) from the slot's stored position, appending to its records; the status
+// into d_status[u].  The caller keeps the plies within SC_MAX_STACK
 namespace chess { struct Position; }
-int launch_root_replay(const sc_move *d_stack, const int32_t *d_off, int n, void *d_rec, chess::Position *d_root_pos,
-                       int32_t *d_status, cudaStream_t st);
-// an evaluator's slot table: slot g's records at d_rec + replay_scratch_bytes(g * (SC_MAX_STACK + 1)), its final
-// position in d_slot_pos[g] and its plies in d_slot_plies[g].  One thread per update u: replays d_stack[d_off[u],
-// d_off[u+1]) into slot d_slot[u], from the initial position or (d_append[u] != 0) from the slot's stored position,
-// appending to its records; the status into d_status[u].  The caller keeps the plies within SC_MAX_STACK
 int launch_slot_replay(const sc_move *d_stack, const int32_t *d_off, const int32_t *d_slot, const int8_t *d_append,
                        int n, void *d_rec, chess::Position *d_slot_pos, int32_t *d_slot_plies, int32_t *d_status,
                        cudaStream_t st);
-// sc_predict_stack / sc_predict_path / an evaluator's leaves, one thread per leaf: leaf i starts from root d_root[i] of
-// the sc_set_roots table above (d_root_off = the d_off it was built from), or of a slot table when d_slot_plies is
-// given (d_root_rec / d_root_pos: its records and positions), or from the initial position when d_root == nullptr (no
-// table is then read), replays d_path[d_off[i], d_off[i+1]) and packs the game as host::pack_position does with d_n_hist[i]
-// history slots (nullptr: min(SC_LOOKBACK, plies + 1)) into d_pos[i], its python-chess ep_square into d_ep[i], and its
-// status into d_status[i] (after a rejected move the leaf is packed from the moves before it).  d_scratch:
-// replay_scratch_bytes(d_off[n] + n) bytes, the path's records
-int launch_path_replay(const void *d_root_rec, const int32_t *d_root_off, const int32_t *d_slot_plies,
-                       const chess::Position *d_root_pos, const int32_t *d_root, const sc_move *d_path,
-                       const int32_t *d_off, const int8_t *d_n_hist, int n, void *d_scratch, sc_position *d_pos,
-                       int8_t *d_ep, int32_t *d_status, cudaStream_t st);
+// sc_predict_stack / sc_predict_path / an evaluator's leaves, one thread per leaf: leaf i starts from slot d_root[i] of
+// a slot table as above (d_slot_rec / d_slot_plies / d_slot_pos: its records, plies and positions), or from the initial
+// position when d_root == nullptr (no table is then read), replays d_path[d_off[i], d_off[i+1]) and packs the game as
+// host::pack_position does with d_n_hist[i] history slots (nullptr: min(SC_LOOKBACK, plies + 1)) into d_pos[i], its
+// python-chess ep_square into d_ep[i], and its status into d_status[i] (after a rejected move the leaf is packed from
+// the moves before it).  d_scratch: replay_scratch_bytes(d_off[n] + n) bytes, the path's records
+int launch_path_replay(const void *d_slot_rec, const int32_t *d_slot_plies, const chess::Position *d_slot_pos,
+                       const int32_t *d_root, const sc_move *d_path, const int32_t *d_off, const int8_t *d_n_hist, int n,
+                       void *d_scratch, sc_position *d_pos, int8_t *d_ep, int32_t *d_status, cudaStream_t st);
 
 // ---- tower_f32.cu -------------------------------------------------------------------------
 // C[M][N] = gather_taps(A)[M][TAPS*K] * W[TAPS*K][ldw] + bias ; A is [rows][lda] fp32

@@ -186,6 +186,39 @@ struct SeW {
     uint16_t *w1s[2] = {nullptr, nullptr}, *w2s[2] = {nullptr, nullptr};  // latency kernel: sliced per cluster rank (CL = 8, 4)
 };
 
+// root slots (sc_set_roots' roots, an evaluator's slots; launch_slot_replay): per slot SC_MAX_STACK + 1 replay
+// records, the final position and the plies on the device, room for `cap` slots; and the plies on the host, one entry
+// per slot in use (-1: an evaluator slot without a root)
+struct SlotTable {
+    void *d_rec = nullptr;
+    chess::Position *d_pos = nullptr;
+    int32_t *d_plies = nullptr;
+    int cap = 0;
+    std::vector<int32_t> plies;
+
+    // room for n_slots slots on the device; grows only, and the device contents are not kept when it grows
+    int reserve(int n_slots)
+    {
+        if (n_slots <= cap) return SC_OK;
+        release();
+        SCB_CUDA(cudaMalloc(&d_rec, replay_scratch_bytes((int64_t)n_slots * (SC_MAX_STACK + 1))));
+        SCB_CUDA(cudaMalloc(&d_pos, sizeof(chess::Position) * (size_t)n_slots));
+        SCB_CUDA(cudaMalloc(&d_plies, sizeof(int32_t) * (size_t)n_slots));
+        cap = n_slots;
+        return SC_OK;
+    }
+    void release()
+    {
+        cudaFree(d_rec);
+        cudaFree(d_pos);
+        cudaFree(d_plies);
+        d_rec = nullptr;
+        d_pos = nullptr;
+        d_plies = nullptr;
+        cap = 0;
+    }
+};
+
 }  // namespace scb
 
 using namespace scb;
@@ -281,24 +314,18 @@ struct sc_engine {
     int8_t *d_pred_ep = nullptr;
     uint8_t *d_pred_out = nullptr, *h_pred_out = nullptr;
     float last_movegen_ms = 0.f;
-    // sc_predict_stack, set up by its first call: stacks / offsets / n_hist of calls that do not fit the small staging
-    // buffer, the replay's per-leaf status (copied back to h_replay_status) and its scratch, grown to the largest call
+    // sc_predict_stack, set up by its first call: stacks / offsets / root indices / n_hist of calls that do not fit the
+    // small staging buffer, the replay's per-leaf status (copied back to h_replay_status) and its scratch, grown to the
+    // largest call
     sc_move *d_stack = nullptr;
-    int32_t *d_stack_off = nullptr, *d_replay_status = nullptr, *h_replay_status = nullptr;
+    int32_t *d_stack_off = nullptr, *d_path_root = nullptr, *d_replay_status = nullptr, *h_replay_status = nullptr;
     int8_t *d_stack_nhist = nullptr;
     void *d_replay_scratch = nullptr;
     size_t replay_scratch_cap = 0;
     cudaEvent_t ev_replay_t[2] = {nullptr, nullptr};  // timing: around the replay kernel
     float last_replay_ms = 0.f;
-    // sc_set_roots' table, set up by its first call: per root its final position and the offsets of its moves (device,
-    // and a host copy in root_off), every root's replay records (grown to the largest call); n_roots == 0: no roots.
-    // d_path_root: sc_predict_path's root indices of calls that do not fit the small staging buffer
-    chess::Position *d_root_pos = nullptr;
-    int32_t *d_root_off = nullptr, *d_path_root = nullptr;
-    void *d_root_rec = nullptr;
-    size_t root_rec_cap = 0;
-    std::vector<int32_t> root_off;
-    int n_roots = 0;
+    // sc_set_roots' table: root r in slot r, roots.plies.size() roots (0: no roots), grown to the largest call
+    SlotTable roots;
     float last_path_ms = 0.f;  // timing: the path-replay kernel (between ev_replay_t)
     // an sc_evaluator owns the stream: every other call that uses the device returns SC_E_STATE
     std::atomic<bool> evaluator{false};
@@ -842,24 +869,13 @@ static int predict_stack_setup(sc_engine *e, int64_t positions)
     if (!e->d_stack) {
         SCB_CHECK(dev_alloc(e, &e->d_stack, (size_t)e->max_batch * SC_MAX_STACK));
         SCB_CHECK(dev_alloc(e, &e->d_stack_off, (size_t)e->max_batch + 1));
+        SCB_CHECK(dev_alloc(e, &e->d_path_root, (size_t)e->max_batch));
         SCB_CHECK(dev_alloc(e, &e->d_stack_nhist, (size_t)e->max_batch));
         SCB_CHECK(dev_alloc(e, &e->d_replay_status, (size_t)e->max_batch));
         SCB_CUDA(cudaMallocHost(&e->h_replay_status, sizeof(int32_t) * (size_t)e->max_batch));
         for (cudaEvent_t &ev : e->ev_replay_t) SCB_CUDA(cudaEventCreate(&ev));
     }
     return grow_records(&e->d_replay_scratch, &e->replay_scratch_cap, positions);
-}
-
-// sc_set_roots' table (first call), with room for the records of `positions` replayed positions
-static int roots_setup(sc_engine *e, int64_t positions)
-{
-    SCB_CHECK(predict_stack_setup(e, 0));
-    if (!e->d_root_pos) {
-        SCB_CHECK(dev_alloc(e, &e->d_root_pos, (size_t)e->max_batch));
-        SCB_CHECK(dev_alloc(e, &e->d_root_off, (size_t)e->max_batch + 1));
-        SCB_CHECK(dev_alloc(e, &e->d_path_root, (size_t)e->max_batch));
-    }
-    return grow_records(&e->d_root_rec, &e->root_rec_cap, positions);
 }
 
 // copies host arrays to the device on `st` and puts the address each is read from in dev[]: through the pinned small
@@ -951,14 +967,31 @@ static std::string replay_error(const char *what, const char *unit, int index, i
            ": move rejected, " + replay_reason(status);
 }
 
-// an evaluator's root slots (engine_backend_create): per slot SC_MAX_STACK + 1 replay records, the final position and
-// the plies on the device, and the plies on the host (-1: the slot has no root)
-struct SlotTable {
-    void *d_rec = nullptr;
-    chess::Position *d_pos = nullptr;
-    int32_t *d_plies = nullptr;
-    std::vector<int32_t> plies;
-};
+// n root updates of `t` in one launch_slot_replay (slot / append nullptr: update u replays into slot u from the initial
+// position), after the host-side checks; waits for it and leaves the statuses in e->h_replay_status.  t.plies is the
+// caller's to update
+static int replay_into_slots(sc_engine *e, SlotTable &t, int n, const int32_t *slot, const int8_t *append,
+                             const int32_t *off, const sc_move *mv)
+{
+    cudaStream_t st = e->stream;
+    SCB_CUDA(cudaSetDevice(e->device));
+    SCB_CHECK(predict_stack_setup(e, 0));
+    const void *d[4];
+    SCB_CHECK(stage_inputs(e, n,
+                           {{off, sizeof(int32_t) * ((size_t)n + 1), e->d_stack_off},
+                            {slot, slot ? sizeof(int32_t) * (size_t)n : 0, e->d_path_root},
+                            {append, append ? (size_t)n : 0, e->d_stack_nhist},
+                            {mv, sizeof(sc_move) * (size_t)off[n], e->d_stack}},
+                           d, st));
+    SCB_CHECK(launch_slot_replay(static_cast<const sc_move *>(d[3]), static_cast<const int32_t *>(d[0]),
+                                 static_cast<const int32_t *>(d[1]), static_cast<const int8_t *>(d[2]), n, t.d_rec,
+                                 t.d_pos, t.d_plies, e->d_replay_status, st));
+    e->launches += 1;
+    SCB_CUDA(cudaMemcpyAsync(e->h_replay_status, e->d_replay_status, sizeof(int32_t) * (size_t)n, cudaMemcpyDeviceToHost,
+                             st));
+    SCB_CUDA(cudaStreamSynchronize(st));
+    return SC_OK;
+}
 
 // SC_E_STATE while an evaluator owns the engine
 static int check_owner(const sc_engine *e, const char *what)
@@ -1064,20 +1097,16 @@ static int predict_collect(sc_engine *e, const char *what, int n, sc_move *moves
     return SC_OK;
 }
 
-// sc_predict_stack, sc_predict_path and an evaluator's pass after their own argument checks: leaf i is root root[i]
-// of sc_set_roots' table or, with `slots`, of that slot table (root == nullptr: the initial position) followed by
-// mv[off[i], off[i+1]).  The move lists' checks, the replay into d_pos /
-// d_pred_ep, sc_predict's launches and the results.  off_name / mv_name: the two arrays in messages; replay_ms: where
-// timing puts the replay kernel's time
-static int predict_replay(sc_engine *e, const char *what, int n, const int32_t *root, const SlotTable *slots,
+// sc_predict_stack, sc_predict_path and an evaluator's pass after their own argument checks: leaf i is slot root[i]
+// of `roots` (root == roots == nullptr: the initial position) followed by mv[off[i], off[i+1]).  The move lists'
+// checks, the replay into d_pos / d_pred_ep, sc_predict's launches and the results.  off_name / mv_name: the two arrays
+// in messages; replay_ms: where timing puts the replay kernel's time
+static int predict_replay(sc_engine *e, const char *what, int n, const int32_t *root, const SlotTable *roots,
                           const sc_move *mv, const int32_t *off, const char *off_name, const char *mv_name,
                           const int8_t *n_hist, sc_position *pos_out, sc_move *moves_out, int32_t *move_cnt_out,
                           float *priors_out, float *value_out, float *replay_ms, void *stream)
 {
-    const int32_t *ro = e->root_off.data();
-    auto root_plies = [&](int i) {
-        return !root ? 0 : slots ? slots->plies[root[i]] : ro[root[i] + 1] - ro[root[i]];
-    };
+    auto root_plies = [&](int i) { return root ? roots->plies[root[i]] : 0; };
     SCB_CHECK(check_move_lists(what, "leaf", off_name, mv_name, n, mv, off, n_hist, root_plies));
     cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
     SCB_CUDA(cudaSetDevice(e->device));
@@ -1092,8 +1121,8 @@ static int predict_replay(sc_engine *e, const char *what, int n, const int32_t *
                            d, st));
     // the packed leaves and their ep squares go where sc_predict's kernels read them on the device
     if (e->timing) SCB_CUDA(cudaEventRecord(e->ev_replay_t[0], st));
-    SCB_CHECK(launch_path_replay(slots ? slots->d_rec : e->d_root_rec, e->d_root_off, slots ? slots->d_plies : nullptr,
-                                 slots ? slots->d_pos : e->d_root_pos, static_cast<const int32_t *>(d[1]),
+    SCB_CHECK(launch_path_replay(roots ? roots->d_rec : nullptr, roots ? roots->d_plies : nullptr,
+                                 roots ? roots->d_pos : nullptr, static_cast<const int32_t *>(d[1]),
                                  static_cast<const sc_move *>(d[2]), static_cast<const int32_t *>(d[0]),
                                  static_cast<const int8_t *>(d[3]), n, e->d_replay_scratch, e->d_pos, e->d_pred_ep,
                                  e->d_replay_status, st));
@@ -1117,12 +1146,12 @@ static int predict_replay(sc_engine *e, const char *what, int n, const int32_t *
     return rc;
 }
 
-// the engine behind an sc_evaluator (host/evaluator.hpp): its slot table, the root updates' launch, and each pass of
-// leaves through predict_replay.  The dispatcher thread is the only caller
+// the engine behind an sc_evaluator (host/evaluator.hpp): its slot table, the root updates through replay_into_slots,
+// and each pass of leaves through predict_replay.  The dispatcher thread is the only caller
 class EngineBackend : public EvalBackend {
     sc_engine *e_;
     SlotTable t_;
-    // one pass: the requests that passed their checks, as predict_replay / launch_slot_replay take them
+    // one pass: the requests that passed their checks, as predict_replay / replay_into_slots take them
     std::vector<int32_t> root_, off_;
     std::vector<sc_move> mv_;
     std::vector<int8_t> flag_;  // update: append; leaf: n_hist
@@ -1145,27 +1174,6 @@ class EngineBackend : public EvalBackend {
         off_.push_back((int32_t)mv_.size());
         flag_.push_back(flag);
     }
-    // the updates' one launch; statuses in e_->h_replay_status
-    int launch_updates(int n)
-    {
-        cudaStream_t st = e_->stream;
-        SCB_CUDA(cudaSetDevice(e_->device));
-        const void *d[4];
-        SCB_CHECK(stage_inputs(e_, n,
-                               {{off_.data(), sizeof(int32_t) * ((size_t)n + 1), e_->d_stack_off},
-                                {root_.data(), sizeof(int32_t) * (size_t)n, e_->d_path_root},
-                                {flag_.data(), (size_t)n, e_->d_stack_nhist},
-                                {mv_.data(), sizeof(sc_move) * mv_.size(), e_->d_stack}},
-                               d, st));
-        SCB_CHECK(launch_slot_replay(static_cast<const sc_move *>(d[3]), static_cast<const int32_t *>(d[0]),
-                                     static_cast<const int32_t *>(d[1]), static_cast<const int8_t *>(d[2]), n, t_.d_rec,
-                                     t_.d_pos, t_.d_plies, e_->d_replay_status, st));
-        e_->launches += 1;
-        SCB_CUDA(cudaMemcpyAsync(e_->h_replay_status, e_->d_replay_status, sizeof(int32_t) * (size_t)n,
-                                 cudaMemcpyDeviceToHost, st));
-        SCB_CUDA(cudaStreamSynchronize(st));
-        return SC_OK;
-    }
 
 public:
     explicit EngineBackend(sc_engine *e) : e_(e) {}
@@ -1173,18 +1181,13 @@ public:
     {
         cudaSetDevice(e_->device);
         cudaStreamSynchronize(e_->stream);
-        if (t_.d_rec) cudaFree(t_.d_rec);
-        if (t_.d_pos) cudaFree(t_.d_pos);
-        if (t_.d_plies) cudaFree(t_.d_plies);
+        t_.release();
         e_->evaluator = false;
     }
     int setup(int n_slots)
     {
         SCB_CUDA(cudaSetDevice(e_->device));
-        SCB_CHECK(roots_setup(e_, 0));  // the staging buffers of sc_set_roots / sc_predict_path
-        SCB_CUDA(cudaMalloc(&t_.d_rec, replay_scratch_bytes((int64_t)n_slots * (SC_MAX_STACK + 1))));
-        SCB_CUDA(cudaMalloc(&t_.d_pos, sizeof(chess::Position) * (size_t)n_slots));
-        SCB_CUDA(cudaMalloc(&t_.d_plies, sizeof(int32_t) * (size_t)n_slots));
+        SCB_CHECK(t_.reserve(n_slots));
         t_.plies.assign((size_t)n_slots, -1);
         return SC_OK;
     }
@@ -1212,7 +1215,7 @@ public:
             add(r->slot, r->moves, r->len, r->append);
         }
         if (run.empty()) return;
-        const int rc = launch_updates((int)run.size());
+        const int rc = replay_into_slots(e_, t_, (int)run.size(), root_.data(), flag_.data(), off_.data(), mv_.data());
         for (size_t i = 0; i < run.size(); i++) {
             RootUpdate *r = run[i];
             const int32_t status = e_->h_replay_status[i];
@@ -1461,7 +1464,7 @@ int sc_destroy(sc_engine *e)
     if (e->h_pred_out) cudaFreeHost(e->h_pred_out);
     if (e->h_replay_status) cudaFreeHost(e->h_replay_status);
     if (e->d_replay_scratch) cudaFree(e->d_replay_scratch);
-    if (e->d_root_rec) cudaFree(e->d_root_rec);
+    e->roots.release();
     for (cudaEvent_t ev : {e->ev_gen_fork, e->ev_gen_done, e->ev_gen_t[0], e->ev_gen_t[1], e->ev_replay_t[0], e->ev_replay_t[1]})
         if (ev) cudaEventDestroy(ev);
     if (e->gen_stream) cudaStreamDestroy(e->gen_stream);
@@ -1651,28 +1654,18 @@ int sc_set_roots(sc_engine *e, int n_roots, const sc_move *stack, const int32_t 
         SCB_CHECK(check_move_lists("sc_set_roots", "root", "stack_off", "stack", n_roots, stack, stack_off, nullptr,
                                    [](int) { return 0; }));
     NvtxRange nv_call("sc_set_roots");
-    e->n_roots = 0;
+    e->roots.plies.clear();
     if (n_roots == 0) return SC_OK;
-    cudaStream_t st = e->stream;
     SCB_CUDA(cudaSetDevice(e->device));
-    const int total = stack_off[n_roots];
-    SCB_CHECK(roots_setup(e, (int64_t)total + n_roots));
-    // the offsets stay on the device with the table: sc_predict_path finds each root's records through them
-    SCB_CUDA(cudaMemcpyAsync(e->d_root_off, stack_off, sizeof(int32_t) * ((size_t)n_roots + 1), cudaMemcpyHostToDevice, st));
-    if (total) SCB_CUDA(cudaMemcpyAsync(e->d_stack, stack, sizeof(sc_move) * (size_t)total, cudaMemcpyHostToDevice, st));
-    SCB_CHECK(launch_root_replay(e->d_stack, e->d_root_off, n_roots, e->d_root_rec, e->d_root_pos, e->d_replay_status, st));
-    e->launches += 1;
-    SCB_CUDA(cudaMemcpyAsync(e->h_replay_status, e->d_replay_status, sizeof(int32_t) * (size_t)n_roots,
-                             cudaMemcpyDeviceToHost, st));
-    SCB_CUDA(cudaStreamSynchronize(st));
+    SCB_CHECK(e->roots.reserve(n_roots));
+    SCB_CHECK(replay_into_slots(e, e->roots, n_roots, nullptr, nullptr, stack_off, stack));
     for (int r = 0; r < n_roots; r++) {
         const int32_t status = e->h_replay_status[r];
         if (!status) continue;
         set_error(replay_error("sc_set_roots", "root", r, status >> 3, status));
         return SC_E_INVAL;
     }
-    e->root_off.assign(stack_off, stack_off + n_roots + 1);
-    e->n_roots = n_roots;
+    for (int r = 0; r < n_roots; r++) e->roots.plies.push_back(stack_off[r + 1] - stack_off[r]);
     return SC_OK;
 }
 
@@ -1686,20 +1679,21 @@ int sc_predict_path(sc_engine *e, int n, const int32_t *root, const sc_move *pat
         set_error("sc_predict_path: bad argument");
         return SC_E_INVAL;
     }
-    if (e->n_roots == 0) {
+    const int n_roots = (int)e->roots.plies.size();
+    if (n_roots == 0) {
         set_error("sc_predict_path: no roots are set (sc_set_roots)");
         return SC_E_STATE;
     }
     if (n == 0) return SC_OK;
     for (int i = 0; i < n; i++) {
-        if (root[i] < 0 || root[i] >= e->n_roots) {
+        if (root[i] < 0 || root[i] >= n_roots) {
             set_error("sc_predict_path: root[" + std::to_string(i) + "] = " + std::to_string(root[i]) + " is not in 0.." +
-                      std::to_string(e->n_roots - 1));
+                      std::to_string(n_roots - 1));
             return SC_E_INVAL;
         }
     }
     NvtxRange nv_call("sc_predict_path");
-    return predict_replay(e, "sc_predict_path", n, root, nullptr, path, path_off, "path_off", "path", n_hist, pos_out,
+    return predict_replay(e, "sc_predict_path", n, root, &e->roots, path, path_off, "path_off", "path", n_hist, pos_out,
                           moves_out, move_cnt_out, priors_out, value_out, &e->last_path_ms, stream);
 }
 

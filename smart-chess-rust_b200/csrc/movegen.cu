@@ -60,9 +60,9 @@ __global__ void __launch_bounds__(MOVEGEN_THREADS) legal_moves_kernel(const sc_p
 // ---- sc_predict_stack / sc_set_roots / sc_predict_path: replay and pack ---------------------------------------------
 // Serial per leaf: each ply depends on the last.  What the repetition walk needs of every replayed position goes to a
 // global scratch rather than a per-thread array (local memory is reserved for every resident thread), and
-// chess::is_repetition walks it exactly as the host Game walks its stack.  sc_set_roots keeps these records of each
-// root game in a persistent table; sc_predict_path continues a stored root's final position with the leaf's path and
-// walks the root's records, then the path's.
+// chess::is_repetition walks it exactly as the host Game walks its stack.  sc_set_roots and an evaluator keep these
+// records of each root game in a persistent slot table; sc_predict_path and an evaluator's leaves continue a stored
+// root's final position with the leaf's path and walk the root's records, then the path's.
 
 namespace {
 
@@ -89,19 +89,8 @@ struct RootPathRecords {
 };
 using PathHistory = PlyHistory<RootPathRecords>;
 
-// where path_replay_kernel finds the records and the plies of root r.  sc_set_roots' table: root r's records at
-// off[r] + r, off[r + 1] - off[r] plies
-struct OffsetRoots {
-    const int32_t *off;
-    __device__ int64_t base(int r) const { return off[r] + r; }
-    __device__ int plies(int r) const { return off[r + 1] - off[r]; }
-};
-// an evaluator's slot table: slot r's records at r * (SC_MAX_STACK + 1), n[r] plies
-struct SlotRoots {
-    const int32_t *n;
-    __device__ int64_t base(int r) const { return (int64_t)r * (SC_MAX_STACK + 1); }
-    __device__ int plies(int r) const { return n[r]; }
-};
+// a slot table (sc_set_roots' roots, an evaluator's slots): slot g's records start at record slot_base(g)
+__device__ __forceinline__ int64_t slot_base(int g) { return (int64_t)g * (SC_MAX_STACK + 1); }
 
 // the replay's checks (Board.push verifies no legality either; from/to < 64 and promo are checked on the host)
 __device__ int replay_reject(const chess::Position &p, const sc_move &m)
@@ -163,26 +152,10 @@ __device__ __forceinline__ void pack_replayed(const History &h, const chess::Pos
 
 constexpr int REPLAY_THREADS = 32;
 
-// sc_set_roots, one thread per root: root r's records (plies + 1) at rec + off[r] + r, its final position and status
-__global__ void __launch_bounds__(REPLAY_THREADS) root_replay_kernel(const sc_move *__restrict__ stack,
-                                                                     const int32_t *__restrict__ off, int n,
-                                                                     ReplayPly *__restrict__ rec,
-                                                                     chess::Position *__restrict__ root_pos,
-                                                                     int32_t *__restrict__ status)
-{
-    const int r = blockIdx.x * blockDim.x + threadIdx.x;
-    if (r >= n) return;
-    const int base = off[r];
-    int len = off[r + 1] - base;
-    chess::Position p;
-    p.set_start();
-    status[r] = replay_moves(p, stack + base, len, rec + base + r, 0);
-    root_pos[r] = p;
-}
-
-// an evaluator's root updates, one thread per updated slot: update u replays stack[off[u], off[u+1]) into slot slot[u],
-// from the initial position or (append[u]) from the slot's stored position after its n_plies[slot] moves, and keeps
-// the records from that ply on, the final position, the plies and status[u]
+// sc_set_roots' and an evaluator's root updates, one thread per updated slot: update u replays stack[off[u], off[u+1])
+// into slot slot[u] (slot == nullptr: slot u), from the initial position or (append[u]; append == nullptr: none) from
+// the slot's stored position after its n_plies[slot] moves, and keeps the records from that ply on, the final
+// position, the plies and status[u]
 __global__ void __launch_bounds__(REPLAY_THREADS) slot_replay_kernel(const sc_move *__restrict__ stack,
                                                                      const int32_t *__restrict__ off,
                                                                      const int32_t *__restrict__ slot,
@@ -194,26 +167,25 @@ __global__ void __launch_bounds__(REPLAY_THREADS) slot_replay_kernel(const sc_mo
 {
     const int u = blockIdx.x * blockDim.x + threadIdx.x;
     if (u >= n) return;
-    const int g = slot[u], base = off[u];
+    const int g = slot ? slot[u] : u, base = off[u];
     int len = off[u + 1] - base, ply0 = 0;
     chess::Position p;
-    if (append[u]) {
+    if (append && append[u]) {
         p = slot_pos[g];
         ply0 = n_plies[g];
     } else {
         p.set_start();
     }
-    status[u] = replay_moves(p, stack + base, len, rec + SlotRoots{}.base(g) + ply0, ply0);
+    status[u] = replay_moves(p, stack + base, len, rec + slot_base(g) + ply0, ply0);
     slot_pos[g] = p;
     n_plies[g] = ply0 + len;
 }
 
-// sc_predict_stack / sc_predict_path / an evaluator's leaves, one thread per leaf: root[i]'s stored position (root ==
-// nullptr: the initial position) continued with path[off[i], off[i+1]) (records in the per-call scratch), packed over
-// the root's records and the path's
-template <class Roots>
+// sc_predict_stack / sc_predict_path / an evaluator's leaves, one thread per leaf: slot root[i]'s stored position (root
+// == nullptr: the initial position) continued with path[off[i], off[i+1]) (records in the per-call scratch), packed
+// over the slot's records and the path's
 __global__ void __launch_bounds__(REPLAY_THREADS) path_replay_kernel(
-    const ReplayPly *__restrict__ root_rec, Roots roots,
+    const ReplayPly *__restrict__ root_rec, const int32_t *__restrict__ root_n_plies,
     const chess::Position *__restrict__ root_pos, const int32_t *__restrict__ root, const sc_move *__restrict__ path,
     const int32_t *__restrict__ off, const int8_t *__restrict__ n_hist, int n, ReplayPly *__restrict__ scratch,
     sc_position *__restrict__ pos, int8_t *__restrict__ ep, int32_t *__restrict__ status)
@@ -228,8 +200,8 @@ __global__ void __launch_bounds__(REPLAY_THREADS) path_replay_kernel(
     int root_plies = 0;
     if (root) {
         const int r = root[i];
-        root_plies = roots.plies(r);
-        rh = root_rec + roots.base(r);
+        root_plies = root_n_plies[r];
+        rh = root_rec + slot_base(r);
         p = root_pos[r];
     } else {
         p.set_start();
@@ -242,16 +214,6 @@ __global__ void __launch_bounds__(REPLAY_THREADS) path_replay_kernel(
 
 size_t replay_scratch_bytes(int64_t positions) { return sizeof(ReplayPly) * (size_t)positions; }
 
-int launch_root_replay(const sc_move *d_stack, const int32_t *d_off, int n, void *d_rec, chess::Position *d_root_pos,
-                       int32_t *d_status, cudaStream_t st)
-{
-    if (n <= 0) return SC_OK;
-    root_replay_kernel<<<(n + REPLAY_THREADS - 1) / REPLAY_THREADS, REPLAY_THREADS, 0, st>>>(
-        d_stack, d_off, n, static_cast<ReplayPly *>(d_rec), d_root_pos, d_status);
-    SCB_CUDA(cudaGetLastError());
-    return SC_OK;
-}
-
 int launch_slot_replay(const sc_move *d_stack, const int32_t *d_off, const int32_t *d_slot, const int8_t *d_append,
                        int n, void *d_rec, chess::Position *d_slot_pos, int32_t *d_slot_plies, int32_t *d_status,
                        cudaStream_t st)
@@ -263,21 +225,14 @@ int launch_slot_replay(const sc_move *d_stack, const int32_t *d_off, const int32
     return SC_OK;
 }
 
-int launch_path_replay(const void *d_root_rec, const int32_t *d_root_off, const int32_t *d_slot_plies,
-                       const chess::Position *d_root_pos, const int32_t *d_root, const sc_move *d_path,
-                       const int32_t *d_off, const int8_t *d_n_hist, int n, void *d_scratch, sc_position *d_pos,
-                       int8_t *d_ep, int32_t *d_status, cudaStream_t st)
+int launch_path_replay(const void *d_slot_rec, const int32_t *d_slot_plies, const chess::Position *d_slot_pos,
+                       const int32_t *d_root, const sc_move *d_path, const int32_t *d_off, const int8_t *d_n_hist, int n,
+                       void *d_scratch, sc_position *d_pos, int8_t *d_ep, int32_t *d_status, cudaStream_t st)
 {
     if (n <= 0) return SC_OK;
-    const dim3 grid((n + REPLAY_THREADS - 1) / REPLAY_THREADS);
-    const ReplayPly *rec = static_cast<const ReplayPly *>(d_root_rec);
-    ReplayPly *scratch = static_cast<ReplayPly *>(d_scratch);
-    if (d_slot_plies)
-        path_replay_kernel<<<grid, REPLAY_THREADS, 0, st>>>(rec, SlotRoots{d_slot_plies}, d_root_pos, d_root, d_path,
-                                                            d_off, d_n_hist, n, scratch, d_pos, d_ep, d_status);
-    else
-        path_replay_kernel<<<grid, REPLAY_THREADS, 0, st>>>(rec, OffsetRoots{d_root_off}, d_root_pos, d_root, d_path,
-                                                            d_off, d_n_hist, n, scratch, d_pos, d_ep, d_status);
+    path_replay_kernel<<<(n + REPLAY_THREADS - 1) / REPLAY_THREADS, REPLAY_THREADS, 0, st>>>(
+        static_cast<const ReplayPly *>(d_slot_rec), d_slot_plies, d_slot_pos, d_root, d_path, d_off, d_n_hist, n,
+        static_cast<ReplayPly *>(d_scratch), d_pos, d_ep, d_status);
     SCB_CUDA(cudaGetLastError());
     return SC_OK;
 }
