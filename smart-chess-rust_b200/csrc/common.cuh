@@ -36,22 +36,21 @@ constexpr int LD_POLICY = 80;    // row stride of the policy logits buffer [B][6
 constexpr int N_VALUE_HIDDEN = 128;
 constexpr float LN_EPS = 1e-6f;  // timm LayerNorm2d
 
+// operand type of the tensor-core modes (tower_bf16.cu below)
+enum TcOp { TC_OP_BF16 = 0, TC_OP_FP16 = 1, TC_OP_E4M3 = 2 };
+// channels per K chunk (one 128-byte swizzle row): 64 16-bit or 128 8-bit elements
+constexpr int tc_op_bk(TcOp op) { return op == TC_OP_E4M3 ? 128 : 64; }
+
 // ---- encode.cu ---------------------------------------------------------------------------
 // planes: one warp per position. out element (b, s, c), s = rank*8+file, c < ld.
 int launch_encode_i8(const sc_position *d_pos, int n, int8_t *out, int32_t *meta_out, cudaStream_t st);
 int launch_encode_f32(const sc_position *d_pos, int n, float *out /*[n][64][112]*/, float *meta_out /*[n][8]*/,
                       cudaStream_t st);
-int launch_encode_bf16(const sc_position *d_pos, int n, __nv_bfloat16 *out /*[n][64][128]*/,
-                       float *meta_out /*[n][8]*/, cudaStream_t st);
-int launch_encode_fp16(const sc_position *d_pos, int n, __half *out /*[n][64][128]*/, float *meta_out /*[n][8]*/,
-                       cudaStream_t st);
-int launch_encode_e4m3(const sc_position *d_pos, int n, uint8_t *out /*[n][64][128]*/, float *meta_out /*[n][8]*/,
-                       cudaStream_t st);
+// tensor-core modes: [n][64][128] in operand type op (bf16 / fp16 bits, e4m3 bytes)
+int launch_encode_tc(TcOp op, const sc_position *d_pos, int n, void *out, float *meta_out /*[n][8]*/, cudaStream_t st);
 // NCHW float planes (sc_forward_only input) -> NHWC
 int launch_nchw_to_nhwc_f32(const float *in, int n, float *out, cudaStream_t st);
-int launch_nchw_to_nhwc_bf16(const float *in, int n, __nv_bfloat16 *out, cudaStream_t st);
-int launch_nchw_to_nhwc_fp16(const float *in, int n, __half *out, cudaStream_t st);
-int launch_nchw_to_nhwc_e4m3(const float *in, int n, uint8_t *out, cudaStream_t st);
+int launch_nchw_to_nhwc_tc(TcOp op, const float *in, int n, void *out, cudaStream_t st);
 
 // ---- policy.cu ----------------------------------------------------------------------------
 // logits [n][64][LD_POLICY] fp32 (square-major) -> per-leaf log-sum-exp, legal-move gather,
@@ -121,9 +120,6 @@ int launch_value_finish(const float *hidden_pre, int n_split, int n, const float
 // bf16, and then every operand buffer below (weights, activations; typed __nv_bfloat16) holds fp16 bit patterns, or
 // e4m3 bytes ([..][k] with k one byte each).  e4m3 weights come with `scale`: per output channel a power of two that the
 // epilogue multiplies the accumulator by.
-enum TcOp { TC_OP_BF16 = 0, TC_OP_FP16 = 1, TC_OP_E4M3 = 2 };
-// channels per K chunk (one 128-byte swizzle row): 64 16-bit or 128 8-bit elements
-constexpr int tc_op_bk(TcOp op) { return op == TC_OP_E4M3 ? 128 : 64; }
 struct TcConv;  // opaque per-layer state (tensor maps)
 enum { TC_EPI_LN = 0, TC_EPI_LN_SE = 1, TC_EPI_LN73 = 2, TC_EPI_RAW = 3 };
 // w: bf16 [taps][bn][k_per_tap] (K-major B operand); bn = 256 (tower / head 1x1 convs),
@@ -191,7 +187,8 @@ struct LatLayerDesc {
     const void *se_w1s8, *se_w2s8, *se_w1s4, *se_w2s4;
     const float *se_b1, *se_b2;
 };
-int lat_tower_create(LatTower **out, const LatLayerDesc *descs, int n, int boards_alloc, bool fp16);
+// op: TC_OP_BF16 or TC_OP_FP16 (there is no e4m3 latency kernel)
+int lat_tower_create(LatTower **out, const LatLayerDesc *descs, int n, int boards_alloc, TcOp op);
 // largest batch the latency kernel takes (one wave of clusters); 0 if it cannot run on this device
 int lat_tower_max_boards(const LatTower *t);
 // SC_E_STATE (no message) when the batch does not fit: run the throughput kernel instead

@@ -193,26 +193,15 @@ int launch_encode_f32(const sc_position *d_pos, int n, float *out, float *meta_o
     return SC_OK;
 }
 
-int launch_encode_bf16(const sc_position *d_pos, int n, __nv_bfloat16 *out, float *meta_out, cudaStream_t st)
+int launch_encode_tc(TcOp op, const sc_position *d_pos, int n, void *out, float *meta_out, cudaStream_t st)
 {
     if (n <= 0) return SC_OK;
-    encode_16bit_kernel<0x3F80u><<<n, ENC_WARPS * 32, 0, st>>>(d_pos, n, reinterpret_cast<uint16_t *>(out), meta_out);
-    SCB_CUDA(cudaGetLastError());
-    return SC_OK;
-}
-
-int launch_encode_fp16(const sc_position *d_pos, int n, __half *out, float *meta_out, cudaStream_t st)
-{
-    if (n <= 0) return SC_OK;
-    encode_16bit_kernel<0x3C00u><<<n, ENC_WARPS * 32, 0, st>>>(d_pos, n, reinterpret_cast<uint16_t *>(out), meta_out);
-    SCB_CUDA(cudaGetLastError());
-    return SC_OK;
-}
-
-int launch_encode_e4m3(const sc_position *d_pos, int n, uint8_t *out, float *meta_out, cudaStream_t st)
-{
-    if (n <= 0) return SC_OK;
-    encode_e4m3_kernel<<<n, ENC_WARPS * 32, 0, st>>>(d_pos, n, out, meta_out);
+    if (op == TC_OP_E4M3)
+        encode_e4m3_kernel<<<n, ENC_WARPS * 32, 0, st>>>(d_pos, n, static_cast<uint8_t *>(out), meta_out);
+    else if (op == TC_OP_FP16)
+        encode_16bit_kernel<0x3C00u><<<n, ENC_WARPS * 32, 0, st>>>(d_pos, n, static_cast<uint16_t *>(out), meta_out);
+    else
+        encode_16bit_kernel<0x3F80u><<<n, ENC_WARPS * 32, 0, st>>>(d_pos, n, static_cast<uint16_t *>(out), meta_out);
     SCB_CUDA(cudaGetLastError());
     return SC_OK;
 }
@@ -251,26 +240,15 @@ int launch_nchw_to_nhwc_f32(const float *in, int n, float *out, cudaStream_t st)
     return SC_OK;
 }
 
-int launch_nchw_to_nhwc_bf16(const float *in, int n, __nv_bfloat16 *out, cudaStream_t st)
+int launch_nchw_to_nhwc_tc(TcOp op, const float *in, int n, void *out, cudaStream_t st)
 {
     if (n <= 0) return SC_OK;
-    nchw_to_nhwc_kernel<__nv_bfloat16, C_IN_PAD><<<n, 256, 0, st>>>(in, n, out);
-    SCB_CUDA(cudaGetLastError());
-    return SC_OK;
-}
-
-int launch_nchw_to_nhwc_fp16(const float *in, int n, __half *out, cudaStream_t st)
-{
-    if (n <= 0) return SC_OK;
-    nchw_to_nhwc_kernel<__half, C_IN_PAD><<<n, 256, 0, st>>>(in, n, out);
-    SCB_CUDA(cudaGetLastError());
-    return SC_OK;
-}
-
-int launch_nchw_to_nhwc_e4m3(const float *in, int n, uint8_t *out, cudaStream_t st)
-{
-    if (n <= 0) return SC_OK;
-    nchw_to_nhwc_kernel<__nv_fp8_e4m3, C_IN_PAD><<<n, 256, 0, st>>>(in, n, reinterpret_cast<__nv_fp8_e4m3 *>(out));
+    if (op == TC_OP_E4M3)
+        nchw_to_nhwc_kernel<__nv_fp8_e4m3, C_IN_PAD><<<n, 256, 0, st>>>(in, n, static_cast<__nv_fp8_e4m3 *>(out));
+    else if (op == TC_OP_FP16)
+        nchw_to_nhwc_kernel<__half, C_IN_PAD><<<n, 256, 0, st>>>(in, n, static_cast<__half *>(out));
+    else
+        nchw_to_nhwc_kernel<__nv_bfloat16, C_IN_PAD><<<n, 256, 0, st>>>(in, n, static_cast<__nv_bfloat16 *>(out));
     SCB_CUDA(cudaGetLastError());
     return SC_OK;
 }

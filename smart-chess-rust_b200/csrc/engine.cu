@@ -125,25 +125,26 @@ static uint16_t f2h(float f)
     return r;
 }
 
-// The weights of a 16-bit tensor-core engine that become MMA / SE operands, rounded to its operand type.  An fp16 engine
-// cannot represent a weight beyond +-65504: `bad` records one, and the load then fails naming the tensor (a bf16 engine
-// has the fp32 exponent range and takes every finite weight).
-struct Op16Weights {
-    bool fp16;
-    bool bad = false;
-    uint16_t operator()(float f)
-    {
-        if (!fp16) return f2bf(f);
-        if (fabsf(f) > 65504.f) bad = true;
-        return f2h(f);
-    }
-    int check(const std::string &tensor) const
-    {
-        if (!bad) return SC_OK;
-        set_error("weight blob: " + tensor + " has a weight beyond the fp16 range (|w| > 65504)");
-        return SC_E_IO;
-    }
-};
+static uint8_t f2e4m3(float f) { return (uint8_t)__nv_cvt_float_to_fp8(f, __NV_SATFINITE, __NV_E4M3); }
+
+// one weight as an operand of type op, round to nearest even: bf16 or fp16 bits, or the e4m3 byte (saturated to +-448)
+static uint16_t op_weight(TcOp op, float f)
+{
+    return op == TC_OP_FP16 ? f2h(f) : op == TC_OP_E4M3 ? f2e4m3(f) : f2bf(f);
+}
+
+// An fp16 engine cannot represent a weight beyond +-65504: the load fails naming the tensor (bf16 has the fp32 exponent
+// range and takes every finite weight, e4m3 weights are scaled into range)
+static int check_op_range(TcOp op, const float *w, size_t n, const std::string &tensor)
+{
+    if (op != TC_OP_FP16) return SC_OK;
+    for (size_t i = 0; i < n; i++)
+        if (fabsf(w[i]) > 65504.f) {
+            set_error("weight blob: " + tensor + " has a weight beyond the fp16 range (|w| > 65504)");
+            return SC_E_IO;
+        }
+    return SC_OK;
+}
 
 // fp8 mode: the e4m3 weights of one output channel whose largest |w| is amax carry the scale s = 2^ceil(log2(amax / 448))
 // (1 for an all-zero channel): w / s is at most 448 and is rounded to e4m3 (round to nearest even).  A power of two
@@ -154,20 +155,6 @@ static float e4m3_scale(float amax)
     int e;
     const float f = frexpf(amax, &e);  // amax = f 2^e, f in [0.5, 1); 448 = 0.875 2^9
     return ldexpf(1.f, f <= 0.875f ? e - 9 : e - 8);
-}
-static uint8_t f2e4m3(float f) { return (uint8_t)__nv_cvt_float_to_fp8(f, __NV_SATFINITE, __NV_E4M3); }
-
-// rows x k fp32 weights (row r at w[r * k], one output channel each) -> e4m3 bytes and the rows' scales
-static void quantize_e4m3(const std::vector<float> &w, int rows, size_t k, std::vector<uint8_t> &q, std::vector<float> &scale)
-{
-    q.assign(w.size(), 0);
-    scale.assign((size_t)rows, 1.f);
-    for (int r = 0; r < rows; r++) {
-        float amax = 0.f;
-        for (size_t i = 0; i < k; i++) amax = fmaxf(amax, fabsf(w[r * k + i]));
-        scale[r] = e4m3_scale(amax);
-        for (size_t i = 0; i < k; i++) q[r * k + i] = f2e4m3(w[r * k + i] / scale[r]);
-    }
 }
 
 struct ConvW {
@@ -383,6 +370,37 @@ static int upload_vec(sc_engine *e, const Blob &b, const std::string &name, size
     return upload(e, out, h);
 }
 
+// fp32 weights in the tensor-core B-operand layout [taps][rows][k] (one output channel per row) -> the device operand in
+// the engine's operand type, and for e4m3 the rows' scales over all taps x k of their weights (*d_scale: nullptr for the
+// 16-bit types)
+static int pack_tc_weights(sc_engine *e, const std::vector<float> &w, int taps, int rows, size_t k,
+                           const std::string &tensor, __nv_bfloat16 **d_w, float **d_scale)
+{
+    SCB_CHECK(check_op_range(e->op, w.data(), w.size(), tensor));
+    std::vector<float> scale;
+    if (e->op == TC_OP_E4M3) {
+        scale.resize((size_t)rows);
+        for (int r = 0; r < rows; r++) {
+            float amax = 0.f;
+            for (int t = 0; t < taps; t++)
+                for (size_t i = 0; i < k; i++) amax = fmaxf(amax, fabsf(w[((size_t)t * rows + r) * k + i]));
+            scale[r] = e4m3_scale(amax);
+        }
+    }
+    const size_t es = e->op == TC_OP_E4M3 ? 1 : 2;
+    std::vector<uint8_t> h(w.size() * es);
+    for (size_t i = 0; i < w.size(); i++) {
+        const uint16_t q = op_weight(e->op, scale.empty() ? w[i] : w[i] / scale[i / k % rows]);
+        memcpy(&h[i * es], &q, es);  // little-endian: an e4m3 byte is q's low byte
+    }
+    uint8_t *d = nullptr;
+    SCB_CHECK(upload(e, &d, h));
+    *d_w = reinterpret_cast<__nv_bfloat16 *>(d);
+    *d_scale = nullptr;
+    if (!scale.empty()) SCB_CHECK(upload(e, d_scale, scale));
+    return SC_OK;
+}
+
 // conv weight [cout][cin][k][k] + bias + LayerNorm gamma/beta -> device layouts
 static int load_conv(sc_engine *e, const Blob &b, const std::string &wname, const std::string &lnname, int taps,
                      int cin, int cout, ConvW &c, int epi = TC_EPI_LN)
@@ -437,36 +455,13 @@ static int load_conv(sc_engine *e, const Blob &b, const std::string &wname, cons
     } else {
         // B operand, K-major: [tap][bn rows][cin_pad]; bn = 256, or 80 for the 73-wide policy conv
         const int bn = cout == C_TOWER ? C_TOWER : LD_POLICY;
-        if (e->op == TC_OP_E4M3) {
-            // per output channel [taps][cin_pad] -> e4m3 with the channel's scale, then [tap][bn][cin_pad]
-            const size_t k = (size_t)taps * c.cin_pad;
-            std::vector<float> wc((size_t)bn * k, 0.f);
-            for (int co = 0; co < cout; co++)
-                for (int ci = 0; ci < cin; ci++)
-                    for (int t = 0; t < taps; t++) wc[co * k + (size_t)t * c.cin_pad + ci] = w->data[((size_t)co * cin + ci) * taps + t];
-            std::vector<uint8_t> q, h(wc.size());
-            std::vector<float> sc;
-            quantize_e4m3(wc, bn, k, q, sc);
-            for (int co = 0; co < bn; co++)
-                for (int t = 0; t < taps; t++)
-                    memcpy(&h[((size_t)t * bn + co) * c.cin_pad], &q[co * k + (size_t)t * c.cin_pad], (size_t)c.cin_pad);
-            uint8_t *d = nullptr;
-            SCB_CHECK(upload(e, &d, h));
-            SCB_CHECK(upload(e, &c.scale, sc));
-            c.w_bf16 = reinterpret_cast<__nv_bfloat16 *>(d);
-            return tc_conv_create(&c.tc, c.w_bf16, taps, c.cin_pad, bn, epi, c.bias, c.gamma, c.beta, TC_OP_E4M3, c.scale);
-        }
-        std::vector<uint16_t> h((size_t)taps * bn * c.cin_pad, 0);
-        Op16Weights cv{e->op == TC_OP_FP16};
+        std::vector<float> h((size_t)taps * bn * c.cin_pad, 0.f);
         for (int co = 0; co < cout; co++)
             for (int ci = 0; ci < cin; ci++)
                 for (int t = 0; t < taps; t++)
-                    h[((size_t)t * bn + co) * c.cin_pad + ci] = cv(w->data[((size_t)co * cin + ci) * taps + t]);
-        SCB_CHECK(cv.check(wname + ".weight"));
-        uint16_t *d = nullptr;
-        SCB_CHECK(upload(e, &d, h));
-        c.w_bf16 = reinterpret_cast<__nv_bfloat16 *>(d);
-        SCB_CHECK(tc_conv_create(&c.tc, c.w_bf16, taps, c.cin_pad, bn, epi, c.bias, c.gamma, c.beta, e->op));
+                    h[((size_t)t * bn + co) * c.cin_pad + ci] = w->data[((size_t)co * cin + ci) * taps + t];
+        SCB_CHECK(pack_tc_weights(e, h, taps, bn, c.cin_pad, wname + ".weight", &c.w_bf16, &c.scale));
+        SCB_CHECK(tc_conv_create(&c.tc, c.w_bf16, taps, c.cin_pad, bn, epi, c.bias, c.gamma, c.beta, e->op, c.scale));
     }
     return SC_OK;
 }
@@ -503,19 +498,19 @@ static int load_weights(sc_engine *e, const Blob &b)
         } else {
             // packed so that epilogue thread j (fc1) / channel c (fc2) reads 8 consecutive inputs
             // with one coalesced 16-byte load: w1p[q][j][i] = fc1[j][8q+i], w2p[q][c][i] = fc2[c][8q+i]
-            // (fp8 mode: bf16, the SE runs on the CUDA cores)
+            // in the type the kernels park values in: the operand type, bf16 for e4m3 (the SE runs on the CUDA cores)
+            const TcOp park = e->op == TC_OP_FP16 ? TC_OP_FP16 : TC_OP_BF16;
+            SCB_CHECK(check_op_range(park, f1->data, f1->numel, p + "se.fc1.weight"));
+            SCB_CHECK(check_op_range(park, f2->data, f2->numel, p + "se.fc2.weight"));
             std::vector<uint16_t> w1p((size_t)C_TOWER * C_SE), w2p((size_t)C_SE * C_TOWER);
-            Op16Weights cv1{e->op == TC_OP_FP16}, cv2{e->op == TC_OP_FP16};
             for (int q = 0; q < C_TOWER / 8; q++)
                 for (int j = 0; j < C_SE; j++)
                     for (int k = 0; k < 8; k++)
-                        w1p[((size_t)q * C_SE + j) * 8 + k] = cv1(f1->data[(size_t)j * C_TOWER + 8 * q + k]);
+                        w1p[((size_t)q * C_SE + j) * 8 + k] = op_weight(park, f1->data[(size_t)j * C_TOWER + 8 * q + k]);
             for (int q = 0; q < C_SE / 8; q++)
                 for (int c = 0; c < C_TOWER; c++)
                     for (int k = 0; k < 8; k++)
-                        w2p[((size_t)q * C_TOWER + c) * 8 + k] = cv2(f2->data[(size_t)c * C_SE + 8 * q + k]);
-            SCB_CHECK(cv1.check(p + "se.fc1.weight"));
-            SCB_CHECK(cv2.check(p + "se.fc2.weight"));
+                        w2p[((size_t)q * C_TOWER + c) * 8 + k] = op_weight(park, f2->data[(size_t)c * C_SE + 8 * q + k]);
             SCB_CHECK(upload(e, &e->se[i].w1p, w1p));
             SCB_CHECK(upload(e, &e->se[i].w2p, w2p));
             // latency kernel: the same numbers sliced per cluster rank r -- fc1 COLUMNS (input channels) [r * NC, +NC)
@@ -528,12 +523,12 @@ static int load_weights(sc_engine *e, const Blob &b)
                         for (int j = 0; j < C_SE; j++)
                             for (int k = 0; k < 8; k++)
                                 a[(((size_t)r * (NC / 8) + q) * C_SE + j) * 8 + k] =
-                                    cv1(f1->data[(size_t)j * C_TOWER + r * NC + 8 * q + k]);
+                                    op_weight(park, f1->data[(size_t)j * C_TOWER + r * NC + 8 * q + k]);
                     for (int q = 0; q < C_SE / 8; q++)
                         for (int c = 0; c < NC; c++)
                             for (int k = 0; k < 8; k++)
                                 b[(((size_t)r * (C_SE / 8) + q) * NC + c) * 8 + k] =
-                                    cv2(f2->data[(size_t)(r * NC + c) * C_SE + 8 * q + k]);
+                                    op_weight(park, f2->data[(size_t)(r * NC + c) * C_SE + 8 * q + k]);
                 }
                 SCB_CHECK(upload(e, &e->se[i].w1s[v], a));
                 SCB_CHECK(upload(e, &e->se[i].w2s[v], b));
@@ -565,34 +560,17 @@ static int load_weights(sc_engine *e, const Blob &b)
                     for (int s = 0; s < 64; s++)
                         h[((size_t)s * C_TOWER + c) * N_VALUE_HIDDEN + j] = fc->data[(size_t)j * KT + c * 64 + s];
             SCB_CHECK(upload(e, &e->vfc_w_f32, h));
-        } else if (e->op == TC_OP_E4M3) {
-            // the B operand below in e4m3, with the hidden units' scales
-            std::vector<float> wf((size_t)N_VALUE_HIDDEN * KV);
-            for (int j = 0; j < N_VALUE_HIDDEN; j++)
-                for (int c = 0; c < C_TOWER; c++)
-                    for (int s = 0; s < 64; s++) wf[(size_t)j * KV + (size_t)s * C_TOWER + c] = fc->data[(size_t)j * KT + c * 64 + s];
-            std::vector<uint8_t> q;
-            std::vector<float> sc;
-            quantize_e4m3(wf, N_VALUE_HIDDEN, KV, q, sc);
-            uint8_t *d = nullptr;
-            SCB_CHECK(upload(e, &d, q));
-            SCB_CHECK(upload(e, &e->v_scale, sc));
-            SCB_CHECK(tc_conv_create(&e->vfc_tc, reinterpret_cast<__nv_bfloat16 *>(d), 1, KV, N_VALUE_HIDDEN, TC_EPI_RAW,
-                                     nullptr, nullptr, nullptr, TC_OP_E4M3, e->v_scale));
         } else {
-            // B operand of the value FC GEMM, K-major: [128][16384] with k' = s*256 + c
-            // (the meta columns stay fp32: the fused value tail applies them)
-            std::vector<uint16_t> h((size_t)N_VALUE_HIDDEN * KV);
-            Op16Weights cv{e->op == TC_OP_FP16};
+            // B operand of the value FC GEMM, K-major: [128][16384] with k' = s*256 + c (fp8 mode: with the hidden units'
+            // scales; the meta columns stay fp32: the fused value tail applies them)
+            std::vector<float> h((size_t)N_VALUE_HIDDEN * KV);
             for (int j = 0; j < N_VALUE_HIDDEN; j++)
                 for (int c = 0; c < C_TOWER; c++)
-                    for (int s = 0; s < 64; s++)
-                        h[(size_t)j * KV + (size_t)s * C_TOWER + c] = cv(fc->data[(size_t)j * KT + c * 64 + s]);
-            SCB_CHECK(cv.check("value_head.ffn.0.weight"));
-            uint16_t *d = nullptr;
-            SCB_CHECK(upload(e, &d, h));
-            SCB_CHECK(tc_conv_create(&e->vfc_tc, reinterpret_cast<__nv_bfloat16 *>(d), 1, KV, N_VALUE_HIDDEN, TC_EPI_RAW,
-                                     nullptr, nullptr, nullptr, e->op));
+                    for (int s = 0; s < 64; s++) h[(size_t)j * KV + (size_t)s * C_TOWER + c] = fc->data[(size_t)j * KT + c * 64 + s];
+            __nv_bfloat16 *d = nullptr;
+            SCB_CHECK(pack_tc_weights(e, h, 1, N_VALUE_HIDDEN, KV, "value_head.ffn.0.weight", &d, &e->v_scale));
+            SCB_CHECK(tc_conv_create(&e->vfc_tc, d, 1, KV, N_VALUE_HIDDEN, TC_EPI_RAW, nullptr, nullptr, nullptr, e->op,
+                                     e->v_scale));
         }
     }
     SCB_CHECK(upload_vec(e, b, "value_head.ffn.0.bias", N_VALUE_HIDDEN, &e->v_b1));
@@ -827,9 +805,7 @@ static int encode_for_mode(sc_engine *e, const sc_position *d_pos, int n, cudaSt
     NvtxRange nv("scb200: encode planes");
     e->launches += 1;
     if (e->mode == SC_MODE_FP32 && !e->fp32_tc) return launch_encode_f32(d_pos, n, e->f_planes, e->d_meta, st);
-    if (e->op == TC_OP_FP16) return launch_encode_fp16(d_pos, n, reinterpret_cast<__half *>(e->h_planes), e->d_meta, st);
-    if (e->op == TC_OP_E4M3) return launch_encode_e4m3(d_pos, n, reinterpret_cast<uint8_t *>(e->h_planes), e->d_meta, st);
-    return launch_encode_bf16(d_pos, n, e->h_planes, e->d_meta, st);
+    return launch_encode_tc(e->op, d_pos, n, e->h_planes, e->d_meta, st);
 }
 
 // sc_predict's buffers, stream and events (first call)
@@ -1421,7 +1397,7 @@ int sc_create(const char *weights_blob_path, int device, int mode, int max_batch
                 }
                 lat_layer(e->pol1, e->h_x, e->h_t, nullptr, 0, 0, nullptr);
                 lat_layer(e->val1, e->h_x, e->h_y, nullptr, 1, 0, nullptr);
-                if ((rc = lat_tower_create(&e->lat, ld.data(), (int)ld.size(), e->alloc_boards, e->op == TC_OP_FP16)) != SC_OK) break;
+                if ((rc = lat_tower_create(&e->lat, ld.data(), (int)ld.size(), e->alloc_boards, e->op)) != SC_OK) break;
                 e->lat_max_boards = lat_tower_max_boards(e->lat);
             }
         }
@@ -1961,12 +1937,8 @@ int sc_forward_only(sc_engine *e, int n, const float *planes, const float *meta,
     SCB_CUDA(cudaMemcpy2DAsync(e->d_meta, 8 * 4, meta, SC_N_META * 4, SC_N_META * 4, (size_t)n, cudaMemcpyHostToDevice, st));
     if (e->mode == SC_MODE_FP32 && !e->fp32_tc)
         SCB_CHECK(launch_nchw_to_nhwc_f32(d_nchw, n, e->f_planes, st));
-    else if (e->op == TC_OP_FP16)
-        SCB_CHECK(launch_nchw_to_nhwc_fp16(d_nchw, n, reinterpret_cast<__half *>(e->h_planes), st));
-    else if (e->op == TC_OP_E4M3)
-        SCB_CHECK(launch_nchw_to_nhwc_e4m3(d_nchw, n, reinterpret_cast<uint8_t *>(e->h_planes), st));
     else
-        SCB_CHECK(launch_nchw_to_nhwc_bf16(d_nchw, n, e->h_planes, st));
+        SCB_CHECK(launch_nchw_to_nhwc_tc(e->op, d_nchw, n, e->h_planes, st));
     e->launches += 1;
     if (e->timing) SCB_CUDA(cudaEventRecord(e->ev[0], st));
     SCB_CHECK(run_network(e, n, st));

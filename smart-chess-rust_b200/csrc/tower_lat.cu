@@ -629,7 +629,7 @@ template <int CL> constexpr int lat_smem_bytes()
 struct LatTower {
     LatLayer *d_layers[2] = {nullptr, nullptr};  // [0]: CL = 8, [1]: CL = 4
     int n_layers = 0;
-    bool fp16 = false;                           // operand type OpFp16 instead of OpBf16
+    TcOp op = TC_OP_BF16;                        // TC_OP_BF16 (OpBf16) or TC_OP_FP16 (OpFp16)
     int max_tiles[2] = {0, 0};                   // co-resident clusters of 8 / 4 CTAs
     bool one_board = true;                       // one-board tiles (M64) while there are clusters for them
 };
@@ -655,11 +655,16 @@ template <int CL, class OT> static int lat_max_clusters(int *out)
     return SC_OK;
 }
 
-int lat_tower_create(LatTower **out, const LatLayerDesc *descs, int n, int boards_alloc, bool fp16)
+int lat_tower_create(LatTower **out, const LatLayerDesc *descs, int n, int boards_alloc, TcOp op)
 {
+    if (op != TC_OP_BF16 && op != TC_OP_FP16) {
+        set_error("lat_tower_create: no latency kernel for this operand type");
+        return SC_E_INVAL;
+    }
+    const bool fp16 = op == TC_OP_FP16;
     LatTower *t = new LatTower();
     t->n_layers = n;
-    t->fp16 = fp16;
+    t->op = op;
     const CUtensorMapDataType dt = fp16 ? OpFp16::TMAP : OpBf16::TMAP;
     for (int v = 0; v < 2; v++) {
         const int CL = v == 0 ? 8 : 4, NC = 256 / CL;
@@ -810,7 +815,8 @@ int lat_tower_launch(LatTower *t, int n_boards, cudaStream_t st, int max_layers)
     if (n_boards <= 0) return SC_OK;
     // one-board tiles (half the operand traffic per CTA) while every board can have a cluster -- 8 CTAs per board, then 4
     // (measured, n = 16: 0.418 ms against 0.433 ms for two boards per 8-CTA cluster) -- then two-board tiles
-    return t->fp16 ? lat_dispatch<OpFp16>(t, n_boards, st, max_layers) : lat_dispatch<OpBf16>(t, n_boards, st, max_layers);
+    return t->op == TC_OP_FP16 ? lat_dispatch<OpFp16>(t, n_boards, st, max_layers)
+                               : lat_dispatch<OpBf16>(t, n_boards, st, max_layers);
 }
 
 }  // namespace scb

@@ -3,61 +3,32 @@
 fp16 mode rounds exactly where bf16 mode rounds, to fp16 instead of bf16 (round to nearest even): the conv, SE and
 value-FC weights, each layer's stored output, the SE layers' parked z and the residual stream x.  Everything else is the
 same fp32 arithmetic.  fp16 keeps 11 significant bits where bf16 keeps 8, so its error against the fp32 oracle should be
-about 1/8 of bf16's; these tests hold it to at most 1/3, and check the per-layer rounding, the bit-identity of the
-kernels and launch structures, the drivers and the weight range check.
+about 1/8 of bf16's; these tests hold it to at most 1/3, and check the bit-identity of the latency and throughput kernels,
+the per-layer rounding, the launch structures, the network variants, the drivers and the weight range check.  The
+per-layer and heads references and the launch-variant and driver checks are test_gpu_layer_reference's, shared with
+the other tensor-core modes.
 """
+import functools
 import json
 import os
 
 import numpy as np
 import pytest
+import scb200
 import torch
 import torch.nn.functional as F
 
 from conftest import games_to_batch
 from test_gpu_bench_config import batch2048, net19  # noqa: F401  (fixtures)
-from test_gpu_layer_reference import (  # noqa: F401  (fixtures and dtype-free helpers)
-    LAT_SHAPES, PLANES, X, T, Y, BIT_EQUAL_MIN, _batch, _engine_tensors, _layers, _norm, _nhwc_to_nchw, games, nets)
+from test_gpu_layer_reference import (  # noqa: F401  (fixtures)
+    FP16, LAT_SHAPES, LAUNCH_VARIANTS, _batch, _engine as _engine_any, _engine_tensors, _eval as _eval_any,
+    check_launch_variant, check_selfplay_arena_and_game, games, nets, run_heads, run_latency_layers,
+    run_throughput_layers)
 
 pytestmark = pytest.mark.gpu
 
-
-# ---- fp16 arithmetic of the reference ---------------------------------------------------------------------------
-def _rnd16(t):
-    return t.to(torch.float16).to(torch.float64)
-
-
-def _u16_to_f64(u):
-    return torch.from_numpy(u.view(np.float16).astype(np.float64))
-
-
-def _ulp16(v):
-    """Spacing of fp16 numbers at |v|: 2^(e - 11) for normal numbers, 2^-24 below 2^-14 (0 at 0)."""
-    m, e = np.frexp(np.abs(v))
-    return np.where(v == 0, 0.0, np.ldexp(1.0, np.maximum(e - 11, -24)))
-
-
-def _conv_bias(sd, conv, x):
-    w = _rnd16(sd[conv + ".weight"].double())
-    return F.conv2d(x, w, sd[conv + ".bias"].double(), padding=w.shape[-1] // 2)
-
-
-def _layer_reference(sd, layer, inp, resid):
-    """One layer in float64 on the kernel's inputs, fp16 where the kernel rounds -> (out before the final rounding,
-    z, gate, a = conv + bias).  (test_gpu_layer_reference's bf16 version with the operand type swapped.)"""
-    conv, norm, _, _, relu, se = layer
-    a = _conv_bias(sd, conv, inp)
-    z = _norm(sd, norm, a)
-    if se is None:
-        return (z.clamp_min(0) if relu else z), None, None, a
-    if se == "residual":
-        gate = torch.ones(z.shape[0], z.shape[1], 1, 1, dtype=torch.float64)
-    else:
-        m = z.mean(dim=(2, 3))
-        h = (m @ _rnd16(sd[se + "fc1.weight"].double()).reshape(128, 256).T + sd[se + "fc1.bias"].double()).clamp_min(0)
-        gate = torch.sigmoid(h @ _rnd16(sd[se + "fc2.weight"].double()).reshape(256, 128).T + sd[se + "fc2.bias"].double())
-        gate = gate[:, :, None, None]
-    return (gate * _rnd16(z) + resid).clamp_min(0), z, gate, a
+_engine = functools.partial(_engine_any, mode=scb200.SC_MODE_FP16)
+_eval = functools.partial(_eval_any, mode=scb200.SC_MODE_FP16)
 
 
 def forward_fp16_operands(sd, planes, meta):
@@ -99,26 +70,6 @@ def forward_fp16_operands(sd, planes, meta):
     z = F.relu(F.linear(torch.cat((rnd(z), meta.float()), dim=1), w1, sd[vh + "ffn.0.bias"]))
     v = torch.tanh(F.linear(z, sd[vh + "ffn.2.weight"], sd[vh + "ffn.2.bias"]))
     return logp, v * (meta[:, 0:1].float() * 2 - 1)
-
-
-def _engine(blob, monkeypatch, env=None, max_batch=512, mode=None):
-    import scb200
-
-    for k in ("SCB200_LATENCY", "SCB200_LAT_CLUSTER", "SCB200_LAT_ONE_BOARD", "SCB200_TOWER", "SCB200_TOWER_GROUP",
-              "SCB200_FUSE_GATHER", "SCB200_FUSE_VALUE"):
-        monkeypatch.delenv(k, raising=False)
-    for k, v in (env or {}).items():
-        monkeypatch.setenv(k, v)
-    return scb200.Engine(blob, 0, scb200.SC_MODE_FP16 if mode is None else mode, max_batch)
-
-
-def _eval(blob, monkeypatch, pos, moves, off, env=None, mode=None, max_batch=2048):
-    e = _engine(blob, monkeypatch, env, max_batch, mode)
-    try:
-        pri, val = e.eval(pos, moves, off)
-        return pri.copy(), val.copy()
-    finally:
-        e.close()
 
 
 # ---- 1. the bench workload against the oracle -------------------------------------------------------------------
@@ -178,115 +129,20 @@ def test_fp16_mode_deviation_is_operand_rounding(co, nets, games, monkeypatch): 
 
 
 # ---- 3. every layer against float64 -----------------------------------------------------------------------------
-def _check_layers(tag, sd, stressed, e, pos, which, boards=None):
-    """test_gpu_layer_reference._check_layers with fp16 rounding: layer k from the k - 1 call's buffers."""
-    import net
-
-    n = len(pos)
-    boards = np.arange(n) if boards is None else np.asarray(boards)
-    planes, _ = e.encode_only(pos)
-    prev = [np.zeros((n, 64, 256), np.uint16) for _ in range(3)]
-    prev_planes = net.planes_i8_hwc_to_nchw(planes[boards]).double()
-    failures = []
-    for k, layer in enumerate(_layers(sd), start=1):
-        cur = e.debug_tower(pos, k, which)
-        conv, _, reads, writes, _, se = layer
-        for b in (X, T, Y):
-            if b != writes:
-                assert np.array_equal(cur[b], prev[b]), f"{tag} which={which} layer {k} ({conv}) changed buffer {'xty'[b]}"
-        inp = prev_planes if reads == PLANES else _nhwc_to_nchw(_u16_to_f64(prev[reads][boards]))
-        resid = _nhwc_to_nchw(_u16_to_f64(prev[X][boards])) if se is not None else None
-        ref, z, gate, a = _layer_reference(sd, layer, inp, resid)
-        got = _nhwc_to_nchw(_u16_to_f64(cur[writes][boards])).numpy()
-        ref = ref.numpy()
-        err = np.abs(got - ref)
-        if layer[1] + ".weight" in sd:
-            scale = np.abs(sd[layer[1] + ".weight"].double().numpy()).reshape(1, -1, 1, 1)
-        else:
-            scale = a.std(dim=1, unbiased=False, keepdim=True).numpy()
-        g = 1.0 if gate is None else gate.numpy()
-        floor = 2e-5 * scale * g + 1e-6
-        if k - 1 in stressed:
-            ratio = stressed[k - 1] / a.std(dim=1, unbiased=False, keepdim=True).numpy()
-            shift_tol = (1e-3 + 4 * ratio * 2.0 ** -24) * scale * g
-        else:
-            shift_tol = 0.0
-        tol = _ulp16(ref) + floor + shift_tol
-        if z is not None:
-            tol = tol + gate.numpy() * _ulp16(z.numpy())
-        want = _rnd16(torch.from_numpy(ref)).numpy()
-        live = (want != 0) | (got != 0)
-        equal = float((got == want)[live].mean())
-        print(f"{tag} which={which} n={n} layer {k:2d} {conv:22s} max err / bound {float(np.max(err / tol)):6.3f}  "
-              f"bit-equal {equal:.5f} of {live.mean():.2f}")
-        assert np.isfinite(got).all(), f"{tag} layer {k} ({conv}): non-finite output"
-        if not (err <= tol).all():
-            i = np.unravel_index(np.argmax(err - tol), err.shape)
-            failures.append(f"layer {k} ({conv}): {int((err > tol).sum())} elements out of bound, worst at {i}: "
-                            f"got {got[i]:.6g} ref {ref[i]:.6g}")
-        if k - 1 not in stressed and equal < BIT_EQUAL_MIN:
-            failures.append(f"layer {k} ({conv}): bit-equal fraction {equal:.4f} < {BIT_EQUAL_MIN}")
-        prev = cur
-    assert not failures, f"{tag} which={which} n={n}:\n" + "\n".join(failures)
-
-
 @pytest.mark.parametrize("tag", ["n2", "stress"])
 def test_fp16_throughput_kernel_layers(nets, games, monkeypatch, tag):  # noqa: F811
-    sd, blob, stressed = nets[tag]
-    e = _engine(blob, monkeypatch)
-    try:
-        for n in (1, 3, 6):
-            pos, _, _ = _batch(games, n)
-            _check_layers(tag, sd, stressed, e, pos, 0)
-        pos, _, _ = _batch(games, 333)
-        _check_layers(tag, sd, stressed, e, pos, 0, boards=[0, 1, 2, 3, 127, 128, 329, 330, 331, 332])
-    finally:
-        e.close()
+    run_throughput_layers(FP16, nets, games, monkeypatch, tag, (1, 3, 6), [0, 1, 2, 3, 127, 128, 329, 330, 331, 332])
 
 
 @pytest.mark.parametrize("shape", sorted(LAT_SHAPES))
 @pytest.mark.parametrize("tag", ["n2", "stress"])
 def test_fp16_latency_kernel_layers(nets, games, monkeypatch, tag, shape):  # noqa: F811
-    sd, blob, stressed = nets[tag]
-    e = _engine(blob, monkeypatch, LAT_SHAPES[shape], max_batch=16)
-    try:
-        for n in (1, 5):
-            pos, _, _ = _batch(games, n)
-            _check_layers(f"{tag}/{shape}", sd, stressed, e, pos, 1)
-    finally:
-        e.close()
-
-
-def _heads_reference(sd, t, y, meta):
-    lg = _conv_bias(sd, "policy_head.model.2", t)
-    lg = _norm(sd, "policy_head.model.3", lg)
-    logp = torch.log_softmax(lg.flatten(1), dim=1)
-    w1 = sd["value_head.ffn.0.weight"].double()
-    w1 = torch.cat((_rnd16(w1[:, :64 * 256]), w1[:, 64 * 256:]), dim=1)
-    hid = (torch.cat((y.flatten(1), meta), dim=1) @ w1.T + sd["value_head.ffn.0.bias"].double()).clamp_min(0)
-    v = torch.tanh(hid @ sd["value_head.ffn.2.weight"].double().T + sd["value_head.ffn.2.bias"].double())
-    return logp.numpy(), (v[:, 0] * (meta[:, 0] * 2 - 1)).numpy()
+    run_latency_layers(FP16, nets, games, monkeypatch, tag, shape)
 
 
 @pytest.mark.parametrize("tag", ["n2", "stress"])
 def test_fp16_heads_from_tower_buffers(nets, games, monkeypatch, tag):  # noqa: F811
-    import net
-
-    sd, blob, _ = nets[tag]
-    e = _engine(blob, monkeypatch)
-    try:
-        for n in (37, 333):
-            pos, _, _ = _batch(games, n)
-            planes, meta = e.encode_only(pos)
-            _, t, y = e.debug_tower(pos, len(_layers(sd)), 0)
-            lp, v = e.forward_only(net.planes_i8_hwc_to_nchw(planes).numpy(), meta.astype(np.float32))
-            lp_ref, v_ref = _heads_reference(sd, _nhwc_to_nchw(_u16_to_f64(t)), _nhwc_to_nchw(_u16_to_f64(y)),
-                                             torch.from_numpy(meta).double())
-            dl, dv = float(np.abs(lp - lp_ref).max()), float(np.abs(v - v_ref).max())
-            print(f"fp16 {tag} heads n={n}: max |d logp| {dl:.2e}  max |d value| {dv:.2e}")
-            assert dl <= 1e-4 and dv <= 1e-5, (tag, n, dl, dv)
-    finally:
-        e.close()
+    run_heads(FP16, nets, games, monkeypatch, tag)
 
 
 # ---- 4. latency kernel == throughput kernel ---------------------------------------------------------------------
@@ -317,22 +173,9 @@ def test_fp16_latency_equals_throughput(nets, games, monkeypatch, env):  # noqa:
 
 
 # ---- 5. launch structures and fused paths -----------------------------------------------------------------------
-@pytest.mark.parametrize("env", [{"SCB200_TOWER": "0"}, {"SCB200_TOWER_GROUP": "0"}, {"SCB200_FUSE_GATHER": "0"},
-                                 {"SCB200_FUSE_VALUE": "0"}])
+@pytest.mark.parametrize("env", LAUNCH_VARIANTS)
 def test_fp16_launch_variants_bit_identical(net19, batch2048, monkeypatch, env):  # noqa: F811
-    """Per-layer launches, other tile groupings and the stand-alone value tail give the same bits as the defaults.  The
-    stand-alone legal-move gather (policy.cu) is the fused epilogue's arithmetic in another kernel, not the same
-    instruction sequence: as in bf16 mode (test_fused_policy_gather_matches_standalone_kernel) the values are bit-equal
-    and the priors agree to 2e-6."""
-    games, pos, moves, off, mv_all, lp, v, pri_ref = batch2048
-    for n in (2048, 100):
-        a = _eval(net19[1], monkeypatch, pos[:n], moves[: off[n]], off[: n + 1], env={"SCB200_LATENCY": "0"})
-        b = _eval(net19[1], monkeypatch, pos[:n], moves[: off[n]], off[: n + 1], env=dict(env, SCB200_LATENCY="0"))
-        assert np.array_equal(a[1], b[1]), (env, n)
-        if "SCB200_FUSE_GATHER" in env:
-            assert np.abs(a[0] - b[0]).max() < 2e-6, (env, n)
-        else:
-            assert np.array_equal(a[0], b[0]), (env, n)
+    check_launch_variant(scb200.SC_MODE_FP16, net19, batch2048, monkeypatch, env)
 
 
 # ---- 6. network variants ----------------------------------------------------------------------------------------
@@ -377,38 +220,7 @@ def test_fp16_variant_networks(co, net_golden, tmp_path, tag, monkeypatch):
 
 # ---- 7. drivers -------------------------------------------------------------------------------------------------
 def test_fp16_selfplay_arena_and_game(co, nets, monkeypatch, tmp_path):  # noqa: F811
-    import scb200
-
-    blob = nets["n2"][1]
-    eng = _engine(blob, monkeypatch, max_batch=64)
-    try:
-        runs = []
-        for _ in range(2):
-            sp = scb200.SelfPlay(eng, n_trees=32, rollout_num=30, num_steps=12, cpuct=2.5, with_noise=False,
-                                 temperature_switch=3, temperature=0.0, keep_traces=True, pipeline_groups=2, seed=0)
-            st = sp.run(max_games=32)
-            assert st["games_finished"] == 32
-            runs.append([sp.trace(k) for k in range(32)])
-            sp.close()
-        assert runs[0] == runs[1]
-        for tr in runs[0]:
-            g = co.Game()
-            for mv, _, ch in tr["steps"]:
-                assert mv in g.legal_uci()
-                g.push(mv)
-        mirror = scb200.game_selfplay(eng, rollout_num=30, num_steps=12, cpuct=2.5, temperature_switch=3, seed=0)
-        assert mirror == runs[0][0]
-        eb = _engine(blob, monkeypatch, max_batch=64, mode=scb200.SC_MODE_BF16)
-        try:
-            a = scb200.Arena(eng, eb, n_trees=16, rollout=20, cpuct=1.5, temperature=0.0, temperature_switch=0,
-                             max_plies=6, seed=1, keep_traces=True, n_threads=2)
-            st = a.run(max_games=16)
-            a.close()
-            assert st["games_finished"] == 16 and st["moves"] == 16 * 6
-        finally:
-            eb.close()
-    finally:
-        eng.close()
+    check_selfplay_arena_and_game(scb200.SC_MODE_FP16, co, nets, monkeypatch)
 
 
 def test_fp16_golden_game_first_divergence(tmp_path):

@@ -3,180 +3,37 @@
 Numerics (DESIGN.md section 3.6): the weights of every tensor-core layer are e4m3 (round to nearest even) with a
 power-of-two scale per output channel, s = 2^ceil(log2(amax / 448)); the epilogue forms a = acc * s + bias and then
 runs the bf16 mode's fp32 LayerNorm / SE / residual / ReLU; each layer's output is stored as e4m3 (round to nearest
-even, saturated to +-448).  The SE layers park their LayerNorm output in bf16 and keep bf16 SE weights.  These tests
-emulate exactly that in float64, layer by layer, and check batch independence, the launch variants, the entry points,
-the drivers and the end-to-end accuracy on the bench batch.
+even, saturated to +-448).  The SE layers park their LayerNorm output in bf16 and keep bf16 SE weights.  The kernels
+are checked layer by layer against a float64 emulation of exactly that (test_gpu_layer_reference's, with the e4m3
+format), and these tests check batch independence, the launch variants, the entry points, the drivers and the
+end-to-end accuracy on the bench batch.
 """
+import functools
+
 import numpy as np
 import pytest
-import torch
-import torch.nn.functional as F
+import scb200
 
 from test_gpu_bench_config import batch2048, net19  # noqa: F401  (fixtures)
-from test_gpu_fp16 import _eval, _engine as _engine_any, _u16_to_f64
-from test_gpu_layer_reference import (  # noqa: F401  (fixtures and dtype-free helpers)
-    PLANES, X, T, Y, BIT_EQUAL_MIN, _batch, _layers, _norm, _nhwc_to_nchw, _ulp_bf16, _bf16, games, nets)
+from test_gpu_layer_reference import (  # noqa: F401  (fixtures)
+    FP8, LAUNCH_VARIANTS, _batch, _engine as _engine_any, _eval, check_launch_variant, check_selfplay_arena_and_game,
+    games, nets, run_heads, run_throughput_layers)
 
 pytestmark = pytest.mark.gpu
 
-E4M3_MAX = 448.0
-
-
-# ---- e4m3 arithmetic of the reference ---------------------------------------------------------------------------
-def _rnd8(t):
-    """round to e4m3 (nearest even), saturating at +-448 (cvt.rn.satfinite)"""
-    return t.clamp(-E4M3_MAX, E4M3_MAX).to(torch.float8_e4m3fn).to(torch.float64)
-
-
-def _ulp8(v):
-    """Spacing of e4m3 numbers at |v|: 2^(e - 4) for normal numbers (|v| >= 2^-6), 2^-9 below (0 at 0)."""
-    m, e = np.frexp(np.abs(v))
-    return np.where(v == 0, 0.0, np.ldexp(1.0, np.maximum(e - 4, -9)))
-
-
-def _scaled_weight(w):
-    """[cout, ...] fp32 weights -> the engine's e4m3 weights times their per-output-channel power-of-two scale,
-    float64: per channel s = 2^ceil(log2(amax / 448)) (1 when all zero), then e4m3(w / s) * s"""
-    w = w.double()
-    amax = w.abs().reshape(w.shape[0], -1).amax(dim=1).numpy()
-    m, e = np.frexp(amax)
-    s = np.where(amax > 0, np.ldexp(1.0, np.where(m <= 0.875, e - 9, e - 8)), 1.0)
-    s = torch.from_numpy(s).reshape((-1,) + (1,) * (w.dim() - 1))
-    return _rnd8(w / s) * s
-
-
-def _conv_bias(sd, conv, x):
-    w = _scaled_weight(sd[conv + ".weight"])
-    return F.conv2d(x, w, sd[conv + ".bias"].double(), padding=w.shape[-1] // 2)
-
-
-def _layer_reference(sd, layer, inp, resid):
-    """One layer in float64 on the kernel's e4m3 inputs -> (out before the final rounding, z, gate, a = conv + bias).
-    The SE layers' z is parked in bf16 and their SE weights are bf16, as in bf16 mode."""
-    conv, norm, _, _, relu, se = layer
-    a = _conv_bias(sd, conv, inp)
-    z = _norm(sd, norm, a)
-    if se is None:
-        return (z.clamp_min(0) if relu else z), None, None, a
-    if se == "residual":
-        gate = torch.ones(z.shape[0], z.shape[1], 1, 1, dtype=torch.float64)
-    else:
-        m = z.mean(dim=(2, 3))
-        h = (m @ _bf16(sd[se + "fc1.weight"].double()).reshape(128, 256).T + sd[se + "fc1.bias"].double()).clamp_min(0)
-        gate = torch.sigmoid(h @ _bf16(sd[se + "fc2.weight"].double()).reshape(256, 128).T + sd[se + "fc2.bias"].double())
-        gate = gate[:, :, None, None]
-    return (gate * _bf16(z) + resid).clamp_min(0), z, gate, a
-
-
-def _engine(blob, monkeypatch, env=None, max_batch=512):
-    import scb200
-
-    return _engine_any(blob, monkeypatch, env, max_batch, scb200.SC_MODE_FP8)
+_engine = functools.partial(_engine_any, mode=scb200.SC_MODE_FP8)
 
 
 # ---- 1 / 2. every layer against float64, on all test nets -------------------------------------------------------
-def _check_layers(tag, sd, stressed, e, pos, boards=None):
-    """test_gpu_fp16._check_layers with e4m3 rounding: layer k from the k - 1 call's buffers.  Bound: one e4m3 ulp of
-    the (saturated) reference, the fp32-accumulation floor of test_gpu_layer_reference and, for SE layers, the bf16
-    park's ulp times the gate; at least BIT_EQUAL_MIN of the live elements bit-equal."""
-    import net
-
-    n = len(pos)
-    boards = np.arange(n) if boards is None else np.asarray(boards)
-    planes, _ = e.encode_only(pos)
-    prev = [np.zeros((n, 64, 256), np.uint16) for _ in range(3)]
-    prev_planes = net.planes_i8_hwc_to_nchw(planes[boards]).double()
-    failures = []
-    for k, layer in enumerate(_layers(sd), start=1):
-        cur = e.debug_tower(pos, k, 0)
-        conv, _, reads, writes, _, se = layer
-        for b in (X, T, Y):
-            if b != writes:
-                assert np.array_equal(cur[b], prev[b]), f"{tag} layer {k} ({conv}) changed buffer {'xty'[b]}"
-        inp = prev_planes if reads == PLANES else _nhwc_to_nchw(_u16_to_f64(prev[reads][boards]))
-        resid = _nhwc_to_nchw(_u16_to_f64(prev[X][boards])) if se is not None else None
-        ref, z, gate, a = _layer_reference(sd, layer, inp, resid)
-        got = _nhwc_to_nchw(_u16_to_f64(cur[writes][boards])).numpy()
-        ref = ref.clamp(-E4M3_MAX, E4M3_MAX).numpy()
-        err = np.abs(got - ref)
-        if layer[1] + ".weight" in sd:
-            scale = np.abs(sd[layer[1] + ".weight"].double().numpy()).reshape(1, -1, 1, 1)
-        else:
-            scale = a.std(dim=1, unbiased=False, keepdim=True).numpy()
-        g = 1.0 if gate is None else gate.numpy()
-        floor = 2e-5 * scale * g + 1e-6
-        if k - 1 in stressed:
-            ratio = stressed[k - 1] / a.std(dim=1, unbiased=False, keepdim=True).numpy()
-            shift_tol = (1e-3 + 4 * ratio * 2.0 ** -24) * scale * g
-        else:
-            shift_tol = 0.0
-        tol = _ulp8(ref) + floor + shift_tol
-        if z is not None:
-            tol = tol + gate.numpy() * _ulp_bf16(z.numpy())
-        want = _rnd8(torch.from_numpy(ref)).numpy()
-        live = (want != 0) | (got != 0)
-        equal = float((got == want)[live].mean())
-        sat = float((np.abs(got) == E4M3_MAX).mean())
-        print(f"{tag} n={n} layer {k:2d} {conv:22s} max err / bound {float(np.max(err / tol)):6.3f}  "
-              f"bit-equal {equal:.5f} of {live.mean():.2f}  saturated {sat:.2e}")
-        assert np.isfinite(got).all(), f"{tag} layer {k} ({conv}): non-finite output"
-        if not (err <= tol).all():
-            i = np.unravel_index(np.argmax(err - tol), err.shape)
-            failures.append(f"layer {k} ({conv}): {int((err > tol).sum())} elements out of bound, worst at {i}: "
-                            f"got {got[i]:.6g} ref {ref[i]:.6g}")
-        if k - 1 not in stressed and equal < BIT_EQUAL_MIN:
-            failures.append(f"layer {k} ({conv}): bit-equal fraction {equal:.4f} < {BIT_EQUAL_MIN}")
-        prev = cur
-    assert not failures, f"{tag} n={n}:\n" + "\n".join(failures)
-
-
 @pytest.mark.parametrize("tag", ["n2", "stress", "bn_se", "ln_nose", "bn_nose"])
 def test_fp8_tower_layers(nets, games, monkeypatch, tag):  # noqa: F811
-    sd, blob, stressed = nets[tag]
-    e = _engine(blob, monkeypatch)
-    try:
-        for n in (1, 6):
-            pos, _, _ = _batch(games, n)
-            _check_layers(tag, sd, stressed, e, pos)
-        if tag in ("n2", "stress"):
-            pos, _, _ = _batch(games, 333)
-            _check_layers(tag, sd, stressed, e, pos, boards=[0, 1, 2, 3, 127, 128, 329, 330, 331, 332])
-    finally:
-        e.close()
-
-
-def _heads_reference(sd, t, y, meta):
-    lg = _conv_bias(sd, "policy_head.model.2", t)
-    lg = _norm(sd, "policy_head.model.3", lg)
-    logp = torch.log_softmax(lg.flatten(1), dim=1)
-    w1 = sd["value_head.ffn.0.weight"].double()
-    w1 = torch.cat((_scaled_weight(w1[:, :64 * 256]), w1[:, 64 * 256:]), dim=1)
-    hid = (torch.cat((y.flatten(1), meta), dim=1) @ w1.T + sd["value_head.ffn.0.bias"].double()).clamp_min(0)
-    v = torch.tanh(hid @ sd["value_head.ffn.2.weight"].double().T + sd["value_head.ffn.2.bias"].double())
-    return logp.numpy(), (v[:, 0] * (meta[:, 0] * 2 - 1)).numpy()
+    boards = [0, 1, 2, 3, 127, 128, 329, 330, 331, 332] if tag in ("n2", "stress") else None
+    run_throughput_layers(FP8, nets, games, monkeypatch, tag, (1, 6), boards)
 
 
 @pytest.mark.parametrize("tag", ["n2", "stress", "bn_se", "ln_nose", "bn_nose"])
 def test_fp8_heads_from_tower_buffers(nets, games, monkeypatch, tag):  # noqa: F811
-    """the policy conv (e4m3, scaled) + LayerNorm(73) + log-softmax and the value FC (e4m3, scaled per hidden unit) +
-    tail, from the tower's own e4m3 t / y buffers, against float64, at the fp16 test's tolerances"""
-    import net
-
-    sd, blob, _ = nets[tag]
-    e = _engine(blob, monkeypatch)
-    try:
-        for n in (37, 333):
-            pos, _, _ = _batch(games, n)
-            planes, meta = e.encode_only(pos)
-            _, t, y = e.debug_tower(pos, len(_layers(sd)), 0)
-            lp, v = e.forward_only(net.planes_i8_hwc_to_nchw(planes).numpy(), meta.astype(np.float32))
-            lp_ref, v_ref = _heads_reference(sd, _nhwc_to_nchw(_u16_to_f64(t)), _nhwc_to_nchw(_u16_to_f64(y)),
-                                             torch.from_numpy(meta).double())
-            dl, dv = float(np.abs(lp - lp_ref).max()), float(np.abs(v - v_ref).max())
-            print(f"fp8 {tag} heads n={n}: max |d logp| {dl:.2e}  max |d value| {dv:.2e}")
-            assert dl <= 1e-4 and dv <= 1e-5, (tag, n, dl, dv)
-    finally:
-        e.close()
+    run_heads(FP8, nets, games, monkeypatch, tag)
 
 
 def test_fp8_has_no_latency_kernel(nets, games, monkeypatch):  # noqa: F811
@@ -209,22 +66,9 @@ def test_fp8_rows_do_not_depend_on_the_batch(net19, batch2048, monkeypatch):  # 
         e.close()
 
 
-@pytest.mark.parametrize("env", [{"SCB200_TOWER": "0"}, {"SCB200_TOWER_GROUP": "0"}, {"SCB200_FUSE_GATHER": "0"},
-                                 {"SCB200_FUSE_VALUE": "0"}])
+@pytest.mark.parametrize("env", LAUNCH_VARIANTS)
 def test_fp8_launch_variants_bit_identical(net19, batch2048, monkeypatch, env):  # noqa: F811
-    """per-layer launches, other tile groupings and the stand-alone value tail give the same bits; the stand-alone
-    legal-move gather gives the same values and priors within 2e-6, as in bf16 mode"""
-    import scb200
-
-    games, pos, moves, off, mv_all, lp, v, pri_ref = batch2048
-    for n in (2048, 100):
-        a = _eval(net19[1], monkeypatch, pos[:n], moves[: off[n]], off[: n + 1], mode=scb200.SC_MODE_FP8)
-        b = _eval(net19[1], monkeypatch, pos[:n], moves[: off[n]], off[: n + 1], env=env, mode=scb200.SC_MODE_FP8)
-        assert np.array_equal(a[1], b[1]), (env, n)
-        if "SCB200_FUSE_GATHER" in env:
-            assert np.abs(a[0] - b[0]).max() < 2e-6, (env, n)
-        else:
-            assert np.array_equal(a[0], b[0]), (env, n)
+    check_launch_variant(scb200.SC_MODE_FP8, net19, batch2048, monkeypatch, env)
 
 
 # ---- 4. entry points and drivers --------------------------------------------------------------------------------
@@ -282,35 +126,7 @@ def test_fp8_predict_path_and_evaluator_equal_eval(nets, monkeypatch):  # noqa: 
 
 
 def test_fp8_selfplay_arena_and_game(co, nets, monkeypatch):  # noqa: F811
-    import scb200
-
-    blob = nets["n2"][1]
-    eng = _engine(blob, monkeypatch, max_batch=64)
-    try:
-        sp = scb200.SelfPlay(eng, n_trees=32, rollout_num=30, num_steps=12, cpuct=2.5, with_noise=False,
-                             temperature_switch=3, temperature=0.0, keep_traces=True, pipeline_groups=2, seed=0)
-        st = sp.run(max_games=32)
-        assert st["games_finished"] == 32
-        traces = [sp.trace(k) for k in range(32)]
-        sp.close()
-        for tr in traces:
-            g = co.Game()
-            for mv, _, ch in tr["steps"]:
-                assert mv in g.legal_uci()
-                g.push(mv)
-        mirror = scb200.game_selfplay(eng, rollout_num=30, num_steps=12, cpuct=2.5, temperature_switch=3, seed=0)
-        assert mirror == traces[0]
-        eb = _engine_any(blob, monkeypatch, max_batch=64, mode=scb200.SC_MODE_BF16)
-        try:
-            a = scb200.Arena(eng, eb, n_trees=16, rollout=20, cpuct=1.5, temperature=0.0, temperature_switch=0,
-                             max_plies=6, seed=1, keep_traces=True, n_threads=2)
-            st = a.run(max_games=16)
-            a.close()
-            assert st["games_finished"] == 16 and st["moves"] == 16 * 6
-        finally:
-            eb.close()
-    finally:
-        eng.close()
+    check_selfplay_arena_and_game(scb200.SC_MODE_FP8, co, nets, monkeypatch)
 
 
 # ---- 5. accuracy on the bench batch -----------------------------------------------------------------------------
