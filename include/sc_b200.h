@@ -155,6 +155,30 @@ int sc_predict_path(sc_engine *e, int n, const int32_t *root, const sc_move *pat
                     const int8_t *n_hist, sc_position *pos_out, sc_move *moves_out, int32_t *move_cnt_out,
                     float *priors_out, float *value_out, void *stream);
 
+/* -------- evaluation cache: the reference's search calls Game::predict at every level of every descent
+ * (src/mcts.rs:152) and evaluates a move's subtree again after the move (mcts.rs:309-323).  With a cache, sc_predict,
+ * sc_predict_stack, sc_predict_path and the batching evaluator answer a leaf they have evaluated before from a table in
+ * device memory, and evaluate identical leaves of one call (one evaluator pass) once.  The key is the packed leaf as
+ * the device reads it (the sc_position row) and its ep byte, confirmed on all 545 bytes, so every output, status and
+ * message is the same as without a cache; the table's contents only change the speed.  A full bucket keeps its
+ * entries that the same call reads, and the new result is then not stored.  A call with a cache waits once more for
+ * the device (after the lookup).  sc_eval*, the batched drivers and sc_game_selfplay do not use it.
+ * sc_set_eval_cache: a table of at least `entries` results (rounded up to whole buckets of 4; about 2.6 KB each), empty,
+ * with the counts reset; 0 frees it (the default is no cache).  SC_E_INVAL for entries < 0 or > SC_MAX_CACHE_ENTRIES,
+ * SC_E_CUDA (and no cache) if the allocation fails, SC_E_STATE while an evaluator owns the engine.
+ * sc_eval_cache_stats: the counts since the table was set; may be called from any thread at any time. */
+#define SC_MAX_CACHE_ENTRIES (1 << 22)
+typedef struct sc_eval_cache_counts {
+    int64_t entries;    /* capacity in use (0 = no cache) */
+    int64_t lookups;    /* leaves probed */
+    int64_t hits;       /* answered from the table */
+    int64_t duplicates; /* answered by an identical leaf evaluated in the same call / pass */
+    int64_t inserts;    /* results stored */
+    int64_t evictions;  /* stored results replaced by an insert */
+} sc_eval_cache_counts;
+int sc_set_eval_cache(sc_engine *e, int64_t entries);
+int sc_eval_cache_stats(const sc_engine *e, sc_eval_cache_counts *out);
+
 /* -------- batching evaluator: many host threads, each running one game's sequential search through the one-leaf
  * interface (src/game.rs:3-15), share one engine.  Each call carries one leaf or one root update and blocks until it is
  * done; one dispatcher thread takes every request pending when the device becomes free (up to max_batch leaves),

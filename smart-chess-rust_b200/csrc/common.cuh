@@ -195,4 +195,36 @@ int lat_tower_max_boards(const LatTower *t);
 int lat_tower_launch(LatTower *t, int n_boards, cudaStream_t st, int max_layers = 0);
 void lat_tower_destroy(LatTower *t);
 
+// ---- eval_cache.cu: sc_set_eval_cache's table of stored leaf results and its per-call scratch ----------------------
+constexpr int CACHE_WAYS = 4;  // entries per bucket
+struct EvalCache {
+    int64_t entries = 0, n_buckets = 0;  // 0: no cache
+    void *ent = nullptr;                 // [entries] stored results (key, count, termination code, value, moves, priors)
+    uint64_t *hash = nullptr;            // [entries] hash of the stored key, 0 = empty
+    unsigned long long *stamp = nullptr; // [entries] the last call that hit or claimed the entry
+    unsigned long long calls = 0;        // calls probed since the table was created
+    // per call, max_batch rows: see cache_probe_kernel
+    uint64_t *row_hash = nullptr;
+    int32_t *row_src = nullptr, *row_owner = nullptr, *miss_row = nullptr, *claim = nullptr;
+    unsigned long long *dedup_key = nullptr;
+    int32_t *dedup_row = nullptr;
+    sc_position *miss_pos = nullptr;     // the misses' leaves and ep bytes, compacted in row order
+    int8_t *miss_ep = nullptr;
+    uint8_t *miss_out = nullptr;         // the misses' moves, counts and termination codes (sc_engine::d_pred_out's layout)
+    float *miss_priors = nullptr, *miss_value = nullptr;
+    int32_t *h_counts = nullptr;         // pinned: misses, hits, duplicates, inserts, evictions of the last probe
+};
+size_t eval_cache_entry_bytes();
+// a table of at least `entries` entries (whole buckets), cleared on `st`, and the scratch for calls of up to max_batch
+// leaves; the caller releases a partly built one
+int eval_cache_create(EvalCache *c, int64_t entries, int max_batch, cudaStream_t st);
+void eval_cache_release(EvalCache *c);
+// the probe of n leaves (d_ep == nullptr: -1 for all); writes h_counts, the misses first
+int launch_cache_probe(EvalCache *c, const sc_position *d_pos, const int8_t *d_ep, int n, cudaStream_t st);
+// after the network has written the m misses' results to miss_out / miss_priors / miss_value: the n leaves' moves,
+// counts and termination codes into d_out (d_pred_out's layout for n leaves), priors (strided by SC_MAX_MOVES, the
+// first count of each row) and values, then the misses' inserts.  ep: the call had ep bytes
+int launch_cache_finish(const EvalCache *c, int n, int m, bool ep, uint8_t *d_out, float *d_priors, float *d_value,
+                        cudaStream_t st);
+
 }  // namespace scb

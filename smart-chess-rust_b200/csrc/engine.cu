@@ -316,6 +316,11 @@ struct sc_engine {
     float last_path_ms = 0.f;  // timing: the path-replay kernel (between ev_replay_t)
     // an sc_evaluator owns the stream: every other call that uses the device returns SC_E_STATE
     std::atomic<bool> evaluator{false};
+    // sc_set_eval_cache's table (cache.entries == 0: none) and its counts, read by sc_eval_cache_stats from any thread
+    EvalCache cache;
+    mutable std::mutex cache_mu;
+    sc_eval_cache_counts cache_counts{};
+    bool net_ran = true;  // the last predict_launch ran the network (not an all-hit call): timing reports 0 otherwise
 };
 
 namespace scb {
@@ -977,12 +982,17 @@ static int check_owner(const sc_engine *e, const char *what)
     return SC_E_STATE;
 }
 
-static int finish_timing(sc_engine *e, cudaStream_t st)
+// net_ran: the call ran the network (an sc_predict* call whose leaves were all answered by the cache did not; its tower
+// time is 0)
+static int finish_timing(sc_engine *e, cudaStream_t st, bool net_ran = true)
 {
     if (!e->timing) return SC_OK;
     SCB_CUDA(cudaEventRecord(e->ev[3], st));
     SCB_CUDA(cudaEventSynchronize(e->ev[3]));
-    SCB_CUDA(cudaEventElapsedTime(&e->last_tower_ms, e->ev[1], e->ev[2]));
+    if (net_ran)
+        SCB_CUDA(cudaEventElapsedTime(&e->last_tower_ms, e->ev[1], e->ev[2]));
+    else
+        e->last_tower_ms = 0.f;
     SCB_CUDA(cudaEventElapsedTime(&e->last_total_ms, e->ev[0], e->ev[3]));
     if (e->timing >= 2) {
         float tot = 0.f;
@@ -997,20 +1007,17 @@ static int finish_timing(sc_engine *e, cudaStream_t st)
     return SC_OK;
 }
 
-// sc_predict and sc_predict_stack once the packed leaves are on the device (d_pos / d_ep, as the kernels read them):
-// the legal moves, the encoder, the network and the gather, and the copies back, all queued on `st`.  Up to
-// SC_SMALL_N leaves write values and strided priors straight into the pinned small output buffer.
-static int predict_launch(sc_engine *e, int n, const sc_position *d_pos, const int8_t *d_ep, float *priors_out,
-                          float *value_out, cudaStream_t st)
+// the legal moves, the encoder, the network and the gather of n packed leaves on the device (d_pos / d_ep, as the
+// kernels read them), queued on `st`: moves, counts and termination codes into d_out ([moves n x SC_MAX_MOVES | counts
+// n | termination codes n]), priors strided by SC_MAX_MOVES into d_priors, values into d_value
+static int predict_network(sc_engine *e, int n, const sc_position *d_pos, const int8_t *d_ep, uint8_t *d_out,
+                           float *d_priors, float *d_value, cudaStream_t st)
 {
     const size_t mv_b = sizeof(sc_move) * (size_t)n * SC_MAX_MOVES;
-    const bool small = n <= SC_SMALL_N;
-    float *d_value = small ? e->h_small_out : e->d_value, *d_priors = small ? e->h_small_out + n : e->d_priors;
-    if (e->timing) SCB_CUDA(cudaEventRecord(e->ev[0], st));
     // the legal moves on their own stream next to the encoder and the tower (they do not depend on the network); the
     // policy head's gather waits for them
-    sc_move *d_moves = reinterpret_cast<sc_move *>(e->d_pred_out);
-    int32_t *d_cnt = reinterpret_cast<int32_t *>(e->d_pred_out + mv_b), *d_term = d_cnt + n;
+    sc_move *d_moves = reinterpret_cast<sc_move *>(d_out);
+    int32_t *d_cnt = reinterpret_cast<int32_t *>(d_out + mv_b), *d_term = d_cnt + n;
     SCB_CUDA(cudaEventRecord(e->ev_gen_fork, st));
     SCB_CUDA(cudaStreamWaitEvent(e->gen_stream, e->ev_gen_fork, 0));
     if (e->timing) SCB_CUDA(cudaEventRecord(e->ev_gen_t[0], e->gen_stream));
@@ -1031,6 +1038,54 @@ static int predict_launch(sc_engine *e, int n, const sc_position *d_pos, const i
         SCB_CHECK(launch_policy_gather(e->logits, d_pos, d_moves, nullptr, d_cnt, n, d_priors, st));
         e->launches += 1;
     }
+    return SC_OK;
+}
+
+// predict_launch with an evaluation cache: the probe, one wait for its miss count m, the network on the m misses
+// (nothing of it when m == 0), and the finish kernel, which writes predict_network's outputs for the n leaves
+static int predict_cached(sc_engine *e, int n, const sc_position *d_pos, const int8_t *d_ep, float *d_priors,
+                          float *d_value, cudaStream_t st)
+{
+    EvalCache &c = e->cache;
+    SCB_CHECK(launch_cache_probe(&c, d_pos, d_ep, n, st));
+    e->launches += 1;
+    SCB_CUDA(cudaStreamSynchronize(st));
+    const int32_t *k = c.h_counts;
+    const int m = k[0];
+    {
+        std::lock_guard<std::mutex> lock(e->cache_mu);
+        e->cache_counts.lookups += n;
+        e->cache_counts.hits += k[1];
+        e->cache_counts.duplicates += k[2];
+        e->cache_counts.inserts += k[3];
+        e->cache_counts.evictions += k[4];
+    }
+    e->net_ran = m > 0;
+    if (m > 0)
+        SCB_CHECK(predict_network(e, m, c.miss_pos, d_ep ? c.miss_ep : nullptr, c.miss_out, c.miss_priors, c.miss_value,
+                                  st));
+    else
+        e->kev_used = 0;
+    SCB_CHECK(launch_cache_finish(&c, n, m, d_ep != nullptr, e->d_pred_out, d_priors, d_value, st));
+    e->launches += 1;
+    return SC_OK;
+}
+
+// sc_predict and sc_predict_stack once the packed leaves are on the device (d_pos / d_ep, as the kernels read them):
+// predict_network, through the evaluation cache if the engine has one, and the copies back, all queued on `st`.  Up
+// to SC_SMALL_N leaves write values and strided priors straight into the pinned small output buffer.
+static int predict_launch(sc_engine *e, int n, const sc_position *d_pos, const int8_t *d_ep, float *priors_out,
+                          float *value_out, cudaStream_t st)
+{
+    const size_t mv_b = sizeof(sc_move) * (size_t)n * SC_MAX_MOVES;
+    const bool small = n <= SC_SMALL_N;
+    float *d_value = small ? e->h_small_out : e->d_value, *d_priors = small ? e->h_small_out + n : e->d_priors;
+    if (e->timing) SCB_CUDA(cudaEventRecord(e->ev[0], st));
+    e->net_ran = true;
+    if (e->cache.entries)
+        SCB_CHECK(predict_cached(e, n, d_pos, d_ep, d_priors, d_value, st));
+    else
+        SCB_CHECK(predict_network(e, n, d_pos, d_ep, e->d_pred_out, d_priors, d_value, st));
     // results: moves, counts and termination codes in one copy, the full SC_MAX_MOVES stride of every leaf
     SCB_CUDA(cudaMemcpyAsync(e->h_pred_out, e->d_pred_out, mv_b + 2 * sizeof(int32_t) * (size_t)n, cudaMemcpyDeviceToHost, st));
     if (!small) {
@@ -1048,9 +1103,10 @@ static int predict_collect(sc_engine *e, const char *what, int n, sc_move *moves
 {
     const size_t mv_b = sizeof(sc_move) * (size_t)n * SC_MAX_MOVES, cnt_b = sizeof(int32_t) * (size_t)n;
     const bool small = n <= SC_SMALL_N;
-    SCB_CHECK(finish_timing(e, st));
+    SCB_CHECK(finish_timing(e, st, e->net_ran));
     SCB_CUDA(cudaStreamSynchronize(st));
-    if (e->timing) SCB_CUDA(cudaEventElapsedTime(&e->last_movegen_ms, e->ev_gen_t[0], e->ev_gen_t[1]));
+    if (e->timing && e->net_ran) SCB_CUDA(cudaEventElapsedTime(&e->last_movegen_ms, e->ev_gen_t[0], e->ev_gen_t[1]));
+    if (e->timing && !e->net_ran) e->last_movegen_ms = 0.f;
     memcpy(moves_out, e->h_pred_out, mv_b);
     memcpy(move_cnt_out, e->h_pred_out + mv_b, cnt_b);
     if (small) {
@@ -1441,6 +1497,7 @@ int sc_destroy(sc_engine *e)
     if (e->h_replay_status) cudaFreeHost(e->h_replay_status);
     if (e->d_replay_scratch) cudaFree(e->d_replay_scratch);
     e->roots.release();
+    eval_cache_release(&e->cache);
     for (cudaEvent_t ev : {e->ev_gen_fork, e->ev_gen_done, e->ev_gen_t[0], e->ev_gen_t[1], e->ev_replay_t[0], e->ev_replay_t[1]})
         if (ev) cudaEventDestroy(ev);
     if (e->gen_stream) cudaStreamDestroy(e->gen_stream);
@@ -1995,6 +2052,45 @@ int sc_debug_tower(sc_engine *e, int n, const sc_position *pos, int n_layers, in
     if (t_out) SCB_CUDA(cudaMemcpyAsync(t_out, e->h_t, bytes, cudaMemcpyDeviceToHost, st));
     if (y_out) SCB_CUDA(cudaMemcpyAsync(y_out, e->h_y, bytes, cudaMemcpyDeviceToHost, st));
     SCB_CUDA(cudaStreamSynchronize(st));
+    return SC_OK;
+}
+
+int sc_set_eval_cache(sc_engine *e, int64_t entries)
+{
+    if (!e || entries < 0 || entries > SC_MAX_CACHE_ENTRIES) {
+        set_error("sc_set_eval_cache: bad argument (entries must be in 0..SC_MAX_CACHE_ENTRIES = " +
+                  std::to_string(SC_MAX_CACHE_ENTRIES) + ")");
+        return SC_E_INVAL;
+    }
+    SCB_CHECK(check_owner(e, "sc_set_eval_cache"));
+    SCB_CUDA(cudaSetDevice(e->device));
+    {
+        std::lock_guard<std::mutex> lock(e->cache_mu);
+        e->cache_counts = sc_eval_cache_counts{};
+    }
+    eval_cache_release(&e->cache);
+    if (entries == 0) return SC_OK;
+    const int rc = eval_cache_create(&e->cache, entries, e->max_batch, e->stream);
+    if (rc != SC_OK) {
+        const std::string msg = g_err;
+        eval_cache_release(&e->cache);
+        cudaGetLastError();  // a failed allocation is not sticky: the engine stays usable, without a cache
+        set_error("sc_set_eval_cache: " + msg);
+        return rc;
+    }
+    std::lock_guard<std::mutex> lock(e->cache_mu);
+    e->cache_counts.entries = e->cache.entries;
+    return SC_OK;
+}
+
+int sc_eval_cache_stats(const sc_engine *e, sc_eval_cache_counts *out)
+{
+    if (!e || !out) {
+        set_error("sc_eval_cache_stats: bad argument");
+        return SC_E_INVAL;
+    }
+    std::lock_guard<std::mutex> lock(e->cache_mu);
+    *out = e->cache_counts;
     return SC_OK;
 }
 

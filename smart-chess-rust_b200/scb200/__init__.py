@@ -7,6 +7,7 @@ CPU box), but creating an Engine without an sm_100 device raises.
 from .binding import (  # noqa: F401
     Engine,
     Evaluator,
+    EvalCacheCounts,
     SelfPlay,
     Arena,
     elo,
@@ -24,6 +25,7 @@ from .binding import (  # noqa: F401
     SC_MODE_FP8,
     SC_MAX_MOVES,
     SC_MAX_STACK,
+    SC_MAX_CACHE_ENTRIES,
     POSITION_DTYPE,
     MOVE_DTYPE,
     lib_path,

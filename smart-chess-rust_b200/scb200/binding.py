@@ -33,7 +33,9 @@ DECLARED_SYMBOLS = [
     "sc_predict_timing", "sc_predict_stack", "sc_predict_stack_timing", "sc_set_roots", "sc_predict_path",
     "sc_predict_path_timing", "sc_evaluator_create", "sc_evaluator_destroy", "sc_evaluator_set_root",
     "sc_evaluator_extend_root", "sc_evaluator_predict", "sc_evaluator_stats", "sc_game_selfplay_many",
+    "sc_set_eval_cache", "sc_eval_cache_stats",
 ]
+SC_MAX_CACHE_ENTRIES = 1 << 22
 
 
 class SelfPlayConfig(C.Structure):
@@ -49,6 +51,15 @@ class EvaluatorCounts(C.Structure):
     """struct sc_evaluator_counts"""
     _fields_ = [("passes", C.c_int64), ("leaves", C.c_int64), ("largest_batch", C.c_int64),
                 ("root_updates", C.c_int64), ("wait_seconds", C.c_double)]
+
+    def as_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_}
+
+
+class EvalCacheCounts(C.Structure):
+    """struct sc_eval_cache_counts"""
+    _fields_ = [("entries", C.c_int64), ("lookups", C.c_int64), ("hits", C.c_int64), ("duplicates", C.c_int64),
+                ("inserts", C.c_int64), ("evictions", C.c_int64)]
 
     def as_dict(self):
         return {k: getattr(self, k) for k, _ in self._fields_}
@@ -107,6 +118,8 @@ def load_library():
         L.sc_evaluator_extend_root.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int]
         L.sc_evaluator_predict.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int] + [C.c_void_p] * 5
         L.sc_evaluator_stats.argtypes = [C.c_void_p, C.POINTER(EvaluatorCounts)]
+        L.sc_set_eval_cache.argtypes = [C.c_void_p, C.c_int64]
+        L.sc_eval_cache_stats.argtypes = [C.c_void_p, C.POINTER(EvalCacheCounts)]
         L.sc_game_selfplay_many.argtypes = [C.c_void_p, C.POINTER(SelfPlayConfig), C.c_int, C.c_void_p, C.c_char_p,
                                             C.c_int64, C.c_void_p, C.POINTER(EvaluatorCounts)]
         L.sc_eval_device.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,
@@ -437,6 +450,18 @@ class Engine:
         _check(load_library().sc_debug_tower(self._h, n, _ptr(positions), n_layers, which, _ptr(out[0]), _ptr(out[1]),
                                              _ptr(out[2])), "sc_debug_tower")
         return out
+
+    def set_eval_cache(self, entries: int):
+        """sc_set_eval_cache: predict(), predict_stack(), predict_path() and an Evaluator on this engine answer repeated
+        leaves from a device table of at least `entries` results (bit-identical outputs); 0 frees it.  The table starts
+        empty and the counts at zero."""
+        _check(load_library().sc_set_eval_cache(self._h, int(entries)), "sc_set_eval_cache")
+
+    def eval_cache_stats(self):
+        """{entries, lookups, hits, duplicates, inserts, evictions} since the last set_eval_cache() (any thread)"""
+        c = EvalCacheCounts()
+        _check(load_library().sc_eval_cache_stats(self._h, C.byref(c)), "sc_eval_cache_stats")
+        return c.as_dict()
 
     def launch_count(self) -> int:
         return int(load_library().sc_launch_count(self._h))
