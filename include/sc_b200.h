@@ -399,6 +399,16 @@ int sc_random_positions(int n, uint64_t seed, int max_ply, sc_position *pos_out,
 int sc_debug_tower(sc_engine *e, int n, const sc_position *pos, int n_layers, int which, uint16_t *x_out,
                    uint16_t *t_out, uint16_t *y_out);
 
+/* Test hook (SC_MODE_FP32 and SC_MODE_FP32_FFMA engines; SC_E_INVAL for every other mode): encodes n leaves, zeroes the
+ * fp32 activation buffers (and an SC_MODE_FP32 engine's operand planes) and runs the first n_layers layers (0 = all) in
+ * sc_debug_tower's order with the kernels and launches of sc_eval.  Copies the buffers whose pointers are not NULL:
+ * x, t, y as fp32 [n][64][256] (x = block input / output, t = conv1 output / policy head input, y = conv2 output
+ * before the SE and residual / value head input), and on an SC_MODE_FP32 engine the bf16x3 operand planes of x and t
+ * the split GEMMs read, as bf16 bit patterns [n][64][3 * 256] (hi, mid, lo planes of 256 channels each).  Plane
+ * pointers on an SC_MODE_FP32_FFMA engine get SC_E_INVAL.  Lets the tests check each fp32 layer. */
+int sc_debug_tower_f32(sc_engine *e, int n, const sc_position *pos, int n_layers, float *x_out, float *t_out,
+                       float *y_out, uint16_t *px_out, uint16_t *pt_out);
+
 /* Test hook: one Dirichlet(alpha) sample of size n from the driver's root-noise sampler (src/mcts.rs:123-130
  * uses rand_distr::Dirichlet(0.3)); lets the tests check its moments. */
 int sc_test_dirichlet(uint64_t seed, float alpha, int n, float *out);

@@ -645,18 +645,16 @@ static int kev_mark(sc_engine *e, cudaStream_t st)
     return SC_OK;
 }
 
-// the network on n boards; planes already in f_planes / h_planes, meta in d_meta.
-// `gather` (16-bit modes only): the policy head's epilogue turns the logits into legal-move priors itself; the caller
-// then skips launch_policy_gather.  Returns through *fused whether that happened.
-// `gather_ready` (with `gather`): the policy head waits for this event first (sc_predict's legal moves)
-static int run_network(sc_engine *e, int n, cudaStream_t st, const TcGather *gather = nullptr,
-                       cudaEvent_t gather_ready = nullptr)
+// the fp32 modes' network on n boards up to the value FC's split sums: the bf16x3 split GEMMs with fp32 LayerNorm / SE
+// (fp32_tc), or every layer FFMA.  max_layers > 0 returns after the first max_layers tower layers in sc_debug_tower's
+// order -- stem, conv1 and conv2 (+ SE + residual) of each block, the policy and the value 1x1 convolution --
+// for sc_debug_tower_f32; 0 runs it all
+static int run_network_f32(sc_engine *e, int n, cudaStream_t st, int max_layers)
 {
-    NvtxRange nv_net("scb200: network (tower + heads)");
     const int rows = n * 64;
-    e->kev_used = 0;
-    if (e->timing) SCB_CUDA(cudaEventRecord(e->ev[1], st));
-    if (e->mode == SC_MODE_FP32 && e->fp32_tc) {
+    int layers = 0;
+    auto stop = [&] { return ++layers == max_layers; };  // after each tower layer: were those the first max_layers?
+    if (e->fp32_tc) {
         const int nb = e->alloc_boards;
         // 256-wide convolution: split GEMM on the tensor cores (fp32 out, + bias), then LayerNorm (+ReLU) in fp32;
         // `planes` = also emit the result as bf16x3 operand planes for the next convolution
@@ -669,24 +667,30 @@ static int run_network(sc_engine *e, int n, cudaStream_t st, const TcGather *gat
             return SC_OK;
         };
         SCB_CHECK(conv(e->stem, e->h_planes, e->f_x, 1, e->p_x, false));
+        if (stop()) return SC_OK;
         for (int i = 0; i < e->n_blocks; i++) {
             SCB_CHECK(conv(e->conv1[i], e->p_x, e->f_t, 1, e->p_t, true));
+            if (stop()) return SC_OK;
             SCB_CHECK(conv(e->conv2[i], e->p_t, e->f_y, 0, nullptr, true));
             SCB_CHECK(launch_se_res_f32(e->f_y, e->f_x, e->f_x, n, e->se[i].w1t, e->se[i].b1, e->se[i].w2t, e->se[i].b2, st,
                                         e->p_x));
             e->launches += 1;
+            if (stop()) return SC_OK;
         }
         e->timed_flops_per_leaf = 2.0 * 64 * 256 * 9.0 * 256 * 2 * e->n_blocks;
         if (e->timing) SCB_CUDA(cudaEventRecord(e->ev[2], st));
         SCB_CHECK(conv(e->pol1, e->p_x, e->f_t, 0, nullptr, false));
+        if (stop()) return SC_OK;
         SCB_CHECK(launch_gemm_f32(1, e->f_t, C_TOWER, e->pol2.w_f32, e->pol2.ldw, e->pol2.bias, e->logits, LD_POLICY,
                                   rows, C_POLICY, C_TOWER, st));
         SCB_CHECK(launch_ln_f32(e->logits, rows, C_POLICY, LD_POLICY, e->pol2.gamma, e->pol2.beta, 0, st));
+        e->launches += 2;
         SCB_CHECK(conv(e->val1, e->p_x, e->f_y, 1, nullptr, false));
+        if (stop()) return SC_OK;
         SCB_CHECK(launch_gemm_f32(1, e->f_y, 64 * C_TOWER, e->vfc_w_f32, N_VALUE_HIDDEN, nullptr, e->vpre,
                                   N_VALUE_HIDDEN, n, N_VALUE_HIDDEN, 64 * C_TOWER, st, e->vsplit));
-        e->launches += 3;
-    } else if (e->mode == SC_MODE_FP32) {
+        e->launches += 1;
+    } else {
         auto conv = [&](const ConvW &c, const float *in, int lda, float *out, int relu) -> int {
             SCB_CHECK(launch_gemm_f32(c.taps, in, lda, c.w_f32, c.ldw, c.bias, out, C_TOWER, rows, c.cout, c.cin, st));
             SCB_CHECK(launch_ln_f32(out, rows, c.cout, C_TOWER, c.gamma, c.beta, relu, st));
@@ -694,6 +698,7 @@ static int run_network(sc_engine *e, int n, cudaStream_t st, const TcGather *gat
             return SC_OK;
         };
         SCB_CHECK(conv(e->stem, e->f_planes, C_IN, e->f_x, 1));
+        if (stop()) return SC_OK;
         for (int i = 0; i < e->n_blocks; i++) {
             SCB_CHECK(kev_mark(e, st));
             SCB_CHECK(launch_gemm_f32(9, e->f_x, C_TOWER, e->conv1[i].w_f32, e->conv1[i].ldw, e->conv1[i].bias, e->f_t,
@@ -701,6 +706,7 @@ static int run_network(sc_engine *e, int n, cudaStream_t st, const TcGather *gat
             SCB_CHECK(kev_mark(e, st));
             SCB_CHECK(launch_ln_f32(e->f_t, rows, C_TOWER, C_TOWER, e->conv1[i].gamma, e->conv1[i].beta, 1, st));
             e->launches += 2;
+            if (stop()) return SC_OK;
             SCB_CHECK(kev_mark(e, st));
             SCB_CHECK(launch_gemm_f32(9, e->f_t, C_TOWER, e->conv2[i].w_f32, e->conv2[i].ldw, e->conv2[i].bias, e->f_y,
                                       C_TOWER, rows, C_TOWER, C_TOWER, st));
@@ -710,18 +716,38 @@ static int run_network(sc_engine *e, int n, cudaStream_t st, const TcGather *gat
             SCB_CHECK(launch_se_res_f32(e->f_y, e->f_x, e->f_x, n, e->se[i].w1t, e->se[i].b1, e->se[i].w2t,
                                         e->se[i].b2, st));
             e->launches += 1;
+            if (stop()) return SC_OK;
         }
         if (e->timing) SCB_CUDA(cudaEventRecord(e->ev[2], st));
         // policy head
         SCB_CHECK(conv(e->pol1, e->f_x, C_TOWER, e->f_t, 0));
+        if (stop()) return SC_OK;
         SCB_CHECK(launch_gemm_f32(1, e->f_t, C_TOWER, e->pol2.w_f32, e->pol2.ldw, e->pol2.bias, e->logits, LD_POLICY,
                                   rows, C_POLICY, C_TOWER, st));
         SCB_CHECK(launch_ln_f32(e->logits, rows, C_POLICY, LD_POLICY, e->pol2.gamma, e->pol2.beta, 0, st));
+        e->launches += 2;
         // value head
         SCB_CHECK(conv(e->val1, e->f_x, C_TOWER, e->f_y, 1));
+        if (stop()) return SC_OK;
         SCB_CHECK(launch_gemm_f32(1, e->f_y, 64 * C_TOWER, e->vfc_w_f32, N_VALUE_HIDDEN, nullptr, e->vpre,
                                   N_VALUE_HIDDEN, n, N_VALUE_HIDDEN, 64 * C_TOWER, st, e->vsplit));
-        e->launches += 3;
+        e->launches += 1;
+    }
+    return SC_OK;
+}
+
+// the network on n boards; planes already in f_planes / h_planes, meta in d_meta.
+// `gather` (16-bit modes only): the policy head's epilogue turns the logits into legal-move priors itself; the caller
+// then skips launch_policy_gather.  Returns through *fused whether that happened.
+// `gather_ready` (with `gather`): the policy head waits for this event first (sc_predict's legal moves)
+static int run_network(sc_engine *e, int n, cudaStream_t st, const TcGather *gather = nullptr,
+                       cudaEvent_t gather_ready = nullptr)
+{
+    NvtxRange nv_net("scb200: network (tower + heads)");
+    e->kev_used = 0;
+    if (e->timing) SCB_CUDA(cudaEventRecord(e->ev[1], st));
+    if (e->mode == SC_MODE_FP32) {
+        SCB_CHECK(run_network_f32(e, n, st, 0));
     } else {
         const int nb = e->alloc_boards;
         int trc = SC_E_STATE;
@@ -2051,6 +2077,42 @@ int sc_debug_tower(sc_engine *e, int n, const sc_position *pos, int n_layers, in
     if (x_out) SCB_CUDA(cudaMemcpyAsync(x_out, e->h_x, bytes, cudaMemcpyDeviceToHost, st));
     if (t_out) SCB_CUDA(cudaMemcpyAsync(t_out, e->h_t, bytes, cudaMemcpyDeviceToHost, st));
     if (y_out) SCB_CUDA(cudaMemcpyAsync(y_out, e->h_y, bytes, cudaMemcpyDeviceToHost, st));
+    SCB_CUDA(cudaStreamSynchronize(st));
+    return SC_OK;
+}
+
+int sc_debug_tower_f32(sc_engine *e, int n, const sc_position *pos, int n_layers, float *x_out, float *t_out,
+                       float *y_out, uint16_t *px_out, uint16_t *pt_out)
+{
+    SCB_CHECK(check_owner(e, "sc_debug_tower_f32"));
+    if (!e || e->mode != SC_MODE_FP32 || n <= 0 || n > e->max_batch || !pos || n_layers < 0) {
+        set_error("sc_debug_tower_f32: bad argument (SC_MODE_FP32 / SC_MODE_FP32_FFMA engines only)");
+        return SC_E_INVAL;
+    }
+    if (!e->fp32_tc && (px_out || pt_out)) {
+        set_error("sc_debug_tower_f32: an SC_MODE_FP32_FFMA engine has no operand planes");
+        return SC_E_INVAL;
+    }
+    cudaStream_t st = e->stream;
+    SCB_CUDA(cudaSetDevice(e->device));
+    const size_t act = (size_t)e->alloc_boards * 64 * C_TOWER;
+    SCB_CUDA(cudaMemsetAsync(e->f_x, 0, act * sizeof(float), st));
+    SCB_CUDA(cudaMemsetAsync(e->f_t, 0, act * sizeof(float), st));
+    SCB_CUDA(cudaMemsetAsync(e->f_y, 0, act * sizeof(float), st));
+    if (e->fp32_tc) {
+        SCB_CUDA(cudaMemsetAsync(e->p_x, 0, act * 3 * sizeof(__nv_bfloat16), st));
+        SCB_CUDA(cudaMemsetAsync(e->p_t, 0, act * 3 * sizeof(__nv_bfloat16), st));
+    }
+    SCB_CUDA(cudaMemcpyAsync(e->d_pos, pos, sizeof(sc_position) * (size_t)n, cudaMemcpyHostToDevice, st));
+    SCB_CHECK(encode_for_mode(e, e->d_pos, n, st));
+    e->kev_used = 0;
+    SCB_CHECK(run_network_f32(e, n, st, n_layers));
+    const size_t count = (size_t)n * 64 * C_TOWER;
+    if (x_out) SCB_CUDA(cudaMemcpyAsync(x_out, e->f_x, count * sizeof(float), cudaMemcpyDeviceToHost, st));
+    if (t_out) SCB_CUDA(cudaMemcpyAsync(t_out, e->f_t, count * sizeof(float), cudaMemcpyDeviceToHost, st));
+    if (y_out) SCB_CUDA(cudaMemcpyAsync(y_out, e->f_y, count * sizeof(float), cudaMemcpyDeviceToHost, st));
+    if (px_out) SCB_CUDA(cudaMemcpyAsync(px_out, e->p_x, count * 3 * 2, cudaMemcpyDeviceToHost, st));
+    if (pt_out) SCB_CUDA(cudaMemcpyAsync(pt_out, e->p_t, count * 3 * 2, cudaMemcpyDeviceToHost, st));
     SCB_CUDA(cudaStreamSynchronize(st));
     return SC_OK;
 }

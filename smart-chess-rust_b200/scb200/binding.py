@@ -33,7 +33,7 @@ DECLARED_SYMBOLS = [
     "sc_predict_timing", "sc_predict_stack", "sc_predict_stack_timing", "sc_set_roots", "sc_predict_path",
     "sc_predict_path_timing", "sc_evaluator_create", "sc_evaluator_destroy", "sc_evaluator_set_root",
     "sc_evaluator_extend_root", "sc_evaluator_predict", "sc_evaluator_stats", "sc_game_selfplay_many",
-    "sc_set_eval_cache", "sc_eval_cache_stats",
+    "sc_set_eval_cache", "sc_eval_cache_stats", "sc_debug_tower_f32",
 ]
 SC_MAX_CACHE_ENTRIES = 1 << 22
 
@@ -103,6 +103,7 @@ def load_library():
         L.sc_selfplay_run_many.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.c_int64, C.c_int64, C.c_double,
                                            C.POINTER(SelfPlayStats)]
         L.sc_debug_tower.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.sc_debug_tower_f32.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int] + [C.c_void_p] * 5
         L.sc_eval.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 6
         L.sc_predict.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 7
         L.sc_predict_timing.argtypes = [C.c_void_p, C.POINTER(C.c_float)]
@@ -449,6 +450,18 @@ class Engine:
         out = [np.zeros((n, 64, 256), dtype=np.uint16) for _ in range(3)]
         _check(load_library().sc_debug_tower(self._h, n, _ptr(positions), n_layers, which, _ptr(out[0]), _ptr(out[1]),
                                              _ptr(out[2])), "sc_debug_tower")
+        return out
+
+    def debug_tower_f32(self, positions, n_layers: int, planes: bool = True):
+        """test hook sc_debug_tower_f32 (fp32 engines): (x, t, y, px, pt) after n_layers layers, x / t / y float32
+        [n, 64, 256], px / pt the bf16x3 operand planes of x and t as uint16 [n, 64, 768] (None unless `planes`; an
+        SC_MODE_FP32_FFMA engine has none)"""
+        n = len(positions)
+        positions = np.ascontiguousarray(positions, dtype=POSITION_DTYPE)
+        out = [np.zeros((n, 64, 256), dtype=np.float32) for _ in range(3)]
+        out += [np.zeros((n, 64, 768), dtype=np.uint16) if planes else None for _ in range(2)]
+        _check(load_library().sc_debug_tower_f32(self._h, n, _ptr(positions), n_layers, *[_ptr(a) for a in out]),
+               "sc_debug_tower_f32")
         return out
 
     def set_eval_cache(self, entries: int):
